@@ -21,6 +21,14 @@ on rank 0, the other half of the metric and the TTA configuration, reported unde
   cpu_baseline / --impl reference  the reference has no CPU path and its TensorRT/OpenCV-CUDA engine cannot be built here (SURVEY 8c);
             this arm times the oracle port (PyTorch fp32 on the host cores + NumPy tiling restatement) on a bounded sample.
 Before timing, the run refuses work-skipping development switches and checks one rendered frame against a fresh synchronous render.
+Every timed loop (value, e2e, e2e_sync, of every workload) runs exactly --steps frames.  Untimed warm-up frames before them:
+--warmup for `value`, max(--warmup, 4) for `e2e` (each of its 4 pinned buffer pairs is used once), 2 for `e2e_sync`.
+
+--dump-outputs DIR writes, after the timed steps, what the device-resident path returned for its last timed frame, per workload:
+  DIR/<workload>.npy       float32 [256][W][3] BGR, 256 whole rows of the output frame (values 0..255; the full 4K / 8K frames
+                           would exceed 64 MB as float32)
+  DIR/<workload>_rows.npy  float64 [256], the row indices (a fixed, seeded sample, the same on every run)
+Inputs (synthetic frames, seeded weights) depend only on the arguments, so two builds can be compared output for output.
 """
 from __future__ import annotations
 
@@ -41,6 +49,7 @@ for p in (ROOT, PKG):
         sys.path.insert(0, p)
 
 FRAME_W, FRAME_H, BLEND = 1920, 1080, 1.0 / 16.0
+DUMP_ROWS, DUMP_SEED = 256, 0
 WORKLOADS = {
     "cunet": dict(model="cunet/art", family="cunet", scale=2, noise=3, tile=256, batch=8, tiles=60, tta=False, dom="patch3x3",
                   dom_name="conv3x3_patch_kernel (tcgen05)",
@@ -212,7 +221,7 @@ def measure(wl, args, rank, world, local, dist, heavy=True):
         raise SystemExit(f"build failed: {msgs}")
     if not eng.load(onnx_path, w2x.RenderConfig(deviceId=local, batchSize=BATCH, height=TILE, width=TILE, scaling=SCALE, overlap=(BLEND, BLEND), tta=wl["tta"])):
         raise SystemExit(f"load failed: {msgs}")
-    steps, warmup = (args.steps, args.warmup) if heavy else (max(8, args.steps // 3), max(3, args.warmup // 2))
+    steps, warmup = args.steps, args.warmup
 
     n_in = 4  # distinct input frames, rotated
     frames = [tiling.synthetic_frame(FRAME_W, FRAME_H, rank * 1000 + s) for s in range(n_in)]
@@ -298,7 +307,7 @@ def measure(wl, args, rank, world, local, dist, heavy=True):
     checksum = int(pin_out[(steps - 1) % ring].array[::97, ::89].astype(np.uint64).sum())  # result read on the host
 
     # ---- the literal drop-in call: synchronous render(), pageable host buffers (`e2e_sync`) ----
-    sync_steps = max(4, steps // 4)
+    sync_steps = steps
     page_in = [np.array(f, copy=True) for f in frames]
     page_out = np.empty((FRAME_H * SCALE, FRAME_W * SCALE, 3), np.uint8)
     for i in range(2):
@@ -316,6 +325,8 @@ def measure(wl, args, rank, world, local, dist, heavy=True):
                e2e_sync=dict(value=sync_value, unit=UNIT, ms_per_step=sync_ms / sync_steps, steps=sync_steps,
                              path="w2x_render (trt::Img2Img::render drop-in), pageable host buffers, synchronous, wall clock"),
                fps=(world if heavy else 1) * steps / (ms_max / 1e3), out_mpx=out_mpx)
+    if args.dump_outputs:
+        res["output"] = last
     if rank == 0:
         peaks, peak_kind = _peaks()
         flops_frame = eng.flops_per_tile * wl["tiles"] * (8 if wl["tta"] else 1)  # real tiles per 1080p frame (padding slots excluded)
@@ -353,11 +364,24 @@ def measure(wl, args, rank, world, local, dist, heavy=True):
     return res
 
 
+def dump_outputs(outdir, outputs):
+    """Each workload's last timed frame (u8 BGR [H][W][3]) -> <key>.npy: a fixed, seeded sample of DUMP_ROWS whole rows as
+    float32, and <key>_rows.npy: those row indices as float64.  At most 256 * 7680 * 3 * 4 B = 23.6 MB per workload."""
+    import numpy as np
+    os.makedirs(outdir, exist_ok=True)
+    for key, frame in outputs.items():
+        rows = np.sort(np.random.default_rng(DUMP_SEED).choice(frame.shape[0], min(DUMP_ROWS, frame.shape[0]), replace=False))
+        np.save(os.path.join(outdir, f"{key}.npy"), frame[rows].astype(np.float32))
+        np.save(os.path.join(outdir, f"{key}_rows.npy"), rows.astype(np.float64))
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=32)
-    ap.add_argument("--warmup", type=int, default=4)
+    ap.add_argument("--steps", type=int, default=32, help="timed frames of every timed loop")
+    ap.add_argument("--warmup", type=int, default=4, help="untimed frames before the device-resident timed loop (see the module docstring for the e2e loops)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write each workload's last timed output frame (a fixed row sample, float32) as DIR/<workload>.npy")
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--workload", default="cunet", choices=sorted(WORKLOADS))
     ap.add_argument("--no-cpu-baseline", action="store_true")
@@ -365,6 +389,8 @@ def main():
     ap.add_argument("--batch", type=int, default=0, help="experiment: override the workload's batchSize (the driver line uses the default)")
     ap.add_argument("--layers", action="store_true", help="also print a per-layer profile to stderr")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
     wl = dict(WORKLOADS[args.workload], key=args.workload)
     if args.batch > 0:
         wl["batch"] = args.batch
@@ -391,6 +417,7 @@ def main():
     w2x.lib()  # the shipped library (lib/libw2x.so); raises if it is missing
 
     r = measure(wl, args, rank, world, local, dist, heavy=True)
+    outputs = {args.workload: r.pop("output", None)}
     extra = {}
     if rank == 0 and world == 1 and not args.only and args.batch == 0:
         for key in ("swin", "cunet_tta", "cunet"):
@@ -398,6 +425,7 @@ def main():
                 continue
             w2 = dict(WORKLOADS[key], key=key)
             x = measure(w2, args, rank, world, local, dist, heavy=False)
+            outputs[key] = x.pop("output", None)
             extra[key] = {"workload": w2["name"], "value": x["value"], "unit": UNIT, "ms_per_step": x["ms_per_step"], "steps": x["steps"], "warmup": x["warmup"],
                           "fps": x["fps"], "e2e": x["e2e"], "e2e_sync": x["e2e_sync"], "stage_ms_last_frame": x["stage"], "roofline": x.get("roofline"),
                           "roofline_tiling": x.get("roofline_tiling"), "gpu_launches": x["launches"], "clocks": x["clocks"]}
@@ -417,6 +445,8 @@ def main():
             line["workloads"] = extra
         if not args.no_cpu_baseline:
             line["cpu_baseline"] = cpu_baseline_block(wl, passes=3)
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, outputs)
         print(json.dumps(line), flush=True)
     if world > 1:
         dist.barrier()
@@ -424,4 +454,5 @@ def main():
 
 
 if __name__ == "__main__":
+    sys.dont_write_bytecode = True  # the benchmark writes nothing into the tree it runs from
     main()

@@ -20,7 +20,8 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 GOLD = np.load(os.path.join(HERE, "golden", "ref_goldens.npz"))
 GRIDS = json.load(open(os.path.join(HERE, "golden", "tile_grid.json")))
 HASHES = json.load(open(os.path.join(HERE, "golden", "ref_hashes.json")))
-live = pytest.mark.skipif(not ref.available(), reason="oracle/_ref is not built (needs /root/reference): golden vectors cover this")
+live = pytest.mark.skipif(not ref.available(), reason="oracle/_ref is not built: needs the upstream waifu2x-tensorrt sources "
+                          "(make -C oracle REF=<checkout>); the golden tests cover the cases stored under tests/golden")
 
 
 # ---------------------------------------------------------------------------------------------------------------------

@@ -10,7 +10,8 @@ import refcases
 from oracle import ref
 
 cv2 = pytest.importorskip("cv2")
-pytestmark = pytest.mark.skipif(not ref.available(), reason="oracle/_ref is not built (needs /root/reference)")
+pytestmark = pytest.mark.skipif(not ref.available(), reason="oracle/_ref is not built: needs the upstream waifu2x-tensorrt sources "
+                                "(make -C oracle REF=<checkout>)")
 
 
 def test_copy_make_border_replicate():
