@@ -1,7 +1,7 @@
 /*
  * w2x_dev.h -- development / test hooks of the B200-native waifu2x engine.  NOT part of the drop-in boundary (include/w2x.h).
  *
- * w2x_selftest_conv and w2x_run_conv_layer are exported by the shipped library (lib/libw2x.so): they run the product's own layer
+ * w2x_selftest_conv, w2x_run_conv_layer and w2x_run_conv_layer_f32 are exported by the shipped library (lib/libw2x.so): they run the product's own layer
  * kernels on caller-supplied or random data so that tests can compare single layers with an independent fp32 reference.
  * The w2x_probe_* micro-benchmarks and every switch that alters or skips kernel work (W2X_DBG, W2X_CONV_IMPL, W2X_NO_PATCH,
  * W2X_NO_FUSE_FIRST, W2X_NO_EPI_GROUPS, W2X_NO_HEAD_KERNEL, W2X_NO_PDL) exist only in the W2X_DEV build, lib/libw2x_dev.so.
@@ -29,6 +29,12 @@ extern "C" {
  * All tensors NHWC fp16 (raw bits).  Returns 1 on success. */
 W2X_API int w2x_run_conv_layer(int device, int kind, int head, int n, int h, int w, int cin, int cout, const uint16_t* in_nhwc,
                                const uint16_t* weights, const float* bias, const uint16_t* skip_nhwc, uint16_t* out_nhwc);
+
+/* The same layer kinds 0-4 through the tf32 kernel of `--precision tf32` engines (kernels/conv_tf32_sm100.cu: tcgen05 kind::tf32, fp32
+ * accumulate): every tensor is NHWC fp32, the weights are the fp32 packed operand of a tf32 build (same layouts as above; the tensor core
+ * uses their TF32 part).  Returns 1 on success. */
+W2X_API int w2x_run_conv_layer_f32(int device, int kind, int n, int h, int w, int cin, int cout, const float* in_nhwc, const float* weights,
+                                   const float* bias, const float* skip_nhwc, float* out_nhwc);
 
 /* The fused MLP half of a SwinUNet block (kernels/swin_mlp_sm100.cu; replaces a slice of the engine enqueued at img2img_infer.cpp:80):
  * x[tokens][c] (NHWC fp16 bits, updated in place) += fc2(GELU(fc1(LayerNorm(x)))), c = 96 or 192, w1 = [2c][c], w2 = [c][2c] fp16 bits

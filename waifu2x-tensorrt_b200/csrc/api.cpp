@@ -276,6 +276,17 @@ int w2x_run_conv_layer(int device, int kind, int head, int n, int h, int w, int 
     }
 }
 
+int w2x_run_conv_layer_f32(int device, int kind, int n, int h, int w, int cin, int cout, const float* in_nhwc, const float* weights, const float* bias,
+                           const float* skip_nhwc, float* out_nhwc) {
+    try {
+        runConvLayerF32(device, kind, n, h, w, cin, cout, in_nhwc, weights, bias, skip_nhwc, out_nhwc);
+        return 1;
+    } catch (const std::exception& ex) {
+        std::fprintf(stderr, "w2x_run_conv_layer_f32: %s\n", ex.what());
+        return 0;
+    }
+}
+
 int w2x_run_swin_mlp(int device, long long tokens, int c, int variant, uint16_t* x, const float* gamma, const float* beta, float eps, const uint16_t* w1,
                      const float* b1, const uint16_t* w2, const float* b2, int reps, float* ms_out) {
     void* bufs[7] = {};

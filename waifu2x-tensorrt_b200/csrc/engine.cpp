@@ -113,7 +113,7 @@ Act Engine::allocAct(int h, int w, int c) {
     if (h <= 0 || w <= 0) throw Error("tile size too small for this model");
     Act a;
     a.n = batch; a.h = h; a.w = w; a.c = c;
-    a.p = (__half*)dalloc(a.elems() * sizeof(__half) + 256);
+    a.p = (__half*)dalloc(a.elems() * elemBytes + 256);
     return a;
 }
 
@@ -132,6 +132,7 @@ void Engine::unload() {
     if (d2hStream) cudaStreamSynchronize(d2hStream);
     for (auto& L : layers) {
         if (L.plan) igemmDestroyPlan(L.plan);
+        if (L.tf32) tf32DestroyPlan(L.tf32);
         if (L.head) convHeadDestroyPlan(L.head);
         if (L.mlp) swinMlpDestroyPlan(L.mlp);
         if (L.attn) swinAttnDestroyPlan(L.attn);
@@ -144,9 +145,12 @@ void Engine::unload() {
     freep(dTileMap); tileMapCap = 0;
     for (cudaEvent_t e : bandEv) cudaEventDestroy(e);
     bandEv.clear();
-    freep(dSlots); freep(dTileOut); freep(dTtaMean); freep(dRampX); freep(dRampY); freep(dFrameIn); freep(dFrameOut); freep(dUnpacked);
+    freep(dSlots);
+    if (dTileOut) { cudaFree(dTileOut); dTileOut = nullptr; } freep(dTtaMean); freep(dRampX); freep(dRampY); freep(dFrameIn); freep(dFrameOut);
+    if (dUnpacked) { cudaFree(dUnpacked); dUnpacked = nullptr; }
     unpackedCap = 0;
-    freep(dBandTiles); freep(dBandMap); freep(dBandSlots); freep(dBandMean);
+    if (dBandTiles) { cudaFree(dBandTiles); dBandTiles = nullptr; }
+    freep(dBandMap); freep(dBandSlots); freep(dBandMean);
     bandTilesCap = bandMapCap = bandSlotCap = bandMeanCap = 0;
     if (evBandModel) { cudaEventDestroy(evBandModel); evBandModel = nullptr; }
     slotCap = tileOutCap = ttaCap = frameInCap = frameOutCap = 0;
@@ -186,8 +190,8 @@ bool Engine::build(const std::string& onnxPath, const w2x_build_config& bc) {
             ELOG(W2X_ERROR, "Failed to set cuda device to device id " + std::to_string(bc.deviceId) + ": " + cudaGetErrorString(e) + ".");
             return false;
         }
-        if (bc.precision != W2X_PRECISION_FP16) {
-            ELOG(W2X_ERROR, "Failed to set precision: the tf32 kernel set is not available in this build (fp16 storage, fp32 accumulate only)");
+        if (bc.precision != W2X_PRECISION_FP16 && bc.precision != W2X_PRECISION_TF32) {
+            ELOG(W2X_ERROR, "Failed to set precision: unknown precision " + std::to_string(bc.precision) + ".");
             return false;
         }
         OnnxGraph g;
@@ -195,6 +199,10 @@ bool Engine::build(const std::string& onnxPath, const w2x_build_config& bc) {
             g = parseOnnx(readFile(onnxPath));
         } catch (const std::exception& ex) {
             ELOG(W2X_ERROR, std::string("Failed to parse ONNX model: ") + ex.what() + ".");
+            return false;
+        }
+        if (bc.precision == W2X_PRECISION_TF32 && isSwinGraph(g)) {
+            ELOG(W2X_ERROR, "Failed to set precision: tf32 is not available for swin_unet models.");
             return false;
         }
         PackedModel pm = packFromOnnx(g, bc.precision);
@@ -227,6 +235,19 @@ static std::string findEngine(const std::string& modelPath, const w2x_render_con
 // ------------------------------------------------------------------------------------------------
 bool Engine::load(const std::string& onnxPath, const w2x_render_config& rc) {
     try {
+        if (rc.precision != W2X_PRECISION_FP16 && rc.precision != W2X_PRECISION_TF32) {
+            ELOG(W2X_ERROR, "Failed to set precision: unknown precision " + std::to_string(rc.precision) + ".");
+            return false;
+        }
+        if (rc.precision == W2X_PRECISION_TF32) {
+            // no tf32 engine file can exist for a SwinUNet (build refuses it): say why rather than that none was found
+            bool swin = false;
+            try { swin = isSwinGraph(parseOnnx(readFile(onnxPath))); } catch (const std::exception&) {}
+            if (swin) {
+                ELOG(W2X_ERROR, "Failed to set precision: tf32 is not available for swin_unet models.");
+                return false;
+            }
+        }
         std::string enginePath;
         try {
             enginePath = findEngine(onnxPath, rc);
@@ -243,12 +264,17 @@ bool Engine::load(const std::string& onnxPath, const w2x_render_config& rc) {
             ELOG(W2X_ERROR, "Failed to set input tensor shape.");
             return false;
         }
-        if (rc.precision != W2X_PRECISION_FP16) {
-            ELOG(W2X_ERROR, "precision tf32 is not available in this build");
-            return false;
-        }
         unload();
         model = deserializePack(readFile(enginePath));
+        if ((int)model.precision != rc.precision) {
+            ELOG(W2X_ERROR, "Engine file \"" + enginePath + "\" was packed for another precision.");
+            return false;
+        }
+        if (model.arch == ARCH_SWINUNET && model.precision == W2X_PRECISION_TF32) {
+            ELOG(W2X_ERROR, "Failed to set precision: tf32 is not available for swin_unet models.");
+            return false;
+        }
+        elemBytes = model.precision == W2X_PRECISION_TF32 ? 4 : 2;
         if ((int)model.scale != rc.scaling) {
             ELOG(W2X_ERROR, "Render scaling " + std::to_string(rc.scaling) + " does not match the model's scale " + std::to_string(model.scale) + ".");
             return false;
@@ -297,14 +323,15 @@ void Engine::buildPlanCunet() {
             const uint32_t want = (i == 7 && !up) ? (uint32_t)L_CONV3 : kinds[i];
             const PackedLayer& L = model.layers[i];
             if (L.kind != want) throw Error("pack file layer " + std::to_string(i) + " ('" + L.name + "') has an unexpected kind");
-            if (L.w.size() != (size_t)L.npad * L.ktot || L.bias.size() != L.npad) throw Error("pack file layer '" + L.name + "' is truncated");
+            if (L.weightCount() != (size_t)L.npad * L.ktot || L.bias.size() != L.npad) throw Error("pack file layer '" + L.name + "' is truncated");
         }
     }
     // weights -> HBM
     for (const auto& L : model.layers) {
-        __half* w = (__half*)dalloc(L.w.size() * 2);
+        const size_t wBytes = L.weightCount() * elemBytes;
+        __half* w = (__half*)dalloc(wBytes);
         float* b = (float*)dalloc(L.bias.size() * 4);
-        uploadAsync(w, L.w.data(), L.w.size() * 2);
+        uploadAsync(w, tf32() ? (const void*)L.wf.data() : (const void*)L.w.data(), wBytes);
         uploadAsync(b, L.bias.data(), L.bias.size() * 4);
         dW.push_back(w);
         dBias.push_back(b);
@@ -319,6 +346,14 @@ void Engine::buildPlanCunet() {
         return v;
     };
     const float S = 0.1f;
+    // fused squeeze: the conv epilogue accumulates exact fixed-point channel sums (int64 atomics) per image
+    auto fuseSqueeze = [&](LayerExec& E, const PackedLayer& L) {
+        E.sePartialBytes = (size_t)batch * L.npad * sizeof(long long);
+        E.sePartial = (long long*)dalloc(E.sePartialBytes);
+        E.p.se_sum = E.sePartial;
+        E.seFused = true;
+    };
+    // The plan below is the same for both precisions; only the kernel behind each layer differs.
     auto push = [&](int li, const ConvParams& p, double flops, bool fin = false) {
         LayerExec E;
         const PackedLayer& L = model.layers[li];
@@ -326,18 +361,19 @@ void Engine::buildPlanCunet() {
         E.p = p;
         E.flops = flops;
         E.isFinal = fin;
-        if (useDirect) E.impl = IMPL_DIRECT;
-        else if (L.kind == L_CONV3 && L.cin == 4 && L.npad == 32 && p.mode == EPI_STORE) E.impl = IMPL_FIRST;
+        const bool rgbFirst = L.kind == L_CONV3 && L.cin == 4 && L.npad == 32 && p.mode == EPI_STORE;
+        if (tf32() && rgbFirst) E.impl = IMPL_FIRST_F32;
+        else if (tf32()) {
+            E.impl = IMPL_TF32;
+            if (L.se_r) fuseSqueeze(E, L);
+            E.tf32 = tf32CreatePlan(asF32(E.p));
+        }
+        else if (useDirect) E.impl = IMPL_DIRECT;
+        else if (rgbFirst) E.impl = IMPL_FIRST;
         else if (convHeadSupported(p) && !devEnv("W2X_NO_HEAD_KERNEL")) { E.impl = IMPL_HEAD; E.head = convHeadCreatePlan(p); }
         else if (igemmSupported(p)) {
             E.impl = IMPL_IGEMM;
-            if (L.se_r) {
-                // fused squeeze: the conv epilogue accumulates exact fixed-point channel sums (int64 atomics) per image
-                E.sePartialBytes = (size_t)batch * L.npad * sizeof(long long);
-                E.sePartial = (long long*)dalloc(E.sePartialBytes);
-                E.p.se_sum = E.sePartial;
-                E.seFused = true;
-            }
+            if (L.se_r) fuseSqueeze(E, L);
             // a UNet's second convolution computes its RGB first layer on the fly (fusedFirstProducer): the 32-channel tensor
             // between them never touches HBM and the first layer's launch disappears
             static const bool noFuse = devEnv("W2X_NO_FUSE_FIRST") != nullptr;
@@ -377,10 +413,10 @@ void Engine::buildPlanCunet() {
         const PackedLayer& L = model.layers[li];
         LayerExec& prod = layers[seLayerIdx];
         if (!prod.seR) throw Error("internal: SE fold without an SE producer");
-        __half* wImg = (__half*)dalloc((size_t)batch * L.w.size() * 2);
+        __half* wImg = (__half*)dalloc((size_t)batch * L.weightCount() * elemBytes);
         prod.foldJobs.push_back({dW[li], wImg, (int)L.npad, (int)L.ktot, (int)L.cin});
         p.w = wImg;
-        p.w_img_stride = (long long)L.w.size();
+        p.w_img_stride = (long long)L.weightCount();
     };
     auto down2 = [&](int li, const Act& in, int seProducer = -1) {
         const PackedLayer& L = model.layers[li];
@@ -440,16 +476,27 @@ void Engine::buildPlanCunet() {
     Act c5 = conv3(20, u4, 64);
     if (z1.h - 40 != c5.h - 2) throw Error("tile size is not supported by this model (head crop mismatch)");
     actOut = conv3(21, c5, 3, EPI_FINAL, 1.f, &z1, 20, true);
+    for (const auto& L : layers)  // the fp32 kernels take SE scales through the consumers' weights only (launchSeScale is fp16)
+        if (tf32() && L.seR && (!L.seFused || L.foldJobs.empty())) throw Error("internal: tf32 SE layer '" + L.name + "' is not fused and folded");
     outTile = actOut.h;
     const int expect = up ? 2 * tile - 72 : tile - 56;
     if (outTile != expect) throw Error("internal: output tile size mismatch");
 }
 
-void Engine::launchLayer(LayerExec& L, cudaStream_t s, __half* outp, int nImg, const __half* inOverride) {
+void Engine::launchLayer(LayerExec& L, cudaStream_t s, void* outp, int nImg, const void* inOverride) {
     switch (L.impl) {
         case IMPL_SKIP: break;  // computed inside the next layer's kernel
-        case IMPL_IGEMM: igemmLaunch(L.plan, s, outp, nImg, inOverride); break;
-        case IMPL_HEAD: launchConvHead(L.head, s, outp, nImg); break;
+        case IMPL_IGEMM: igemmLaunch(L.plan, s, static_cast<__half*>(outp), nImg, static_cast<const __half*>(inOverride)); break;
+        case IMPL_TF32: tf32Launch(L.tf32, s, static_cast<float*>(outp), nImg); break;
+        case IMPL_FIRST_F32: {
+            ConvParamsF32 p = asF32(L.p);
+            p.gn = nImg;
+            if (outp) p.out = static_cast<float*>(outp);
+            if (inOverride) p.in = static_cast<const float*>(inOverride);
+            launchConvFirstF32(p, s);
+            break;
+        }
+        case IMPL_HEAD: launchConvHead(L.head, s, static_cast<__half*>(outp), nImg); break;
         case IMPL_SWIN_MLP: swinMlpLaunch(L.mlp, s, (long long)nImg * L.tokH * L.tokW); break;
         case IMPL_SWIN_ATTN: swinAttnLaunch(L.attn, s, nImg); break;
         case IMPL_LAYERNORM:
@@ -461,8 +508,8 @@ void Engine::launchLayer(LayerExec& L, cudaStream_t s, __half* outp, int nImg, c
         default: {
             ConvParams p = L.p;
             p.gn = nImg;
-            if (outp) p.out = outp;
-            if (inOverride) p.in = inOverride;
+            if (outp) p.out = static_cast<__half*>(outp);
+            if (inOverride) p.in = static_cast<const __half*>(inOverride);
             if (L.impl == IMPL_FIRST) launchConvFirst(p, s);
             else launchConvDirect(p, s);
         }
@@ -761,9 +808,11 @@ int Engine::layerKernel(int index, char* buf, int cap) const {
     if (index < 0 || index >= (int)layers.size()) return 0;
     const LayerExec& L = layers[index];
     if (L.plan) igemmDescribe(L.plan, buf, cap);
+    else if (L.tf32) tf32Describe(L.tf32, buf, cap);
     else if (L.mlp) swinMlpDescribe(L.mlp, buf, cap);
     else if (L.attn) swinAttnDescribe(L.attn, buf, cap);
-    else std::snprintf(buf, cap, "%s", L.impl == IMPL_FIRST ? "first-layer mma.sync" : L.impl == IMPL_LAYERNORM ? "layernorm" :
+    else std::snprintf(buf, cap, "%s", L.impl == IMPL_FIRST ? "first-layer mma.sync" : L.impl == IMPL_FIRST_F32 ? "first-layer fp32 (CUDA cores)" :
+                                       L.impl == IMPL_LAYERNORM ? "layernorm" :
                                        L.impl == IMPL_ATTENTION ? "window-attention mma.sync" :
                                        L.impl == IMPL_HEAD ? "head kernel, taps in N (tcgen05)" : L.impl == IMPL_SKIP ? "fused into the next layer" : "direct (reference kernel)");
     return 1;
@@ -781,18 +830,28 @@ double Engine::flopsPerTile() const {
 bool Engine::frameWideUnpack() const {
     if (layers.size() < 2) return false;
     const int impl = layers[0].impl;
-    return impl == IMPL_FIRST || impl == IMPL_DIRECT || (impl == IMPL_SKIP && layers[1].plan != nullptr);
+    return impl == IMPL_FIRST || impl == IMPL_FIRST_F32 || impl == IMPL_DIRECT || (impl == IMPL_SKIP && layers[1].plan != nullptr);
 }
 
 // inTiles: this batch's unpacked tiles inside the frame-wide buffer (nullptr: the per-batch input tensor actIn)
-void Engine::runModel(cudaStream_t s, __half* finalOut, int nImages, const __half* inTiles) {
+void Engine::launchSe(const LayerExec& L, int n, cudaStream_t s) {
+    if (!L.seFused) launchSeSqueeze(L.p.out, n, L.p.out_h, L.p.out_w, L.p.out_c, L.sePartial, s);
+    launchSeExcite(L.sePartial, n, L.p.out_c, L.seR, L.p.out_h * L.p.out_w, L.seW1, L.seB1, L.seW2, L.seB2, L.seScale, s);
+    if (L.foldJobs.empty()) launchSeScale(L.p.out, n, L.p.out_h, L.p.out_w, L.p.out_c, L.seScale, s);
+    for (const auto& j : L.foldJobs) {
+        if (tf32()) launchScaleWeightsF32(static_cast<const float*>(j.w), static_cast<float*>(j.wOut), L.seScale, n, j.npad, j.ktot, j.cin, s);
+        else launchScaleWeights(static_cast<const __half*>(j.w), static_cast<__half*>(j.wOut), L.seScale, n, j.npad, j.ktot, j.cin, s);
+    }
+}
+
+void Engine::runModel(cudaStream_t s, void* finalOut, int nImages, const void* inTiles) {
     const int n = (nImages > 0 && nImages < batch) ? nImages : batch;
     // SE accumulators are cleared up front so that the layer chain below is kernel -> kernel only (programmatic dependent launch)
     for (auto& L : layers)
         if (L.seR) W2X_CUDA(cudaMemsetAsync(L.sePartial, 0, L.sePartialBytes, s));
     for (size_t li = 0; li < layers.size(); ++li) {
         LayerExec& L = layers[li];
-        __half* outp = (L.isFinal && finalOut) ? finalOut : L.p.out;
+        void* outp = (L.isFinal && finalOut) ? finalOut : static_cast<void*>(L.p.out);
         // the layer that reads the model input: layer 0, or its fused consumer (layer 1) when layer 0 runs inside it
         const bool readsInput = inTiles && (li == 0 || (li == 1 && layers[0].impl == IMPL_SKIP));
         launchLayer(L, s, outp, n, readsInput ? inTiles : nullptr);
@@ -803,11 +862,8 @@ void Engine::runModel(cudaStream_t s, __half* finalOut, int nImages, const __hal
             if (de != cudaSuccess) throw Error("layer '" + L.name + "': " + cudaGetErrorString(de));
         }
         if (L.seR) {
-            if (!L.seFused) { launchSeSqueeze(L.p.out, n, L.p.out_h, L.p.out_w, L.p.out_c, L.sePartial, s); ++launches; }
-            launchSeExcite(L.sePartial, n, L.p.out_c, L.seR, L.p.out_h * L.p.out_w, L.seW1, L.seB1, L.seW2, L.seB2, L.seScale, s);
-            ++launches;
-            if (L.foldJobs.empty()) { launchSeScale(L.p.out, n, L.p.out_h, L.p.out_w, L.p.out_c, L.seScale, s); ++launches; }
-            for (const auto& j : L.foldJobs) { launchScaleWeights(j.w, j.wOut, L.seScale, n, j.npad, j.ktot, j.cin, s); ++launches; }
+            launchSe(L, n, s);
+            launches += (L.seFused ? 0 : 1) + 1 + (L.foldJobs.empty() ? 1 : (long long)L.foldJobs.size());
         }
     }
     W2X_CUDA(cudaGetLastError());
@@ -877,16 +933,16 @@ void Engine::ensureFrameBuffers(int w, int h) {
         if (need > unpackedCap) {
             if (dUnpacked) cudaFree(dUnpacked);
             dUnpacked = nullptr;
-            W2X_CUDA(cudaMalloc(&dUnpacked, need * sizeof(__half)));
+            W2X_CUDA(cudaMalloc(&dUnpacked, need * elemBytes));
             unpackedCap = need;
             // a fused RGB first layer reads the buffer through a tensor map of its own
-            if (layers[0].impl == IMPL_SKIP) igemmSetFusedFrameInput(layers[1].plan, dUnpacked, stepCount);
+            if (layers[0].impl == IMPL_SKIP) igemmSetFusedFrameInput(layers[1].plan, static_cast<const __half*>(dUnpacked), stepCount);
         }
     }
     const size_t tileElems = (size_t)outTile * outTile * 4;
     if ((size_t)stepCount * tileElems > tileOutCap) {
         if (dTileOut) cudaFree(dTileOut);
-        W2X_CUDA(cudaMalloc(&dTileOut, (size_t)stepCount * tileElems * sizeof(__half)));
+        W2X_CUDA(cudaMalloc(&dTileOut, (size_t)stepCount * tileElems * elemBytes));
         tileOutCap = (size_t)stepCount * tileElems;
     }
     if (cfg.tta && (size_t)grid.count * tileElems > ttaCap) {
@@ -926,7 +982,7 @@ void Engine::renderOnStream(const uint8_t* dSrc, int w, int h, size_t srcPitch, 
         sp.rampx = dRampX; sp.rampy = dRampY;
         sp.dst = dDst; sp.pitch = dstPitch;
         sp.tiles = cfg.tta ? (const void*)dTtaMean : (const void*)dTileOut;
-        sp.f32 = cfg.tta ? 1 : 0;
+        sp.f32 = (cfg.tta || tf32()) ? 1 : 0;
         sp.tile_map = cfg.tta ? nullptr : dTileMap;
         sp.y_begin = yBegin; sp.y_end = yEnd;
         launchStitch(sp, s);
@@ -951,7 +1007,7 @@ void Engine::renderOnStream(const uint8_t* dSrc, int w, int h, size_t srcPitch, 
     const bool frameWide = frameWideUnpack();
     if (frameWide)
         span(0, [&] {
-            launchUnpack(dSrc, w, h, srcPitch, dSlots, realSteps, tile, dUnpacked, s);
+            unpackTiles(dSrc, w, h, srcPitch, dSlots, realSteps, dUnpacked, s);
             ++launches;
         });
     for (int b = 0; b < batchCount; ++b) {
@@ -960,10 +1016,10 @@ void Engine::renderOnStream(const uint8_t* dSrc, int w, int h, size_t srcPitch, 
         if (nReal <= 0) continue;
         if (!frameWide)
             span(0, [&] {
-                launchUnpack(dSrc, w, h, srcPitch, dSlots + (size_t)b * batch, nReal, tile, actIn.p, s);
+                unpackTiles(dSrc, w, h, srcPitch, dSlots + (size_t)b * batch, nReal, actIn.p, s);
                 ++launches;
             });
-        span(1, [&] { runModel(s, dTileOut + (size_t)b * batch * tileElems, nReal, frameWide ? dUnpacked + (size_t)b * batch * inElems : nullptr); });
+        span(1, [&] { runModel(s, elemAt(dTileOut, (size_t)b * batch * tileElems), nReal, frameWide ? elemAt(dUnpacked, (size_t)b * batch * inElems) : nullptr); });
         if (progressive) {
             // output rows that only depend on tile rows finished with this batch: stitch them now, hand the caller an event to copy after
             for (const RowBand& rb : rowBands) {
@@ -990,11 +1046,21 @@ void Engine::renderOnStream(const uint8_t* dSrc, int w, int h, size_t srcPitch, 
     }
     if (cfg.tta)
         span(4, [&] {
-            launchTtaReduce(dTileOut, grid.count, outTile, dTtaMean, s);
+            ttaReduce(dTileOut, grid.count, dTtaMean, s);
             ++launches;
         });
     span(2, [&] { stitchRows(0, h * scale); });
     W2X_CUDA(cudaGetLastError());
+}
+
+void Engine::unpackTiles(const uint8_t* src, int w, int h, size_t pitch, const TileSlot* slots, int n, void* out, cudaStream_t s) {
+    if (tf32()) launchUnpack(src, w, h, pitch, slots, n, tile, static_cast<float*>(out), s);
+    else launchUnpack(src, w, h, pitch, slots, n, tile, static_cast<__half*>(out), s);
+}
+
+void Engine::ttaReduce(const void* outs, int tiles, float* mean, cudaStream_t s) {
+    if (tf32()) launchTtaReduce(static_cast<const float*>(outs), tiles, outTile, mean, s);
+    else launchTtaReduce(static_cast<const __half*>(outs), tiles, outTile, mean, s);
 }
 
 int Engine::lastStageMs(float* out, int n) {
@@ -1142,7 +1208,8 @@ bool Engine::renderBanded(Engine* const* es, int count, const uint8_t* src, int 
         for (int r = 0; r < count; ++r) {
             if (!es[r] || !es[r]->isLoaded) throw Error("no engine loaded");
             if (es[r]->tile != e0.tile || es[r]->outTile != e0.outTile || es[r]->scale != e0.scale || es[r]->batch != e0.batch ||
-                es[r]->cfg.overlapX != e0.cfg.overlapX || es[r]->cfg.overlapY != e0.cfg.overlapY || es[r]->cfg.tta != e0.cfg.tta)
+                es[r]->cfg.overlapX != e0.cfg.overlapX || es[r]->cfg.overlapY != e0.cfg.overlapY || es[r]->cfg.tta != e0.cfg.tta ||
+                es[r]->elemBytes != e0.elemBytes)
                 throw Error("row-band render needs identically configured engines");
         }
         const int scale = e0.scale, outT = e0.outTile, tile = e0.tile, batch = e0.batch;
@@ -1152,7 +1219,7 @@ bool Engine::renderBanded(Engine* const* es, int count, const uint8_t* src, int 
         if (g.count <= 0) throw Error("frame is too small for the configured tile overlap");
         const int bands = std::min(count, g.ny);
         const size_t tileElems = (size_t)outT * outT * 4;
-        const size_t elemBytes = tta ? sizeof(float) : sizeof(__half);  // stitched tiles: the fp16 model outputs, or the f32 TTA means
+        const size_t elemBytes = tta ? sizeof(float) : e0.elemBytes;  // stitched tiles: the model outputs, or the f32 TTA means
         const int sty = outT - g.outOvY;
         const int cw = w * scale, ch = h * scale;
         struct Band { int j0, j1, own, steps, yBegin, yEnd, inY0, inY1; };
@@ -1186,7 +1253,7 @@ bool Engine::renderBanded(Engine* const* es, int count, const uint8_t* src, int 
             const int bandH = b.inY1 - b.inY0;
             grow(e.dFrameIn, e.frameInCap, (size_t)w * 3 * bandH, 1);
             grow(e.dFrameOut, e.frameOutCap, (size_t)cw * 3 * (size_t)(b.yEnd - b.yBegin), 1);
-            grow(e.dBandTiles, e.bandTilesCap, (size_t)b.steps * tileElems + (tta ? 0 : (size_t)g.nx * tileElems), sizeof(__half));
+            grow(e.dBandTiles, e.bandTilesCap, (size_t)b.steps * tileElems + (tta ? 0 : (size_t)g.nx * tileElems), e.elemBytes);
             if (tta) grow(e.dBandMean, e.bandMeanCap, (size_t)(b.own + g.nx) * tileElems, sizeof(float));
             grow(e.dBandMap, e.bandMapCap, (size_t)g.count, sizeof(int));
             grow(e.dBandSlots, e.bandSlotCap, (size_t)b.steps, sizeof(TileSlot));
@@ -1212,13 +1279,13 @@ bool Engine::renderBanded(Engine* const* es, int count, const uint8_t* src, int 
             for (int bi = 0; bi < b.steps / batch; ++bi) {
                 const int nReal = std::min(batch, realSteps - bi * batch);
                 if (nReal <= 0) break;
-                launchUnpack(e.dFrameIn, w, bandH, (size_t)w * 3, e.dBandSlots + (size_t)bi * batch, nReal, tile, e.actIn.p, e.stream);
+                e.unpackTiles(e.dFrameIn, w, bandH, (size_t)w * 3, e.dBandSlots + (size_t)bi * batch, nReal, e.actIn.p, e.stream);
                 ++e.launches;
                 W2X_CUDA(cudaGetLastError());
-                e.runModel(e.stream, e.dBandTiles + (size_t)bi * batch * tileElems, nReal);
+                e.runModel(e.stream, e.elemAt(e.dBandTiles, (size_t)bi * batch * tileElems), nReal);
             }
             if (tta) {
-                launchTtaReduce(e.dBandTiles, b.own, outT, e.dBandMean, e.stream);
+                e.ttaReduce(e.dBandTiles, b.own, e.dBandMean, e.stream);
                 ++e.launches;
             }
             W2X_CUDA(cudaEventRecord(e.evBandModel, e.stream));
@@ -1249,7 +1316,7 @@ bool Engine::renderBanded(Engine* const* es, int count, const uint8_t* src, int 
                 W2X_CUDA(cudaMemcpy2DAsync(dstRow, tileBytes, srcRow, tileBytes, stripBytes, (size_t)g.nx, cudaMemcpyDefault, e.stream));
             }
             StitchParams sp{};
-            sp.tiles = tilesBase; sp.f32 = tta ? 1 : 0; sp.tile_map = e.dBandMap;
+            sp.tiles = tilesBase; sp.f32 = elemBytes == 4 ? 1 : 0; sp.tile_map = e.dBandMap;
             sp.outT = outT; sp.nx = g.nx; sp.ny = g.ny; sp.ovx = g.outOvX; sp.ovy = g.outOvY;
             sp.cw = cw; sp.ch = ch; sp.rampx = e.dRampX; sp.rampy = e.dRampY;
             // the band's output rows land at the top of its (band-sized) output buffer
@@ -1310,16 +1377,18 @@ bool Engine::infer(const float* inNchw, int n, float* outNchw) {
         W2X_CUDA(cudaSetDevice(cfg.deviceId));
         const size_t inElems = (size_t)n * 3 * tile * tile, outElems = (size_t)n * 3 * outTile * outTile;
         float *dIn = nullptr, *dOut = nullptr;
-        __half* dOutH = nullptr;
+        void* dOutH = nullptr;  // model output, engine elements
         W2X_CUDA(cudaMalloc(&dIn, inElems * 4));
         W2X_CUDA(cudaMalloc(&dOut, outElems * 4));
-        W2X_CUDA(cudaMalloc(&dOutH, (size_t)batch * outTile * outTile * 4 * 2));
+        W2X_CUDA(cudaMalloc(&dOutH, (size_t)batch * outTile * outTile * 4 * elemBytes));
         try {
             W2X_CUDA(cudaMemcpyAsync(dIn, inNchw, inElems * 4, cudaMemcpyHostToDevice, stream));
-            W2X_CUDA(cudaMemsetAsync(actIn.p, 0, actIn.elems() * 2, stream));
-            launchNchwToNhwc4(dIn, n, tile, actIn.p, stream);
+            W2X_CUDA(cudaMemsetAsync(actIn.p, 0, actIn.elems() * elemBytes, stream));
+            if (tf32()) launchNchwToNhwc4(dIn, n, tile, reinterpret_cast<float*>(actIn.p), stream);
+            else launchNchwToNhwc4(dIn, n, tile, actIn.p, stream);
             runModel(stream, dOutH, n);
-            launchNhwc4ToNchw(dOutH, n, outTile, dOut, stream);
+            if (tf32()) launchNhwc4ToNchw(static_cast<const float*>(dOutH), n, outTile, dOut, stream);
+            else launchNhwc4ToNchw(static_cast<const __half*>(dOutH), n, outTile, dOut, stream);
             launches += 2;
             W2X_CUDA(cudaMemcpyAsync(outNchw, dOut, outElems * 4, cudaMemcpyDeviceToHost, stream));
             W2X_CUDA(cudaStreamSynchronize(stream));
@@ -1351,12 +1420,7 @@ int Engine::profileLayers(int repeats, char (*names)[48], float* ms, double* flo
             for (int r = 0; r < repeats; ++r) {
                 if (L.seR) W2X_CUDA(cudaMemsetAsync(L.sePartial, 0, L.sePartialBytes, stream));
                 launchLayer(L, stream, nullptr, batch);
-                if (L.seR) {
-                    if (!L.seFused) launchSeSqueeze(L.p.out, L.p.gn, L.p.out_h, L.p.out_w, L.p.out_c, L.sePartial, stream);
-                    launchSeExcite(L.sePartial, L.p.gn, L.p.out_c, L.seR, L.p.out_h * L.p.out_w, L.seW1, L.seB1, L.seW2, L.seB2, L.seScale, stream);
-                    if (L.foldJobs.empty()) launchSeScale(L.p.out, L.p.gn, L.p.out_h, L.p.out_w, L.p.out_c, L.seScale, stream);
-                    for (const auto& j : L.foldJobs) launchScaleWeights(j.w, j.wOut, L.seScale, L.p.gn, j.npad, j.ktot, j.cin, stream);
-                }
+                if (L.seR) launchSe(L, L.p.gn, stream);
             }
             W2X_CUDA(cudaEventRecord(e1, stream));
             W2X_CUDA(cudaEventSynchronize(e1));
@@ -1365,8 +1429,8 @@ int Engine::profileLayers(int repeats, char (*names)[48], float* ms, double* flo
             std::snprintf(names[i], 48, "%s", L.name.c_str());
             if (std::getenv("W2X_VERBOSE")) {
                 char d[256] = "";
-                if (L.plan) igemmDescribe(L.plan, d, sizeof(d));
-                std::fprintf(stderr, "[w2x] %-28s %s\n", L.name.c_str(), L.plan ? d : (L.impl == IMPL_FIRST ? "first-layer mma.sync" : L.impl == IMPL_HEAD ? "head kernel, taps in N (tcgen05)" : L.impl == IMPL_SKIP ? "fused into the next layer" : "direct"));
+                layerKernel(i, d, sizeof(d));
+                std::fprintf(stderr, "[w2x] %-28s %s\n", L.name.c_str(), d);
             }
             ms[i] = t / repeats;
             flops[i] = L.flops * batch;
@@ -1445,6 +1509,51 @@ void runConvLayer(int device, int kind, int impl, int n, int h, int w, int cin, 
         W2X_CUDA(cudaDeviceSynchronize());
         W2X_CUDA(cudaGetLastError());
         W2X_CUDA(cudaMemcpy(outData, out.p, out.elems() * 2, cudaMemcpyDeviceToHost));
+    } catch (...) {
+        cleanup();
+        throw;
+    }
+    cleanup();
+}
+
+void runConvLayerF32(int device, int kind, int n, int h, int w, int cin, int cout, const float* in, const float* wPacked, const float* bias,
+                     const float* skipData, float* outData) {
+    W2X_CUDA(cudaSetDevice(device));
+    std::vector<void*> bufs;
+    Tf32Plan* plan = nullptr;
+    auto cleanup = [&] {
+        if (plan) tf32DestroyPlan(plan);
+        for (void* b : bufs) cudaFree(b);
+    };
+    try {
+        auto dmal = [&](size_t bytes) { void* p = nullptr; W2X_CUDA(cudaMalloc(&p, bytes + 256)); bufs.push_back(p); return p; };
+        auto up = [&](const void* src, size_t bytes) { void* d = dmal(bytes); W2X_CUDA(cudaMemcpy(d, src, bytes, cudaMemcpyHostToDevice)); return d; };
+        int npad = 0, ktot = 0;
+        Act out{}, skip{};
+        convLayerGeometry(kind, n, h, w, cin, cout, npad, ktot, out, skip);
+        if (!in || !wPacked || !bias || !outData || (skip.n && !skipData)) throw Error("null argument");
+        // the ConvParams builders take the nominal fp16 pointer type of the engine's plan (see Act)
+        Act inA{nullptr, n, h, w, cin};
+        inA.p = (__half*)up(in, inA.elems() * 4);
+        const __half* dWt = (const __half*)up(wPacked, (size_t)npad * ktot * 4);
+        float* dB = (float*)up(bias, (size_t)npad * 4);
+        if (skip.n) skip.p = (__half*)up(skipData, skip.elems() * 4);
+        out.p = (__half*)dmal(out.elems() * 4);
+        W2X_CUDA(cudaMemset(out.p, 0, out.elems() * 4));
+        ConvParams p{};
+        if (kind == 0) p = makeConv3Params(inA, out, dWt, dB, npad, EPI_STORE, 0.1f, cout);
+        else if (kind == 1) p = makeDown2Params(inA, out, dWt, dB, npad, 0.1f);
+        else if (kind == 2) p = makeUp2Params(inA, out, dWt, dB, cout, 0.1f, &skip, 4);
+        else if (kind == 3) p = makeUp4Params(inA, out, dWt, dB);
+        else {
+            p = makeConv3Params(inA, out, dWt, dB, npad, EPI_FINAL, 1.f, 4);
+            p.skip = skip.p; p.skip_h = skip.h; p.skip_w = skip.w; p.skip_c = 4; p.skip_off = 20;
+        }
+        plan = tf32CreatePlan(asF32(p));
+        tf32Launch(plan, nullptr);
+        W2X_CUDA(cudaDeviceSynchronize());
+        W2X_CUDA(cudaGetLastError());
+        W2X_CUDA(cudaMemcpy(outData, out.p, out.elems() * 4, cudaMemcpyDeviceToHost));
     } catch (...) {
         cleanup();
         throw;

@@ -4,6 +4,7 @@
 #include <cuda_fp16.h>
 #include <cuda_runtime.h>
 
+#include <cstring>
 #include <string>
 #include <vector>
 
@@ -19,19 +20,31 @@ namespace w2x {
         if (_e != cudaSuccess) throw ::w2x::Error(std::string(#expr) + ": " + cudaGetErrorString(_e)); \
     } while (0)
 
+// Activation tensor NHWC [n][h][w][c].  Its elements are the engine's (Engine::elemBytes): fp16, or fp32 in a tf32 engine, where the
+// pointer (like every activation / weight pointer of the plan and of ConvParams) is nominal and the kernels read it as float (asF32).
 struct Act {
     __half* p = nullptr;
     int n = 0, h = 0, w = 0, c = 0;
     size_t elems() const { return (size_t)n * h * w * c; }
 };
 
-enum ConvImpl { IMPL_DIRECT = 0, IMPL_FIRST = 1, IMPL_IGEMM = 2, IMPL_LAYERNORM = 3, IMPL_ATTENTION = 4, IMPL_HEAD = 5, IMPL_SKIP = 6, IMPL_SWIN_MLP = 7, IMPL_SWIN_ATTN = 8 };
+enum ConvImpl { IMPL_DIRECT = 0, IMPL_FIRST = 1, IMPL_IGEMM = 2, IMPL_LAYERNORM = 3, IMPL_ATTENTION = 4, IMPL_HEAD = 5, IMPL_SKIP = 6, IMPL_SWIN_MLP = 7, IMPL_SWIN_ATTN = 8,
+                IMPL_TF32 = 9, IMPL_FIRST_F32 = 10 };
+
+// the plan's ConvParams of a tf32 engine, as the fp32 kernels take them (same layout; the pointers address fp32 data)
+inline ConvParamsF32 asF32(const ConvParams& p) {
+    static_assert(sizeof(ConvParams) == sizeof(ConvParamsF32), "ConvParamsT layouts differ");
+    ConvParamsF32 q;
+    std::memcpy(static_cast<void*>(&q), &p, sizeof q);
+    return q;
+}
 
 struct LayerExec {
     std::string name;
     ConvParams p{};
     int impl = IMPL_DIRECT;
     IgemmPlan* plan = nullptr;
+    Tf32Plan* tf32 = nullptr;  // IMPL_TF32
     HeadPlan* head = nullptr;  // IMPL_HEAD
     SwinMlpPlan* mlp = nullptr;  // IMPL_SWIN_MLP: LayerNorm + fc1 + GELU + fc2 + residual in one kernel (the two preceding layers are IMPL_SKIP)
     SwinAttnPlan* attn = nullptr;  // IMPL_SWIN_ATTN: LayerNorm + QKV + window attention + proj + residual in one kernel (three preceding layers are IMPL_SKIP)
@@ -43,7 +56,7 @@ struct LayerExec {
     long long* sePartial = nullptr;  // [batch][C] exact fixed-point channel sums (2^10 scale, kSeFixedScale)
     float* seScale = nullptr;
     int seBlocks = 0;
-    struct FoldJob { const __half* w; __half* wOut; int npad, ktot, cin; };
+    struct FoldJob { const void* w; void* wOut; int npad, ktot, cin; };  // engine element type
     std::vector<FoldJob> foldJobs;  // consumers that take this layer's SE scale through per-image weights
     bool seFused = false;        // squeeze sums come from the conv epilogue (ConvParams::se_sum)
     size_t sePartialBytes = 0;
@@ -99,8 +112,14 @@ private:
     void uploadAsync(void* dst, const void* src, size_t bytes);
     void buildPlanCunet();
     void buildPlanSwin();
-    void launchLayer(LayerExec& L, cudaStream_t s, __half* outOverride, int nImages, const __half* inOverride = nullptr);
-    void runModel(cudaStream_t s, __half* finalOut, int nImages = 0, const __half* inTiles = nullptr);
+    void launchLayer(LayerExec& L, cudaStream_t s, void* outOverride, int nImages, const void* inOverride = nullptr);
+    void runModel(cudaStream_t s, void* finalOut, int nImages = 0, const void* inTiles = nullptr);
+    void launchSe(const LayerExec& L, int nImages, cudaStream_t s);  // squeeze (unless fused) -> excite -> scale or fold into the consumers
+    bool tf32() const { return elemBytes == 4; }
+    // element `i` of an activation / tile buffer of this engine's element type
+    void* elemAt(void* base, size_t i) const { return static_cast<uint8_t*>(base) + i * elemBytes; }
+    void unpackTiles(const uint8_t* src, int w, int h, size_t pitch, const TileSlot* slots, int n, void* out, cudaStream_t s);
+    void ttaReduce(const void* outs, int tiles, float* mean, cudaStream_t s);
     bool frameWideUnpack() const;
     void ensureFrameBuffers(int w, int h);
     struct RowBand { int y0, y1, batch; };             // output rows [y0, y1) are final once batch `batch` has run (row-major tile order)
@@ -121,11 +140,12 @@ private:
     w2x_render_config cfg{};
     PackedModel model;
     int tile = 0, outTile = 0, scale = 1, batch = 1;
+    size_t elemBytes = 2;            // activations, weights and model outputs: 2 (fp16) or 4 (fp32, --precision tf32)
     bool useDirect = false;
     bool debugSync = false;      // W2X_DEBUG_SYNC: synchronise + check after every layer (names the failing kernel)
 
     std::vector<void*> allocs;       // freed in unload()
-    std::vector<__half*> dW;         // per layer
+    std::vector<__half*> dW;         // per layer (engine element type)
     std::vector<float*> dBias;
     std::vector<LayerExec> layers;
     Act actIn;                       // [batch][tile][tile][4]
@@ -143,9 +163,9 @@ private:
     std::vector<RowBand> rowBands;
     std::vector<cudaEvent_t> bandEv;
     size_t slotCap = 0;
-    __half* dUnpacked = nullptr;     // [steps][tile][tile][4] fp16: every tile of the frame, unpacked by one launch
+    void* dUnpacked = nullptr;       // [steps][tile][tile][4] engine elements: every tile of the frame, unpacked by one launch
     size_t unpackedCap = 0;
-    __half* dTileOut = nullptr;      // [steps][outT][outT][4] fp16
+    void* dTileOut = nullptr;        // [steps][outT][outT][4] engine elements
     size_t tileOutCap = 0;
     float* dTtaMean = nullptr;       // [tiles][outT][outT][4] f32 (TTA only)
     size_t ttaCap = 0;
@@ -171,7 +191,7 @@ private:
     cudaEvent_t nextEvent();
     cudaEvent_t timerEv[16] = {};
     // row-band mode
-    __half* dBandTiles = nullptr;
+    void* dBandTiles = nullptr;
     size_t bandTilesCap = 0;
     int* dBandMap = nullptr;
     size_t bandMapCap = 0;
@@ -187,6 +207,9 @@ private:
 // Single-layer test hooks, see include/w2x_dev.h.  impl: 0 = the kernel the planner picks, 1 = head kernel, 2 = scalar reference.
 void runConvLayer(int device, int kind, int impl, int n, int h, int w, int cin, int cout, const uint16_t* in, const uint16_t* wPacked,
                   const float* bias, const uint16_t* skip, uint16_t* out);
+// the same layer kinds through the tf32 kernel: fp32 NHWC tensors and fp32 packed weights
+void runConvLayerF32(int device, int kind, int n, int h, int w, int cin, int cout, const float* in, const float* wPacked, const float* bias,
+                     const float* skip, float* out);
 double selftestConv(int device, int kind, int n, int h, int w, int cin, int cout, unsigned seed);
 
 }  // namespace w2x

@@ -24,9 +24,11 @@ struct ConvTap {
     int c0, dx, dz, dy;  // offsets along (c, x, z, y) of the 5-D view
 };
 
-struct ConvParams {
+// T is the activation / weight element type: __half for the fp16 kernels, float for the tf32 kernel (conv_tf32_sm100.cu)
+template <typename T>
+struct ConvParamsT {
     // A operand view (element strides; c is contiguous)
-    const __half* in;
+    const T* in;
     long long sx, sz, sy, sn;
     int dimc, dimx, dimz, dimy;  // view extents (for the TMA map)
     int cin;                     // channels per tap
@@ -36,17 +38,17 @@ struct ConvParams {
     // GEMM extents
     int gx, gy, gn;  // pixel grid per image (x, y) and image count
     int npad, ktot;
-    const __half* w;    // B: [npad][ktot], K-major
+    const T* w;         // B: [npad][ktot], K-major
     long long w_img_stride;  // elements between per-image copies of B (SE scale folded into the weights), 0 = shared
     const float* bias;  // [npad]
     // epilogue
     int mode;
     float slope;  // LeakyReLU negative slope; 1.0f = linear
     int act;      // ActKind (EPI_STORE only)
-    __half* out;
+    T* out;
     int out_h, out_w, out_c;
     int cout;  // EPI_STORE: channels stored (4 or a multiple of 8); EPI_D2S: channels per phase
-    const __half* skip;
+    const T* skip;
     int skip_h, skip_w, skip_c, skip_off;
     const float* skip_scale;  // optional per-(img, channel) multiplier applied to skip (SE fold), or nullptr
     long long* se_sum;        // optional [gn][npad] int64: fused SE squeeze = sum over the image of round(activation * 2^10) (kSeFixedScale),
@@ -54,6 +56,8 @@ struct ConvParams {
                               // tile or on the image's batch slot); the buffer must be zeroed before the launch
     int se_slots;             // unused (kept for ABI stability of the struct inside this library)
 };
+using ConvParams = ConvParamsT<__half>;
+using ConvParamsF32 = ConvParamsT<float>;
 
 #ifdef __CUDACC__
 
@@ -231,6 +235,16 @@ void launchLayerNorm(const __half* x, __half* y, long long tokens, int c, const 
 void launchWindowAttention(const __half* qkv, __half* out, int n, int h, int w, int c, int heads, int window, int shift,
                            const float* relpos, cudaStream_t s);
 
+// tf32 path (kernels/conv_tf32_sm100.cu): fp32 NHWC activations and fp32 K-major weights, tcgen05 kind::tf32 MMAs, fp32 epilogues
+struct Tf32Plan;                                                  // opaque: tensor maps + launch geometry
+bool tf32Supported(const ConvParamsF32& p);
+Tf32Plan* tf32CreatePlan(const ConvParamsF32& p);                 // throws w2x::Error when unsupported
+void tf32DestroyPlan(Tf32Plan* plan);
+void tf32Launch(const Tf32Plan* plan, cudaStream_t s, float* outOverride = nullptr, int nImages = 0);
+const char* tf32Describe(const Tf32Plan* plan, char* buf, int cap);
+void launchConvFirstF32(const ConvParamsF32& p, cudaStream_t s);  // cin=4 -> 32 first layer on the CUDA cores (fp32 FMA)
+void launchScaleWeightsF32(const float* w, float* wOut, const float* scale, int nimg, int npad, int ktot, int cin, cudaStream_t s);
+
 // squeeze/excite
 constexpr float kSeFixedScale = 1024.f;  // 2^10 fixed-point resolution of the squeeze sums: 32 fp16-range values cannot overflow int32
 void launchSeSqueeze(const __half* x, int n, int h, int w, int c, long long* sums, cudaStream_t s);  // sums must be zeroed
@@ -244,6 +258,8 @@ void launchScaleWeights(const __half* w, __half* wOut, const float* scale, int n
 struct TileSlot { int x, y, aug, valid; };  // input rect origin, D4 op, 0 = zero dummy slot (img2img_render.cpp:281)
 void launchUnpack(const uint8_t* frame, int w, int h, size_t pitch, const TileSlot* slots, int nslots, int tile,
                   __half* out, cudaStream_t s);
+void launchUnpack(const uint8_t* frame, int w, int h, size_t pitch, const TileSlot* slots, int nslots, int tile,
+                  float* out, cudaStream_t s);  // tf32 engines: the reference's convertTo(CV_32F, 1/255) blob exactly
 struct StitchParams {
     const void* tiles;   // [count][outT][outT][4] fp16 or f32
     int f32;             // element type of tiles
@@ -259,8 +275,11 @@ struct StitchParams {
 };
 void launchStitch(const StitchParams& p, cudaStream_t s);
 void launchTtaReduce(const __half* outs, int tiles, int outT, float* mean, cudaStream_t s);
-// NCHW f32 <-> NHWC4 fp16 (Img2Img::infer host entry, tests)
+void launchTtaReduce(const float* outs, int tiles, int outT, float* mean, cudaStream_t s);
+// NCHW f32 <-> NHWC4 fp16 / f32 (Img2Img::infer host entry, tests)
 void launchNchwToNhwc4(const float* in, int n, int t, __half* out, cudaStream_t s);
 void launchNhwc4ToNchw(const __half* in, int n, int t, float* out, cudaStream_t s);
+void launchNchwToNhwc4(const float* in, int n, int t, float* out, cudaStream_t s);
+void launchNhwc4ToNchw(const float* in, int n, int t, float* out, cudaStream_t s);
 
 }  // namespace w2x

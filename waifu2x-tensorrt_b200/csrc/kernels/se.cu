@@ -4,6 +4,7 @@
 #include <cuda_fp16.h>
 #include <cuda_runtime.h>
 
+#include "../model_pack.h"
 #include "conv_params.h"
 #include "launch.h"
 
@@ -107,6 +108,23 @@ void launchScaleWeights(const __half* w, __half* wOut, const float* scale, int n
     const int total = npad * ktot;  // even; k and k+1 share a tap because cin is even
     dim3 grid((total / 2 + 255) / 256, nimg);
     launchPdl(scale_weights_kernel, grid, dim3(256), 0, s, w, wOut, scale, total, ktot, cin);
+}
+
+// fp32 twin for tf32 engines: the scaled weights are rounded to nearest TF32 like the packed ones (model_pack.h: roundToTf32)
+__global__ void __launch_bounds__(256) scale_weights_f32_kernel(const float* __restrict__ w, float* __restrict__ wOut, const float* __restrict__ scale,
+                                                                int total, int ktot, int cin) {
+    pdlLaunchDependents();
+    pdlWait();
+    const int img = blockIdx.y;
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= total) return;
+    wOut[(size_t)img * total + i] = roundToTf32(w[i] * scale[(size_t)img * cin + (i % ktot) % cin]);
+}
+
+void launchScaleWeightsF32(const float* w, float* wOut, const float* scale, int nimg, int npad, int ktot, int cin, cudaStream_t s) {
+    const int total = npad * ktot;
+    dim3 grid((total + 255) / 256, nimg);
+    launchPdl(scale_weights_f32_kernel, grid, dim3(256), 0, s, w, wOut, scale, total, ktot, cin);
 }
 
 void launchSeScale(__half* x, int n, int h, int w, int c, const float* scale, cudaStream_t s) {

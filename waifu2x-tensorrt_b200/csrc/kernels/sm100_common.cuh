@@ -134,6 +134,21 @@ __device__ __forceinline__ void ummaLoHi(uint32_t tmemD, uint32_t aLo, uint32_t 
         "r"(aLo), "r"(aHi), "r"(bLo), "r"(bHi), "r"(idesc), "r"(accumulate)
         : "memory");
 }
+// the same with kind::tf32 (fp32 operands in shared memory, TF32 multiply, fp32 accumulate): one K step is 8 elements = 32 bytes,
+// like the 16 fp16 elements of kind::f16, so the descriptors advance exactly as for fp16
+__device__ __forceinline__ void ummaTf32LoHi(uint32_t tmemD, uint32_t aLo, uint32_t aHi, uint32_t bLo, uint32_t bHi, uint32_t idesc, uint32_t accumulate) {
+    asm volatile(
+        "{\n\t"
+        ".reg .pred p;\n\t"
+        ".reg .b64 da, db;\n\t"
+        "setp.ne.b32 p, %6, 0;\n\t"
+        "mov.b64 da, {%1, %2};\n\t"
+        "mov.b64 db, {%3, %4};\n\t"
+        "tcgen05.mma.cta_group::1.kind::tf32 [%0], da, db, %5, p;\n\t"
+        "}" ::"r"(tmemD),
+        "r"(aLo), "r"(aHi), "r"(bLo), "r"(bHi), "r"(idesc), "r"(accumulate)
+        : "memory");
+}
 // one elected lane of a fully converged warp
 __device__ __forceinline__ bool electOne() {
     uint32_t pred;
@@ -182,6 +197,11 @@ __device__ __forceinline__ uint64_t makeDesc(uint32_t smemAddr, uint32_t hi) {
 // instruction descriptor (cute::UMMA::InstrDescriptor): D=F32 [4,6), A=B=F16 (0), K-major both, N>>3 [17,23), M>>4 [24,29)
 __host__ __device__ __forceinline__ uint32_t instrDescF16(int m, int n) {
     return (1u << 4) | ((uint32_t)(n >> 3) << 17) | ((uint32_t)(m >> 4) << 24);
+}
+
+// the same with A=B=TF32 (format 2 in bits [7,10) and [10,13))
+__host__ __device__ __forceinline__ uint32_t instrDescTf32(int m, int n) {
+    return instrDescF16(m, n) | (2u << 7) | (2u << 10);
 }
 
 __device__ __forceinline__ uint4 ldsV4(uint32_t addr) {

@@ -2,7 +2,7 @@
 // /root/reference/src/tensorrt/img2img_render.cpp and img2img_infer.cpp (SURVEY 2.1 table).
 //
 //   unpack     : padRoi (:68-105) + applyAugmentation (:134-177) + cvtColor BGR2RGB (:227) + split/convertTo(1/255)
-//                (infer.cpp:5-21) -> fp16 RGB0 NHWC4 tile batch, one pass, no intermediate mats.
+//                (infer.cpp:5-21) -> fp16 (f32 for tf32 engines) RGB0 NHWC4 tile batch, one pass, no intermediate mats.
 //   stitch     : applyWeights (:107-121) + canvas add (:329-330) + convertTo(8U, 255) (:342) + RGB2BGR (:343).
 //                Gather formulation: each output pixel is owned by exactly one thread, which sums the <= 4 covering
 //                tiles in the reference's tile order (column-major), so no zero-filled f32 canvas and no RMW passes.
@@ -48,6 +48,29 @@ __device__ __forceinline__ void revSrcIndex(int k, int r, int c, int n, int& rr,
     }
 }
 
+// one RGB0 pixel of an NHWC4 tensor: fp16 (fp16 engines) or f32 (tf32 engines)
+__device__ __forceinline__ void storePx(__half* out, size_t i, float r, float g, float b) {
+    Half4 o;
+    o.a = __floats2half2_rn(r, g);
+    o.b = __floats2half2_rn(b, 0.f);
+    reinterpret_cast<Half4*>(out)[i] = o;
+}
+__device__ __forceinline__ void storePx(float* out, size_t i, float r, float g, float b) {
+    reinterpret_cast<float4*>(out)[i] = make_float4(r, g, b, 0.f);
+}
+template <typename T> struct Px4;
+template <> struct Px4<__half> {
+    using type = Half4;
+    __device__ __forceinline__ static float3 rgb(const Half4& v) {
+        const float2 p0 = __half22float2(v.a), p1 = __half22float2(v.b);
+        return make_float3(p0.x, p0.y, p1.x);
+    }
+};
+template <> struct Px4<float> {
+    using type = float4;
+    __device__ __forceinline__ static float3 rgb(const float4& v) { return make_float3(v.x, v.y, v.z); }
+};
+
 // ---- unpack ---------------------------------------------------------------------------------------
 // grid: (tile/32 x tile/32 blocks of 32 x 32 output pixels, nslots), 256 threads.  Under every D4 augmentation the source of a
 // 32 x 32 output block is a 32 x 32 block of the (replicate-padded) frame, so the block first stages those 32 source rows (96
@@ -57,9 +80,10 @@ __device__ __forceinline__ void revSrcIndex(int k, int r, int c, int n, int& rr,
 constexpr int kUB = 32;             // block edge
 constexpr int kURow = 104;          // staged bytes per source row: 96 + up to 3 alignment bytes, rounded up to a word multiple
 
+template <typename T>
 __global__ void __launch_bounds__(256) unpack_kernel(const uint8_t* __restrict__ frame, int w, int h, size_t pitch,
                                                      const TileSlot* __restrict__ slots, int tile, int wordOk,
-                                                     __half* __restrict__ out) {
+                                                     T* __restrict__ out) {
     __shared__ __align__(16) uint8_t sm[kUB * kURow];
     __shared__ int smOff[kUB];      // byte offset of local source column 0 inside each staged row (fast path: alignment slack)
     const int blocksPerSide = (tile + kUB - 1) / kUB;
@@ -68,15 +92,12 @@ __global__ void __launch_bounds__(256) unpack_kernel(const uint8_t* __restrict__
     const int r0 = br * kUB, c0 = bc * kUB;
     const int tx = threadIdx.x & 31, ty = threadIdx.x >> 5;
     const TileSlot ts = slots[slot];
-    Half4* outp = reinterpret_cast<Half4*>(out) + (size_t)slot * tile * tile;
+    T* outp = out + (size_t)slot * tile * tile * 4;
     if (!ts.valid) {  // padding slot of the last batch (render.cpp:281): a zero tile
-        Half4 z;
-        z.a = __floats2half2_rn(0.f, 0.f);
-        z.b = z.a;
 #pragma unroll
         for (int i = 0; i < 4; ++i) {
             const int r = r0 + ty + 8 * i, c = c0 + tx;
-            if (r < tile && c < tile) outp[(size_t)r * tile + c] = z;
+            if (r < tile && c < tile) storePx(outp, (size_t)r * tile + c, 0.f, 0.f, 0.f);
         }
         return;
     }
@@ -122,20 +143,23 @@ __global__ void __launch_bounds__(256) unpack_kernel(const uint8_t* __restrict__
         const int lr = rr - rrMin;
         const uint8_t* px = sm + lr * kURow + smOff[lr] + (cc - ccMin) * 3;
         const float b = __fmul_rn((float)px[0], k), g = __fmul_rn((float)px[1], k), rch = __fmul_rn((float)px[2], k);
-        Half4 o;
-        o.a = __floats2half2_rn(rch, g);
-        o.b = __floats2half2_rn(b, 0.f);
-        outp[(size_t)r * tile + c] = o;
+        storePx(outp, (size_t)r * tile + c, rch, g, b);
     }
 }
 
-void launchUnpack(const uint8_t* frame, int w, int h, size_t pitch, const TileSlot* slots, int nslots, int tile,
-                  __half* out, cudaStream_t s) {
+template <typename T>
+void launchUnpackT(const uint8_t* frame, int w, int h, size_t pitch, const TileSlot* slots, int nslots, int tile, T* out, cudaStream_t s) {
     if (nslots <= 0) return;
     const int side = (tile + kUB - 1) / kUB;
     dim3 grid(side * side, nslots);
     const int wordOk = (reinterpret_cast<uintptr_t>(frame) & 3) == 0 ? 1 : 0;
-    unpack_kernel<<<grid, 256, 0, s>>>(frame, w, h, pitch, slots, tile, wordOk, out);
+    unpack_kernel<T><<<grid, 256, 0, s>>>(frame, w, h, pitch, slots, tile, wordOk, out);
+}
+void launchUnpack(const uint8_t* frame, int w, int h, size_t pitch, const TileSlot* slots, int nslots, int tile, __half* out, cudaStream_t s) {
+    launchUnpackT(frame, w, h, pitch, slots, nslots, tile, out, s);
+}
+void launchUnpack(const uint8_t* frame, int w, int h, size_t pitch, const TileSlot* slots, int nslots, int tile, float* out, cudaStream_t s) {
+    launchUnpackT(frame, w, h, pitch, slots, nslots, tile, out, s);
 }
 
 // ---- stitch + pack ----------------------------------------------------------------------------------
@@ -296,8 +320,10 @@ void launchStitch(const StitchParams& pin, cudaStream_t s) {
 // Block = 32 x 32 output pixels of one tile.  For each augmentation the 32 x 32 source block of that model output (again a square
 // block, see unpack) is staged in shared memory with coalesced 8-byte loads (256 contiguous bytes per row), so the transposed
 // augmentations gather from shared memory instead of striding through HBM; every thread then adds its four pixels in index order.
-__global__ void __launch_bounds__(256) tta_reduce_kernel(const __half* __restrict__ outs, int outT, float* __restrict__ mean) {
-    __shared__ Half4 sm[kUB][kUB + 1];
+template <typename T>
+__global__ void __launch_bounds__(256) tta_reduce_kernel(const T* __restrict__ outs, int outT, float* __restrict__ mean) {
+    using P = typename Px4<T>::type;
+    __shared__ P sm[kUB][kUB + 1];
     const int tile = blockIdx.y;
     const int side = (outT + kUB - 1) / kUB;
     const int br = blockIdx.x / side, bc = blockIdx.x - br * side;
@@ -312,7 +338,7 @@ __global__ void __launch_bounds__(256) tta_reduce_kernel(const __half* __restric
         revSrcIndex(k, r1, c1, outT, rb, cb);
         const int rrMin = min(ra, rb), ccMin = min(ca, cb);
         const int rows = abs(ra - rb) + 1, cols = abs(ca - cb) + 1;
-        const Half4* src = reinterpret_cast<const Half4*>(outs) + ((size_t)tile * 8 + k) * plane;
+        const P* src = reinterpret_cast<const P*>(outs) + ((size_t)tile * 8 + k) * plane;
         __syncthreads();  // the previous augmentation's reads of sm are done
         for (int lr = ty; lr < rows; lr += 8)
             if (tx < cols) sm[lr][tx] = src[(size_t)(rrMin + lr) * outT + ccMin + tx];
@@ -323,11 +349,10 @@ __global__ void __launch_bounds__(256) tta_reduce_kernel(const __half* __restric
             if (r >= outT || c >= outT) continue;
             int rr, cc;
             revSrcIndex(k, r, c, outT, rr, cc);
-            const Half4 v = sm[rr - rrMin][cc - ccMin];
-            const float2 p0 = __half22float2(v.a), p1 = __half22float2(v.b);
-            ar[i] = __fadd_rn(ar[i], p0.x);
-            ag[i] = __fadd_rn(ag[i], p0.y);
-            ab[i] = __fadd_rn(ab[i], p1.x);
+            const float3 v = Px4<T>::rgb(sm[rr - rrMin][cc - ccMin]);
+            ar[i] = __fadd_rn(ar[i], v.x);
+            ag[i] = __fadd_rn(ag[i], v.y);
+            ab[i] = __fadd_rn(ab[i], v.z);
         }
     }
     const float k8 = 0.125f;
@@ -340,45 +365,51 @@ __global__ void __launch_bounds__(256) tta_reduce_kernel(const __half* __restric
     }
 }
 
-void launchTtaReduce(const __half* outs, int tiles, int outT, float* mean, cudaStream_t s) {
+template <typename T>
+void launchTtaReduceT(const T* outs, int tiles, int outT, float* mean, cudaStream_t s) {
     if (tiles <= 0) return;
     const int side = (outT + kUB - 1) / kUB;
     dim3 grid(side * side, tiles);
-    tta_reduce_kernel<<<grid, 256, 0, s>>>(outs, outT, mean);
+    tta_reduce_kernel<T><<<grid, 256, 0, s>>>(outs, outT, mean);
 }
+void launchTtaReduce(const __half* outs, int tiles, int outT, float* mean, cudaStream_t s) { launchTtaReduceT(outs, tiles, outT, mean, s); }
+void launchTtaReduce(const float* outs, int tiles, int outT, float* mean, cudaStream_t s) { launchTtaReduceT(outs, tiles, outT, mean, s); }
 
 // ---- layout helpers for the Img2Img::infer-shaped entry point ---------------------------------------------
-__global__ void nchw_to_nhwc4_kernel(const float* __restrict__ in, int t, __half* __restrict__ out) {
+template <typename T>
+__global__ void nchw_to_nhwc4_kernel(const float* __restrict__ in, int t, T* __restrict__ out) {
     const int n = blockIdx.y;
     const int idx = blockIdx.x * blockDim.x + threadIdx.x;
     if (idx >= t * t) return;
     const size_t plane = (size_t)t * t;
     const float* b = in + (size_t)n * 3 * plane;
-    Half4 o{__floats2half2_rn(b[idx], b[plane + idx]), __floats2half2_rn(b[2 * plane + idx], 0.f)};
-    reinterpret_cast<Half4*>(out)[(size_t)n * plane + idx] = o;
+    storePx(out, (size_t)n * plane + idx, b[idx], b[plane + idx], b[2 * plane + idx]);
 }
 
-__global__ void nhwc4_to_nchw_kernel(const __half* __restrict__ in, int t, float* __restrict__ out) {
+template <typename T>
+__global__ void nhwc4_to_nchw_kernel(const T* __restrict__ in, int t, float* __restrict__ out) {
     const int n = blockIdx.y;
     const int idx = blockIdx.x * blockDim.x + threadIdx.x;
     if (idx >= t * t) return;
     const size_t plane = (size_t)t * t;
-    const Half4 v = reinterpret_cast<const Half4*>(in)[(size_t)n * plane + idx];
-    const float2 p0 = __half22float2(v.a), p1 = __half22float2(v.b);
+    const float3 v = Px4<T>::rgb(reinterpret_cast<const typename Px4<T>::type*>(in)[(size_t)n * plane + idx]);
     float* b = out + (size_t)n * 3 * plane;
-    b[idx] = p0.x;
-    b[plane + idx] = p0.y;
-    b[2 * plane + idx] = p1.x;
+    b[idx] = v.x;
+    b[plane + idx] = v.y;
+    b[2 * plane + idx] = v.z;
 }
 
 void launchNchwToNhwc4(const float* in, int n, int t, __half* out, cudaStream_t s) {
-    dim3 grid((t * t + 255) / 256, n);
-    nchw_to_nhwc4_kernel<<<grid, 256, 0, s>>>(in, t, out);
+    nchw_to_nhwc4_kernel<<<dim3((t * t + 255) / 256, n), 256, 0, s>>>(in, t, out);
 }
-
+void launchNchwToNhwc4(const float* in, int n, int t, float* out, cudaStream_t s) {
+    nchw_to_nhwc4_kernel<<<dim3((t * t + 255) / 256, n), 256, 0, s>>>(in, t, out);
+}
 void launchNhwc4ToNchw(const __half* in, int n, int t, float* out, cudaStream_t s) {
-    dim3 grid((t * t + 255) / 256, n);
-    nhwc4_to_nchw_kernel<<<grid, 256, 0, s>>>(in, t, out);
+    nhwc4_to_nchw_kernel<<<dim3((t * t + 255) / 256, n), 256, 0, s>>>(in, t, out);
+}
+void launchNhwc4ToNchw(const float* in, int n, int t, float* out, cudaStream_t s) {
+    nhwc4_to_nchw_kernel<<<dim3((t * t + 255) / 256, n), 256, 0, s>>>(in, t, out);
 }
 
 }  // namespace w2x

@@ -363,7 +363,8 @@ inline float W4(const OnnxTensor* t, int a, int b, int c, int d) {
     return t->data[(((size_t)a * s[1] + b) * s[2] + c) * s[3] + d];
 }
 
-PackedLayer packLayer(const ConvNode& c, int cinStore = 0, int npadTo = 0) {
+// tf32: the GEMM weights are stored as fp32 rounded to nearest TF32 (PackedLayer::wf) instead of fp16 bits (PackedLayer::w)
+PackedLayer packLayer(const ConvNode& c, bool tf32, int cinStore = 0, int npadTo = 0) {
     PackedLayer L;
     L.name = c.name;
     L.cout = (uint32_t)c.cout;
@@ -371,52 +372,53 @@ PackedLayer packLayer(const ConvNode& c, int cinStore = 0, int npadTo = 0) {
     if (cinp < c.cin || (cinp % 4)) throw Error("pack: unsupported cin in " + c.name);
     L.cin = (uint32_t)cinp;
     auto bias = [&](int co) { return c.b ? c.b->data[(size_t)co] : 0.0f; };
+    std::vector<float> w;  // [npad][ktot]
     if (!c.transpose && c.kh == 3 && c.kw == 3 && c.stride == 1 && c.pad == 0) {
         L.kind = L_CONV3; L.taps = 9;
         L.npad = (uint32_t)(npadTo > 0 ? npadTo : (c.cout + 15) / 16 * 16);
         L.ktot = 9 * L.cin;
-        L.w.assign((size_t)L.npad * L.ktot, 0);
+        w.assign((size_t)L.npad * L.ktot, 0.f);
         L.bias.assign(L.npad, 0.f);
         for (int co = 0; co < c.cout; ++co) {
             L.bias[co] = bias(co);
             for (int ky = 0; ky < 3; ++ky)
                 for (int kx = 0; kx < 3; ++kx)
                     for (int ci = 0; ci < c.cin; ++ci)
-                        L.w[(size_t)co * L.ktot + (ky * 3 + kx) * L.cin + ci] = floatToHalfBits(W4(c.w, co, ci, ky, kx));
+                        w[(size_t)co * L.ktot + (ky * 3 + kx) * L.cin + ci] = W4(c.w, co, ci, ky, kx);
         }
     } else if (!c.transpose && c.kh == 2 && c.kw == 2 && c.stride == 2 && c.pad == 0) {
         L.kind = L_DOWN2; L.taps = 4;
         L.npad = (uint32_t)((c.cout + 15) / 16 * 16);
         L.ktot = 4 * L.cin;
-        L.w.assign((size_t)L.npad * L.ktot, 0);
+        w.assign((size_t)L.npad * L.ktot, 0.f);
         L.bias.assign(L.npad, 0.f);
         for (int co = 0; co < c.cout; ++co) {
             L.bias[co] = bias(co);
             for (int dy = 0; dy < 2; ++dy)
                 for (int dx = 0; dx < 2; ++dx)
                     for (int ci = 0; ci < c.cin; ++ci)
-                        L.w[(size_t)co * L.ktot + (dy * 2 + dx) * L.cin + ci] = floatToHalfBits(W4(c.w, co, ci, dy, dx));
+                        w[(size_t)co * L.ktot + (dy * 2 + dx) * L.cin + ci] = W4(c.w, co, ci, dy, dx);
         }
     } else if (c.transpose && c.kh == 2 && c.kw == 2 && c.stride == 2 && c.pad == 0) {
         if (c.cout % 8) throw Error("pack: convT 2x2 cout must be a multiple of 8 in " + c.name);
         L.kind = L_UP2; L.taps = 1;
         L.npad = (uint32_t)(4 * c.cout);
         L.ktot = L.cin;
-        L.w.assign((size_t)L.npad * L.ktot, 0);
+        w.assign((size_t)L.npad * L.ktot, 0.f);
         L.bias.assign(L.npad, 0.f);
         for (int q = 0; q < 4; ++q)
             for (int co = 0; co < c.cout; ++co) {
                 const int n = q * c.cout + co;
                 L.bias[n] = bias(co);
                 for (int ci = 0; ci < c.cin; ++ci)
-                    L.w[(size_t)n * L.ktot + ci] = floatToHalfBits(W4(c.w, ci, co, q >> 1, q & 1));
+                    w[(size_t)n * L.ktot + ci] = W4(c.w, ci, co, q >> 1, q & 1);
             }
     } else if (c.transpose && c.kh == 4 && c.kw == 4 && c.stride == 2 && c.pad == 3) {
         if (c.cout > 4) throw Error("pack: convT 4x4 head supports cout <= 4 in " + c.name);
         L.kind = L_UP4; L.taps = 4;
         L.npad = 16;
         L.ktot = 4 * L.cin;
-        L.w.assign((size_t)L.npad * L.ktot, 0);
+        w.assign((size_t)L.npad * L.ktot, 0.f);
         L.bias.assign(L.npad, 0.f);
         for (int py = 0; py < 2; ++py)
             for (int px = 0; px < 2; ++px)
@@ -426,12 +428,19 @@ PackedLayer packLayer(const ConvNode& c, int cinStore = 0, int npadTo = 0) {
                     for (int wy = 0; wy < 2; ++wy)
                         for (int wx = 0; wx < 2; ++wx)
                             for (int ci = 0; ci < c.cin; ++ci)
-                                L.w[(size_t)n * L.ktot + (wy * 2 + wx) * L.cin + ci] =
-                                    floatToHalfBits(W4(c.w, ci, co, 2 + py - 2 * wy, 2 + px - 2 * wx));
+                                w[(size_t)n * L.ktot + (wy * 2 + wx) * L.cin + ci] =
+                                    W4(c.w, ci, co, 2 + py - 2 * wy, 2 + px - 2 * wx);
                 }
     } else {
         throw Error("pack: unsupported convolution '" + c.name + "' (k=" + std::to_string(c.kh) + " s=" +
                     std::to_string(c.stride) + " p=" + std::to_string(c.pad) + (c.transpose ? " transposed)" : ")"));
+    }
+    if (tf32) {
+        L.wf.resize(w.size());
+        for (size_t i = 0; i < w.size(); ++i) L.wf[i] = roundToTf32(w[i]);
+    } else {
+        L.w.resize(w.size());
+        for (size_t i = 0; i < w.size(); ++i) L.w[i] = floatToHalfBits(w[i]);
     }
     return L;
 }
@@ -595,8 +604,8 @@ PackedModel packSwin(const OnnxGraph& g, int precision) {
         throw Error("pack: unexpected swin_unet patch embedding");
     const int C = c1.conv.cout;
     m.dim = (uint32_t)C;
-    m.layers.push_back(packLayer(c0.conv, 0, 64));   // 3 -> 64 stored channels (zero weights above cout)
-    m.layers.push_back(packLayer(c1.conv, 64, 0));   // 64 stored -> C
+    m.layers.push_back(packLayer(c0.conv, false, 0, 64));   // 3 -> 64 stored channels (zero weights above cout)
+    m.layers.push_back(packLayer(c1.conv, false, 64, 0));   // 64 stored -> C
     auto block = [&](int dim) {
         const Rec& n1 = need(R_LN, "norm1");
         const Rec& qkv = need(R_LIN, "qkv");
@@ -641,7 +650,7 @@ PackedModel packSwin(const OnnxGraph& g, int precision) {
     auto down = [&](int cin, int cout) {
         const Rec& r = need(R_CONV, "patch down conv");
         if (r.conv.kh != 2 || r.conv.stride != 2 || r.conv.cin != cin || r.conv.cout != cout) throw Error("pack: unexpected PatchDown " + r.name);
-        m.layers.push_back(packLayer(r.conv));
+        m.layers.push_back(packLayer(r.conv, false));
     };
     auto upl = [&](int cin, int cout) {
         const Rec& r = need(R_LIN, "patch up linear");
@@ -709,11 +718,19 @@ void composeUpToImage(const PackedLayer& U, const PackedLayer& L, std::vector<ui
             }
 }
 
-PackedModel packFromOnnx(const OnnxGraph& g, int precision) {
+bool isSwinGraph(const OnnxGraph& g) {
     // SwinUNet exports carry LayerNorm (fused, or decomposed into ... Sqrt -> Div -> Mul -> Add below opset 17) and an Erf GELU / Softmax;
     // the cunet family has none of these
     for (const auto& n : g.nodes)
-        if (n.op == "LayerNormalization" || n.op == "Softmax" || n.op == "Erf") return packSwin(g, precision);
+        if (n.op == "LayerNormalization" || n.op == "Softmax" || n.op == "Erf") return true;
+    return false;
+}
+
+PackedModel packFromOnnx(const OnnxGraph& g, int precision) {
+    if (isSwinGraph(g)) {
+        if (precision == W2X_PRECISION_TF32) throw Error("tf32 is not available for swin_unet models");
+        return packSwin(g, precision);
+    }
     std::vector<ConvNode> convs = collectConvs(g);
     PackedModel m;
     m.precision = (uint32_t)precision;
@@ -736,7 +753,7 @@ PackedModel packFromOnnx(const OnnxGraph& g, int precision) {
             ++i;
             continue;
         }
-        m.layers.push_back(packLayer(c));
+        m.layers.push_back(packLayer(c, precision == W2X_PRECISION_TF32));
     }
     // template: UNet1 (8 layers) + UNet2 (14 layers), SURVEY 2.2
     const bool up = m.layers.size() > 7 && m.layers[7].kind == L_UP4;
@@ -806,7 +823,8 @@ PackedModel packFromOnnx(const OnnxGraph& g, int precision) {
 }
 
 // ------------------------------------------------------------------------------------------------
-// Flat file:  "W2XPACK2" | arch scale offset precision dim nlayers | per layer: header + blobs (4-byte aligned)
+// Flat file:  "W2XPACK2" | arch scale offset precision dim nlayers | per layer: header + blobs (4-byte aligned); the GEMM weight blob
+// holds fp16 bits (precision FP16) or fp32 values (precision TF32)
 // ------------------------------------------------------------------------------------------------
 namespace {
 void put32(std::vector<uint8_t>& o, uint32_t v) { for (int i = 0; i < 4; ++i) o.push_back((uint8_t)(v >> (8 * i))); }
@@ -843,7 +861,9 @@ std::vector<uint8_t> serializePack(const PackedModel& m) {
         put32(o, L.kind); put32(o, L.cin); put32(o, L.cout); put32(o, L.npad); put32(o, L.ktot); put32(o, L.taps); put32(o, L.se_r);
         put32(o, L.heads); put32(o, L.window); put32(o, L.upscale);
         uint32_t e; std::memcpy(&e, &L.eps, 4); put32(o, e);
-        putVec(o, L.w); putVec(o, L.bias); putVec(o, L.se_w1); putVec(o, L.se_b1); putVec(o, L.se_w2); putVec(o, L.se_b2);
+        if (m.precision == W2X_PRECISION_TF32) putVec(o, L.wf);
+        else putVec(o, L.w);
+        putVec(o, L.bias); putVec(o, L.se_w1); putVec(o, L.se_b1); putVec(o, L.se_w2); putVec(o, L.se_b2);
         putVec(o, L.gamma); putVec(o, L.beta); putVec(o, L.relpos);
     }
     return o;
@@ -864,9 +884,11 @@ PackedModel deserializePack(const std::vector<uint8_t>& blob) {
         L.kind = in.u32(); L.cin = in.u32(); L.cout = in.u32(); L.npad = in.u32(); L.ktot = in.u32(); L.taps = in.u32(); L.se_r = in.u32();
         L.heads = in.u32(); L.window = in.u32(); L.upscale = in.u32();
         const uint32_t e = in.u32(); std::memcpy(&L.eps, &e, 4);
-        in.vec(L.w); in.vec(L.bias); in.vec(L.se_w1); in.vec(L.se_b1); in.vec(L.se_w2); in.vec(L.se_b2);
+        if (m.precision == W2X_PRECISION_TF32) in.vec(L.wf);
+        else in.vec(L.w);
+        in.vec(L.bias); in.vec(L.se_w1); in.vec(L.se_b1); in.vec(L.se_w2); in.vec(L.se_b2);
         in.vec(L.gamma); in.vec(L.beta); in.vec(L.relpos);
-        if (L.w.size() != (size_t)L.npad * L.ktot || L.bias.size() != L.npad) throw Error("pack file: layer '" + L.name + "' has inconsistent sizes");
+        if (L.weightCount() != (size_t)L.npad * L.ktot || L.bias.size() != L.npad) throw Error("pack file: layer '" + L.name + "' has inconsistent sizes");
     }
     return m;
 }

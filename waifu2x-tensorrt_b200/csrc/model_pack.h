@@ -1,9 +1,10 @@
 // ONNX import + kernel-native weight packing ("build" in the B200 engine).
 // Replaces nvonnxparser::parseFromFile + buildSerializedNetwork (/root/reference/src/tensorrt/img2img_build.cpp:87-147):
-// instead of a TensorRT plan the artefact is a flat file of fp16 GEMM-operand matrices laid out exactly as the
-// tcgen05 implicit-GEMM kernels consume them.
+// instead of a TensorRT plan the artefact is a flat file of fp16 (tf32 packs: fp32) GEMM-operand matrices laid out exactly as
+// the tcgen05 implicit-GEMM kernels consume them.
 #pragma once
 #include <cstdint>
+#include <cstring>
 #include <string>
 #include <vector>
 
@@ -61,13 +62,15 @@ struct PackedLayer {
     uint32_t ktot = 0;   // GEMM K (= taps * cin)
     uint32_t taps = 0;
     uint32_t se_r = 0;   // squeeze/excite hidden width (0 = no SE after this layer)
-    std::vector<uint16_t> w;     // fp16 bits, [npad][ktot] K-major
+    std::vector<uint16_t> w;     // fp16 bits, [npad][ktot] K-major (fp16 packs)
+    std::vector<float> wf;       // the same as fp32 rounded to nearest TF32 (tf32 packs; w is then empty)
     std::vector<float> bias;     // [npad]
     std::vector<float> se_w1, se_b1, se_w2, se_b2;  // [r][c], [r], [c][r], [c]
     // SwinUNet
     uint32_t heads = 0, window = 0, upscale = 0;     // L_ATTN: heads, window; L_TOIMG: pixel-shuffle factor
     float eps = 0.f;                                 // L_LN
     std::vector<float> gamma, beta, relpos;          // L_LN: [c], [c];  L_ATTN: [heads][n][n]
+    size_t weightCount() const { return w.empty() ? wf.size() : w.size(); }
 };
 
 struct PackedModel {
@@ -76,7 +79,8 @@ struct PackedModel {
     std::vector<PackedLayer> layers;
 };
 
-PackedModel packFromOnnx(const OnnxGraph& g, int precision);
+bool isSwinGraph(const OnnxGraph& g);
+PackedModel packFromOnnx(const OnnxGraph& g, int precision);  // precision W2X_PRECISION_TF32: fp32 weights (PackedLayer::wf), cunet only
 // PatchUp (L_UPLIN: rows q0 * cout + c, q0 = dy * 2 + dx) followed by ToImage with pixel shuffle 2 (L_TOIMG: rows q1 * 4 + c3) and nothing in
 // between is one linear map with a pixel shuffle of 4: w [64][K] fp16 bits (row (oy * 4 + ox) * 4 + c3, oy = 2 dy + ey, ox = 2 dx + ex; rows with
 // c3 = 3 are zero), b [64].  Composed in double precision from the packed fp16 weights, rounded to fp16 once.
@@ -86,5 +90,27 @@ PackedModel deserializePack(const std::vector<uint8_t>& blob);
 
 uint16_t floatToHalfBits(float f);
 float halfBitsToFloat(uint16_t h);
+
+#ifdef __CUDACC__
+#define W2X_HOST_DEVICE __host__ __device__
+#else
+#define W2X_HOST_DEVICE
+#endif
+// round to nearest even TF32 (8-bit exponent, 10-bit mantissa: the low 13 bits of the fp32 pattern cleared); inf / nan unchanged
+inline W2X_HOST_DEVICE float roundToTf32(float f) {
+#ifdef __CUDA_ARCH__
+    uint32_t u = __float_as_uint(f);
+#else
+    uint32_t u;
+    std::memcpy(&u, &f, 4);
+#endif
+    if ((u & 0x7f800000u) != 0x7f800000u) u = (u + 0xfffu + ((u >> 13) & 1u)) & 0xffffe000u;
+#ifdef __CUDA_ARCH__
+    return __uint_as_float(u);
+#else
+    std::memcpy(&f, &u, 4);
+    return f;
+#endif
+}
 
 }  // namespace w2x

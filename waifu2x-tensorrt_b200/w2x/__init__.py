@@ -135,6 +135,7 @@ _SIGNATURES = {
     "w2x_infer": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_void_p]),
     "w2x_selftest_conv": (C.c_double, [C.c_int] * 7 + [C.c_uint]),
     "w2x_run_conv_layer": (C.c_int, [C.c_int] * 8 + [C.c_void_p, C.c_void_p, C.POINTER(C.c_float), C.c_void_p, C.c_void_p]),
+    "w2x_run_conv_layer_f32": (C.c_int, [C.c_int] * 7 + [C.c_void_p, C.c_void_p, C.POINTER(C.c_float), C.c_void_p, C.c_void_p]),
     "w2x_swin_attn_prepare": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p]),
     "w2x_compose_up_to_image": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p]),
     "w2x_run_swin_attn": (C.c_int, [C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_float, C.c_void_p,
@@ -300,6 +301,25 @@ def run_conv_layer(kind: int, x: np.ndarray, w_packed: np.ndarray, bias: np.ndar
                                   _ptr(sk) if sk is not None else None, _ptr(out))
     if not ok:
         raise RuntimeError("w2x_run_conv_layer failed")
+    return out
+
+
+def run_conv_layer_f32(kind: int, x: np.ndarray, w_packed: np.ndarray, bias: np.ndarray, cout: int, skip: Optional[np.ndarray] = None,
+                       device: int = 0) -> np.ndarray:
+    """run_conv_layer through the tf32 kernel of --precision tf32 engines (include/w2x_dev.h: w2x_run_conv_layer_f32): x, skip and the
+    result are float32 NHWC, w_packed float32 [npad][ktot] (the tensor core uses its TF32 part)."""
+    x = np.ascontiguousarray(x, np.float32)
+    n, h, w, cin = x.shape
+    shape = {0: (n, h - 2, w - 2, cout), 1: (n, h // 2, w // 2, cout), 2: (n, 2 * h, 2 * w, cout), 3: (n, 2 * h - 4, 2 * w - 4, 4),
+             4: (n, h - 2, w - 2, 4)}[kind]
+    out = np.zeros(shape, np.float32)
+    wp = np.ascontiguousarray(w_packed, np.float32)
+    b = np.ascontiguousarray(bias, np.float32)
+    sk = np.ascontiguousarray(skip, np.float32) if skip is not None else None
+    ok = lib().w2x_run_conv_layer_f32(device, kind, n, h, w, cin, cout, _ptr(x), _ptr(wp), b.ctypes.data_as(C.POINTER(C.c_float)),
+                                      _ptr(sk) if sk is not None else None, _ptr(out))
+    if not ok:
+        raise RuntimeError("w2x_run_conv_layer_f32 failed")
     return out
 
 
