@@ -91,6 +91,19 @@ W2X_API int w2x_render(w2x_engine* e, const uint8_t* src_bgr, int width, int hei
 
 /* ---- extensions (not in the reference) ------------------------------------------------------------- */
 
+/* Images with an alpha channel: src BGRA u8 HWC (w x h, row pitch src_stride >= 4 * width) -> dst BGRA (w*scaling x h*scaling, pitch
+ * dst_stride >= 4 * width * scaling), synchronous, with any loaded engine (fp16 or tf32, with or without TTA).
+ *  - Every alpha byte 255: B, G, R are byte-identical to w2x_render of the B, G, R planes, alpha is 255, and the model runs once.
+ *  - Some alpha byte 0: before the model, the colour of the transparent pixels (alpha == 0) is replaced by a bleed of the visible
+ *    colour: `offset / scale` rounds (the model's input border, w2x_pack_info), each of which gives every transparent pixel with a
+ *    known 8-neighbour the rounded-half-up integer mean of its known neighbours; pixels still unknown become (0, 0, 0).  So the
+ *    colour under alpha == 0 never reaches the output.  B, G, R out are w2x_render of the bled frame.
+ *  - Some alpha byte < 255: the alpha plane goes through the same model, tiles, TTA and blending as a grey image (B = G = R = alpha),
+ *    in the same batches as the colour tiles; output alpha = saturate(rint(255 * (r + g + b) / 3)) of its blended canvas.
+ * Returns 0 and logs the reason on failure (no engine loaded, null pointers, strides below 4 bytes per pixel). */
+W2X_API int w2x_render_bgra(w2x_engine* e, const uint8_t* src_bgra, int width, int height, size_t src_stride,
+                            uint8_t* dst_bgra, size_t dst_stride);
+
 /* Same as w2x_render but src/dst are DEVICE pointers on cfg.deviceId; enqueued on the engine's stream,
  * returns without synchronising (w2x_sync to wait).  Used for the HBM-resident `value` measurement. */
 W2X_API int w2x_render_device(w2x_engine* e, const uint8_t* d_src_bgr, int width, int height, size_t src_stride,

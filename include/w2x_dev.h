@@ -15,6 +15,10 @@
 extern "C" {
 #endif
 
+/* The colour bleed of w2x_render_bgra on host buffers: src BGRA (w x h, pitch src_stride >= 4 * width), `rounds` rounds ->
+ * dst BGRA packed (pitch 4 * width), alpha bytes copied from src.  Returns 1 on success. */
+W2X_API int w2x_alpha_bleed(int device, const uint8_t* src_bgra, int width, int height, size_t src_stride, int rounds, uint8_t* dst_bgra);
+
 /* One layer of the dense model path (SURVEY 8a row a17; replaces a slice of the engine enqueued at img2img_infer.cpp:80) on
  * caller-supplied host data, through the kernel the execution planner picks for that shape (head != 0: kinds 3 / 4 through the
  * dedicated head kernels).  Weights are the packed GEMM operand B[npad][ktot] (fp16 bits, K-major) and bias[npad] that `build`

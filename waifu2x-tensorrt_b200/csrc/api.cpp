@@ -2,6 +2,7 @@
 #include <cuda_fp16.h>
 #include <cuda_runtime.h>
 
+#include <algorithm>
 #include <cstring>
 #include <filesystem>
 
@@ -70,6 +71,11 @@ int w2x_load(w2x_engine* e, const char* onnx_path, const w2x_render_config* cfg)
 int w2x_render(w2x_engine* e, const uint8_t* src, int width, int height, size_t src_stride, uint8_t* dst, size_t dst_stride) {
     if (!e || !src || !dst) return 0;
     return e->impl.render(src, width, height, src_stride, dst, dst_stride) ? 1 : 0;
+}
+
+int w2x_render_bgra(w2x_engine* e, const uint8_t* src, int width, int height, size_t src_stride, uint8_t* dst, size_t dst_stride) {
+    if (!e) return 0;
+    return e->impl.renderBgra(src, width, height, src_stride, dst, dst_stride) ? 1 : 0;
 }
 
 int w2x_render_device(w2x_engine* e, const uint8_t* src, int width, int height, size_t src_stride, uint8_t* dst, size_t dst_stride) {
@@ -234,6 +240,29 @@ int w2x_stitch_tiles(int device, const uint16_t* tiles, int count, int out_tile,
         return 1;
     } catch (const std::exception& ex) {
         std::fprintf(stderr, "w2x_stitch_tiles: %s\n", ex.what());
+        return 0;
+    }
+}
+
+int w2x_alpha_bleed(int device, const uint8_t* src, int width, int height, size_t src_stride, int rounds, uint8_t* dst) {
+    try {
+        if (!src || !dst || width <= 0 || height <= 0 || src_stride < (size_t)width * 4 || rounds < 0) throw Error("invalid argument");
+        W2X_CUDA(cudaSetDevice(device));
+        DevBufs b;
+        const size_t row = (size_t)width * 4, bytes = row * height;
+        uint8_t* dSrc = b.alloc<uint8_t>(bytes);
+        uint8_t* dBuf[2] = {b.alloc<uint8_t>(bytes), b.alloc<uint8_t>(bytes)};
+        W2X_CUDA(cudaMemcpy2D(dSrc, row, src, src_stride, row, height, cudaMemcpyHostToDevice));
+        const uint8_t* in = dSrc;
+        for (int r = 0; r < std::max(rounds, 1); ++r) {   // the engine's sequence (Engine::renderOnStream)
+            launchAlphaBleedRound(in, dBuf[r & 1], width, height, rounds > 0 ? 1 : 0, r + 1 >= rounds ? dSrc : nullptr, nullptr);
+            in = dBuf[r & 1];
+        }
+        W2X_CUDA(cudaGetLastError());
+        W2X_CUDA(cudaMemcpy(dst, in, bytes, cudaMemcpyDeviceToHost));
+        return 1;
+    } catch (const std::exception& ex) {
+        std::fprintf(stderr, "w2x_alpha_bleed: %s\n", ex.what());
         return 0;
     }
 }

@@ -149,6 +149,8 @@ void Engine::unload() {
     if (dTileOut) { cudaFree(dTileOut); dTileOut = nullptr; } freep(dTtaMean); freep(dRampX); freep(dRampY); freep(dFrameIn); freep(dFrameOut);
     if (dUnpacked) { cudaFree(dUnpacked); dUnpacked = nullptr; }
     unpackedCap = 0;
+    freep(dAlphaFlags); freep(dBleed[0]); freep(dBleed[1]);
+    bleedCap = 0;
     if (dBandTiles) { cudaFree(dBandTiles); dBandTiles = nullptr; }
     freep(dBandMap); freep(dBandSlots); freep(dBandMean);
     bandTilesCap = bandMapCap = bandSlotCap = bandMeanCap = 0;
@@ -170,6 +172,7 @@ void Engine::unload() {
     if (h2dStream) { cudaStreamDestroy(h2dStream); h2dStream = nullptr; }
     if (d2hStream) { cudaStreamDestroy(d2hStream); d2hStream = nullptr; }
     frameW = frameH = 0;
+    framePasses = 1;
     isLoaded = false;
 }
 
@@ -872,14 +875,16 @@ void Engine::runModel(cudaStream_t s, void* finalOut, int nImages, const void* i
 // ------------------------------------------------------------------------------------------------
 // render (img2img_render.cpp:224-348)
 // ------------------------------------------------------------------------------------------------
-void Engine::ensureFrameBuffers(int w, int h) {
-    if (w == frameW && h == frameH) return;
+void Engine::ensureFrameBuffers(int w, int h, int passes) {
+    if (w == frameW && h == frameH && passes == framePasses) return;
     if (w <= 0 || h <= 0) throw Error("invalid frame size");
     W2X_CUDA(cudaStreamSynchronize(stream));
     grid = calculateTiles(w, h, w * scale, h * scale, tile, tile, outTile, outTile, scale, cfg.overlapX, cfg.overlapY);
     if (grid.count <= 0) throw Error("frame is too small for the configured tile overlap");
     const int stepsPerTile = cfg.tta ? 8 : 1;
-    batchCount = (int)std::lround(std::ceil((double)(grid.count * stepsPerTile) / batch));  // render.cpp:249
+    // a BGRA frame with an alpha pass: the alpha steps follow the colour steps in the same order (alpha slot = colour slot +
+    // count * stepsPerTile), and the batches are padded once per frame
+    batchCount = (int)std::lround(std::ceil((double)(grid.count * stepsPerTile * passes) / batch));  // render.cpp:249
     stepCount = batchCount * batch;
     // Tile order.  The reference walks its column-major tile list (render.cpp:264-265).  A tile's result does not depend on its batch
     // or slot (exact integer SE sums), so without TTA the tiles are processed ROW by row instead: the output rows above the next tile row
@@ -891,10 +896,10 @@ void Engine::ensureFrameBuffers(int w, int h) {
     if (!cfg.tta) {
         tileMapHost.assign((size_t)grid.count, 0);
         for (int step = 0; step < stepCount; ++step) {
-            if (step < grid.count) {
-                const int j = step / grid.nx, i = step - j * grid.nx, ti = i * grid.ny + j;
-                slots[step] = {grid.inRects[ti].x, grid.inRects[ti].y, 0, 1};
-                tileMapHost[ti] = step;
+            if (step < grid.count * passes) {
+                const int q = step % grid.count, j = q / grid.nx, i = q - j * grid.nx, ti = i * grid.ny + j;
+                slots[step] = {grid.inRects[ti].x, grid.inRects[ti].y, 0, step < grid.count ? 1 : kSlotAlpha};
+                if (step < grid.count) tileMapHost[ti] = step;
             } else {
                 slots[step] = {0, 0, 0, 0};  // zero dummy tile, render.cpp:281
             }
@@ -909,7 +914,7 @@ void Engine::ensureFrameBuffers(int w, int h) {
     } else {
         for (int step = 0; step < stepCount; ++step) {
             const int ti = step / stepsPerTile, aug = step % stepsPerTile;  // render.cpp:264-265
-            if (ti < grid.count) slots[step] = {grid.inRects[ti].x, grid.inRects[ti].y, aug, 1};
+            if (ti < grid.count * passes) slots[step] = {grid.inRects[ti % grid.count].x, grid.inRects[ti % grid.count].y, aug, ti < grid.count ? 1 : kSlotAlpha};
             else slots[step] = {0, 0, 0, 0};  // zero dummy tile, render.cpp:281
         }
     }
@@ -945,10 +950,10 @@ void Engine::ensureFrameBuffers(int w, int h) {
         W2X_CUDA(cudaMalloc(&dTileOut, (size_t)stepCount * tileElems * elemBytes));
         tileOutCap = (size_t)stepCount * tileElems;
     }
-    if (cfg.tta && (size_t)grid.count * tileElems > ttaCap) {
+    if (cfg.tta && (size_t)grid.count * passes * tileElems > ttaCap) {
         if (dTtaMean) cudaFree(dTtaMean);
-        W2X_CUDA(cudaMalloc(&dTtaMean, (size_t)grid.count * tileElems * sizeof(float)));
-        ttaCap = (size_t)grid.count * tileElems;
+        W2X_CUDA(cudaMalloc(&dTtaMean, (size_t)grid.count * passes * tileElems * sizeof(float)));
+        ttaCap = (size_t)grid.count * passes * tileElems;
     }
     if (rampXLen != grid.outOvX) {
         if (dRampX) { cudaFree(dRampX); dRampX = nullptr; }
@@ -968,26 +973,11 @@ void Engine::ensureFrameBuffers(int w, int h) {
     W2X_CUDA(cudaStreamSynchronize(stream));
     frameW = w;
     frameH = h;
+    framePasses = passes;
 }
 
 void Engine::renderOnStream(const uint8_t* dSrc, int w, int h, size_t srcPitch, uint8_t* dDst, size_t dstPitch, cudaStream_t s, bool timed,
-                            std::vector<BandDone>* bands) {
-    ensureFrameBuffers(w, h);
-    const bool progressive = bands != nullptr && !cfg.tta && !rowBands.empty();
-    if (bands) bands->clear();
-    auto stitchRows = [&](int yBegin, int yEnd) {
-        StitchParams sp{};
-        sp.outT = outTile; sp.nx = grid.nx; sp.ny = grid.ny; sp.ovx = grid.outOvX; sp.ovy = grid.outOvY;
-        sp.cw = w * scale; sp.ch = h * scale;
-        sp.rampx = dRampX; sp.rampy = dRampY;
-        sp.dst = dDst; sp.pitch = dstPitch;
-        sp.tiles = cfg.tta ? (const void*)dTtaMean : (const void*)dTileOut;
-        sp.f32 = (cfg.tta || tf32()) ? 1 : 0;
-        sp.tile_map = cfg.tta ? nullptr : dTileMap;
-        sp.y_begin = yBegin; sp.y_end = yEnd;
-        launchStitch(sp, s);
-        ++launches;
-    };
+                            std::vector<BandDone>* bands, int pixelBytes) {
     if (timed) { evUsed = 0; spans.clear(); }
     auto span = [&](int kind, auto&& fn) {
         if (!timed) { fn(); return; }
@@ -999,15 +989,72 @@ void Engine::renderOnStream(const uint8_t* dSrc, int w, int h, size_t srcPitch, 
         W2X_CUDA(cudaEventRecord(e1, s));
         spans.push_back({kind, i0, evUsed - 1});
     };
+    int passes = 1;
+    if (pixelBytes == 4) {
+        // The alpha plane decides the schedule: no alpha < 255, no alpha pass; some alpha == 0, the colour bleed first.  Both count as
+        // unpack time.
+        if (!dAlphaFlags) W2X_CUDA(cudaMalloc(&dAlphaFlags, 2 * sizeof(int)));
+        int flags[2] = {0, 0};
+        span(0, [&] {
+            W2X_CUDA(cudaMemsetAsync(dAlphaFlags, 0, 2 * sizeof(int), s));
+            launchAlphaScan(dSrc, (size_t)w * h, dAlphaFlags, s);
+            ++launches;
+        });
+        W2X_CUDA(cudaMemcpyAsync(flags, dAlphaFlags, sizeof flags, cudaMemcpyDeviceToHost, s));
+        W2X_CUDA(cudaStreamSynchronize(s));
+        passes = flags[0] ? 2 : 1;
+        if (flags[1]) {
+            const size_t bytes = (size_t)w * h * 4;
+            if (bytes > bleedCap) {
+                for (auto*& b : dBleed) {
+                    if (b) cudaFree(b);
+                    b = nullptr;
+                }
+                bleedCap = 0;
+                for (auto*& b : dBleed) W2X_CUDA(cudaMalloc(&b, bytes));
+                bleedCap = bytes;
+            }
+            // rounds = the model's input-side border (the halo of every tile): colour from farther away cannot reach an output pixel
+            const int rounds = (int)(model.offset / std::max<uint32_t>(model.scale, 1));
+            span(0, [&] {
+                const uint8_t* in = dSrc;
+                for (int r = 0; r < std::max(rounds, 1); ++r) {
+                    uint8_t* out = dBleed[r & 1];
+                    launchAlphaBleedRound(in, out, w, h, rounds > 0 ? 1 : 0, r + 1 >= rounds ? dSrc : nullptr, s);
+                    ++launches;
+                    in = out;
+                }
+                dSrc = in;
+            });
+        }
+    }
+    ensureFrameBuffers(w, h, passes);
+    const bool progressive = pixelBytes == 3 && bands != nullptr && !cfg.tta && !rowBands.empty();
+    if (bands) bands->clear();
+    auto stitchRows = [&](int yBegin, int yEnd) {
+        StitchParams sp{};
+        sp.outT = outTile; sp.nx = grid.nx; sp.ny = grid.ny; sp.ovx = grid.outOvX; sp.ovy = grid.outOvY;
+        sp.cw = w * scale; sp.ch = h * scale;
+        sp.rampx = dRampX; sp.rampy = dRampY;
+        sp.dst = dDst; sp.pitch = dstPitch;
+        sp.tiles = cfg.tta ? (const void*)dTtaMean : (const void*)dTileOut;
+        sp.f32 = (cfg.tta || tf32()) ? 1 : 0;
+        sp.tile_map = cfg.tta ? nullptr : dTileMap;
+        sp.y_begin = yBegin; sp.y_end = yEnd;
+        sp.bgra = pixelBytes == 4 ? 1 : 0;
+        sp.alpha_off = passes == 2 ? grid.count : 0;   // TTA: index of the reduced alpha tile; else the alpha step of the tile's slot
+        launchStitch(sp, s);
+        ++launches;
+    };
     const size_t tileElems = (size_t)outTile * outTile * 4;
     const size_t inElems = (size_t)tile * tile * 4;
     // real (non-padding) slots: the reference computes the zero padding tiles of the last batch and discards them (:281,:298)
-    const int realSteps = grid.count * (cfg.tta ? 8 : 1);
+    const int realSteps = grid.count * (cfg.tta ? 8 : 1) * passes;
     // all tiles of the frame are unpacked by ONE launch into a frame-wide buffer; the batches then chain kernel -> kernel
     const bool frameWide = frameWideUnpack();
     if (frameWide)
         span(0, [&] {
-            unpackTiles(dSrc, w, h, srcPitch, dSlots, realSteps, dUnpacked, s);
+            unpackTiles(dSrc, w, h, srcPitch, dSlots, realSteps, dUnpacked, s, pixelBytes);
             ++launches;
         });
     for (int b = 0; b < batchCount; ++b) {
@@ -1016,7 +1063,7 @@ void Engine::renderOnStream(const uint8_t* dSrc, int w, int h, size_t srcPitch, 
         if (nReal <= 0) continue;
         if (!frameWide)
             span(0, [&] {
-                unpackTiles(dSrc, w, h, srcPitch, dSlots + (size_t)b * batch, nReal, actIn.p, s);
+                unpackTiles(dSrc, w, h, srcPitch, dSlots + (size_t)b * batch, nReal, actIn.p, s, pixelBytes);
                 ++launches;
             });
         span(1, [&] { runModel(s, elemAt(dTileOut, (size_t)b * batch * tileElems), nReal, frameWide ? elemAt(dUnpacked, (size_t)b * batch * inElems) : nullptr); });
@@ -1046,16 +1093,16 @@ void Engine::renderOnStream(const uint8_t* dSrc, int w, int h, size_t srcPitch, 
     }
     if (cfg.tta)
         span(4, [&] {
-            ttaReduce(dTileOut, grid.count, dTtaMean, s);
+            ttaReduce(dTileOut, grid.count * passes, dTtaMean, s);
             ++launches;
         });
     span(2, [&] { stitchRows(0, h * scale); });
     W2X_CUDA(cudaGetLastError());
 }
 
-void Engine::unpackTiles(const uint8_t* src, int w, int h, size_t pitch, const TileSlot* slots, int n, void* out, cudaStream_t s) {
-    if (tf32()) launchUnpack(src, w, h, pitch, slots, n, tile, static_cast<float*>(out), s);
-    else launchUnpack(src, w, h, pitch, slots, n, tile, static_cast<__half*>(out), s);
+void Engine::unpackTiles(const uint8_t* src, int w, int h, size_t pitch, const TileSlot* slots, int n, void* out, cudaStream_t s, int pixelBytes) {
+    if (tf32()) launchUnpack(src, w, h, pitch, slots, n, tile, static_cast<float*>(out), s, pixelBytes);
+    else launchUnpack(src, w, h, pitch, slots, n, tile, static_cast<__half*>(out), s, pixelBytes);
 }
 
 void Engine::ttaReduce(const void* outs, int tiles, float* mean, cudaStream_t s) {
@@ -1141,6 +1188,40 @@ bool Engine::render(const uint8_t* src, int w, int h, size_t srcStride, uint8_t*
             W2X_CUDA(cudaStreamSynchronize(d2hStream));
         }
         W2X_CUDA(cudaStreamSynchronize(stream));  // the sync the reference leaves commented out (render.cpp:345)
+        return true;
+    } catch (const std::exception& ex) {
+        ELOG(W2X_ERROR, std::string("Render failed unexpectedly: ") + ex.what() + ".");
+        return false;
+    }
+}
+
+bool Engine::renderBgra(const uint8_t* src, int w, int h, size_t srcStride, uint8_t* dst, size_t dstStride) {
+    try {
+        if (!isLoaded) throw Error("no engine loaded");
+        if (!src || !dst) throw Error("null image pointer");
+        if (w <= 0 || h <= 0) throw Error("invalid frame size");
+        if (srcStride < (size_t)w * 4 || dstStride < (size_t)w * scale * 4) throw Error("row stride is smaller than 4 bytes per pixel");
+        W2X_CUDA(cudaSetDevice(cfg.deviceId));
+        const size_t ipitch = (size_t)w * 4, opitch = (size_t)w * scale * 4;
+        const size_t inBytes = ipitch * h, outBytes = opitch * h * scale;
+        if (inBytes > frameInCap) {
+            if (dFrameIn) cudaFree(dFrameIn);
+            dFrameIn = nullptr;
+            frameInCap = 0;
+            W2X_CUDA(cudaMalloc(&dFrameIn, inBytes));
+            frameInCap = inBytes;
+        }
+        if (outBytes > frameOutCap) {
+            if (dFrameOut) cudaFree(dFrameOut);
+            dFrameOut = nullptr;
+            frameOutCap = 0;
+            W2X_CUDA(cudaMalloc(&dFrameOut, outBytes));
+            frameOutCap = outBytes;
+        }
+        W2X_CUDA(cudaMemcpy2DAsync(dFrameIn, ipitch, src, srcStride, ipitch, h, cudaMemcpyHostToDevice, stream));
+        renderOnStream(dFrameIn, w, h, ipitch, dFrameOut, opitch, stream, true, nullptr, 4);
+        W2X_CUDA(cudaMemcpy2DAsync(dst, dstStride, dFrameOut, opitch, opitch, (size_t)h * scale, cudaMemcpyDeviceToHost, stream));
+        W2X_CUDA(cudaStreamSynchronize(stream));
         return true;
     } catch (const std::exception& ex) {
         ELOG(W2X_ERROR, std::string("Render failed unexpectedly: ") + ex.what() + ".");

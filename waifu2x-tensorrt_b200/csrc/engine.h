@@ -83,6 +83,9 @@ public:
     bool load(const std::string& onnxPath, const w2x_render_config& cfg);
     bool render(const uint8_t* src, int w, int h, size_t srcStride, uint8_t* dst, size_t dstStride);
     bool renderDevice(const uint8_t* dSrc, int w, int h, size_t srcStride, uint8_t* dDst, size_t dstStride);
+    // BGRA host buffers (w x h, pitch >= 4w) -> BGRA (w*scale x h*scale, pitch >= 4*w*scale), synchronous like render: the B, G, R of
+    // the colour-bled frame through the render pipeline, the alpha plane as a second model pass in the same batches (none when opaque)
+    bool renderBgra(const uint8_t* src, int w, int h, size_t srcStride, uint8_t* dst, size_t dstStride);
     int submit(const uint8_t* src, int w, int h, size_t srcStride, uint8_t* dst, size_t dstStride);
     bool wait(int ticket);
     // one image sharded over several engines (one per GPU) by bands of tile rows, seam rows exchanged peer-to-peer
@@ -118,15 +121,17 @@ private:
     bool tf32() const { return elemBytes == 4; }
     // element `i` of an activation / tile buffer of this engine's element type
     void* elemAt(void* base, size_t i) const { return static_cast<uint8_t*>(base) + i * elemBytes; }
-    void unpackTiles(const uint8_t* src, int w, int h, size_t pitch, const TileSlot* slots, int n, void* out, cudaStream_t s);
+    void unpackTiles(const uint8_t* src, int w, int h, size_t pitch, const TileSlot* slots, int n, void* out, cudaStream_t s, int pixelBytes = 3);
     void ttaReduce(const void* outs, int tiles, float* mean, cudaStream_t s);
     bool frameWideUnpack() const;
-    void ensureFrameBuffers(int w, int h);
+    // passes: 1 = the colour tiles, 2 = the colour tiles followed by the alpha tiles of a BGRA frame (renderBgra)
+    void ensureFrameBuffers(int w, int h, int passes = 1);
     struct RowBand { int y0, y1, batch; };             // output rows [y0, y1) are final once batch `batch` has run (row-major tile order)
     struct BandDone { int y0, y1; cudaEvent_t ev; };   // ... and have been stitched when `ev` fires
     // bands != nullptr (and no TTA): stitch progressively, one launch per finished tile row, and report the bands instead of one stitch at the end
+    // pixelBytes 4: packed BGRA frames (dSrcPitch = 4w): alpha scan, colour bleed and alpha pass as the frame needs them; no bands
     void renderOnStream(const uint8_t* dSrc, int w, int h, size_t srcPitch, uint8_t* dDst, size_t dstPitch, cudaStream_t s, bool timed,
-                        std::vector<BandDone>* bands = nullptr);
+                        std::vector<BandDone>* bands = nullptr, int pixelBytes = 3);
     void* dalloc(size_t bytes);
     Act allocAct(int h, int w, int c);
 
@@ -154,7 +159,7 @@ private:
     long long launches = 0;
 
     // frame-level state
-    int frameW = 0, frameH = 0;
+    int frameW = 0, frameH = 0, framePasses = 1;
     TileGrid grid;
     int stepCount = 0, batchCount = 0;
     TileSlot* dSlots = nullptr;
@@ -174,6 +179,10 @@ private:
     // host-buffer paths
     uint8_t *dFrameIn = nullptr, *dFrameOut = nullptr;
     size_t frameInCap = 0, frameOutCap = 0;
+    // BGRA frames: alpha-scan flags (2 ints) and the two ping-pong buffers of the colour bleed
+    int* dAlphaFlags = nullptr;
+    uint8_t* dBleed[2] = {nullptr, nullptr};
+    size_t bleedCap = 0;
     // pipelined submit
     static constexpr int kSlots = 3;
     struct PipeSlot {

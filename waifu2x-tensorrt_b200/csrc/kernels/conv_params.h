@@ -255,11 +255,15 @@ void launchSeScale(__half* x, int n, int h, int w, int c, const float* scale, cu
 void launchScaleWeights(const __half* w, __half* wOut, const float* scale, int nimg, int npad, int ktot, int cin, cudaStream_t s);
 
 // tiling (kernels/tiling.cu)
-struct TileSlot { int x, y, aug, valid; };  // input rect origin, D4 op, 0 = zero dummy slot (img2img_render.cpp:281)
+// input rect origin, D4 op, valid: 0 = zero dummy slot (img2img_render.cpp:281), 1 = the frame's B, G, R bytes, kSlotAlpha = the
+// alpha byte of a BGRA frame as R = G = B (the alpha pass of Engine::renderBgra)
+struct TileSlot { int x, y, aug, valid; };
+constexpr int kSlotAlpha = 2;
+// pixelBytes: 3 = BGR frame, 4 = BGRA frame
 void launchUnpack(const uint8_t* frame, int w, int h, size_t pitch, const TileSlot* slots, int nslots, int tile,
-                  __half* out, cudaStream_t s);
+                  __half* out, cudaStream_t s, int pixelBytes = 3);
 void launchUnpack(const uint8_t* frame, int w, int h, size_t pitch, const TileSlot* slots, int nslots, int tile,
-                  float* out, cudaStream_t s);  // tf32 engines: the reference's convertTo(CV_32F, 1/255) blob exactly
+                  float* out, cudaStream_t s, int pixelBytes = 3);  // tf32 engines: the reference's convertTo(CV_32F, 1/255) blob exactly
 struct StitchParams {
     const void* tiles;   // [count][outT][outT][4] fp16 or f32
     int f32;             // element type of tiles
@@ -272,8 +276,17 @@ struct StitchParams {
     // (i, j) lives at slot tile_map[i * ny + j] of `tiles` (nullptr = identity, the reference's column-major order)
     int y_begin, y_end;
     const int* tile_map;
+    // BGRA canvas (4-byte pixels); alpha_off > 0: the alpha pass's tile of reference tile t is at slot(t) + alpha_off, else alpha = 255
+    int bgra, alpha_off;
 };
 void launchStitch(const StitchParams& p, cudaStream_t s);
+// BGRA frames (kernels/alpha.cu), packed w x h x 4 bytes on the device.
+// flags[0] = 1 if some alpha < 255, flags[1] = 1 if some alpha == 0; flags must be zeroed
+void launchAlphaScan(const uint8_t* bgra, size_t pixels, int* flags, cudaStream_t s);
+// One Jacobi round of the colour bleed: a pixel is known when its alpha byte is > 0; a known pixel keeps B, G, R, an unknown one with
+// n > 0 known 8-neighbours takes their per-channel mean (2 sum + n) / 2n (grow != 0) and becomes known, any other is (0, 0, 0).  The
+// output alpha byte is 255 / 0 for known / unknown, or, when alphaOf != nullptr (last round), alphaOf's alpha byte.
+void launchAlphaBleedRound(const uint8_t* in, uint8_t* out, int w, int h, int grow, const uint8_t* alphaOf, cudaStream_t s);
 void launchTtaReduce(const __half* outs, int tiles, int outT, float* mean, cudaStream_t s);
 void launchTtaReduce(const float* outs, int tiles, int outT, float* mean, cudaStream_t s);
 // NCHW f32 <-> NHWC4 fp16 / f32 (Img2Img::infer host entry, tests)

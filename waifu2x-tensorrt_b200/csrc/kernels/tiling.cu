@@ -74,17 +74,21 @@ template <> struct Px4<float> {
 // ---- unpack ---------------------------------------------------------------------------------------
 // grid: (tile/32 x tile/32 blocks of 32 x 32 output pixels, nslots), 256 threads.  Under every D4 augmentation the source of a
 // 32 x 32 output block is a 32 x 32 block of the (replicate-padded) frame, so the block first stages those 32 source rows (96
-// bytes each) in shared memory with coalesced loads -- 32-bit words from the 4-byte-aligned start of each row segment when the
-// segment lies inside the frame, clamped byte loads on border blocks -- and then every thread converts four pixels, reading the
-// staged bytes at the mirrored / transposed position, and writes them with 8-byte stores (256 contiguous bytes per warp).
+// bytes each, 128 for BGRA) in shared memory with coalesced loads -- 32-bit words from the 4-byte-aligned start of each row segment
+// when the segment lies inside the frame, clamped byte loads on border blocks -- and then every thread converts four pixels, reading
+// the staged bytes at the mirrored / transposed position, and writes them with 8-byte stores (256 contiguous bytes per warp).
+// PS = source bytes per pixel: 3 (BGR) or 4 (BGRA; a slot with valid == kSlotAlpha reads the alpha byte into R, G and B).
 constexpr int kUB = 32;             // block edge
-constexpr int kURow = 104;          // staged bytes per source row: 96 + up to 3 alignment bytes, rounded up to a word multiple
+// staged bytes per source row: BGR 96 + up to 3 alignment bytes, rounded up to a word multiple; BGRA rows are word-aligned (128 bytes),
+// padded by one word so that the column reads of the transposed augmentations do not all hit one bank
+template <int PS> constexpr int kURow = PS == 3 ? 104 : 132;
 
-template <typename T>
+template <typename T, int PS>
 __global__ void __launch_bounds__(256) unpack_kernel(const uint8_t* __restrict__ frame, int w, int h, size_t pitch,
                                                      const TileSlot* __restrict__ slots, int tile, int wordOk,
                                                      T* __restrict__ out) {
-    __shared__ __align__(16) uint8_t sm[kUB * kURow];
+    constexpr int kRow = kURow<PS>;
+    __shared__ __align__(16) uint8_t sm[kUB * kRow];
     __shared__ int smOff[kUB];      // byte offset of local source column 0 inside each staged row (fast path: alignment slack)
     const int blocksPerSide = (tile + kUB - 1) / kUB;
     const int slot = blockIdx.y;
@@ -114,20 +118,21 @@ __global__ void __launch_bounds__(256) unpack_kernel(const uint8_t* __restrict__
     for (int lr = ty; lr < rows; lr += 8) {
         const int sy = min(max(ts.y + rrMin + lr, 0), h - 1);
         const uint8_t* rowp = frame + (size_t)sy * pitch;
-        const size_t segStart = (size_t)sy * pitch + (size_t)x0 * 3;   // byte offset of the segment from `frame`
-        // fast path: whole 32-pixel segment inside the row and at least 4 bytes of the row (or the next row) behind it
-        if (inside && wordOk && (size_t)(x0 + kUB) * 3 + 4 <= pitch) {
+        const size_t segStart = (size_t)sy * pitch + (size_t)x0 * PS;  // byte offset of the segment from `frame`
+        // fast path: whole 32-pixel segment inside the row and (BGR) at least 4 bytes of the row (or the next row) behind it; a BGRA
+        // segment is word-aligned (wordOk includes pitch % 4 == 0) and read exactly
+        if (inside && wordOk && (PS == 4 || (size_t)(x0 + kUB) * 3 + 4 <= pitch)) {
             const size_t a = segStart & ~(size_t)3;
-            if (tx < kURow / 4) {
+            if (tx < (PS == 3 ? kRow / 4 : kUB)) {
                 const uint32_t v = *reinterpret_cast<const uint32_t*>(frame + a + 4 * tx);
-                *reinterpret_cast<uint32_t*>(sm + lr * kURow + 4 * tx) = v;
+                *reinterpret_cast<uint32_t*>(sm + lr * kRow + 4 * tx) = v;
             }
             if (tx == 0) smOff[lr] = (int)(segStart - a);
         } else {
-            for (int b = tx; b < cols * 3; b += 32) {
-                const int cc = b / 3, ch = b - cc * 3;
+            for (int b = tx; b < cols * PS; b += 32) {
+                const int cc = b / PS, ch = b - cc * PS;
                 const int sx = min(max(x0 + cc, 0), w - 1);   // BORDER_REPLICATE (padRoi, render.cpp:79-100)
-                sm[lr * kURow + b] = rowp[(size_t)sx * 3 + ch];
+                sm[lr * kRow + b] = rowp[(size_t)sx * PS + ch];
             }
             if (tx == 0) smOff[lr] = 0;
         }
@@ -141,25 +146,34 @@ __global__ void __launch_bounds__(256) unpack_kernel(const uint8_t* __restrict__
         int rr, cc;
         augSrcIndex(ts.aug, r, c, tile, rr, cc);
         const int lr = rr - rrMin;
-        const uint8_t* px = sm + lr * kURow + smOff[lr] + (cc - ccMin) * 3;
+        const uint8_t* px = sm + lr * kRow + smOff[lr] + (cc - ccMin) * PS;
+        if (PS == 4 && ts.valid == kSlotAlpha) {
+            const float a = __fmul_rn((float)px[3], k);
+            storePx(outp, (size_t)r * tile + c, a, a, a);
+            continue;
+        }
         const float b = __fmul_rn((float)px[0], k), g = __fmul_rn((float)px[1], k), rch = __fmul_rn((float)px[2], k);
         storePx(outp, (size_t)r * tile + c, rch, g, b);
     }
 }
 
 template <typename T>
-void launchUnpackT(const uint8_t* frame, int w, int h, size_t pitch, const TileSlot* slots, int nslots, int tile, T* out, cudaStream_t s) {
+void launchUnpackT(const uint8_t* frame, int w, int h, size_t pitch, const TileSlot* slots, int nslots, int tile, T* out, cudaStream_t s,
+                   int pixelBytes) {
     if (nslots <= 0) return;
     const int side = (tile + kUB - 1) / kUB;
     dim3 grid(side * side, nslots);
-    const int wordOk = (reinterpret_cast<uintptr_t>(frame) & 3) == 0 ? 1 : 0;
-    unpack_kernel<T><<<grid, 256, 0, s>>>(frame, w, h, pitch, slots, tile, wordOk, out);
+    const bool aligned = (reinterpret_cast<uintptr_t>(frame) & 3) == 0;
+    if (pixelBytes == 4) unpack_kernel<T, 4><<<grid, 256, 0, s>>>(frame, w, h, pitch, slots, tile, aligned && (pitch & 3) == 0 ? 1 : 0, out);
+    else unpack_kernel<T, 3><<<grid, 256, 0, s>>>(frame, w, h, pitch, slots, tile, aligned ? 1 : 0, out);
 }
-void launchUnpack(const uint8_t* frame, int w, int h, size_t pitch, const TileSlot* slots, int nslots, int tile, __half* out, cudaStream_t s) {
-    launchUnpackT(frame, w, h, pitch, slots, nslots, tile, out, s);
+void launchUnpack(const uint8_t* frame, int w, int h, size_t pitch, const TileSlot* slots, int nslots, int tile, __half* out, cudaStream_t s,
+                  int pixelBytes) {
+    launchUnpackT(frame, w, h, pitch, slots, nslots, tile, out, s, pixelBytes);
 }
-void launchUnpack(const uint8_t* frame, int w, int h, size_t pitch, const TileSlot* slots, int nslots, int tile, float* out, cudaStream_t s) {
-    launchUnpackT(frame, w, h, pitch, slots, nslots, tile, out, s);
+void launchUnpack(const uint8_t* frame, int w, int h, size_t pitch, const TileSlot* slots, int nslots, int tile, float* out, cudaStream_t s,
+                  int pixelBytes) {
+    launchUnpackT(frame, w, h, pitch, slots, nslots, tile, out, s, pixelBytes);
 }
 
 // ---- stitch + pack ----------------------------------------------------------------------------------
@@ -180,7 +194,12 @@ __device__ __forceinline__ void loadTilePx(const void* tiles, size_t idx, float&
 // is computed once per block (threads 0..kSR-1) and broadcast through shared memory, and the tile reads of a warp are 256
 // contiguous bytes.  Along each axis a pixel is covered by at most two tiles (stride = outT - ov > outT / 2).  The packed BGR bytes
 // of a row (768 per block) are staged in shared memory and leave as 16-byte vector stores (scalar on unaligned canvases / tails).
+// PB = output bytes per pixel: 3 (BGR) or 4 (BGRA).  A BGRA pixel blends the alpha pass's tile of the same reference tile (slot +
+// alpha_off) with the same weights in the same order, and packs the mean of its three channels as alpha; without an alpha pass
+// (alpha_off == 0) alpha is 255.
 constexpr int kSW = 256, kSR = 16;
+
+__device__ __forceinline__ uint8_t packU8(float v) { return (uint8_t)min(max(__float2int_rn(__fmul_rn(v, 255.f)), 0), 255); }
 
 struct StitchRow {
     int n;            // covering tile rows (0 past the band end)
@@ -188,9 +207,9 @@ struct StitchRow {
     float wt[2], wb[2];
 };
 
-template <bool F32>
+template <bool F32, int PB>
 __global__ void __launch_bounds__(kSW) stitch_kernel(StitchParams p, int vecOk) {
-    __shared__ __align__(16) uint8_t sm[kSR][kSW * 3];
+    __shared__ __align__(16) uint8_t sm[kSR][kSW * PB];
     __shared__ StitchRow rowInfo[kSR];
     const int ox0 = blockIdx.x * kSW, ox = ox0 + threadIdx.x;
     const int oyBase = p.y_begin + blockIdx.y * kSR;
@@ -252,9 +271,12 @@ __global__ void __launch_bounds__(kSW) stitch_kernel(StitchParams p, int vecOk) 
         const int rn = ri.n;
         if (!live || rn == 0) continue;
         float accr = 0.f, accg = 0.f, accb = 0.f;
+        float alr = 0.f, alg = 0.f, alb = 0.f;   // BGRA: the alpha pass's canvas
+        const bool alpha = PB == 4 && p.alpha_off > 0;
         if (plainX && rn == 1 && ri.wt[0] == 1.f && ri.wb[0] == 1.f) {
             const int slot = p.tile_map ? __ldg(p.tile_map + ti[0] * p.ny + ri.j[0]) : ti[0] * p.ny + ri.j[0];
             loadTilePx<F32>(p.tiles, ((size_t)slot * p.outT + ri.ly[0]) * p.outT + lxs[0], accr, accg, accb);
+            if (alpha) loadTilePx<F32>(p.tiles, ((size_t)(slot + p.alpha_off) * p.outT + ri.ly[0]) * p.outT + lxs[0], alr, alg, alb);
         } else {
 #pragma unroll
             for (int a = 0; a < 2; ++a) {       // tile order of the reference: x outer, y inner (render.cpp:43-44)
@@ -274,33 +296,43 @@ __global__ void __launch_bounds__(kSW) stitch_kernel(StitchParams p, int vecOk) 
                     accr = __fadd_rn(accr, r);
                     accg = __fadd_rn(accg, g);
                     accb = __fadd_rn(accb, b);
+                    if (alpha) {
+                        loadTilePx<F32>(p.tiles, ((size_t)(slot + p.alpha_off) * p.outT + ri.ly[bsel]) * p.outT + lxs[a], r, g, b);
+                        r = __fmul_rn(__fmul_rn(__fmul_rn(__fmul_rn(r, wl), wt), wr), wb);
+                        g = __fmul_rn(__fmul_rn(__fmul_rn(__fmul_rn(g, wl), wt), wr), wb);
+                        b = __fmul_rn(__fmul_rn(__fmul_rn(__fmul_rn(b, wl), wt), wr), wb);
+                        alr = __fadd_rn(alr, r);
+                        alg = __fadd_rn(alg, g);
+                        alb = __fadd_rn(alb, b);
+                    }
                 }
             }
         }
         // convertTo(CV_8UC3, 255): saturate_cast<uchar>(rint(v * 255)) (render.cpp:342), then RGB -> BGR (:343)
-        uint8_t* d = sm[row] + threadIdx.x * 3;
-        d[0] = (uint8_t)min(max(__float2int_rn(__fmul_rn(accb, 255.f)), 0), 255);
-        d[1] = (uint8_t)min(max(__float2int_rn(__fmul_rn(accg, 255.f)), 0), 255);
-        d[2] = (uint8_t)min(max(__float2int_rn(__fmul_rn(accr, 255.f)), 0), 255);
+        uint8_t* d = sm[row] + threadIdx.x * PB;
+        d[0] = packU8(accb);
+        d[1] = packU8(accg);
+        d[2] = packU8(accr);
+        if (PB == 4) d[3] = alpha ? packU8(__fdiv_rn(__fadd_rn(__fadd_rn(alr, alg), alb), 3.f)) : (uint8_t)255;
     }
     __syncthreads();
-    const int nbytes = min(kSW, p.cw - ox0) * 3;
+    const int nbytes = min(kSW, p.cw - ox0) * PB;
     if (nbytes <= 0) return;
     const int rowsHere = min(kSR, p.y_end - oyBase);
     if (vecOk) {
-        const int nvec = nbytes >> 4;                       // 48 vectors per full row: 256 threads cover 5 1/3 rows per pass
+        const int nvec = nbytes >> 4;                       // 48 (BGRA: 64) vectors per full row
         for (int v = threadIdx.x; v < nvec * rowsHere; v += kSW) {
             const int row = v / nvec, c = v - row * nvec;
-            reinterpret_cast<uint4*>(p.dst + (size_t)(oyBase + row) * p.pitch + (size_t)ox0 * 3)[c] = reinterpret_cast<const uint4*>(sm[row])[c];
+            reinterpret_cast<uint4*>(p.dst + (size_t)(oyBase + row) * p.pitch + (size_t)ox0 * PB)[c] = reinterpret_cast<const uint4*>(sm[row])[c];
         }
         const int tail = nbytes - (nvec << 4);
         for (int b = threadIdx.x; b < tail * rowsHere; b += kSW) {
             const int row = b / tail, c = (nvec << 4) + b - row * tail;
-            p.dst[(size_t)(oyBase + row) * p.pitch + (size_t)ox0 * 3 + c] = sm[row][c];
+            p.dst[(size_t)(oyBase + row) * p.pitch + (size_t)ox0 * PB + c] = sm[row][c];
         }
     } else {
         for (int row = 0; row < rowsHere; ++row)
-            for (int b = threadIdx.x; b < nbytes; b += kSW) p.dst[(size_t)(oyBase + row) * p.pitch + (size_t)ox0 * 3 + b] = sm[row][b];
+            for (int b = threadIdx.x; b < nbytes; b += kSW) p.dst[(size_t)(oyBase + row) * p.pitch + (size_t)ox0 * PB + b] = sm[row][b];
     }
 }
 
@@ -309,10 +341,15 @@ void launchStitch(const StitchParams& pin, cudaStream_t s) {
     if (p.y_end <= 0) { p.y_begin = 0; p.y_end = p.ch; }  // whole canvas
     if (p.y_end <= p.y_begin) return;
     dim3 grid((p.cw + kSW - 1) / kSW, (p.y_end - p.y_begin + kSR - 1) / kSR);
-    // 16-byte stores need 16-byte aligned row segments: block columns start at multiples of 768 bytes
+    // 16-byte stores need 16-byte aligned row segments: block columns start at multiples of 768 (BGRA: 1024) bytes
     const int vecOk = ((reinterpret_cast<uintptr_t>(p.dst) & 15) == 0 && (p.pitch & 15) == 0) ? 1 : 0;
-    if (p.f32) stitch_kernel<true><<<grid, kSW, 0, s>>>(p, vecOk);
-    else stitch_kernel<false><<<grid, kSW, 0, s>>>(p, vecOk);
+    if (p.bgra) {
+        if (p.f32) stitch_kernel<true, 4><<<grid, kSW, 0, s>>>(p, vecOk);
+        else stitch_kernel<false, 4><<<grid, kSW, 0, s>>>(p, vecOk);
+    } else {
+        if (p.f32) stitch_kernel<true, 3><<<grid, kSW, 0, s>>>(p, vecOk);
+        else stitch_kernel<false, 3><<<grid, kSW, 0, s>>>(p, vecOk);
+    }
 }
 
 // ---- TTA reduce -------------------------------------------------------------------------------------

@@ -93,7 +93,12 @@ public:
         w2x_set_progress_callback(h_, prog_ ? &Img2Img::onProgress : nullptr, this);
     }
 
-    // extensions (not in the reference): up to three frames in flight, see w2x_submit / w2x_wait in include/w2x.h
+    // extensions (not in the reference): BGRA8 HWC in, BGRA8 HWC out, synchronous, see w2x_render_bgra in include/w2x.h
+    bool renderBgra(const unsigned char* srcBgra, int width, int height, size_t srcStride, unsigned char* dstBgra, size_t dstStride) {
+        return w2x_render_bgra(h_, srcBgra, width, height, srcStride, dstBgra, dstStride) != 0;
+    }
+
+    // up to three frames in flight, see w2x_submit / w2x_wait in include/w2x.h
     int submit(const unsigned char* srcBgr, int width, int height, size_t srcStride, unsigned char* dstBgr, size_t dstStride) {
         return w2x_submit(h_, srcBgr, width, height, srcStride, dstBgr, dstStride);
     }
@@ -134,6 +139,8 @@ public:
         return w2x_pool_submit(h_, srcBgr, width, height, srcStride, dstBgr, dstStride);
     }
     bool wait(int ticket) { return w2x_pool_wait(h_, ticket) != 0; }
+    // the pool's index-th engine (borrowed), e.g. for w2x_render_bgra
+    w2x_engine* engine(int index) const { return w2x_pool_engine(h_, index); }
     void setMessageCallback(MessageCallback cb) {
         msg_ = std::move(cb);
         w2x_pool_set_message_callback(h_, msg_ ? &Img2ImgPool::onMessage : nullptr, this);

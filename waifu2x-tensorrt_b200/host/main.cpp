@@ -41,6 +41,7 @@ struct Options {
     std::string command;  // "render" | "build"
     std::vector<fs::path> inputPaths;
     bool recursive = false, nosuffix = false, tta = false;
+    bool alpha = false;  // extension: still images keep their alpha channel (BGRA through Img2Img::renderBgra, PNG out)
     fs::path outputDirectory;
     double blend = 1.0 / 16.0;
     std::string codec = "libx264", pixelFormat = "yuv420p";
@@ -70,6 +71,7 @@ const char* kUsage =
     "    -i, --input PATH ... REQUIRED   --recursive   -o, --output DIR   --nosuffix\n"
     "    --blend FLOAT:{0.125,0.0625,0.03125,0}=0.0625   --tta\n"
     "    --codec TEXT=libx264   --pix_fmt TEXT=yuv420p   --crf INT:[0,51]=23   --ffmpegDir TEXT\n"
+    "    --alpha                     Keep the alpha channel of still images (extension; videos are rendered without it)\n"
     "  build                         Build model\n";
 
 int toInt(const std::string& name, const std::string& v) {
@@ -158,6 +160,7 @@ Options parse(int argc, char** argv) {
             requireMember(a, o.blend, {1.0 / 8.0, 1.0 / 16.0, 1.0 / 32.0, 0.0});
         }
         else if (inRender && a == "--tta") o.tta = true;
+        else if (inRender && a == "--alpha") o.alpha = true;
         else if (inRender && a == "--codec") o.codec = value();
         else if (inRender && a == "--pix_fmt") o.pixelFormat = value();
         else if (inRender && a == "--crf") { o.crf = toInt(a, value()); if (o.crf < 0 || o.crf > 51) throw ParseError(a + ": value not in range 0 to 51"); }
@@ -302,7 +305,11 @@ int main(int argc, char* argv[]) {
     writer.setFfmpegDir(o.ffmpegDir).setConstantRateFactor(o.crf);
     try {
         for (auto& file : files) {
-            capture.open(file.string());
+            capture.setChannels(3).open(file.string());
+            // --alpha: a still image is decoded again as BGRA (the frame count is known once ffprobe has run)
+            const bool bgra = o.alpha && capture.getFrameCount() == 1;
+            if (bgra) capture.setChannels(4).open(file.string());
+            else if (o.alpha) logLine(trt::Severity::warn, "--alpha applies to still images; " + file.string() + " is rendered without alpha");
             const FrameSize inSize = capture.getFrameSize(), outSize = inSize * o.scale;
             frameIndex = 0;
             frameCount = (size_t)capture.getFrameCount();
@@ -315,8 +322,23 @@ int main(int argc, char* argv[]) {
                 file.replace_extension(".mp4");
                 writer.setFrameRate(capture.getFrameRate()).setPixelFormat(o.pixelFormat).setCodec(o.codec);
             }
-            writer.setFrameSize(outSize).setOutputFile(file.string());
+            writer.setFrameSize(outSize).setOutputFile(file.string()).setChannels(bgra ? 4 : 3);
             writer.open();
+            if (bgra) {  // one frame, synchronously; with a --device list on the pool's first engine
+                in[0].reserve(inSize.bytes(4));
+                out[0].reserve(outSize.bytes(4));
+                if (!capture.read(in[0].p)) throw std::runtime_error("could not read \"" + file.string() + "\"");
+                w2x_engine* e = pool ? pool->engine(0) : engine.handle();
+                if (!w2x_render_bgra(e, in[0].p, inSize.width, inSize.height, (size_t)inSize.width * 4, out[0].p, (size_t)outSize.width * 4))
+                    throw std::runtime_error("render failed");
+                frameIndex = 1;
+                writer.write(out[0].p, outSize);
+                capture.release();
+                writer.release();
+                if (writer.exitStatus() != 0) throw std::runtime_error("ffmpeg failed to encode \"" + file.string() + "\" (exit status " + std::to_string(writer.exitStatus()) + ")");
+                fileIndex++;
+                continue;
+            }
             for (int s = 0; s < kRing; ++s) { in[s].reserve(inSize.bytes()); out[s].reserve(outSize.bytes()); }
 
             std::mutex mu;

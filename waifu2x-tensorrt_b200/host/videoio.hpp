@@ -2,6 +2,7 @@
 // reference's VideoCapture (/root/reference/src/videoio/capture.{h,cpp}) and VideoWriter (writer.{h,cpp}) with the same
 // class names, method names, command lines (capture.cpp:65-68,96-99; writer.cpp:24-33) and error behaviour (std::exception
 // on failure), minus OpenCV: frames are raw BGR8 HWC buffers (cv::Mat overloads appear when <opencv2/core.hpp> was included).
+// setChannels(4) on either class switches the raw frames to BGRA8 (`-pix_fmt bgra` instead of `bgr24`, nothing else changes).
 //
 // Fixes relative to the reference (SURVEY 8f rank 1): the command prefix (`ffmpegDir`) is settable on BOTH classes and is
 // honoured by VideoWriter::open (the reference ignores it, writer.cpp:24); release() uses pclose on every platform (the
@@ -33,7 +34,7 @@ struct FrameSize {  // stands in for cv::Size2i
     bool operator==(const FrameSize& o) const { return width == o.width && height == o.height; }
     bool operator!=(const FrameSize& o) const { return !(*this == o); }
     FrameSize operator*(int s) const { return {width * s, height * s}; }
-    size_t bytes() const { return (size_t)width * height * 3; }
+    size_t bytes(int channels = 3) const { return (size_t)width * height * channels; }
 };
 
 // A path inside the double quotes of the reference's command lines (capture.cpp:65-68,96-99; writer.cpp:24-33).  The reference pastes
@@ -46,6 +47,13 @@ inline std::string quotedPath(const std::string& path) {
         q += c;
     }
     return q + "\"";
+}
+
+// ffmpeg's name of the raw frame layout with `channels` bytes per pixel
+inline const char* rawPixelFormat(int channels) {
+    if (channels == 3) return "bgr24";
+    if (channels == 4) return "bgra";
+    throw std::invalid_argument("channels must be 3 or 4");
 }
 
 class VideoCapture {
@@ -75,7 +83,7 @@ public:
             frameSize.height = std::stoi(props.at("height"));
             frameRate = fraction(props.at("r_frame_rate"));
             frameCount = props.at("nb_frames") == "n/a" ? 1 : std::stoi(props.at("nb_frames"));  // no frame count => an image
-            const std::string cmd = ffmpegDir + "ffmpeg -v error -i " + quotedPath(path) + " -f image2pipe -vcodec rawvideo -pix_fmt bgr24 -";
+            const std::string cmd = ffmpegDir + "ffmpeg -v error -i " + quotedPath(path) + " -f image2pipe -vcodec rawvideo -pix_fmt " + rawPixelFormat(channels) + " -";
             pipe = popen(cmd.c_str(), "r");
             if (!pipe) throw std::runtime_error("could not open ffmpeg with command\"" + cmd + "\"");
             growPipe(pipe);
@@ -89,11 +97,11 @@ public:
 
     [[nodiscard]] bool isOpened() const noexcept { return opened; }
 
-    // capture.cpp:116-128: one blocking read of W*H*3 bytes; false after the last frame
+    // capture.cpp:116-128: one blocking read of W*H*channels bytes; false after the last frame
     bool read(uint8_t* bgr) {
         if (!opened) throw std::runtime_error("video capture is not opened");
         if (frameIndex + 1 >= frameCount) return false;
-        const size_t want = frameSize.bytes();
+        const size_t want = frameSize.bytes(channels);
         size_t got = 0;
         while (got < want) {
             const size_t n = fread(bgr + got, 1, want - got, pipe);
@@ -119,6 +127,9 @@ public:
 
     [[nodiscard]] const std::string& getFfmpegDir() const noexcept { return ffmpegDir; }
     VideoCapture& setFfmpegDir(const std::string& value) { ffmpegDir = value; return *this; }  // missing in the reference (capture.h)
+    // 3 (BGR, the default) or 4 (BGRA); applies from the next open()
+    VideoCapture& setChannels(int value) { rawPixelFormat(value); channels = value; return *this; }
+    [[nodiscard]] int getChannels() const noexcept { return channels; }
     [[nodiscard]] const FrameSize& getFrameSize() const noexcept { return frameSize; }
     [[nodiscard]] double getFrameRate() const noexcept { return frameRate; }
     [[nodiscard]] int getFrameCount() const noexcept { return frameCount; }
@@ -150,6 +161,7 @@ private:
     double frameRate = -1;
     int frameCount = -1;
     int frameIndex = -1;
+    int channels = 3;
 };
 
 class VideoWriter {
@@ -165,7 +177,7 @@ public:
         if (frameSize.width <= 0 || frameSize.height <= 0) throw std::invalid_argument("frame size must be greater than 0");
         if (outputFile.empty()) throw std::invalid_argument("output file is empty");
         const std::string cmd = ffmpegDir + "ffmpeg -v error -y -f rawvideo -vcodec rawvideo -s " + std::to_string(frameSize.width) + "x" +
-                                std::to_string(frameSize.height) + " -pix_fmt bgr24" + (frameRate <= 0 ? "" : " -r " + std::to_string(frameRate)) +
+                                std::to_string(frameSize.height) + " -pix_fmt " + rawPixelFormat(channels) + (frameRate <= 0 ? "" : " -r " + std::to_string(frameRate)) +
                                 " -i -" + (codec.empty() ? "" : " -vcodec " + codec) + (pixelFormat.empty() ? "" : " -pix_fmt " + pixelFormat) +
                                 (crf < 0 ? "" : " -crf " + std::to_string(crf)) + (quality < 0 ? "" : " -q:v " + std::to_string(quality)) +
                                 " " + quotedPath(outputFile);
@@ -181,7 +193,7 @@ public:
     void write(const uint8_t* bgr, const FrameSize& size) {
         if (!opened) throw std::runtime_error("video writer is not opened");
         if (size != frameSize) throw std::invalid_argument("frame size does not match");
-        if (fwrite(bgr, 1, frameSize.bytes(), pipe) != frameSize.bytes()) throw std::runtime_error("could not write frame to pipe");
+        if (fwrite(bgr, 1, frameSize.bytes(channels), pipe) != frameSize.bytes(channels)) throw std::runtime_error("could not write frame to pipe");
     }
 #ifdef OPENCV_CORE_HPP
     void write(const cv::Mat& frame) {
@@ -218,6 +230,9 @@ public:
     VideoWriter& setCodec(const std::string& v) { guard(); codec = v; return *this; }
     VideoWriter& setConstantRateFactor(int v) { guard(); crf = v; return *this; }
     VideoWriter& setQuality(int v) { guard(); quality = v; return *this; }
+    // 3 (BGR, the default) or 4 (BGRA): the layout of the frames given to write()
+    VideoWriter& setChannels(int v) { guard(); rawPixelFormat(v); channels = v; return *this; }
+    [[nodiscard]] int getChannels() const noexcept { return channels; }
 
 private:
     void guard() const {
@@ -231,4 +246,5 @@ private:
     std::string outputFile, pixelFormat, codec;
     int crf = -1, quality = -1;
     int lastStatus = 0;
+    int channels = 3;
 };

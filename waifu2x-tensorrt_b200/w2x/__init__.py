@@ -98,6 +98,7 @@ _SIGNATURES = {
     "w2x_load": (C.c_int, [C.c_void_p, C.c_char_p, C.POINTER(_RenderConfig)]),
     "w2x_render": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_size_t, C.c_void_p, C.c_size_t]),
     "w2x_render_device": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_size_t, C.c_void_p, C.c_size_t]),
+    "w2x_render_bgra": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_size_t, C.c_void_p, C.c_size_t]),
     "w2x_submit": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_size_t, C.c_void_p, C.c_size_t]),
     "w2x_render_banded": (C.c_int, [C.POINTER(C.c_void_p), C.c_int, C.c_void_p, C.c_int, C.c_int, C.c_size_t, C.c_void_p, C.c_size_t]),
     "w2x_wait": (C.c_int, [C.c_void_p, C.c_int]),
@@ -132,6 +133,7 @@ _SIGNATURES = {
     "w2x_unpack_tiles": (C.c_int, [C.c_int, C.c_void_p, C.c_int, C.c_int, C.c_size_t, C.POINTER(_Rect), C.POINTER(C.c_int), C.c_int, C.c_int, C.c_void_p]),
     "w2x_stitch_tiles": (C.c_int, [C.c_int, C.c_void_p] + [C.c_int] * 8 + [C.c_void_p, C.c_size_t]),
     "w2x_tta_reduce": (C.c_int, [C.c_int, C.c_void_p, C.c_int, C.c_int, C.c_void_p]),
+    "w2x_alpha_bleed": (C.c_int, [C.c_int, C.c_void_p, C.c_int, C.c_int, C.c_size_t, C.c_int, C.c_void_p]),
     "w2x_infer": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_void_p]),
     "w2x_selftest_conv": (C.c_double, [C.c_int] * 7 + [C.c_uint]),
     "w2x_run_conv_layer": (C.c_int, [C.c_int] * 8 + [C.c_void_p, C.c_void_p, C.POINTER(C.c_float), C.c_void_p, C.c_void_p]),
@@ -283,6 +285,21 @@ def tta_reduce(outs_f16: np.ndarray, device: int = 0) -> np.ndarray:
     if not lib().w2x_tta_reduce(device, _ptr(t), tiles, ot, _ptr(mean)):
         raise RuntimeError("w2x_tta_reduce failed")
     return mean
+
+
+def _rows_of_pixels(a: np.ndarray, channels: int) -> bool:
+    """a is [H, W, channels] uint8 with contiguous pixels (rows may be strided)."""
+    return a.dtype == np.uint8 and a.ndim == 3 and a.shape[2] == channels and a.strides[2] == 1 and a.strides[1] == channels
+
+
+def alpha_bleed(src_bgra: np.ndarray, rounds: int, device: int = 0) -> np.ndarray:
+    """The colour bleed of w2x_render_bgra (include/w2x_dev.h: w2x_alpha_bleed): uint8 [H, W, 4] BGRA -> uint8 [H, W, 4], alpha unchanged."""
+    src = src_bgra if _rows_of_pixels(src_bgra, 4) else np.ascontiguousarray(src_bgra, dtype=np.uint8)
+    h, w = src.shape[:2]
+    out = np.empty((h, w, 4), np.uint8)
+    if not lib().w2x_alpha_bleed(device, _ptr(src), w, h, src.strides[0], int(rounds), _ptr(out)):
+        raise RuntimeError("w2x_alpha_bleed failed")
+    return out
 
 
 def run_conv_layer(kind: int, x: np.ndarray, w_packed: np.ndarray, bias: np.ndarray, cout: int, skip: Optional[np.ndarray] = None,
@@ -448,6 +465,19 @@ class Img2Img:
         return dst if ok else None
 
     # extensions
+    def render_bgra(self, src: np.ndarray, dst: Optional[np.ndarray] = None) -> Optional[np.ndarray]:
+        """src: uint8 [H, W, 4] BGRA (rows may be strided).  Returns dst (uint8 [H*s, W*s, 4] BGRA; a caller's dst may have strided rows)
+        or None on failure (the reason in last_error)."""
+        if not _rows_of_pixels(src, 4):
+            src = np.ascontiguousarray(src, dtype=np.uint8)
+        h, w = src.shape[:2]
+        if dst is None:
+            dst = np.empty((h * self.scaling, w * self.scaling, 4), np.uint8)
+        elif not _rows_of_pixels(dst, 4):
+            raise ValueError("dst must be uint8 [H, W, 4] with contiguous pixels")
+        ok = self._l.w2x_render_bgra(self._h, _ptr(src), w, h, src.strides[0], _ptr(dst), dst.strides[0])
+        return dst if ok else None
+
     def infer(self, x_nchw: np.ndarray) -> Optional[np.ndarray]:
         x = np.ascontiguousarray(x_nchw, dtype=np.float32)
         n = x.shape[0]
