@@ -163,20 +163,39 @@ def test_colour_under_alpha_zero_does_not_matter(built_lib, alpha_models):
 
 
 def test_interleaved_calls_equal_fresh_engines(built_lib, alpha_models):
+    """render, submit, render_bgra and render_banded (over this engine and a second one) in one sequence on frames that grow, shrink and
+    grow again: every call returns what the same call returns on fresh engines."""
+    import w2x
+    from test_gpu_engine_state import _submit
     e, _, _ = _make("cunet2x_t64_b3", alpha_models)
     _, path = alpha_models[("cunet", 2)]
+    e2 = _engine(path, 2, 64, 3)
     opaque = masked_frame(150, 97, 6)
     opaque[..., 3] = 255
     calls = [("bgr", tiling.synthetic_frame(150, 97, 7)), ("bgra", masked_frame(131, 70, 8)), ("bgra", opaque),
              ("bgr", tiling.synthetic_frame(131, 70, 9)), ("bgra", masked_frame(150, 97, 10)), ("bgra", opaque[:70, :131].copy()),
-             ("bgr", tiling.synthetic_frame(150, 97, 11))]
-    got = [e.render(f) if k == "bgr" else e.render_bgra(f) for k, f in calls]
+             ("bgr", tiling.synthetic_frame(150, 97, 11)), ("submit", tiling.synthetic_frame(210, 160, 12)),
+             ("banded", tiling.synthetic_frame(96, 150, 13)), ("bgra", masked_frame(230, 170, 14)), ("submit", tiling.synthetic_frame(90, 60, 15)),
+             ("banded", tiling.synthetic_frame(240, 180, 16)), ("bgr", tiling.synthetic_frame(100, 70, 17))]
+
+    def call(k, engines, f):
+        if k == "bgr":
+            return engines[0].render(f)
+        if k == "bgra":
+            return engines[0].render_bgra(f)
+        if k == "submit":
+            return _submit(engines[0], f)
+        return w2x.render_banded(engines, f)
+
+    got = [call(k, [e, e2], f) for k, f in calls]
     for (k, f), g in zip(calls, got):
-        fresh = _engine(path, 2, 64, 3)
-        want = fresh.render(f) if k == "bgr" else fresh.render_bgra(f)
-        fresh.close()
+        fresh = [_engine(path, 2, 64, 3) for _ in range(2 if k == "banded" else 1)]
+        want = call(k, fresh, f)
+        for x in fresh:
+            x.close()
         assert g is not None and np.array_equal(g, want), (k, f.shape)
     e.close()
+    e2.close()
 
 
 def test_strided_host_buffers(built_lib, alpha_models):

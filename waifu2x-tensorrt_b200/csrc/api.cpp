@@ -5,6 +5,7 @@
 #include <algorithm>
 #include <cstring>
 #include <filesystem>
+#include <memory>
 
 #include "engine.h"
 #include "pool.h"
@@ -25,16 +26,11 @@ void setErr(char* err, int cap, const std::string& s) {
     }
 }
 
-struct DevBufs {
-    std::vector<void*> v;
-    ~DevBufs() { for (void* p : v) cudaFree(p); }
-    template <class T> T* alloc(size_t count) {
-        void* p = nullptr;
-        W2X_CUDA(cudaMalloc(&p, count * sizeof(T) + 16));
-        v.push_back(p);
-        return (T*)p;
-    }
-};
+// device memory for `count` elements of T, owned by `bufs`
+template <class T> T* alloc(std::vector<DeviceBuffer>& bufs, size_t count) {
+    bufs.emplace_back(count * sizeof(T) + 16);
+    return bufs.back().get<T>();
+}
 }  // namespace
 
 extern "C" {
@@ -197,15 +193,15 @@ int w2x_unpack_tiles(int device, const uint8_t* src, int width, int height, size
     try {
         if (!src || !rects || !out || n <= 0 || tile <= 0) return 0;
         W2X_CUDA(cudaSetDevice(device));
-        DevBufs b;
-        uint8_t* dSrc = b.alloc<uint8_t>((size_t)width * 3 * height);
+        std::vector<DeviceBuffer> b;
+        uint8_t* dSrc = alloc<uint8_t>(b, (size_t)width * 3 * height);
         W2X_CUDA(cudaMemcpy2D(dSrc, (size_t)width * 3, src, src_stride, (size_t)width * 3, height, cudaMemcpyHostToDevice));
         std::vector<TileSlot> slots(n);
         for (int i = 0; i < n; ++i) slots[i] = {rects[i].x, rects[i].y, aug ? aug[i] : 0, 1};
-        TileSlot* dSlots = b.alloc<TileSlot>(n);
+        TileSlot* dSlots = alloc<TileSlot>(b, n);
         W2X_CUDA(cudaMemcpy(dSlots, slots.data(), sizeof(TileSlot) * n, cudaMemcpyHostToDevice));
         const size_t elems = (size_t)n * tile * tile * 4;
-        __half* dOut = b.alloc<__half>(elems);
+        __half* dOut = alloc<__half>(b, elems);
         launchUnpack(dSrc, width, height, (size_t)width * 3, dSlots, n, tile, dOut, nullptr);
         W2X_CUDA(cudaGetLastError());
         W2X_CUDA(cudaMemcpy(out, dOut, elems * 2, cudaMemcpyDeviceToHost));
@@ -221,16 +217,16 @@ int w2x_stitch_tiles(int device, const uint16_t* tiles, int count, int out_tile,
     try {
         if (!tiles || !dst || count != nx * ny) return 0;
         W2X_CUDA(cudaSetDevice(device));
-        DevBufs b;
+        std::vector<DeviceBuffer> b;
         const size_t elems = (size_t)count * out_tile * out_tile * 4;
-        __half* dT = b.alloc<__half>(elems);
+        __half* dT = alloc<__half>(b, elems);
         W2X_CUDA(cudaMemcpy(dT, tiles, elems * 2, cudaMemcpyHostToDevice));
         std::vector<float> rx = blendRamp(overlap_x), ry = blendRamp(overlap_y);
-        float* dRx = b.alloc<float>(rx.size() + 1);
-        float* dRy = b.alloc<float>(ry.size() + 1);
+        float* dRx = alloc<float>(b, rx.size() + 1);
+        float* dRy = alloc<float>(b, ry.size() + 1);
         if (!rx.empty()) W2X_CUDA(cudaMemcpy(dRx, rx.data(), rx.size() * 4, cudaMemcpyHostToDevice));
         if (!ry.empty()) W2X_CUDA(cudaMemcpy(dRy, ry.data(), ry.size() * 4, cudaMemcpyHostToDevice));
-        uint8_t* dDst = b.alloc<uint8_t>((size_t)canvas_w * 3 * canvas_h);
+        uint8_t* dDst = alloc<uint8_t>(b, (size_t)canvas_w * 3 * canvas_h);
         StitchParams sp{};
         sp.tiles = dT; sp.f32 = 0; sp.outT = out_tile; sp.nx = nx; sp.ny = ny; sp.ovx = overlap_x; sp.ovy = overlap_y;
         sp.cw = canvas_w; sp.ch = canvas_h; sp.rampx = dRx; sp.rampy = dRy; sp.dst = dDst; sp.pitch = (size_t)canvas_w * 3;
@@ -248,10 +244,10 @@ int w2x_alpha_bleed(int device, const uint8_t* src, int width, int height, size_
     try {
         if (!src || !dst || width <= 0 || height <= 0 || src_stride < (size_t)width * 4 || rounds < 0) throw Error("invalid argument");
         W2X_CUDA(cudaSetDevice(device));
-        DevBufs b;
+        std::vector<DeviceBuffer> b;
         const size_t row = (size_t)width * 4, bytes = row * height;
-        uint8_t* dSrc = b.alloc<uint8_t>(bytes);
-        uint8_t* dBuf[2] = {b.alloc<uint8_t>(bytes), b.alloc<uint8_t>(bytes)};
+        uint8_t* dSrc = alloc<uint8_t>(b, bytes);
+        uint8_t* dBuf[2] = {alloc<uint8_t>(b, bytes), alloc<uint8_t>(b, bytes)};
         W2X_CUDA(cudaMemcpy2D(dSrc, row, src, src_stride, row, height, cudaMemcpyHostToDevice));
         const uint8_t* in = dSrc;
         for (int r = 0; r < std::max(rounds, 1); ++r) {   // the engine's sequence (Engine::renderOnStream)
@@ -271,10 +267,10 @@ int w2x_tta_reduce(int device, const uint16_t* outs, int tiles, int out_tile, fl
     try {
         if (!outs || !mean || tiles <= 0) return 0;
         W2X_CUDA(cudaSetDevice(device));
-        DevBufs b;
+        std::vector<DeviceBuffer> b;
         const size_t plane = (size_t)out_tile * out_tile * 4;
-        __half* dIn = b.alloc<__half>(plane * 8 * tiles);
-        float* dOut = b.alloc<float>(plane * tiles);
+        __half* dIn = alloc<__half>(b, plane * 8 * tiles);
+        float* dOut = alloc<float>(b, plane * tiles);
         W2X_CUDA(cudaMemcpy(dIn, outs, plane * 8 * tiles * 2, cudaMemcpyHostToDevice));
         launchTtaReduce(dIn, tiles, out_tile, dOut, nullptr);
         W2X_CUDA(cudaGetLastError());
@@ -318,45 +314,39 @@ int w2x_run_conv_layer_f32(int device, int kind, int n, int h, int w, int cin, i
 
 int w2x_run_swin_mlp(int device, long long tokens, int c, int variant, uint16_t* x, const float* gamma, const float* beta, float eps, const uint16_t* w1,
                      const float* b1, const uint16_t* w2, const float* b2, int reps, float* ms_out) {
-    void* bufs[7] = {};
-    SwinMlpPlan* plan = nullptr;
-    cudaEvent_t e0 = nullptr, e1 = nullptr;
-    int ok = 0;
     try {
         if (tokens < 1 || !x || !gamma || !beta || !w1 || !b1 || !w2 || !b2 || !swinMlpSupported(c, 2 * c)) throw Error("invalid argument");
         W2X_CUDA(cudaSetDevice(device));
         const size_t C = (size_t)c;
         const size_t sizes[7] = {(size_t)tokens * C * 2, C * 4, C * 4, 2 * C * C * 2, 2 * C * 4, 2 * C * C * 2, C * 4};
         const void* host[7] = {x, gamma, beta, w1, b1, w2, b2};
+        DeviceBuffer bufs[7];
         for (int i = 0; i < 7; ++i) {
-            W2X_CUDA(cudaMalloc(&bufs[i], sizes[i]));
-            W2X_CUDA(cudaMemcpy(bufs[i], host[i], sizes[i], cudaMemcpyHostToDevice));
+            bufs[i].ensure(sizes[i]);
+            W2X_CUDA(cudaMemcpy(bufs[i].get(), host[i], sizes[i], cudaMemcpyHostToDevice));
         }
-        plan = swinMlpCreatePlan((__half*)bufs[0], c, (const float*)bufs[1], (const float*)bufs[2], eps, (const __half*)bufs[3], (const float*)bufs[4],
-                                 (const __half*)bufs[5], (const float*)bufs[6], variant);
-        swinMlpLaunch(plan, nullptr, tokens);
+        std::unique_ptr<SwinMlpPlan, void (*)(SwinMlpPlan*)> plan(
+            swinMlpCreatePlan(bufs[0].get<__half>(), c, bufs[1].get<const float>(), bufs[2].get<const float>(), eps, bufs[3].get<const __half>(),
+                              bufs[4].get<const float>(), bufs[5].get<const __half>(), bufs[6].get<const float>(), variant),
+            swinMlpDestroyPlan);
+        swinMlpLaunch(plan.get(), nullptr, tokens);
         W2X_CUDA(cudaDeviceSynchronize());
-        W2X_CUDA(cudaMemcpy(x, bufs[0], sizes[0], cudaMemcpyDeviceToHost));
+        W2X_CUDA(cudaMemcpy(x, bufs[0].get(), sizes[0], cudaMemcpyDeviceToHost));
         if (ms_out && reps > 0) {
-            W2X_CUDA(cudaEventCreate(&e0));
-            W2X_CUDA(cudaEventCreate(&e1));
+            CudaEvent ev0, ev1;
+            cudaEvent_t e0 = ev0.get(), e1 = ev1.get();
             W2X_CUDA(cudaEventRecord(e0, nullptr));
-            for (int i = 0; i < reps; ++i) swinMlpLaunch(plan, nullptr, tokens);
+            for (int i = 0; i < reps; ++i) swinMlpLaunch(plan.get(), nullptr, tokens);
             W2X_CUDA(cudaEventRecord(e1, nullptr));
             W2X_CUDA(cudaEventSynchronize(e1));
             W2X_CUDA(cudaEventElapsedTime(ms_out, e0, e1));
             *ms_out /= (float)reps;
         }
-        ok = 1;
+        return 1;
     } catch (const std::exception& ex) {
         std::fprintf(stderr, "w2x_run_swin_mlp: %s\n", ex.what());
+        return 0;
     }
-    if (e0) cudaEventDestroy(e0);
-    if (e1) cudaEventDestroy(e1);
-    if (plan) swinMlpDestroyPlan(plan);
-    for (void* b : bufs)
-        if (b) cudaFree(b);
-    return ok;
 }
 
 // host-only hooks for the CPU test suite: the operand preparation of the fused Swin kernels
@@ -400,10 +390,6 @@ int w2x_compose_up_to_image(const uint16_t* w_up, const float* b_up, const uint1
 
 int w2x_run_swin_attn(int device, int n, int h, int w, int c, int heads, int shift, uint16_t* x, const float* gamma, const float* beta, float eps, const uint16_t* wqkv,
                       const float* bqkv, const uint16_t* wproj, const float* bproj, const float* relpos, int reps, float* ms_out) {
-    void* bufs[9] = {};
-    SwinAttnPlan* plan = nullptr;
-    cudaEvent_t e0 = nullptr, e1 = nullptr;
-    int ok = 0;
     try {
         if (n < 1 || !x || !gamma || !beta || !wqkv || !bqkv || !relpos || !swinAttnSupported(c, heads, 6, h, w)) throw Error("invalid argument");
         const bool fuseProj = swinAttnFusesProj(c);
@@ -415,41 +401,40 @@ int w2x_run_swin_attn(int device, int n, int h, int w, int c, int heads, int shi
         const size_t C = (size_t)c;
         const size_t sizes[8] = {(size_t)n * h * w * C * 2, C * 4, C * 4, wR.size() * 2, bR.size() * 4, C * C * 2, C * 4, relR.size() * 4};
         const void* host[8] = {x, gamma, beta, wR.data(), bR.data(), wproj, bproj, relR.data()};
+        DeviceBuffer bufs[9];
         for (int i = 0; i < 8; ++i) {
             if (!host[i]) continue;   // wproj / bproj of the variant that stops at the attention output
-            W2X_CUDA(cudaMalloc(&bufs[i], sizes[i]));
-            W2X_CUDA(cudaMemcpy(bufs[i], host[i], sizes[i], cudaMemcpyHostToDevice));
+            bufs[i].ensure(sizes[i]);
+            W2X_CUDA(cudaMemcpy(bufs[i].get(), host[i], sizes[i], cudaMemcpyHostToDevice));
         }
         if (!fuseProj) {
-            W2X_CUDA(cudaMalloc(&bufs[8], sizes[0]));
-            W2X_CUDA(cudaMemset(bufs[8], 0, sizes[0]));
+            bufs[8].ensure(sizes[0]);
+            W2X_CUDA(cudaMemset(bufs[8].get(), 0, sizes[0]));
         }
         W2X_CUDA(cudaDeviceSynchronize());
-        plan = swinAttnCreatePlan((__half*)bufs[0], n, h, w, c, heads, 6, shift, (const float*)bufs[1], (const float*)bufs[2], eps, (const __half*)bufs[3],
-                                  (const float*)bufs[4], (const __half*)bufs[5], (const float*)bufs[6], (const float*)bufs[7], (__half*)bufs[8]);
-        swinAttnLaunch(plan, nullptr, n);
+        std::unique_ptr<SwinAttnPlan, void (*)(SwinAttnPlan*)> plan(
+            swinAttnCreatePlan(bufs[0].get<__half>(), n, h, w, c, heads, 6, shift, bufs[1].get<const float>(), bufs[2].get<const float>(), eps,
+                               bufs[3].get<const __half>(), bufs[4].get<const float>(), bufs[5].get<const __half>(), bufs[6].get<const float>(),
+                               bufs[7].get<const float>(), bufs[8].get<__half>()),
+            swinAttnDestroyPlan);
+        swinAttnLaunch(plan.get(), nullptr, n);
         W2X_CUDA(cudaDeviceSynchronize());
-        W2X_CUDA(cudaMemcpy(x, fuseProj ? bufs[0] : bufs[8], sizes[0], cudaMemcpyDeviceToHost));
+        W2X_CUDA(cudaMemcpy(x, bufs[fuseProj ? 0 : 8].get(), sizes[0], cudaMemcpyDeviceToHost));
         if (ms_out && reps > 0) {
-            W2X_CUDA(cudaEventCreate(&e0));
-            W2X_CUDA(cudaEventCreate(&e1));
+            CudaEvent ev0, ev1;
+            cudaEvent_t e0 = ev0.get(), e1 = ev1.get();
             W2X_CUDA(cudaEventRecord(e0, nullptr));
-            for (int i = 0; i < reps; ++i) swinAttnLaunch(plan, nullptr, n);
+            for (int i = 0; i < reps; ++i) swinAttnLaunch(plan.get(), nullptr, n);
             W2X_CUDA(cudaEventRecord(e1, nullptr));
             W2X_CUDA(cudaEventSynchronize(e1));
             W2X_CUDA(cudaEventElapsedTime(ms_out, e0, e1));
             *ms_out /= (float)reps;
         }
-        ok = 1;
+        return 1;
     } catch (const std::exception& ex) {
         std::fprintf(stderr, "w2x_run_swin_attn: %s\n", ex.what());
+        return 0;
     }
-    if (e0) cudaEventDestroy(e0);
-    if (e1) cudaEventDestroy(e1);
-    if (plan) swinAttnDestroyPlan(plan);
-    for (void* b : bufs)
-        if (b) cudaFree(b);
-    return ok;
 }
 
 #ifdef W2X_DEV

@@ -6,6 +6,7 @@
 #include <cstdlib>
 #include <cstring>
 #include <filesystem>
+#include <memory>
 #include <random>
 
 namespace w2x {
@@ -103,10 +104,8 @@ void Engine::log(int severity, const std::string& msg, const char* func, int lin
 #define ELOG(sev, msg) log(sev, msg, __FUNCTION__, __LINE__)
 
 void* Engine::dalloc(size_t bytes) {
-    void* p = nullptr;
-    W2X_CUDA(cudaMalloc(&p, bytes ? bytes : 16));
-    allocs.push_back(p);
-    return p;
+    allocs.emplace_back(bytes ? bytes : 16);
+    return allocs.back().get();
 }
 
 Act Engine::allocAct(int h, int w, int c) {
@@ -118,12 +117,8 @@ Act Engine::allocAct(int h, int w, int c) {
 }
 
 cudaEvent_t Engine::nextEvent() {
-    if (evUsed == (int)evPool.size()) {
-        cudaEvent_t e;
-        W2X_CUDA(cudaEventCreate(&e));
-        evPool.push_back(e);
-    }
-    return evPool[evUsed++];
+    if (timing.used == (int)timing.pool.size()) timing.pool.emplace_back();
+    return timing.pool[timing.used++].get();
 }
 
 void Engine::unload() {
@@ -138,41 +133,17 @@ void Engine::unload() {
         if (L.attn) swinAttnDestroyPlan(L.attn);
     }
     layers.clear();
-    for (void* p : allocs) cudaFree(p);
-    allocs.clear();
     dW.clear(); dBias.clear();
-    auto freep = [](auto*& p) { if (p) { cudaFree(p); p = nullptr; } };
-    freep(dTileMap); tileMapCap = 0;
-    for (cudaEvent_t e : bandEv) cudaEventDestroy(e);
-    bandEv.clear();
-    freep(dSlots);
-    if (dTileOut) { cudaFree(dTileOut); dTileOut = nullptr; } freep(dTtaMean); freep(dRampX); freep(dRampY); freep(dFrameIn); freep(dFrameOut);
-    if (dUnpacked) { cudaFree(dUnpacked); dUnpacked = nullptr; }
-    unpackedCap = 0;
-    freep(dAlphaFlags); freep(dBleed[0]); freep(dBleed[1]);
-    bleedCap = 0;
-    if (dBandTiles) { cudaFree(dBandTiles); dBandTiles = nullptr; }
-    freep(dBandMap); freep(dBandSlots); freep(dBandMean);
-    bandTilesCap = bandMapCap = bandSlotCap = bandMeanCap = 0;
-    if (evBandModel) { cudaEventDestroy(evBandModel); evBandModel = nullptr; }
-    slotCap = tileOutCap = ttaCap = frameInCap = frameOutCap = 0;
-    rampXLen = rampYLen = -1;
-    for (auto& s : pipe) {
-        freep(s.dIn); freep(s.dOut);
-        s.inCap = s.outCap = 0;
-        if (s.evH2D) { cudaEventDestroy(s.evH2D); s.evH2D = nullptr; }
-        if (s.evComp) { cudaEventDestroy(s.evComp); s.evComp = nullptr; }
-        if (s.evDone) { cudaEventDestroy(s.evDone); s.evDone = nullptr; }
-        s.busy = false;
-    }
-    for (auto& e : timerEv) if (e) { cudaEventDestroy(e); e = nullptr; }
-    for (auto e : evPool) cudaEventDestroy(e);
-    evPool.clear(); evUsed = 0; spans.clear();
+    allocs.clear();
+    fc = {};
+    staging = {};
+    bgra = {};
+    band = {};
+    pipe = {};
+    timing = {};
     if (stream) { cudaStreamDestroy(stream); stream = nullptr; }
     if (h2dStream) { cudaStreamDestroy(h2dStream); h2dStream = nullptr; }
     if (d2hStream) { cudaStreamDestroy(d2hStream); d2hStream = nullptr; }
-    frameW = frameH = 0;
-    framePasses = 1;
     isLoaded = false;
 }
 
@@ -876,16 +847,21 @@ void Engine::runModel(cudaStream_t s, void* finalOut, int nImages, const void* i
 // render (img2img_render.cpp:224-348)
 // ------------------------------------------------------------------------------------------------
 void Engine::ensureFrameBuffers(int w, int h, int passes) {
-    if (w == frameW && h == frameH && passes == framePasses) return;
+    if (w == fc.w && h == fc.h && passes == fc.passes) return;
     if (w <= 0 || h <= 0) throw Error("invalid frame size");
     W2X_CUDA(cudaStreamSynchronize(stream));
+    // no frame matches the cache until every table below describes the new one: a frame refused here, or a failed allocation, must not
+    // leave the previous key next to this frame's grid
+    fc.w = fc.h = 0;
+    TileGrid& grid = fc.grid;
     grid = calculateTiles(w, h, w * scale, h * scale, tile, tile, outTile, outTile, scale, cfg.overlapX, cfg.overlapY);
     if (grid.count <= 0) throw Error("frame is too small for the configured tile overlap");
     const int stepsPerTile = cfg.tta ? 8 : 1;
     // a BGRA frame with an alpha pass: the alpha steps follow the colour steps in the same order (alpha slot = colour slot +
     // count * stepsPerTile), and the batches are padded once per frame
-    batchCount = (int)std::lround(std::ceil((double)(grid.count * stepsPerTile * passes) / batch));  // render.cpp:249
-    stepCount = batchCount * batch;
+    fc.batchCount = (int)std::lround(std::ceil((double)(grid.count * stepsPerTile * passes) / batch));  // render.cpp:249
+    const int stepCount = fc.batchCount * batch;
+    std::vector<RowBand>& rowBands = fc.rowBands;
     // Tile order.  The reference walks its column-major tile list (render.cpp:264-265).  A tile's result does not depend on its batch
     // or slot (exact integer SE sums), so without TTA the tiles are processed ROW by row instead: the output rows above the next tile row
     // are then final as soon as a tile row is done, which lets render() stitch and download them while later batches still compute.
@@ -918,108 +894,72 @@ void Engine::ensureFrameBuffers(int w, int h, int passes) {
             else slots[step] = {0, 0, 0, 0};  // zero dummy tile, render.cpp:281
         }
     }
-    if ((size_t)stepCount > slotCap) {
-        if (dSlots) cudaFree(dSlots);
-        W2X_CUDA(cudaMalloc(&dSlots, sizeof(TileSlot) * stepCount));
-        slotCap = stepCount;
-    }
-    uploadAsync(dSlots, slots.data(), sizeof(TileSlot) * stepCount);
+    fc.slots.ensure(sizeof(TileSlot) * stepCount);
+    uploadAsync(fc.slots.get(), slots.data(), sizeof(TileSlot) * stepCount);
     if (!tileMapHost.empty()) {
-        if (tileMapHost.size() > tileMapCap) {
-            if (dTileMap) cudaFree(dTileMap);
-            dTileMap = nullptr;
-            W2X_CUDA(cudaMalloc(&dTileMap, sizeof(int) * tileMapHost.size()));
-            tileMapCap = tileMapHost.size();
-        }
-        uploadAsync(dTileMap, tileMapHost.data(), sizeof(int) * tileMapHost.size());
+        fc.tileMap.ensure(sizeof(int) * tileMapHost.size());
+        uploadAsync(fc.tileMap.get(), tileMapHost.data(), sizeof(int) * tileMapHost.size());
     }
-    if (frameWideUnpack()) {
-        const size_t need = (size_t)stepCount * tile * tile * 4;
-        if (need > unpackedCap) {
-            if (dUnpacked) cudaFree(dUnpacked);
-            dUnpacked = nullptr;
-            W2X_CUDA(cudaMalloc(&dUnpacked, need * elemBytes));
-            unpackedCap = need;
-            // a fused RGB first layer reads the buffer through a tensor map of its own
-            if (layers[0].impl == IMPL_SKIP) igemmSetFusedFrameInput(layers[1].plan, static_cast<const __half*>(dUnpacked), stepCount);
-        }
-    }
+    // a fused RGB first layer reads the frame-wide buffer through a tensor map of its own
+    if (frameWideUnpack() && fc.unpacked.ensure((size_t)stepCount * tile * tile * 4 * elemBytes) && layers[0].impl == IMPL_SKIP)
+        igemmSetFusedFrameInput(layers[1].plan, fc.unpacked.get<const __half>(), stepCount);
     const size_t tileElems = (size_t)outTile * outTile * 4;
-    if ((size_t)stepCount * tileElems > tileOutCap) {
-        if (dTileOut) cudaFree(dTileOut);
-        W2X_CUDA(cudaMalloc(&dTileOut, (size_t)stepCount * tileElems * elemBytes));
-        tileOutCap = (size_t)stepCount * tileElems;
-    }
-    if (cfg.tta && (size_t)grid.count * passes * tileElems > ttaCap) {
-        if (dTtaMean) cudaFree(dTtaMean);
-        W2X_CUDA(cudaMalloc(&dTtaMean, (size_t)grid.count * passes * tileElems * sizeof(float)));
-        ttaCap = (size_t)grid.count * passes * tileElems;
-    }
-    if (rampXLen != grid.outOvX) {
-        if (dRampX) { cudaFree(dRampX); dRampX = nullptr; }
-        std::vector<float> r = blendRamp(grid.outOvX);
-        W2X_CUDA(cudaMalloc(&dRampX, std::max<size_t>(r.size(), 1) * 4));
-        if (!r.empty()) uploadAsync(dRampX, r.data(), r.size() * 4);
-        rampXLen = grid.outOvX;
-    }
-    if (rampYLen != grid.outOvY) {
-        if (dRampY) { cudaFree(dRampY); dRampY = nullptr; }
-        std::vector<float> r = blendRamp(grid.outOvY);
-        W2X_CUDA(cudaMalloc(&dRampY, std::max<size_t>(r.size(), 1) * 4));
-        if (!r.empty()) uploadAsync(dRampY, r.data(), r.size() * 4);
-        rampYLen = grid.outOvY;
-    }
+    fc.tileOut.ensure((size_t)stepCount * tileElems * elemBytes);
+    if (cfg.tta) fc.ttaMean.ensure((size_t)grid.count * passes * tileElems * sizeof(float));
+    // a ramp drops its length while it is replaced, so that a failure leaves no length that its buffer does not hold
+    auto ramp = [&](DeviceBuffer& buf, int& len, int overlap) {
+        if (len == overlap) return;
+        len = -1;
+        const std::vector<float> r = blendRamp(overlap);
+        buf.ensure(std::max<size_t>(r.size(), 1) * sizeof(float));
+        uploadAsync(buf.get(), r.data(), r.size() * sizeof(float));
+        len = overlap;
+    };
+    ramp(fc.rampX, fc.rampXLen, grid.outOvX);
+    ramp(fc.rampY, fc.rampYLen, grid.outOvY);
     // the copies above are ordered on `stream` like every kernel that reads them; the sync keeps the staging vectors' lifetime trivial
     W2X_CUDA(cudaStreamSynchronize(stream));
-    frameW = w;
-    frameH = h;
-    framePasses = passes;
+    fc.w = w;
+    fc.h = h;
+    fc.passes = passes;
 }
 
 void Engine::renderOnStream(const uint8_t* dSrc, int w, int h, size_t srcPitch, uint8_t* dDst, size_t dstPitch, cudaStream_t s, bool timed,
                             std::vector<BandDone>* bands, int pixelBytes) {
-    if (timed) { evUsed = 0; spans.clear(); }
+    if (timed) { timing.used = 0; timing.spans.clear(); }
     auto span = [&](int kind, auto&& fn) {
         if (!timed) { fn(); return; }
         cudaEvent_t e0 = nextEvent();
-        const int i0 = evUsed - 1;
+        const int i0 = timing.used - 1;
         W2X_CUDA(cudaEventRecord(e0, s));
         fn();
         cudaEvent_t e1 = nextEvent();
         W2X_CUDA(cudaEventRecord(e1, s));
-        spans.push_back({kind, i0, evUsed - 1});
+        timing.spans.push_back({kind, i0, timing.used - 1});
     };
     int passes = 1;
     if (pixelBytes == 4) {
         // The alpha plane decides the schedule: no alpha < 255, no alpha pass; some alpha == 0, the colour bleed first.  Both count as
         // unpack time.
-        if (!dAlphaFlags) W2X_CUDA(cudaMalloc(&dAlphaFlags, 2 * sizeof(int)));
+        bgra.flags.ensure(2 * sizeof(int));
+        int* dFlags = bgra.flags.get<int>();
         int flags[2] = {0, 0};
         span(0, [&] {
-            W2X_CUDA(cudaMemsetAsync(dAlphaFlags, 0, 2 * sizeof(int), s));
-            launchAlphaScan(dSrc, (size_t)w * h, dAlphaFlags, s);
+            W2X_CUDA(cudaMemsetAsync(dFlags, 0, 2 * sizeof(int), s));
+            launchAlphaScan(dSrc, (size_t)w * h, dFlags, s);
             ++launches;
         });
-        W2X_CUDA(cudaMemcpyAsync(flags, dAlphaFlags, sizeof flags, cudaMemcpyDeviceToHost, s));
+        W2X_CUDA(cudaMemcpyAsync(flags, dFlags, sizeof flags, cudaMemcpyDeviceToHost, s));
         W2X_CUDA(cudaStreamSynchronize(s));
         passes = flags[0] ? 2 : 1;
         if (flags[1]) {
-            const size_t bytes = (size_t)w * h * 4;
-            if (bytes > bleedCap) {
-                for (auto*& b : dBleed) {
-                    if (b) cudaFree(b);
-                    b = nullptr;
-                }
-                bleedCap = 0;
-                for (auto*& b : dBleed) W2X_CUDA(cudaMalloc(&b, bytes));
-                bleedCap = bytes;
-            }
+            for (DeviceBuffer& b : bgra.bleed) b.ensure((size_t)w * h * 4);
             // rounds = the model's input-side border (the halo of every tile): colour from farther away cannot reach an output pixel
             const int rounds = (int)(model.offset / std::max<uint32_t>(model.scale, 1));
             span(0, [&] {
                 const uint8_t* in = dSrc;
                 for (int r = 0; r < std::max(rounds, 1); ++r) {
-                    uint8_t* out = dBleed[r & 1];
+                    uint8_t* out = bgra.bleed[r & 1].get<uint8_t>();
                     launchAlphaBleedRound(in, out, w, h, rounds > 0 ? 1 : 0, r + 1 >= rounds ? dSrc : nullptr, s);
                     ++launches;
                     in = out;
@@ -1029,17 +969,18 @@ void Engine::renderOnStream(const uint8_t* dSrc, int w, int h, size_t srcPitch, 
         }
     }
     ensureFrameBuffers(w, h, passes);
-    const bool progressive = pixelBytes == 3 && bands != nullptr && !cfg.tta && !rowBands.empty();
+    const TileGrid& grid = fc.grid;
+    const bool progressive = pixelBytes == 3 && bands != nullptr && !cfg.tta && !fc.rowBands.empty();
     if (bands) bands->clear();
     auto stitchRows = [&](int yBegin, int yEnd) {
         StitchParams sp{};
         sp.outT = outTile; sp.nx = grid.nx; sp.ny = grid.ny; sp.ovx = grid.outOvX; sp.ovy = grid.outOvY;
         sp.cw = w * scale; sp.ch = h * scale;
-        sp.rampx = dRampX; sp.rampy = dRampY;
+        sp.rampx = fc.rampX.get<float>(); sp.rampy = fc.rampY.get<float>();
         sp.dst = dDst; sp.pitch = dstPitch;
-        sp.tiles = cfg.tta ? (const void*)dTtaMean : (const void*)dTileOut;
+        sp.tiles = cfg.tta ? fc.ttaMean.get() : fc.tileOut.get();
         sp.f32 = (cfg.tta || tf32()) ? 1 : 0;
-        sp.tile_map = cfg.tta ? nullptr : dTileMap;
+        sp.tile_map = cfg.tta ? nullptr : fc.tileMap.get<int>();
         sp.y_begin = yBegin; sp.y_end = yEnd;
         sp.bgra = pixelBytes == 4 ? 1 : 0;
         sp.alpha_off = passes == 2 ? grid.count : 0;   // TTA: index of the reduced alpha tile; else the alpha step of the tile's slot
@@ -1054,37 +995,33 @@ void Engine::renderOnStream(const uint8_t* dSrc, int w, int h, size_t srcPitch, 
     const bool frameWide = frameWideUnpack();
     if (frameWide)
         span(0, [&] {
-            unpackTiles(dSrc, w, h, srcPitch, dSlots, realSteps, dUnpacked, s, pixelBytes);
+            unpackTiles(dSrc, w, h, srcPitch, fc.slots.get<TileSlot>(), realSteps, fc.unpacked.get(), s, pixelBytes);
             ++launches;
         });
-    for (int b = 0; b < batchCount; ++b) {
+    for (int b = 0; b < fc.batchCount; ++b) {
         const auto t0 = std::chrono::steady_clock::now();
         const int nReal = std::min(batch, realSteps - b * batch);
         if (nReal <= 0) continue;
         if (!frameWide)
             span(0, [&] {
-                unpackTiles(dSrc, w, h, srcPitch, dSlots + (size_t)b * batch, nReal, actIn.p, s, pixelBytes);
+                unpackTiles(dSrc, w, h, srcPitch, fc.slots.get<TileSlot>() + (size_t)b * batch, nReal, actIn.p, s, pixelBytes);
                 ++launches;
             });
-        span(1, [&] { runModel(s, elemAt(dTileOut, (size_t)b * batch * tileElems), nReal, frameWide ? elemAt(dUnpacked, (size_t)b * batch * inElems) : nullptr); });
+        span(1, [&] { runModel(s, elemAt(fc.tileOut.get(), (size_t)b * batch * tileElems), nReal, frameWide ? elemAt(fc.unpacked.get(), (size_t)b * batch * inElems) : nullptr); });
         if (progressive) {
             // output rows that only depend on tile rows finished with this batch: stitch them now, hand the caller an event to copy after
-            for (const RowBand& rb : rowBands) {
+            for (const RowBand& rb : fc.rowBands) {
                 if (rb.batch != b) continue;
                 span(2, [&] { stitchRows(rb.y0, rb.y1); });
-                if (bandEv.size() <= bands->size()) {
-                    cudaEvent_t e;
-                    W2X_CUDA(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
-                    bandEv.push_back(e);
-                }
-                cudaEvent_t e = bandEv[bands->size()];
+                if (fc.bandEv.size() <= bands->size()) fc.bandEv.emplace_back(cudaEventDisableTiming);
+                cudaEvent_t e = fc.bandEv[bands->size()].get();
                 W2X_CUDA(cudaEventRecord(e, s));
                 bands->push_back({rb.y0, rb.y1, e});
             }
         }
         if (progCb) {
             const double ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
-            progCb(b + 1, batchCount, 1000.0 / std::max(ms, 1e-6), progUser);  // render.cpp:336-338
+            progCb(b + 1, fc.batchCount, 1000.0 / std::max(ms, 1e-6), progUser);  // render.cpp:336-338
         }
     }
     if (progressive) {
@@ -1093,7 +1030,7 @@ void Engine::renderOnStream(const uint8_t* dSrc, int w, int h, size_t srcPitch, 
     }
     if (cfg.tta)
         span(4, [&] {
-            ttaReduce(dTileOut, grid.count * passes, dTtaMean, s);
+            ttaReduce(fc.tileOut.get(), grid.count * passes, fc.ttaMean.get<float>(), s);
             ++launches;
         });
     span(2, [&] { stitchRows(0, h * scale); });
@@ -1114,13 +1051,15 @@ int Engine::lastStageMs(float* out, int n) {
     if (!stream) return 0;
     cudaStreamSynchronize(stream);
     float acc[5] = {0, 0, 0, 0, 0};  // unpack, model, stitch, total, tta_reduce
+    auto& pool = timing.pool;
+    const auto& spans = timing.spans;
     for (const auto& sp : spans) {
         float ms = 0;
-        if (cudaEventElapsedTime(&ms, evPool[sp.e0], evPool[sp.e1]) == cudaSuccess) acc[sp.kind] += ms;
+        if (cudaEventElapsedTime(&ms, pool[sp.e0].get(), pool[sp.e1].get()) == cudaSuccess) acc[sp.kind] += ms;
     }
     if (!spans.empty()) {
         float ms = 0;
-        if (cudaEventElapsedTime(&ms, evPool[spans.front().e0], evPool[spans.back().e1]) == cudaSuccess) acc[3] = ms;
+        if (cudaEventElapsedTime(&ms, pool[spans.front().e0].get(), pool[spans.back().e1].get()) == cudaSuccess) acc[3] = ms;
     }
     const int k = std::min(n, 5);
     for (int i = 0; i < k; ++i) out[i] = acc[i];
@@ -1130,16 +1069,20 @@ int Engine::lastStageMs(float* out, int n) {
 bool Engine::timerMark(int idx, int which) {
     if (idx < 0 || idx >= 16 || !stream) return false;
     if (cudaSetDevice(cfg.deviceId) != cudaSuccess) return false;
-    if (!timerEv[idx] && cudaEventCreate(&timerEv[idx]) != cudaSuccess) return false;
     cudaStream_t s = which == 1 ? h2dStream : which == 2 ? d2hStream : stream;
-    return cudaEventRecord(timerEv[idx], s) == cudaSuccess;
+    try {
+        return cudaEventRecord(timing.marks[idx].get(), s) == cudaSuccess;
+    } catch (const Error&) {
+        return false;
+    }
 }
 
 float Engine::timerElapsedMs(int i0, int i1) {
-    if (i0 < 0 || i1 < 0 || i0 >= 16 || i1 >= 16 || !timerEv[i0] || !timerEv[i1]) return -1.f;
-    if (cudaEventSynchronize(timerEv[i0]) != cudaSuccess || cudaEventSynchronize(timerEv[i1]) != cudaSuccess) return -1.f;
+    if (i0 < 0 || i1 < 0 || i0 >= 16 || i1 >= 16 || !timing.marks[i0].created() || !timing.marks[i1].created()) return -1.f;
+    cudaEvent_t e0 = timing.marks[i0].get(), e1 = timing.marks[i1].get();
+    if (cudaEventSynchronize(e0) != cudaSuccess || cudaEventSynchronize(e1) != cudaSuccess) return -1.f;
     float ms = -1.f;
-    if (cudaEventElapsedTime(&ms, timerEv[i0], timerEv[i1]) != cudaSuccess) return -1.f;
+    if (cudaEventElapsedTime(&ms, e0, e1) != cudaSuccess) return -1.f;
     return ms;
 }
 
@@ -1158,36 +1101,7 @@ bool Engine::renderDevice(const uint8_t* dSrc, int w, int h, size_t srcStride, u
 bool Engine::render(const uint8_t* src, int w, int h, size_t srcStride, uint8_t* dst, size_t dstStride) {
     try {
         if (!isLoaded) throw Error("no engine loaded");
-        W2X_CUDA(cudaSetDevice(cfg.deviceId));
-        const size_t inBytes = (size_t)w * 3 * h, outBytes = (size_t)w * scale * 3 * h * scale;
-        if (inBytes > frameInCap) {
-            if (dFrameIn) cudaFree(dFrameIn);
-            W2X_CUDA(cudaMalloc(&dFrameIn, inBytes));
-            frameInCap = inBytes;
-        }
-        if (outBytes > frameOutCap) {
-            if (dFrameOut) cudaFree(dFrameOut);
-            W2X_CUDA(cudaMalloc(&dFrameOut, outBytes));
-            frameOutCap = outBytes;
-        }
-        W2X_CUDA(cudaMemcpy2DAsync(dFrameIn, (size_t)w * 3, src, srcStride, (size_t)w * 3, h, cudaMemcpyHostToDevice, stream));  // render.cpp:226
-        // every kernel of the frame is queued first; the output then leaves band by band (rows that are final after a tile row), each copy
-        // ordered behind its band's stitch only, so the download of a band overlaps the batches still computing (the reference downloads
-        // the whole canvas after the last batch, render.cpp:344).  With --tta there is one band: the whole frame after the reduce.
-        std::vector<BandDone> bands;
-        const size_t opitch = (size_t)w * scale * 3;
-        renderOnStream(dFrameIn, w, h, (size_t)w * 3, dFrameOut, opitch, stream, true, &bands);
-        if (bands.empty()) {
-            W2X_CUDA(cudaMemcpy2DAsync(dst, dstStride, dFrameOut, opitch, opitch, (size_t)h * scale, cudaMemcpyDeviceToHost, stream));  // render.cpp:344
-        } else {
-            for (const BandDone& bd : bands) {
-                W2X_CUDA(cudaStreamWaitEvent(d2hStream, bd.ev, 0));
-                W2X_CUDA(cudaMemcpy2DAsync(dst + (size_t)bd.y0 * dstStride, dstStride, dFrameOut + (size_t)bd.y0 * opitch, opitch, opitch, (size_t)(bd.y1 - bd.y0),
-                                           cudaMemcpyDeviceToHost, d2hStream));
-            }
-            W2X_CUDA(cudaStreamSynchronize(d2hStream));
-        }
-        W2X_CUDA(cudaStreamSynchronize(stream));  // the sync the reference leaves commented out (render.cpp:345)
+        renderHostFrame(src, w, h, srcStride, dst, dstStride, 3);
         return true;
     } catch (const std::exception& ex) {
         ELOG(W2X_ERROR, std::string("Render failed unexpectedly: ") + ex.what() + ".");
@@ -1201,32 +1115,37 @@ bool Engine::renderBgra(const uint8_t* src, int w, int h, size_t srcStride, uint
         if (!src || !dst) throw Error("null image pointer");
         if (w <= 0 || h <= 0) throw Error("invalid frame size");
         if (srcStride < (size_t)w * 4 || dstStride < (size_t)w * scale * 4) throw Error("row stride is smaller than 4 bytes per pixel");
-        W2X_CUDA(cudaSetDevice(cfg.deviceId));
-        const size_t ipitch = (size_t)w * 4, opitch = (size_t)w * scale * 4;
-        const size_t inBytes = ipitch * h, outBytes = opitch * h * scale;
-        if (inBytes > frameInCap) {
-            if (dFrameIn) cudaFree(dFrameIn);
-            dFrameIn = nullptr;
-            frameInCap = 0;
-            W2X_CUDA(cudaMalloc(&dFrameIn, inBytes));
-            frameInCap = inBytes;
-        }
-        if (outBytes > frameOutCap) {
-            if (dFrameOut) cudaFree(dFrameOut);
-            dFrameOut = nullptr;
-            frameOutCap = 0;
-            W2X_CUDA(cudaMalloc(&dFrameOut, outBytes));
-            frameOutCap = outBytes;
-        }
-        W2X_CUDA(cudaMemcpy2DAsync(dFrameIn, ipitch, src, srcStride, ipitch, h, cudaMemcpyHostToDevice, stream));
-        renderOnStream(dFrameIn, w, h, ipitch, dFrameOut, opitch, stream, true, nullptr, 4);
-        W2X_CUDA(cudaMemcpy2DAsync(dst, dstStride, dFrameOut, opitch, opitch, (size_t)h * scale, cudaMemcpyDeviceToHost, stream));
-        W2X_CUDA(cudaStreamSynchronize(stream));
+        renderHostFrame(src, w, h, srcStride, dst, dstStride, 4);
         return true;
     } catch (const std::exception& ex) {
         ELOG(W2X_ERROR, std::string("Render failed unexpectedly: ") + ex.what() + ".");
         return false;
     }
+}
+
+void Engine::renderHostFrame(const uint8_t* src, int w, int h, size_t srcStride, uint8_t* dst, size_t dstStride, int pixelBytes) {
+    W2X_CUDA(cudaSetDevice(cfg.deviceId));
+    const size_t ipitch = (size_t)w * pixelBytes, opitch = (size_t)w * scale * pixelBytes;
+    staging.in.ensure(ipitch * h);
+    staging.out.ensure(opitch * h * scale);
+    uint8_t *dIn = staging.in.get<uint8_t>(), *dOut = staging.out.get<uint8_t>();
+    W2X_CUDA(cudaMemcpy2DAsync(dIn, ipitch, src, srcStride, ipitch, h, cudaMemcpyHostToDevice, stream));  // render.cpp:226
+    // every kernel of the frame is queued first; the output then leaves band by band (rows that are final after a tile row), each copy
+    // ordered behind its band's stitch only, so the download of a band overlaps the batches still computing (the reference downloads
+    // the whole canvas after the last batch, render.cpp:344).  With --tta, and for BGRA frames, there is one band: the whole frame.
+    std::vector<BandDone> bands;
+    renderOnStream(dIn, w, h, ipitch, dOut, opitch, stream, true, &bands, pixelBytes);
+    if (bands.empty()) {
+        W2X_CUDA(cudaMemcpy2DAsync(dst, dstStride, dOut, opitch, opitch, (size_t)h * scale, cudaMemcpyDeviceToHost, stream));  // render.cpp:344
+    } else {
+        for (const BandDone& bd : bands) {
+            W2X_CUDA(cudaStreamWaitEvent(d2hStream, bd.ev, 0));
+            W2X_CUDA(cudaMemcpy2DAsync(dst + (size_t)bd.y0 * dstStride, dstStride, dOut + (size_t)bd.y0 * opitch, opitch, opitch, (size_t)(bd.y1 - bd.y0),
+                                       cudaMemcpyDeviceToHost, d2hStream));
+        }
+        W2X_CUDA(cudaStreamSynchronize(d2hStream));
+    }
+    W2X_CUDA(cudaStreamSynchronize(stream));  // the sync the reference leaves commented out (render.cpp:345)
 }
 
 // Pipelined frames: H2D (copy stream) -> compute (engine stream) -> D2H (copy stream), kSlots frames in flight.
@@ -1236,33 +1155,20 @@ int Engine::submit(const uint8_t* src, int w, int h, size_t srcStride, uint8_t* 
         W2X_CUDA(cudaSetDevice(cfg.deviceId));
         const int ticket = nextTicket;
         PipeSlot& ps = pipe[ticket % kSlots];
-        if (!ps.evH2D) {
-            W2X_CUDA(cudaEventCreateWithFlags(&ps.evH2D, cudaEventDisableTiming));
-            W2X_CUDA(cudaEventCreateWithFlags(&ps.evComp, cudaEventDisableTiming));
-            W2X_CUDA(cudaEventCreateWithFlags(&ps.evDone, cudaEventDisableTiming));
-        }
-        if (ps.busy) { W2X_CUDA(cudaEventSynchronize(ps.evDone)); ps.busy = false; }
-        const size_t inBytes = (size_t)w * 3 * h, outBytes = (size_t)w * scale * 3 * h * scale;
-        if (inBytes > ps.inCap) {
-            if (ps.dIn) cudaFree(ps.dIn);
-            W2X_CUDA(cudaMalloc(&ps.dIn, inBytes));
-            ps.inCap = inBytes;
-        }
-        if (outBytes > ps.outCap) {
-            if (ps.dOut) cudaFree(ps.dOut);
-            W2X_CUDA(cudaMalloc(&ps.dOut, outBytes));
-            ps.outCap = outBytes;
-        }
+        if (ps.busy) { W2X_CUDA(cudaEventSynchronize(ps.evDone.get())); ps.busy = false; }
+        ps.in.ensure((size_t)w * 3 * h);
+        ps.out.ensure((size_t)w * scale * 3 * h * scale);
+        uint8_t *dIn = ps.in.get<uint8_t>(), *dOut = ps.out.get<uint8_t>();
         ensureFrameBuffers(w, h);
-        W2X_CUDA(cudaMemcpy2DAsync(ps.dIn, (size_t)w * 3, src, srcStride, (size_t)w * 3, h, cudaMemcpyHostToDevice, h2dStream));
-        W2X_CUDA(cudaEventRecord(ps.evH2D, h2dStream));
-        W2X_CUDA(cudaStreamWaitEvent(stream, ps.evH2D, 0));
-        renderOnStream(ps.dIn, w, h, (size_t)w * 3, ps.dOut, (size_t)w * scale * 3, stream, false);
-        W2X_CUDA(cudaEventRecord(ps.evComp, stream));
-        W2X_CUDA(cudaStreamWaitEvent(d2hStream, ps.evComp, 0));
-        W2X_CUDA(cudaMemcpy2DAsync(dst, dstStride, ps.dOut, (size_t)w * scale * 3, (size_t)w * scale * 3, (size_t)h * scale,
+        W2X_CUDA(cudaMemcpy2DAsync(dIn, (size_t)w * 3, src, srcStride, (size_t)w * 3, h, cudaMemcpyHostToDevice, h2dStream));
+        W2X_CUDA(cudaEventRecord(ps.evH2D.get(), h2dStream));
+        W2X_CUDA(cudaStreamWaitEvent(stream, ps.evH2D.get(), 0));
+        renderOnStream(dIn, w, h, (size_t)w * 3, dOut, (size_t)w * scale * 3, stream, false);
+        W2X_CUDA(cudaEventRecord(ps.evComp.get(), stream));
+        W2X_CUDA(cudaStreamWaitEvent(d2hStream, ps.evComp.get(), 0));
+        W2X_CUDA(cudaMemcpy2DAsync(dst, dstStride, dOut, (size_t)w * scale * 3, (size_t)w * scale * 3, (size_t)h * scale,
                                    cudaMemcpyDeviceToHost, d2hStream));
-        W2X_CUDA(cudaEventRecord(ps.evDone, d2hStream));
+        W2X_CUDA(cudaEventRecord(ps.evDone.get(), d2hStream));
         ps.busy = true;
         ++nextTicket;
         return ticket;
@@ -1318,13 +1224,6 @@ bool Engine::renderBanded(Engine* const* es, int count, const uint8_t* src, int 
             bd[r].inY1 = std::min(h, g.inRects[bd[r].j1 - 1].y + tile);
             if (bd[r].inY1 <= bd[r].inY0) { bd[r].inY0 = std::min(std::max(bd[r].inY0, 0), h - 1); bd[r].inY1 = bd[r].inY0 + 1; }
         }
-        auto grow = [](auto*& p, size_t& cap, size_t need, size_t elem) {
-            if (need <= cap) return;
-            if (p) cudaFree(p);
-            p = nullptr;
-            W2X_CUDA(cudaMalloc((void**)&p, need * elem));
-            cap = need;
-        };
         // ---- phase 1: every band uploads its rows, unpacks and runs the model on its tiles; nothing here waits for a device ----
         for (int r = 0; r < bands; ++r) {
             Engine& e = *es[r];
@@ -1332,51 +1231,52 @@ bool Engine::renderBanded(Engine* const* es, int count, const uint8_t* src, int 
             W2X_CUDA(cudaSetDevice(e.cfg.deviceId));
             e.ensureFrameBuffers(w, h);  // blend ramps for this frame size
             const int bandH = b.inY1 - b.inY0;
-            grow(e.dFrameIn, e.frameInCap, (size_t)w * 3 * bandH, 1);
-            grow(e.dFrameOut, e.frameOutCap, (size_t)cw * 3 * (size_t)(b.yEnd - b.yBegin), 1);
-            grow(e.dBandTiles, e.bandTilesCap, (size_t)b.steps * tileElems + (tta ? 0 : (size_t)g.nx * tileElems), e.elemBytes);
-            if (tta) grow(e.dBandMean, e.bandMeanCap, (size_t)(b.own + g.nx) * tileElems, sizeof(float));
-            grow(e.dBandMap, e.bandMapCap, (size_t)g.count, sizeof(int));
-            grow(e.dBandSlots, e.bandSlotCap, (size_t)b.steps, sizeof(TileSlot));
-            if (!e.evBandModel) W2X_CUDA(cudaEventCreateWithFlags(&e.evBandModel, cudaEventDisableTiming));
+            e.staging.in.ensure((size_t)w * 3 * bandH);
+            e.staging.out.ensure((size_t)cw * 3 * (size_t)(b.yEnd - b.yBegin));
+            e.band.tiles.ensure(((size_t)b.steps * tileElems + (tta ? 0 : (size_t)g.nx * tileElems)) * e.elemBytes);
+            if (tta) e.band.mean.ensure((size_t)(b.own + g.nx) * tileElems * sizeof(float));
+            e.band.map.ensure((size_t)g.count * sizeof(int));
+            e.band.slots.ensure((size_t)b.steps * sizeof(TileSlot));
+            uint8_t* dIn = e.staging.in.get<uint8_t>();
+            TileSlot* dSlots = e.band.slots.get<TileSlot>();
             // model runs in row-major band order (a tile row is contiguous for the seam copy), eight consecutive augmentations per
             // tile with --tta; map: global tile index -> slot of the stitched tile buffer.  The staging vectors live in the engine
             // so that the asynchronous copies below never outlive them.
-            e.bandSlotsHost.assign((size_t)b.steps, TileSlot{0, 0, 0, 0});
-            e.bandMapHost.assign((size_t)g.count, -1);
+            e.band.slotsHost.assign((size_t)b.steps, TileSlot{0, 0, 0, 0});
+            e.band.mapHost.assign((size_t)g.count, -1);
             for (int j = b.j0; j < b.j1; ++j)
                 for (int i = 0; i < g.nx; ++i) {
                     const int s = (j - b.j0) * g.nx + i, t = i * g.ny + j;
-                    for (int a = 0; a < spt; ++a) e.bandSlotsHost[(size_t)s * spt + a] = {g.inRects[t].x, g.inRects[t].y - b.inY0, a, 1};
-                    e.bandMapHost[t] = s;
+                    for (int a = 0; a < spt; ++a) e.band.slotsHost[(size_t)s * spt + a] = {g.inRects[t].x, g.inRects[t].y - b.inY0, a, 1};
+                    e.band.mapHost[t] = s;
                 }
             const int recvSlot = tta ? b.own : b.steps;  // where the seam row received from the band above lands
             if (r > 0)
-                for (int i = 0; i < g.nx; ++i) e.bandMapHost[i * g.ny + b.j0 - 1] = recvSlot + i;
-            W2X_CUDA(cudaMemcpyAsync(e.dBandSlots, e.bandSlotsHost.data(), sizeof(TileSlot) * e.bandSlotsHost.size(), cudaMemcpyHostToDevice, e.stream));
-            W2X_CUDA(cudaMemcpyAsync(e.dBandMap, e.bandMapHost.data(), sizeof(int) * e.bandMapHost.size(), cudaMemcpyHostToDevice, e.stream));
-            W2X_CUDA(cudaMemcpy2DAsync(e.dFrameIn, (size_t)w * 3, src + (size_t)b.inY0 * srcStride, srcStride, (size_t)w * 3, bandH, cudaMemcpyHostToDevice, e.stream));
+                for (int i = 0; i < g.nx; ++i) e.band.mapHost[i * g.ny + b.j0 - 1] = recvSlot + i;
+            W2X_CUDA(cudaMemcpyAsync(dSlots, e.band.slotsHost.data(), sizeof(TileSlot) * e.band.slotsHost.size(), cudaMemcpyHostToDevice, e.stream));
+            W2X_CUDA(cudaMemcpyAsync(e.band.map.get(), e.band.mapHost.data(), sizeof(int) * e.band.mapHost.size(), cudaMemcpyHostToDevice, e.stream));
+            W2X_CUDA(cudaMemcpy2DAsync(dIn, (size_t)w * 3, src + (size_t)b.inY0 * srcStride, srcStride, (size_t)w * 3, bandH, cudaMemcpyHostToDevice, e.stream));
             const int realSteps = b.own * spt;
             for (int bi = 0; bi < b.steps / batch; ++bi) {
                 const int nReal = std::min(batch, realSteps - bi * batch);
                 if (nReal <= 0) break;
-                e.unpackTiles(e.dFrameIn, w, bandH, (size_t)w * 3, e.dBandSlots + (size_t)bi * batch, nReal, e.actIn.p, e.stream);
+                e.unpackTiles(dIn, w, bandH, (size_t)w * 3, dSlots + (size_t)bi * batch, nReal, e.actIn.p, e.stream);
                 ++e.launches;
                 W2X_CUDA(cudaGetLastError());
-                e.runModel(e.stream, e.elemAt(e.dBandTiles, (size_t)bi * batch * tileElems), nReal);
+                e.runModel(e.stream, e.elemAt(e.band.tiles.get(), (size_t)bi * batch * tileElems), nReal);
             }
             if (tta) {
-                e.ttaReduce(e.dBandTiles, b.own, e.dBandMean, e.stream);
+                e.ttaReduce(e.band.tiles.get(), b.own, e.band.mean.get<float>(), e.stream);
                 ++e.launches;
             }
-            W2X_CUDA(cudaEventRecord(e.evBandModel, e.stream));
+            W2X_CUDA(cudaEventRecord(e.band.evModel.get(), e.stream));
         }
         // ---- phase 2: seam exchange (bottom overlap rows of band r-1's last tile row -> band r), stitch own rows, download ----
         for (int r = 0; r < bands; ++r) {
             Engine& e = *es[r];
             const Band& b = bd[r];
             W2X_CUDA(cudaSetDevice(e.cfg.deviceId));
-            uint8_t* tilesBase = tta ? reinterpret_cast<uint8_t*>(e.dBandMean) : reinterpret_cast<uint8_t*>(e.dBandTiles);
+            uint8_t* tilesBase = (tta ? e.band.mean : e.band.tiles).get<uint8_t>();
             if (r > 0 && g.outOvY > 0) {
                 Engine& up = *es[r - 1];
                 if (up.cfg.deviceId != e.cfg.deviceId) {
@@ -1387,8 +1287,8 @@ bool Engine::renderBanded(Engine* const* es, int count, const uint8_t* src, int 
                         (void)cudaGetLastError();
                     }
                 }
-                W2X_CUDA(cudaStreamWaitEvent(e.stream, up.evBandModel, 0));
-                const uint8_t* upBase = tta ? reinterpret_cast<const uint8_t*>(up.dBandMean) : reinterpret_cast<const uint8_t*>(up.dBandTiles);
+                W2X_CUDA(cudaStreamWaitEvent(e.stream, up.band.evModel.get(), 0));
+                const uint8_t* upBase = (tta ? up.band.mean : up.band.tiles).get<const uint8_t>();
                 const size_t tileBytes = tileElems * elemBytes;
                 const size_t rowOff = (size_t)(outT - g.outOvY) * outT * 4 * elemBytes;      // first blended row inside a tile
                 const size_t stripBytes = (size_t)g.outOvY * outT * 4 * elemBytes;           // the overlap rows of one tile: contiguous
@@ -1397,17 +1297,17 @@ bool Engine::renderBanded(Engine* const* es, int count, const uint8_t* src, int 
                 W2X_CUDA(cudaMemcpy2DAsync(dstRow, tileBytes, srcRow, tileBytes, stripBytes, (size_t)g.nx, cudaMemcpyDefault, e.stream));
             }
             StitchParams sp{};
-            sp.tiles = tilesBase; sp.f32 = elemBytes == 4 ? 1 : 0; sp.tile_map = e.dBandMap;
+            sp.tiles = tilesBase; sp.f32 = elemBytes == 4 ? 1 : 0; sp.tile_map = e.band.map.get<int>();
             sp.outT = outT; sp.nx = g.nx; sp.ny = g.ny; sp.ovx = g.outOvX; sp.ovy = g.outOvY;
-            sp.cw = cw; sp.ch = ch; sp.rampx = e.dRampX; sp.rampy = e.dRampY;
+            sp.cw = cw; sp.ch = ch; sp.rampx = e.fc.rampX.get<float>(); sp.rampy = e.fc.rampY.get<float>();
             // the band's output rows land at the top of its (band-sized) output buffer
-            sp.dst = e.dFrameOut - (size_t)b.yBegin * cw * 3; sp.pitch = (size_t)cw * 3;
+            sp.dst = e.staging.out.get<uint8_t>() - (size_t)b.yBegin * cw * 3; sp.pitch = (size_t)cw * 3;
             sp.y_begin = b.yBegin; sp.y_end = b.yEnd;
             launchStitch(sp, e.stream);
             ++e.launches;
             const size_t rows = (size_t)(b.yEnd - b.yBegin);
             if (rows)
-                W2X_CUDA(cudaMemcpy2DAsync(dst + (size_t)b.yBegin * dstStride, dstStride, e.dFrameOut, (size_t)cw * 3, (size_t)cw * 3, rows,
+                W2X_CUDA(cudaMemcpy2DAsync(dst + (size_t)b.yBegin * dstStride, dstStride, e.staging.out.get(), (size_t)cw * 3, (size_t)cw * 3, rows,
                                            cudaMemcpyDeviceToHost, e.stream));
         }
         for (int r = 0; r < bands; ++r) {
@@ -1426,7 +1326,7 @@ bool Engine::wait(int ticket) {
         if (ticket < 0 || ticket >= nextTicket) throw Error("invalid ticket");
         if (nextTicket - ticket > kSlots) return true;  // slot already recycled => that frame completed
         PipeSlot& ps = pipe[ticket % kSlots];
-        if (ps.busy) { W2X_CUDA(cudaEventSynchronize(ps.evDone)); ps.busy = false; }
+        if (ps.busy) { W2X_CUDA(cudaEventSynchronize(ps.evDone.get())); ps.busy = false; }
         return true;
     } catch (const std::exception& ex) {
         ELOG(W2X_ERROR, std::string("Wait failed: ") + ex.what() + ".");
@@ -1457,27 +1357,19 @@ bool Engine::infer(const float* inNchw, int n, float* outNchw) {
         }
         W2X_CUDA(cudaSetDevice(cfg.deviceId));
         const size_t inElems = (size_t)n * 3 * tile * tile, outElems = (size_t)n * 3 * outTile * outTile;
-        float *dIn = nullptr, *dOut = nullptr;
-        void* dOutH = nullptr;  // model output, engine elements
-        W2X_CUDA(cudaMalloc(&dIn, inElems * 4));
-        W2X_CUDA(cudaMalloc(&dOut, outElems * 4));
-        W2X_CUDA(cudaMalloc(&dOutH, (size_t)batch * outTile * outTile * 4 * elemBytes));
-        try {
-            W2X_CUDA(cudaMemcpyAsync(dIn, inNchw, inElems * 4, cudaMemcpyHostToDevice, stream));
-            W2X_CUDA(cudaMemsetAsync(actIn.p, 0, actIn.elems() * elemBytes, stream));
-            if (tf32()) launchNchwToNhwc4(dIn, n, tile, reinterpret_cast<float*>(actIn.p), stream);
-            else launchNchwToNhwc4(dIn, n, tile, actIn.p, stream);
-            runModel(stream, dOutH, n);
-            if (tf32()) launchNhwc4ToNchw(static_cast<const float*>(dOutH), n, outTile, dOut, stream);
-            else launchNhwc4ToNchw(static_cast<const __half*>(dOutH), n, outTile, dOut, stream);
-            launches += 2;
-            W2X_CUDA(cudaMemcpyAsync(outNchw, dOut, outElems * 4, cudaMemcpyDeviceToHost, stream));
-            W2X_CUDA(cudaStreamSynchronize(stream));
-        } catch (...) {
-            cudaFree(dIn); cudaFree(dOut); cudaFree(dOutH);
-            throw;
-        }
-        cudaFree(dIn); cudaFree(dOut); cudaFree(dOutH);
+        DeviceBuffer in(inElems * 4), out(outElems * 4);
+        DeviceBuffer outH((size_t)batch * outTile * outTile * 4 * elemBytes);  // model output, engine elements
+        float *dIn = in.get<float>(), *dOut = out.get<float>();
+        W2X_CUDA(cudaMemcpyAsync(dIn, inNchw, inElems * 4, cudaMemcpyHostToDevice, stream));
+        W2X_CUDA(cudaMemsetAsync(actIn.p, 0, actIn.elems() * elemBytes, stream));
+        if (tf32()) launchNchwToNhwc4(dIn, n, tile, reinterpret_cast<float*>(actIn.p), stream);
+        else launchNchwToNhwc4(dIn, n, tile, actIn.p, stream);
+        runModel(stream, outH.get(), n);
+        if (tf32()) launchNhwc4ToNchw(outH.get<const float>(), n, outTile, dOut, stream);
+        else launchNhwc4ToNchw(outH.get<const __half>(), n, outTile, dOut, stream);
+        launches += 2;
+        W2X_CUDA(cudaMemcpyAsync(outNchw, dOut, outElems * 4, cudaMemcpyDeviceToHost, stream));
+        W2X_CUDA(cudaStreamSynchronize(stream));
         return true;
     } catch (const std::exception& ex) {
         ELOG(W2X_ERROR, std::string("Engine inference failed unexpectedly: ") + ex.what() + ".");
@@ -1489,9 +1381,8 @@ int Engine::profileLayers(int repeats, char (*names)[48], float* ms, double* flo
     try {
         if (!isLoaded) throw Error("no engine loaded");
         W2X_CUDA(cudaSetDevice(cfg.deviceId));
-        cudaEvent_t e0, e1;
-        W2X_CUDA(cudaEventCreate(&e0));
-        W2X_CUDA(cudaEventCreate(&e1));
+        CudaEvent ev0, ev1;
+        cudaEvent_t e0 = ev0.get(), e1 = ev1.get();
         runModel(stream, nullptr);  // warm-up, and populates every activation
         W2X_CUDA(cudaStreamSynchronize(stream));
         int i = 0;
@@ -1517,8 +1408,6 @@ int Engine::profileLayers(int repeats, char (*names)[48], float* ms, double* flo
             flops[i] = L.flops * batch;
             ++i;
         }
-        cudaEventDestroy(e0);
-        cudaEventDestroy(e1);
         return i;
     } catch (const std::exception& ex) {
         ELOG(W2X_ERROR, std::string("Profile failed: ") + ex.what() + ".");
@@ -1541,105 +1430,69 @@ static void convLayerGeometry(int kind, int n, int h, int w, int cin, int cout, 
     else throw Error("bad kind");
 }
 
+// The layer of `kind` on device copies of the host tensors, whose elements are `elemBytes` wide: fp16, or fp32 for the tf32 kernel (the
+// ConvParams builders take the nominal fp16 pointer type of the engine's plan, see Act).  `bufs` owns the device memory; `out` is the
+// zeroed output tensor.
+static ConvParams uploadConvLayer(int kind, int n, int h, int w, int cin, int cout, size_t elemBytes, const void* in, const void* wPacked,
+                                  const float* bias, const void* skipData, const void* outData, std::vector<DeviceBuffer>& bufs, Act& out) {
+    int npad = 0, ktot = 0;
+    Act skip{};
+    convLayerGeometry(kind, n, h, w, cin, cout, npad, ktot, out, skip);
+    if (!in || !wPacked || !bias || !outData || (skip.n && !skipData)) throw Error("null argument");
+    auto dmal = [&](size_t bytes) { bufs.emplace_back(bytes + 256); return bufs.back().get(); };
+    auto up = [&](const void* src, size_t bytes) { void* d = dmal(bytes); W2X_CUDA(cudaMemcpy(d, src, bytes, cudaMemcpyHostToDevice)); return d; };
+    Act inA{nullptr, n, h, w, cin};
+    inA.p = (__half*)up(in, inA.elems() * elemBytes);
+    const __half* dWt = (const __half*)up(wPacked, (size_t)npad * ktot * elemBytes);
+    const float* dB = (const float*)up(bias, (size_t)npad * 4);
+    if (skip.n) skip.p = (__half*)up(skipData, skip.elems() * elemBytes);
+    out.p = (__half*)dmal(out.elems() * elemBytes);
+    W2X_CUDA(cudaMemset(out.p, 0, out.elems() * elemBytes));
+    if (kind == 0) return makeConv3Params(inA, out, dWt, dB, npad, EPI_STORE, 0.1f, cout);
+    if (kind == 1) return makeDown2Params(inA, out, dWt, dB, npad, 0.1f);
+    if (kind == 2) return makeUp2Params(inA, out, dWt, dB, cout, 0.1f, &skip, 4);
+    if (kind == 3) return makeUp4Params(inA, out, dWt, dB);
+    ConvParams p = makeConv3Params(inA, out, dWt, dB, npad, EPI_FINAL, 1.f, 4);
+    p.skip = skip.p; p.skip_h = skip.h; p.skip_w = skip.w; p.skip_c = 4; p.skip_off = 20;
+    return p;
+}
+
 void runConvLayer(int device, int kind, int impl, int n, int h, int w, int cin, int cout, const uint16_t* in, const uint16_t* wPacked,
                   const float* bias, const uint16_t* skipData, uint16_t* outData) {
     W2X_CUDA(cudaSetDevice(device));
-    std::vector<void*> bufs;
-    IgemmPlan* plan = nullptr;
-    HeadPlan* hp = nullptr;
-    auto cleanup = [&] {
-        if (plan) igemmDestroyPlan(plan);
-        if (hp) convHeadDestroyPlan(hp);
-        for (void* b : bufs) cudaFree(b);
-    };
-    try {
-        auto dmal = [&](size_t bytes) { void* p = nullptr; W2X_CUDA(cudaMalloc(&p, bytes + 256)); bufs.push_back(p); return p; };
-        auto up = [&](const void* src, size_t bytes) { void* d = dmal(bytes); W2X_CUDA(cudaMemcpy(d, src, bytes, cudaMemcpyHostToDevice)); return d; };
-        int npad = 0, ktot = 0;
-        Act out{}, skip{};
-        convLayerGeometry(kind, n, h, w, cin, cout, npad, ktot, out, skip);
-        if (!in || !wPacked || !bias || !outData || (skip.n && !skipData)) throw Error("null argument");
-        Act inA{nullptr, n, h, w, cin};
-        inA.p = (__half*)up(in, inA.elems() * 2);
-        __half* dWt = (__half*)up(wPacked, (size_t)npad * ktot * 2);
-        float* dB = (float*)up(bias, (size_t)npad * 4);
-        if (skip.n) skip.p = (__half*)up(skipData, skip.elems() * 2);
-        out.p = (__half*)dmal(out.elems() * 2);
-        W2X_CUDA(cudaMemset(out.p, 0, out.elems() * 2));
-        ConvParams p{};
-        if (kind == 0) p = makeConv3Params(inA, out, dWt, dB, npad, EPI_STORE, 0.1f, cout);
-        else if (kind == 1) p = makeDown2Params(inA, out, dWt, dB, npad, 0.1f);
-        else if (kind == 2) p = makeUp2Params(inA, out, dWt, dB, cout, 0.1f, &skip, 4);
-        else if (kind == 3) p = makeUp4Params(inA, out, dWt, dB);
-        else {
-            p = makeConv3Params(inA, out, dWt, dB, npad, EPI_FINAL, 1.f, 4);
-            p.skip = skip.p; p.skip_h = skip.h; p.skip_w = skip.w; p.skip_c = 4; p.skip_off = 20;
-        }
-        if (impl == 2) {
-            launchConvDirect(p, nullptr);
-        } else if (impl == 1) {
-            if (!convHeadSupported(p)) throw Error("no head kernel for this layer");
-            hp = convHeadCreatePlan(p);
-            launchConvHead(hp, nullptr);
-        } else {
-            plan = igemmCreatePlan(p);
-            // W2X_REPEAT (development build only): back-to-back launches, for steady-state clock / power readings of one layer
-            const int reps = devEnv("W2X_REPEAT") ? std::max(1, std::atoi(devEnv("W2X_REPEAT"))) : 1;
-            for (int r = 0; r < reps; ++r) igemmLaunch(plan, nullptr, nullptr);
-        }
-        W2X_CUDA(cudaDeviceSynchronize());
-        W2X_CUDA(cudaGetLastError());
-        W2X_CUDA(cudaMemcpy(outData, out.p, out.elems() * 2, cudaMemcpyDeviceToHost));
-    } catch (...) {
-        cleanup();
-        throw;
+    std::vector<DeviceBuffer> bufs;
+    Act out{};
+    const ConvParams p = uploadConvLayer(kind, n, h, w, cin, cout, 2, in, wPacked, bias, skipData, outData, bufs, out);
+    std::unique_ptr<IgemmPlan, void (*)(IgemmPlan*)> plan(nullptr, igemmDestroyPlan);
+    std::unique_ptr<HeadPlan, void (*)(HeadPlan*)> hp(nullptr, convHeadDestroyPlan);
+    if (impl == 2) {
+        launchConvDirect(p, nullptr);
+    } else if (impl == 1) {
+        if (!convHeadSupported(p)) throw Error("no head kernel for this layer");
+        hp.reset(convHeadCreatePlan(p));
+        launchConvHead(hp.get(), nullptr);
+    } else {
+        plan.reset(igemmCreatePlan(p));
+        // W2X_REPEAT (development build only): back-to-back launches, for steady-state clock / power readings of one layer
+        const int reps = devEnv("W2X_REPEAT") ? std::max(1, std::atoi(devEnv("W2X_REPEAT"))) : 1;
+        for (int r = 0; r < reps; ++r) igemmLaunch(plan.get(), nullptr, nullptr);
     }
-    cleanup();
+    W2X_CUDA(cudaDeviceSynchronize());
+    W2X_CUDA(cudaGetLastError());
+    W2X_CUDA(cudaMemcpy(outData, out.p, out.elems() * 2, cudaMemcpyDeviceToHost));
 }
 
 void runConvLayerF32(int device, int kind, int n, int h, int w, int cin, int cout, const float* in, const float* wPacked, const float* bias,
                      const float* skipData, float* outData) {
     W2X_CUDA(cudaSetDevice(device));
-    std::vector<void*> bufs;
-    Tf32Plan* plan = nullptr;
-    auto cleanup = [&] {
-        if (plan) tf32DestroyPlan(plan);
-        for (void* b : bufs) cudaFree(b);
-    };
-    try {
-        auto dmal = [&](size_t bytes) { void* p = nullptr; W2X_CUDA(cudaMalloc(&p, bytes + 256)); bufs.push_back(p); return p; };
-        auto up = [&](const void* src, size_t bytes) { void* d = dmal(bytes); W2X_CUDA(cudaMemcpy(d, src, bytes, cudaMemcpyHostToDevice)); return d; };
-        int npad = 0, ktot = 0;
-        Act out{}, skip{};
-        convLayerGeometry(kind, n, h, w, cin, cout, npad, ktot, out, skip);
-        if (!in || !wPacked || !bias || !outData || (skip.n && !skipData)) throw Error("null argument");
-        // the ConvParams builders take the nominal fp16 pointer type of the engine's plan (see Act)
-        Act inA{nullptr, n, h, w, cin};
-        inA.p = (__half*)up(in, inA.elems() * 4);
-        const __half* dWt = (const __half*)up(wPacked, (size_t)npad * ktot * 4);
-        float* dB = (float*)up(bias, (size_t)npad * 4);
-        if (skip.n) skip.p = (__half*)up(skipData, skip.elems() * 4);
-        out.p = (__half*)dmal(out.elems() * 4);
-        W2X_CUDA(cudaMemset(out.p, 0, out.elems() * 4));
-        ConvParams p{};
-        if (kind == 0) p = makeConv3Params(inA, out, dWt, dB, npad, EPI_STORE, 0.1f, cout);
-        else if (kind == 1) p = makeDown2Params(inA, out, dWt, dB, npad, 0.1f);
-        else if (kind == 2) p = makeUp2Params(inA, out, dWt, dB, cout, 0.1f, &skip, 4);
-        else if (kind == 3) p = makeUp4Params(inA, out, dWt, dB);
-        else {
-            p = makeConv3Params(inA, out, dWt, dB, npad, EPI_FINAL, 1.f, 4);
-            p.skip = skip.p; p.skip_h = skip.h; p.skip_w = skip.w; p.skip_c = 4; p.skip_off = 20;
-        }
-        plan = tf32CreatePlan(asF32(p));
-        tf32Launch(plan, nullptr);
-        W2X_CUDA(cudaDeviceSynchronize());
-        W2X_CUDA(cudaGetLastError());
-        W2X_CUDA(cudaMemcpy(outData, out.p, out.elems() * 4, cudaMemcpyDeviceToHost));
-    } catch (...) {
-        cleanup();
-        throw;
-    }
-    cleanup();
+    std::vector<DeviceBuffer> bufs;
+    Act out{};
+    const ConvParams p = uploadConvLayer(kind, n, h, w, cin, cout, 4, in, wPacked, bias, skipData, outData, bufs, out);
+    std::unique_ptr<Tf32Plan, void (*)(Tf32Plan*)> plan(tf32CreatePlan(asF32(p)), tf32DestroyPlan);
+    tf32Launch(plan.get(), nullptr);
+    W2X_CUDA(cudaDeviceSynchronize());
+    W2X_CUDA(cudaGetLastError());
+    W2X_CUDA(cudaMemcpy(outData, out.p, out.elems() * 4, cudaMemcpyDeviceToHost));
 }
 
 // On-device self-check on random data: the tensor-core kernel vs the scalar CUDA-core reference kernel; returns max |diff|.

@@ -4,8 +4,10 @@
 #include <cuda_fp16.h>
 #include <cuda_runtime.h>
 
+#include <array>
 #include <cstring>
 #include <string>
+#include <utility>
 #include <vector>
 
 #include "hostutil.h"
@@ -19,6 +21,72 @@ namespace w2x {
         cudaError_t _e = (expr);                                                                        \
         if (_e != cudaSuccess) throw ::w2x::Error(std::string(#expr) + ": " + cudaGetErrorString(_e)); \
     } while (0)
+
+// Device memory with one owner, freed with it.
+class DeviceBuffer {
+public:
+    DeviceBuffer() = default;
+    explicit DeviceBuffer(size_t bytes) { ensure(bytes); }
+    DeviceBuffer(DeviceBuffer&& o) noexcept : p(std::exchange(o.p, nullptr)), cap(std::exchange(o.cap, 0)) {}
+    DeviceBuffer& operator=(DeviceBuffer&& o) noexcept {
+        if (this != &o) {
+            release();
+            p = std::exchange(o.p, nullptr);
+            cap = std::exchange(o.cap, 0);
+        }
+        return *this;
+    }
+    ~DeviceBuffer() { release(); }
+
+    // At least `bytes`; true when it reallocated (the contents are then undefined).  The old memory is released first, so a failed
+    // allocation leaves the buffer empty rather than a stale capacity over a freed pointer.
+    bool ensure(size_t bytes) {
+        if (bytes <= cap) return false;
+        release();
+        W2X_CUDA(cudaMalloc(&p, bytes));
+        cap = bytes;
+        return true;
+    }
+    template <class T = void> T* get() const { return static_cast<T*>(p); }
+
+private:
+    void release() {
+        if (p) cudaFree(p);
+        p = nullptr;
+        cap = 0;
+    }
+    void* p = nullptr;
+    size_t cap = 0;
+};
+
+// A CUDA event with one owner, created with `flags` on first use and destroyed with it.
+class CudaEvent {
+public:
+    CudaEvent() = default;
+    explicit CudaEvent(unsigned flags) : flags(flags) {}
+    CudaEvent(CudaEvent&& o) noexcept : e(std::exchange(o.e, nullptr)), flags(o.flags) {}
+    CudaEvent& operator=(CudaEvent&& o) noexcept {
+        if (this != &o) {
+            if (e) cudaEventDestroy(e);
+            e = std::exchange(o.e, nullptr);
+            flags = o.flags;
+        }
+        return *this;
+    }
+    ~CudaEvent() {
+        if (e) cudaEventDestroy(e);
+    }
+
+    cudaEvent_t get() {
+        if (!e) W2X_CUDA(cudaEventCreateWithFlags(&e, flags));
+        return e;
+    }
+    bool created() const { return e != nullptr; }
+
+private:
+    cudaEvent_t e = nullptr;
+    unsigned flags = cudaEventDefault;
+};
 
 // Activation tensor NHWC [n][h][w][c].  Its elements are the engine's (Engine::elemBytes): fp16, or fp32 in a tf32 engine, where the
 // pointer (like every activation / weight pointer of the plan and of ConvParams) is nominal and the kernels read it as float (asF32).
@@ -78,6 +146,8 @@ class Engine {
 public:
     Engine();
     ~Engine();
+    Engine(const Engine&) = delete;
+    Engine& operator=(const Engine&) = delete;
 
     bool build(const std::string& onnxPath, const w2x_build_config& cfg);
     bool load(const std::string& onnxPath, const w2x_render_config& cfg);
@@ -132,6 +202,8 @@ private:
     // pixelBytes 4: packed BGRA frames (dSrcPitch = 4w): alpha scan, colour bleed and alpha pass as the frame needs them; no bands
     void renderOnStream(const uint8_t* dSrc, int w, int h, size_t srcPitch, uint8_t* dDst, size_t dstPitch, cudaStream_t s, bool timed,
                         std::vector<BandDone>* bands = nullptr, int pixelBytes = 3);
+    // render / renderBgra: host frame -> staging buffers -> renderOnStream -> host frame, synchronous
+    void renderHostFrame(const uint8_t* src, int w, int h, size_t srcStride, uint8_t* dst, size_t dstStride, int pixelBytes);
     void* dalloc(size_t bytes);
     Act allocAct(int h, int w, int c);
 
@@ -149,7 +221,7 @@ private:
     bool useDirect = false;
     bool debugSync = false;      // W2X_DEBUG_SYNC: synchronise + check after every layer (names the failing kernel)
 
-    std::vector<void*> allocs;       // freed in unload()
+    std::vector<DeviceBuffer> allocs;  // plan lifetime: weights, activations, SE scratch
     std::vector<__half*> dW;         // per layer (engine element type)
     std::vector<float*> dBias;
     std::vector<LayerExec> layers;
@@ -158,59 +230,54 @@ private:
     cudaStream_t stream = nullptr, h2dStream = nullptr, d2hStream = nullptr;
     long long launches = 0;
 
-    // frame-level state
-    int frameW = 0, frameH = 0, framePasses = 1;
-    TileGrid grid;
-    int stepCount = 0, batchCount = 0;
-    TileSlot* dSlots = nullptr;
-    int* dTileMap = nullptr;                     // slot of reference tile ti (row-major processing order without TTA)
-    size_t tileMapCap = 0;
-    std::vector<RowBand> rowBands;
-    std::vector<cudaEvent_t> bandEv;
-    size_t slotCap = 0;
-    void* dUnpacked = nullptr;       // [steps][tile][tile][4] engine elements: every tile of the frame, unpacked by one launch
-    size_t unpackedCap = 0;
-    void* dTileOut = nullptr;        // [steps][outT][outT][4] engine elements
-    size_t tileOutCap = 0;
-    float* dTtaMean = nullptr;       // [tiles][outT][outT][4] f32 (TTA only)
-    size_t ttaCap = 0;
-    float *dRampX = nullptr, *dRampY = nullptr;
-    int rampXLen = -1, rampYLen = -1;
-    // host-buffer paths
-    uint8_t *dFrameIn = nullptr, *dFrameOut = nullptr;
-    size_t frameInCap = 0, frameOutCap = 0;
+    // Each group below is reset by one assignment in unload().
+    // frame cache (ensureFrameBuffers), valid for the frame key w x h, passes; w == 0: no frame
+    struct FrameCache {
+        int w = 0, h = 0, passes = 1;
+        TileGrid grid;
+        int batchCount = 0;
+        std::vector<RowBand> rowBands;
+        std::vector<CudaEvent> bandEv;   // render's per-band events (cudaEventDisableTiming), reused frame after frame
+        DeviceBuffer slots;              // TileSlot [steps]
+        DeviceBuffer tileMap;            // int [tiles]: slot of reference tile ti (row-major processing order without TTA)
+        DeviceBuffer unpacked;           // [steps][tile][tile][4] engine elements: every tile of the frame, unpacked by one launch
+        DeviceBuffer tileOut;            // [steps][outT][outT][4] engine elements
+        DeviceBuffer ttaMean;            // [tiles][outT][outT][4] f32 (TTA only)
+        DeviceBuffer rampX, rampY;       // blend ramps of rampXLen / rampYLen entries
+        int rampXLen = -1, rampYLen = -1;
+    } fc;
+    // host-buffer paths: the frame on the device (render, renderBgra, renderBanded)
+    struct HostStaging { DeviceBuffer in, out; } staging;
     // BGRA frames: alpha-scan flags (2 ints) and the two ping-pong buffers of the colour bleed
-    int* dAlphaFlags = nullptr;
-    uint8_t* dBleed[2] = {nullptr, nullptr};
-    size_t bleedCap = 0;
+    struct BgraScratch { DeviceBuffer flags, bleed[2]; } bgra;
     // pipelined submit
     static constexpr int kSlots = 3;
     struct PipeSlot {
-        uint8_t *dIn = nullptr, *dOut = nullptr;
-        size_t inCap = 0, outCap = 0;
-        cudaEvent_t evH2D = nullptr, evComp = nullptr, evDone = nullptr;
+        DeviceBuffer in, out;
+        CudaEvent evH2D{cudaEventDisableTiming}, evComp{cudaEventDisableTiming}, evDone{cudaEventDisableTiming};
         bool busy = false;
-    } pipe[kSlots];
+    };
+    std::array<PipeSlot, kSlots> pipe;
     int nextTicket = 0;
-    // stage timing
-    std::vector<cudaEvent_t> evPool;
-    int evUsed = 0;
+    // stage timing (renderOnStream's spans) and the caller's timer marks
     struct StageSpan { int kind, e0, e1; };
-    std::vector<StageSpan> spans;
+    struct Timing {
+        std::vector<CudaEvent> pool;
+        int used = 0;
+        std::vector<StageSpan> spans;
+        CudaEvent marks[16];
+    } timing;
     cudaEvent_t nextEvent();
-    cudaEvent_t timerEv[16] = {};
     // row-band mode
-    void* dBandTiles = nullptr;
-    size_t bandTilesCap = 0;
-    int* dBandMap = nullptr;
-    size_t bandMapCap = 0;
-    TileSlot* dBandSlots = nullptr;
-    size_t bandSlotCap = 0;
-    cudaEvent_t evBandModel = nullptr;
-    float* dBandMean = nullptr;                  // --tta in row-band mode: [own tiles + received seam row][outT][outT][4] f32
-    size_t bandMeanCap = 0;
-    std::vector<TileSlot> bandSlotsHost;         // staging of the asynchronous uploads (must outlive them)
-    std::vector<int> bandMapHost;
+    struct BandState {
+        DeviceBuffer tiles;              // engine elements: own model outputs (+ the received seam row without TTA)
+        DeviceBuffer mean;               // --tta: [own tiles + received seam row][outT][outT][4] f32
+        DeviceBuffer map;                // int [tiles]
+        DeviceBuffer slots;              // TileSlot [steps]
+        CudaEvent evModel{cudaEventDisableTiming};
+        std::vector<TileSlot> slotsHost;  // staging of the asynchronous uploads (must outlive them)
+        std::vector<int> mapHost;
+    } band;
 };
 
 // Single-layer test hooks, see include/w2x_dev.h.  impl: 0 = the kernel the planner picks, 1 = head kernel, 2 = scalar reference.
