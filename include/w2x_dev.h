@@ -2,7 +2,8 @@
  * w2x_dev.h -- development / test hooks of the B200-native waifu2x engine.  NOT part of the drop-in boundary (include/w2x.h).
  *
  * w2x_selftest_conv, w2x_run_conv_layer and w2x_run_conv_layer_f32 are exported by the shipped library (lib/libw2x.so): they run the product's own layer
- * kernels on caller-supplied or random data so that tests can compare single layers with an independent fp32 reference.
+ * kernels on caller-supplied or random data so that tests can compare single layers with an independent fp32 reference.  w2x_layer_tensor,
+ * also shipped, reads the per-layer tensors of a loaded engine for the same purpose.
  * The w2x_probe_* micro-benchmarks and every switch that alters or skips kernel work (W2X_DBG, W2X_CONV_IMPL, W2X_NO_PATCH,
  * W2X_NO_FUSE_FIRST, W2X_NO_EPI_GROUPS, W2X_NO_HEAD_KERNEL, W2X_NO_PDL) exist only in the W2X_DEV build, lib/libw2x_dev.so.
  */
@@ -18,6 +19,20 @@ extern "C" {
 /* The colour bleed of w2x_render_bgra on host buffers: src BGRA (w x h, pitch src_stride >= 4 * width), `rounds` rounds ->
  * dst BGRA packed (pitch 4 * width), alpha bytes copied from src.  Returns 1 on success. */
 W2X_API int w2x_alpha_bleed(int device, const uint8_t* src_bgra, int width, int height, size_t src_stride, int rounds, uint8_t* dst_bgra);
+
+/* Read-only view of a loaded CUNet/UpCUNet engine, for per-layer tests: after w2x_infer, w2x_render or w2x_submit + w2x_wait, copy one
+ * tensor of plan layer `index` (the indexing of w2x_layer_kernel) as the last batch left it into dst (cap bytes); dims[4] receives its
+ * shape, unused trailing entries 1.  which:
+ *   0 the layer's output activation [batch][h][w][c], engine elements (fp16 bits, or fp32 in a tf32 engine)
+ *   1 the model input tensor [batch][tile][tile][4] that w2x_infer fills (index ignored; render reads its tiles elsewhere)
+ *   2 SE channel sums, int64 [batch][c], fixed point 2^-10 (SE layers only)
+ *   3 SE gate, float [batch][c] (SE layers only)
+ *   4 the per-image weights this layer reads, [batch][npad][ktot] engine elements (layers with an SE gate folded into their weights)
+ * Slots at and after the image count of the last batch hold stale data.  The call synchronises the engine's streams, launches no kernel
+ * and changes no engine state.  dst == NULL: only the size and dims.  Returns the bytes written (or needed); 0 when the layer has no
+ * such tensor (the output of a layer computed inside the next one, or of the final layer, which goes to the caller); -1 on error
+ * (e.g. a SwinUNet engine), with the message in w2x_last_error. */
+W2X_API long long w2x_layer_tensor(w2x_engine* e, int index, int which, void* dst, size_t cap, int* dims);
 
 /* One layer of the dense model path (SURVEY 8a row a17; replaces a slice of the engine enqueued at img2img_infer.cpp:80) on
  * caller-supplied host data, through the kernel the execution planner picks for that shape (head != 0: kinds 3 / 4 through the

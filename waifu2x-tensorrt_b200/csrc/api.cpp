@@ -159,6 +159,9 @@ int w2x_profile_layers(w2x_engine* e, int repeats, char (*names)[48], float* ms,
     return e ? e->impl.profileLayers(repeats < 1 ? 1 : repeats, names, ms, flops, n) : -1;
 }
 int w2x_layer_kernel(w2x_engine* e, int index, char* buf, int cap) { return e && buf && cap > 0 ? e->impl.layerKernel(index, buf, cap) : 0; }
+long long w2x_layer_tensor(w2x_engine* e, int index, int which, void* dst, size_t cap, int* dims) {
+    return e ? e->impl.layerTensor(index, which, dst, cap, dims) : -1;
+}
 int w2x_infer(w2x_engine* e, const float* in, int n, float* out) { return e && in && out && e->impl.infer(in, n, out) ? 1 : 0; }
 
 // ---- stage entry points ---------------------------------------------------------------------------------

@@ -792,6 +792,57 @@ int Engine::layerKernel(int index, char* buf, int cap) const {
     return 1;
 }
 
+// After the engine's work has finished: copy one tensor that the plan of layer `index` wrote or reads, as the last batch left it.
+// It launches no kernel and changes no engine state.  dst == nullptr: report the size and the shape only.
+long long Engine::layerTensor(int index, int which, void* dst, size_t cap, int* dims) {
+    try {
+        if (!isLoaded) throw Error("no engine loaded");
+        if (model.arch != ARCH_CUNET && model.arch != ARCH_UPCUNET) throw Error("not a CUNet engine");
+        if (which != 1 && (index < 0 || index >= (int)layers.size())) throw Error("layer index " + std::to_string(index) + " is out of range");
+        const void* src = nullptr;
+        size_t bytes = 0;
+        int shape[4] = {batch, 1, 1, 1};
+        if (which == 1) {
+            src = actIn.p;
+            bytes = actIn.elems() * elemBytes;
+            shape[1] = actIn.h; shape[2] = actIn.w; shape[3] = actIn.c;
+        } else {
+            const LayerExec& L = layers[index];
+            if (which == 0 && L.impl != IMPL_SKIP && !L.isFinal) {
+                src = L.p.out;
+                shape[1] = L.p.out_h; shape[2] = L.p.out_w; shape[3] = L.p.out_c;
+                bytes = (size_t)batch * L.p.out_h * L.p.out_w * L.p.out_c * elemBytes;
+            } else if (which == 2 && L.seR) {
+                src = L.sePartial;
+                bytes = L.sePartialBytes;
+                shape[1] = (int)(bytes / ((size_t)batch * sizeof(long long)));
+            } else if (which == 3 && L.seR) {
+                src = L.seScale;
+                shape[1] = L.p.out_c;
+                bytes = (size_t)batch * L.p.out_c * sizeof(float);
+            } else if (which == 4 && L.p.w_img_stride) {
+                src = L.p.w;
+                shape[1] = L.p.npad; shape[2] = (int)model.layers[index].ktot;
+                bytes = (size_t)batch * L.p.w_img_stride * elemBytes;
+            } else if (which < 0 || which > 4) {
+                throw Error("unknown tensor " + std::to_string(which));
+            }
+        }
+        if (dims) std::memcpy(dims, shape, sizeof shape);
+        if (!src || !dst) return (long long)bytes;
+        if (cap < bytes) throw Error("buffer of " + std::to_string(cap) + " bytes is too small for " + std::to_string(bytes));
+        W2X_CUDA(cudaSetDevice(cfg.deviceId));
+        W2X_CUDA(cudaStreamSynchronize(stream));
+        W2X_CUDA(cudaStreamSynchronize(h2dStream));
+        W2X_CUDA(cudaStreamSynchronize(d2hStream));
+        W2X_CUDA(cudaMemcpy(dst, src, bytes, cudaMemcpyDeviceToHost));
+        return (long long)bytes;
+    } catch (const std::exception& ex) {
+        ELOG(W2X_ERROR, std::string("Layer tensor copy failed: ") + ex.what() + ".");
+        return -1;
+    }
+}
+
 double Engine::flopsPerTile() const {
     double f = 0;
     for (const auto& L : layers) f += L.flops;

@@ -172,6 +172,8 @@ public:
     double flopsPerTile() const;
     int lastStageMs(float* out, int n);
     int layerKernel(int index, char* buf, int cap) const;
+    // test hook w2x_layer_tensor (include/w2x_dev.h): a read-only copy of one tensor of a CUNet plan layer
+    long long layerTensor(int index, int which, void* dst, size_t cap, int* dims);
     bool timerMark(int idx, int which);
     float timerElapsedMs(int i0, int i1);
     int device() const { return cfg.deviceId; }

@@ -135,6 +135,7 @@ _SIGNATURES = {
     "w2x_tta_reduce": (C.c_int, [C.c_int, C.c_void_p, C.c_int, C.c_int, C.c_void_p]),
     "w2x_alpha_bleed": (C.c_int, [C.c_int, C.c_void_p, C.c_int, C.c_int, C.c_size_t, C.c_int, C.c_void_p]),
     "w2x_infer": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_void_p]),
+    "w2x_layer_tensor": (C.c_longlong, [C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_size_t, C.POINTER(C.c_int)]),
     "w2x_selftest_conv": (C.c_double, [C.c_int] * 7 + [C.c_uint]),
     "w2x_run_conv_layer": (C.c_int, [C.c_int] * 8 + [C.c_void_p, C.c_void_p, C.POINTER(C.c_float), C.c_void_p, C.c_void_p]),
     "w2x_run_conv_layer_f32": (C.c_int, [C.c_int] * 7 + [C.c_void_p, C.c_void_p, C.POINTER(C.c_float), C.c_void_p, C.c_void_p]),
@@ -530,6 +531,26 @@ class Img2Img:
     def layer_kernel(self, index: int) -> Optional[str]:
         buf = C.create_string_buffer(256)
         return buf.value.decode() if self._l.w2x_layer_kernel(self._h, index, buf, 256) else None
+
+    # which: 0 layer output, 1 model input, 2 SE sums, 3 SE gate, 4 per-image folded weights (include/w2x_dev.h: w2x_layer_tensor)
+    _LAYER_TENSOR_RANK = {0: 4, 1: 4, 2: 2, 3: 2, 4: 3}
+
+    def layer_tensor(self, index: int, which: int = 0) -> Optional[np.ndarray]:
+        """A copy of one tensor of plan layer `index` of a loaded CUNet engine, as the last batch left it: float16 or float32 (the
+        engine's elements) for which 0, 1 and 4, int64 for 2, float32 for 3.  None when the layer has no such tensor."""
+        dims = (C.c_int * 4)()
+        n = self._l.w2x_layer_tensor(self._h, index, which, None, 0, dims)
+        if n < 0:
+            raise RuntimeError(self.last_error)
+        if n == 0:
+            return None
+        shape = tuple(dims[:self._LAYER_TENSOR_RANK[which]])
+        count = int(np.prod(shape))
+        dtype = np.int64 if which == 2 else np.float32 if which == 3 else np.float16 if n == 2 * count else np.float32
+        out = np.empty(shape, dtype)
+        if out.nbytes != n or self._l.w2x_layer_tensor(self._h, index, which, _ptr(out), out.nbytes, dims) != n:
+            raise RuntimeError(self.last_error or "w2x_layer_tensor: unexpected size")
+        return out
 
     def render_device(self, d_src: int, w: int, h: int, d_dst: int) -> bool:
         return bool(self._l.w2x_render_device(self._h, C.c_void_p(d_src), w, h, w * 3, C.c_void_p(d_dst), w * self.scaling * 3))
