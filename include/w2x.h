@@ -104,6 +104,27 @@ W2X_API int w2x_render(w2x_engine* e, const uint8_t* src_bgr, int width, int hei
 W2X_API int w2x_render_bgra(w2x_engine* e, const uint8_t* src_bgra, int width, int height, size_t src_stride,
                             uint8_t* dst_bgra, size_t dst_stride);
 
+/* Output at any size up to the model's: src BGR u8 HWC (w x h, pitch src_stride >= 3 * width) -> dst BGR u8 (dst_width x dst_height,
+ * pitch dst_stride >= 3 * dst_width), synchronous, with any loaded engine, for 1 <= dst_width <= width * scaling and
+ * 1 <= dst_height <= height * scaling.  Let C be the canvas w2x_render returns for src (width * scaling x height * scaling).  Then, per
+ * channel, with the u8 values of C taken as reals:
+ *     dst = clamp(rint(R_y(R_x(C))), 0, 255)
+ * where R is the antialiased bicubic resample of torch.nn.functional.interpolate(mode="bicubic", antialias=True, align_corners=False),
+ * i.e. PIL's BICUBIC reduction (a = -0.5).  On one axis n_in -> n_out, r = n_in / n_out, s = max(r, 1), output index i reads
+ *     c = r * (i + 0.5),  taps j in [max(floor(c - 2s + 0.5), 0), min(floor(c + 2s + 0.5), n_in)),  weight cubic((j - c + 0.5) / s)
+ * normalised to sum 1, cubic(x) = ((a + 2)|x| - (a + 3))x^2 + 1 for |x| < 1, a(|x|^3 - 5|x|^2 + 8|x| - 4) for 1 <= |x| < 2, else 0.
+ * The device computes it in fp32 with no rounding between the two passes (within 1 of the float64 result).
+ *  - dst_width x dst_height == the canvas: byte-identical to w2x_render, and no resample runs.
+ *  - An axis with n_out == n_in has the single weight 1: it is left alone.
+ *  - The resample never enlarges the model's output: larger sizes are refused.  BGR only.
+ * Returns 0 and logs the reason on failure (no engine loaded, null pointers, an output size outside the range above, strides below 3
+ * bytes per pixel). */
+W2X_API int w2x_render_resized(w2x_engine* e, const uint8_t* src_bgr, int width, int height, size_t src_stride, uint8_t* dst_bgr,
+                               int dst_width, int dst_height, size_t dst_stride);
+/* w2x_render_resized through the pipeline of w2x_submit: returns a ticket >= 0 for w2x_wait, or -1 with the reason logged. */
+W2X_API int w2x_submit_resized(w2x_engine* e, const uint8_t* src_bgr, int width, int height, size_t src_stride, uint8_t* dst_bgr,
+                               int dst_width, int dst_height, size_t dst_stride);
+
 /* Same as w2x_render but src/dst are DEVICE pointers on cfg.deviceId; enqueued on the engine's stream,
  * returns without synchronising (w2x_sync to wait).  Used for the HBM-resident `value` measurement. */
 W2X_API int w2x_render_device(w2x_engine* e, const uint8_t* d_src_bgr, int width, int height, size_t src_stride,
@@ -136,6 +157,10 @@ W2X_API void w2x_pool_set_message_callback(w2x_pool* p, w2x_message_cb cb, void*
 W2X_API int w2x_pool_build(w2x_pool* p, const char* onnx_path, const w2x_build_config* cfg);
 W2X_API int w2x_pool_load(w2x_pool* p, const char* onnx_path, const w2x_render_config* cfg);
 W2X_API int w2x_pool_submit(w2x_pool* p, const uint8_t* src_bgr, int width, int height, size_t src_stride, uint8_t* dst_bgr, size_t dst_stride);
+/* w2x_pool_submit with the output of w2x_render_resized; a size the frame's engine refuses fails its w2x_pool_wait, with the reason
+ * logged through the pool's message callback. */
+W2X_API int w2x_pool_submit_resized(w2x_pool* p, const uint8_t* src_bgr, int width, int height, size_t src_stride, uint8_t* dst_bgr,
+                                    int dst_width, int dst_height, size_t dst_stride);
 W2X_API int w2x_pool_wait(w2x_pool* p, int ticket);
 W2X_API int w2x_pool_sync(w2x_pool* p);
 W2X_API void* w2x_host_alloc(size_t bytes);   /* cudaHostAlloc (pinned) */

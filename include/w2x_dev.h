@@ -20,6 +20,16 @@ extern "C" {
  * dst BGRA packed (pitch 4 * width), alpha bytes copied from src.  Returns 1 on success. */
 W2X_API int w2x_alpha_bleed(int device, const uint8_t* src_bgra, int width, int height, size_t src_stride, int rounds, uint8_t* dst_bgra);
 
+/* The resample of w2x_render_resized alone, on host buffers: src BGR (w x h, pitch src_stride >= 3 * width) -> dst BGR (dst_width x
+ * dst_height, pitch dst_stride >= 3 * dst_width; the bytes between rows are left alone), 1 <= dst_width <= width, 1 <= dst_height <= height.
+ * Returns 1 on success. */
+W2X_API int w2x_resample(int device, const uint8_t* src_bgr, int width, int height, size_t src_stride, uint8_t* dst_bgr, int dst_width, int dst_height,
+                         size_t dst_stride);
+/* Host only (no GPU): the resample's table of one axis n_in -> n_out (1 <= n_out <= n_in).  Returns taps, the row length of the weight
+ * table (0 on error).  When weights != NULL and cap >= n_out * taps, also writes first[n_out] (first input index), count[n_out] (inputs
+ * read: first .. first + count - 1, which covers every non-zero weight) and weights[n_out][taps] (fp32, zero past count). */
+W2X_API int w2x_resample_table(int n_in, int n_out, int* first, int* count, float* weights, size_t cap);
+
 /* Read-only view of a loaded CUNet/UpCUNet engine, for per-layer tests: after w2x_infer, w2x_render or w2x_submit + w2x_wait, copy one
  * tensor of plan layer `index` (the indexing of w2x_layer_kernel) as the last batch left it into dst (cap bytes); dims[4] receives its
  * shape, unused trailing entries 1.  which:

@@ -74,6 +74,18 @@ int w2x_render_bgra(w2x_engine* e, const uint8_t* src, int width, int height, si
     return e->impl.renderBgra(src, width, height, src_stride, dst, dst_stride) ? 1 : 0;
 }
 
+int w2x_render_resized(w2x_engine* e, const uint8_t* src, int width, int height, size_t src_stride, uint8_t* dst, int dst_width, int dst_height,
+                       size_t dst_stride) {
+    if (!e) return 0;
+    return e->impl.renderResized(src, width, height, src_stride, dst, dst_width, dst_height, dst_stride) ? 1 : 0;
+}
+
+int w2x_submit_resized(w2x_engine* e, const uint8_t* src, int width, int height, size_t src_stride, uint8_t* dst, int dst_width, int dst_height,
+                       size_t dst_stride) {
+    if (!e) return -1;
+    return e->impl.submitResized(src, width, height, src_stride, dst, dst_width, dst_height, dst_stride);
+}
+
 int w2x_render_device(w2x_engine* e, const uint8_t* src, int width, int height, size_t src_stride, uint8_t* dst, size_t dst_stride) {
     if (!e || !src || !dst) return 0;
     return e->impl.renderDevice(src, width, height, src_stride, dst, dst_stride) ? 1 : 0;
@@ -111,6 +123,17 @@ int w2x_pool_load(w2x_pool* p, const char* onnx_path, const w2x_render_config* c
 int w2x_pool_submit(w2x_pool* p, const uint8_t* src, int width, int height, size_t src_stride, uint8_t* dst, size_t dst_stride) {
     if (!p || !src || !dst) return -1;
     try { return p->impl.submit(src, width, height, src_stride, dst, dst_stride); } catch (...) { return -1; }
+}
+int w2x_pool_submit_resized(w2x_pool* p, const uint8_t* src, int width, int height, size_t src_stride, uint8_t* dst, int dst_width, int dst_height,
+                            size_t dst_stride) {
+    if (!p || !src || !dst) return -1;
+    if (dst_width < 1 || dst_height < 1) {   // the other refusals come from the engine that takes the frame, through w2x_pool_wait
+        if (w2x_engine* e = p->impl.engine(0))
+            e->impl.log(W2X_ERROR, "Submit failed: output size " + std::to_string(dst_width) + "x" + std::to_string(dst_height) + " is below 1x1.",
+                        __FUNCTION__, __LINE__);
+        return -1;
+    }
+    try { return p->impl.submit(src, width, height, src_stride, dst, dst_stride, dst_width, dst_height); } catch (...) { return -1; }
 }
 int w2x_pool_wait(w2x_pool* p, int ticket) {
     try { return p && p->impl.wait(ticket) ? 1 : 0; } catch (...) { return 0; }
@@ -262,6 +285,58 @@ int w2x_alpha_bleed(int device, const uint8_t* src, int width, int height, size_
         return 1;
     } catch (const std::exception& ex) {
         std::fprintf(stderr, "w2x_alpha_bleed: %s\n", ex.what());
+        return 0;
+    }
+}
+
+int w2x_resample(int device, const uint8_t* src, int width, int height, size_t src_stride, uint8_t* dst, int dst_width, int dst_height,
+                 size_t dst_stride) {
+    try {
+        if (!src || !dst || width <= 0 || height <= 0 || src_stride < (size_t)width * 3 || dst_width < 1 || dst_width > width || dst_height < 1 ||
+            dst_height > height || dst_stride < (size_t)dst_width * 3)
+            throw Error("invalid argument");
+        W2X_CUDA(cudaSetDevice(device));
+        const ResampleAxis axes[2] = {resampleAxis(width, dst_width), resampleAxis(height, dst_height)};
+        std::vector<DeviceBuffer> b;
+        ResampleTable t[2];
+        for (int a = 0; a < 2; ++a) {
+            const ResampleAxis& ax = axes[a];
+            int* first = alloc<int>(b, ax.nOut);
+            int* count = alloc<int>(b, ax.nOut);
+            float* w = alloc<float>(b, ax.w.size());
+            W2X_CUDA(cudaMemcpy(first, ax.first.data(), ax.nOut * sizeof(int), cudaMemcpyHostToDevice));
+            W2X_CUDA(cudaMemcpy(count, ax.count.data(), ax.nOut * sizeof(int), cudaMemcpyHostToDevice));
+            W2X_CUDA(cudaMemcpy(w, ax.w.data(), ax.w.size() * sizeof(float), cudaMemcpyHostToDevice));
+            t[a] = {first, count, w, ax.taps};
+        }
+        const size_t row = (size_t)width * 3, orow = (size_t)dst_width * 3;
+        uint8_t* dSrc = alloc<uint8_t>(b, row * height);
+        float* dTmp = alloc<float>(b, (size_t)height * orow);
+        uint8_t* dDst = alloc<uint8_t>(b, orow * dst_height);
+        W2X_CUDA(cudaMemcpy2D(dSrc, row, src, src_stride, row, height, cudaMemcpyHostToDevice));
+        launchResampleH(dSrc, row, 0, height, t[0], dst_width, dTmp, nullptr);   // the engine's sequence (Engine::renderOnStream)
+        launchResampleV(dTmp, dst_width, t[1], 0, dst_height, dDst, orow, nullptr);
+        W2X_CUDA(cudaGetLastError());
+        W2X_CUDA(cudaMemcpy2D(dst, dst_stride, dDst, orow, orow, dst_height, cudaMemcpyDeviceToHost));
+        return 1;
+    } catch (const std::exception& ex) {
+        std::fprintf(stderr, "w2x_resample: %s\n", ex.what());
+        return 0;
+    }
+}
+
+int w2x_resample_table(int n_in, int n_out, int* first, int* count, float* weights, size_t cap) {
+    try {
+        const ResampleAxis ax = resampleAxis(n_in, n_out);
+        if (weights) {
+            if (!first || !count || cap < ax.w.size()) throw Error("weights capacity below n_out * taps");
+            std::memcpy(first, ax.first.data(), ax.first.size() * sizeof(int));
+            std::memcpy(count, ax.count.data(), ax.count.size() * sizeof(int));
+            std::memcpy(weights, ax.w.data(), ax.w.size() * sizeof(float));
+        }
+        return ax.taps;
+    } catch (const std::exception& ex) {
+        std::fprintf(stderr, "w2x_resample_table: %s\n", ex.what());
         return 0;
     }
 }

@@ -138,6 +138,7 @@ void Engine::unload() {
     fc = {};
     staging = {};
     bgra = {};
+    resize = {};
     band = {};
     pipe = {};
     timing = {};
@@ -975,8 +976,38 @@ void Engine::ensureFrameBuffers(int w, int h, int passes) {
     fc.passes = passes;
 }
 
+// Resized output: the tables and buffers of canvas cw x ch -> dw x dh.  Like ensureFrameBuffers, the key is cleared first and set only
+// once every table has been uploaded.
+void Engine::ensureResize(int cw, int ch, int dw, int dh) {
+    if (cw == resize.cw && ch == resize.ch && dw == resize.dw && dh == resize.dh) return;
+    W2X_CUDA(cudaStreamSynchronize(stream));
+    resize.cw = resize.ch = resize.dw = resize.dh = 0;
+    const ResampleAxis axes[2] = {resampleAxis(cw, dw), resampleAxis(ch, dh)};
+    ResampleTable* tables[2] = {&resize.tx, &resize.ty};
+    for (int a = 0; a < 2; ++a) {
+        const ResampleAxis& ax = axes[a];
+        const size_t intBytes = (size_t)ax.nOut * sizeof(int);
+        resize.tables[a].ensure(2 * intBytes + ax.w.size() * sizeof(float));
+        uint8_t* base = resize.tables[a].get<uint8_t>();
+        uploadAsync(base, ax.first.data(), intBytes);
+        uploadAsync(base + intBytes, ax.count.data(), intBytes);
+        uploadAsync(base + 2 * intBytes, ax.w.data(), ax.w.size() * sizeof(float));
+        *tables[a] = {reinterpret_cast<const int*>(base), reinterpret_cast<const int*>(base + intBytes), reinterpret_cast<const float*>(base + 2 * intBytes),
+                      ax.taps};
+    }
+    resize.rowEnd.resize((size_t)dh);
+    for (int i = 0; i < dh; ++i) resize.rowEnd[i] = axes[1].first[i] + axes[1].count[i];
+    resize.canvas.ensure((size_t)cw * 3 * ch);
+    resize.tmp.ensure((size_t)ch * dw * 3 * sizeof(float));
+    W2X_CUDA(cudaStreamSynchronize(stream));   // the staging vectors above end with this call
+    resize.cw = cw;
+    resize.ch = ch;
+    resize.dw = dw;
+    resize.dh = dh;
+}
+
 void Engine::renderOnStream(const uint8_t* dSrc, int w, int h, size_t srcPitch, uint8_t* dDst, size_t dstPitch, cudaStream_t s, bool timed,
-                            std::vector<BandDone>* bands, int pixelBytes) {
+                            std::vector<BandDone>* bands, int pixelBytes, int dstW, int dstH) {
     if (timed) { timing.used = 0; timing.spans.clear(); }
     auto span = [&](int kind, auto&& fn) {
         if (!timed) { fn(); return; }
@@ -1020,15 +1051,25 @@ void Engine::renderOnStream(const uint8_t* dSrc, int w, int h, size_t srcPitch, 
         }
     }
     ensureFrameBuffers(w, h, passes);
+    const int cw = w * scale, ch = h * scale;
+    if (dstW <= 0) dstW = cw;
+    if (dstH <= 0) dstH = ch;
+    // a resized frame is stitched into the engine's canvas and resampled from there into dDst
+    const bool resized = dstW != cw || dstH != ch;
+    if (resized) {
+        if (pixelBytes != 3) throw Error("resized output is BGR only");
+        ensureResize(cw, ch, dstW, dstH);
+    }
     const TileGrid& grid = fc.grid;
     const bool progressive = pixelBytes == 3 && bands != nullptr && !cfg.tta && !fc.rowBands.empty();
     if (bands) bands->clear();
     auto stitchRows = [&](int yBegin, int yEnd) {
         StitchParams sp{};
         sp.outT = outTile; sp.nx = grid.nx; sp.ny = grid.ny; sp.ovx = grid.outOvX; sp.ovy = grid.outOvY;
-        sp.cw = w * scale; sp.ch = h * scale;
+        sp.cw = cw; sp.ch = ch;
         sp.rampx = fc.rampX.get<float>(); sp.rampy = fc.rampY.get<float>();
-        sp.dst = dDst; sp.pitch = dstPitch;
+        sp.dst = resized ? resize.canvas.get<uint8_t>() : dDst;
+        sp.pitch = resized ? (size_t)cw * 3 : dstPitch;
         sp.tiles = cfg.tta ? fc.ttaMean.get() : fc.tileOut.get();
         sp.f32 = (cfg.tta || tf32()) ? 1 : 0;
         sp.tile_map = cfg.tta ? nullptr : fc.tileMap.get<int>();
@@ -1037,6 +1078,20 @@ void Engine::renderOnStream(const uint8_t* dSrc, int w, int h, size_t srcPitch, 
         sp.alpha_off = passes == 2 ? grid.count : 0;   // TTA: index of the reduced alpha tile; else the alpha step of the tile's slot
         launchStitch(sp, s);
         ++launches;
+    };
+    // Canvas rows [y0, y1) have just been stitched: resample them horizontally, then every output row not yet written whose vertical
+    // window ends at or above y1 (a prefix of the rows left, since the windows are monotone).  Returns the output rows written.
+    int rowsOut = 0;
+    auto resampleRows = [&](int y0, int y1) {
+        launchResampleH(resize.canvas.get<uint8_t>(), (size_t)cw * 3, y0, y1, resize.tx, dstW, resize.tmp.get<float>(), s);
+        ++launches;
+        const int i0 = rowsOut;
+        while (rowsOut < dstH && resize.rowEnd[rowsOut] <= y1) ++rowsOut;
+        if (rowsOut > i0) {
+            launchResampleV(resize.tmp.get<float>(), dstW, resize.ty, i0, rowsOut, dDst, dstPitch, s);
+            ++launches;
+        }
+        return std::make_pair(i0, rowsOut);
     };
     const size_t tileElems = (size_t)outTile * outTile * 4;
     const size_t inElems = (size_t)tile * tile * 4;
@@ -1063,11 +1118,16 @@ void Engine::renderOnStream(const uint8_t* dSrc, int w, int h, size_t srcPitch, 
             // output rows that only depend on tile rows finished with this batch: stitch them now, hand the caller an event to copy after
             for (const RowBand& rb : fc.rowBands) {
                 if (rb.batch != b) continue;
-                span(2, [&] { stitchRows(rb.y0, rb.y1); });
+                std::pair<int, int> rows{rb.y0, rb.y1};
+                span(2, [&] {
+                    stitchRows(rb.y0, rb.y1);
+                    if (resized) rows = resampleRows(rb.y0, rb.y1);
+                });
+                if (rows.second <= rows.first) continue;
                 if (fc.bandEv.size() <= bands->size()) fc.bandEv.emplace_back(cudaEventDisableTiming);
                 cudaEvent_t e = fc.bandEv[bands->size()].get();
                 W2X_CUDA(cudaEventRecord(e, s));
-                bands->push_back({rb.y0, rb.y1, e});
+                bands->push_back({rows.first, rows.second, e});
             }
         }
         if (progCb) {
@@ -1084,7 +1144,10 @@ void Engine::renderOnStream(const uint8_t* dSrc, int w, int h, size_t srcPitch, 
             ttaReduce(fc.tileOut.get(), grid.count * passes, fc.ttaMean.get<float>(), s);
             ++launches;
         });
-    span(2, [&] { stitchRows(0, h * scale); });
+    span(2, [&] {
+        stitchRows(0, ch);
+        if (resized) resampleRows(0, ch);
+    });
     W2X_CUDA(cudaGetLastError());
 }
 
@@ -1152,7 +1215,7 @@ bool Engine::renderDevice(const uint8_t* dSrc, int w, int h, size_t srcStride, u
 bool Engine::render(const uint8_t* src, int w, int h, size_t srcStride, uint8_t* dst, size_t dstStride) {
     try {
         if (!isLoaded) throw Error("no engine loaded");
-        renderHostFrame(src, w, h, srcStride, dst, dstStride, 3);
+        renderHostFrame(src, w, h, srcStride, dst, dstStride, 3, w * scale, h * scale);
         return true;
     } catch (const std::exception& ex) {
         ELOG(W2X_ERROR, std::string("Render failed unexpectedly: ") + ex.what() + ".");
@@ -1166,7 +1229,7 @@ bool Engine::renderBgra(const uint8_t* src, int w, int h, size_t srcStride, uint
         if (!src || !dst) throw Error("null image pointer");
         if (w <= 0 || h <= 0) throw Error("invalid frame size");
         if (srcStride < (size_t)w * 4 || dstStride < (size_t)w * scale * 4) throw Error("row stride is smaller than 4 bytes per pixel");
-        renderHostFrame(src, w, h, srcStride, dst, dstStride, 4);
+        renderHostFrame(src, w, h, srcStride, dst, dstStride, 4, w * scale, h * scale);
         return true;
     } catch (const std::exception& ex) {
         ELOG(W2X_ERROR, std::string("Render failed unexpectedly: ") + ex.what() + ".");
@@ -1174,20 +1237,42 @@ bool Engine::renderBgra(const uint8_t* src, int w, int h, size_t srcStride, uint
     }
 }
 
-void Engine::renderHostFrame(const uint8_t* src, int w, int h, size_t srcStride, uint8_t* dst, size_t dstStride, int pixelBytes) {
+void Engine::checkResized(const uint8_t* src, int w, int h, const uint8_t* dst, int dstW, int dstH, size_t dstStride) const {
+    if (!src || !dst) throw Error("null image pointer");
+    if (w <= 0 || h <= 0) throw Error("invalid frame size");
+    if (dstW < 1 || dstW > w * scale || dstH < 1 || dstH > h * scale)
+        throw Error("output size " + std::to_string(dstW) + "x" + std::to_string(dstH) + " is outside 1x1 .. " + std::to_string(w * scale) + "x" +
+                    std::to_string(h * scale) + " (the resample only reduces the model's " + std::to_string(scale) + "x output)");
+    if (dstStride < (size_t)dstW * 3) throw Error("row stride is smaller than 3 bytes per pixel");
+}
+
+bool Engine::renderResized(const uint8_t* src, int w, int h, size_t srcStride, uint8_t* dst, int dstW, int dstH, size_t dstStride) {
+    try {
+        if (!isLoaded) throw Error("no engine loaded");
+        checkResized(src, w, h, dst, dstW, dstH, dstStride);
+        if (srcStride < (size_t)w * 3) throw Error("row stride is smaller than 3 bytes per pixel");
+        renderHostFrame(src, w, h, srcStride, dst, dstStride, 3, dstW, dstH);
+        return true;
+    } catch (const std::exception& ex) {
+        ELOG(W2X_ERROR, std::string("Render failed unexpectedly: ") + ex.what() + ".");
+        return false;
+    }
+}
+
+void Engine::renderHostFrame(const uint8_t* src, int w, int h, size_t srcStride, uint8_t* dst, size_t dstStride, int pixelBytes, int dstW, int dstH) {
     W2X_CUDA(cudaSetDevice(cfg.deviceId));
-    const size_t ipitch = (size_t)w * pixelBytes, opitch = (size_t)w * scale * pixelBytes;
+    const size_t ipitch = (size_t)w * pixelBytes, opitch = (size_t)dstW * pixelBytes;
     staging.in.ensure(ipitch * h);
-    staging.out.ensure(opitch * h * scale);
+    staging.out.ensure(opitch * dstH);
     uint8_t *dIn = staging.in.get<uint8_t>(), *dOut = staging.out.get<uint8_t>();
     W2X_CUDA(cudaMemcpy2DAsync(dIn, ipitch, src, srcStride, ipitch, h, cudaMemcpyHostToDevice, stream));  // render.cpp:226
     // every kernel of the frame is queued first; the output then leaves band by band (rows that are final after a tile row), each copy
     // ordered behind its band's stitch only, so the download of a band overlaps the batches still computing (the reference downloads
     // the whole canvas after the last batch, render.cpp:344).  With --tta, and for BGRA frames, there is one band: the whole frame.
     std::vector<BandDone> bands;
-    renderOnStream(dIn, w, h, ipitch, dOut, opitch, stream, true, &bands, pixelBytes);
+    renderOnStream(dIn, w, h, ipitch, dOut, opitch, stream, true, &bands, pixelBytes, dstW, dstH);
     if (bands.empty()) {
-        W2X_CUDA(cudaMemcpy2DAsync(dst, dstStride, dOut, opitch, opitch, (size_t)h * scale, cudaMemcpyDeviceToHost, stream));  // render.cpp:344
+        W2X_CUDA(cudaMemcpy2DAsync(dst, dstStride, dOut, opitch, opitch, (size_t)dstH, cudaMemcpyDeviceToHost, stream));  // render.cpp:344
     } else {
         for (const BandDone& bd : bands) {
             W2X_CUDA(cudaStreamWaitEvent(d2hStream, bd.ev, 0));
@@ -1203,30 +1288,46 @@ void Engine::renderHostFrame(const uint8_t* src, int w, int h, size_t srcStride,
 int Engine::submit(const uint8_t* src, int w, int h, size_t srcStride, uint8_t* dst, size_t dstStride) {
     try {
         if (!isLoaded) throw Error("no engine loaded");
-        W2X_CUDA(cudaSetDevice(cfg.deviceId));
-        const int ticket = nextTicket;
-        PipeSlot& ps = pipe[ticket % kSlots];
-        if (ps.busy) { W2X_CUDA(cudaEventSynchronize(ps.evDone.get())); ps.busy = false; }
-        ps.in.ensure((size_t)w * 3 * h);
-        ps.out.ensure((size_t)w * scale * 3 * h * scale);
-        uint8_t *dIn = ps.in.get<uint8_t>(), *dOut = ps.out.get<uint8_t>();
-        ensureFrameBuffers(w, h);
-        W2X_CUDA(cudaMemcpy2DAsync(dIn, (size_t)w * 3, src, srcStride, (size_t)w * 3, h, cudaMemcpyHostToDevice, h2dStream));
-        W2X_CUDA(cudaEventRecord(ps.evH2D.get(), h2dStream));
-        W2X_CUDA(cudaStreamWaitEvent(stream, ps.evH2D.get(), 0));
-        renderOnStream(dIn, w, h, (size_t)w * 3, dOut, (size_t)w * scale * 3, stream, false);
-        W2X_CUDA(cudaEventRecord(ps.evComp.get(), stream));
-        W2X_CUDA(cudaStreamWaitEvent(d2hStream, ps.evComp.get(), 0));
-        W2X_CUDA(cudaMemcpy2DAsync(dst, dstStride, dOut, (size_t)w * scale * 3, (size_t)w * scale * 3, (size_t)h * scale,
-                                   cudaMemcpyDeviceToHost, d2hStream));
-        W2X_CUDA(cudaEventRecord(ps.evDone.get(), d2hStream));
-        ps.busy = true;
-        ++nextTicket;
-        return ticket;
+        return submitFrame(src, w, h, srcStride, dst, w * scale, h * scale, dstStride);
     } catch (const std::exception& ex) {
         ELOG(W2X_ERROR, std::string("Submit failed unexpectedly: ") + ex.what() + ".");
         return -1;
     }
+}
+
+int Engine::submitResized(const uint8_t* src, int w, int h, size_t srcStride, uint8_t* dst, int dstW, int dstH, size_t dstStride) {
+    try {
+        if (!isLoaded) throw Error("no engine loaded");
+        checkResized(src, w, h, dst, dstW, dstH, dstStride);
+        if (srcStride < (size_t)w * 3) throw Error("row stride is smaller than 3 bytes per pixel");
+        return submitFrame(src, w, h, srcStride, dst, dstW, dstH, dstStride);
+    } catch (const std::exception& ex) {
+        ELOG(W2X_ERROR, std::string("Submit failed unexpectedly: ") + ex.what() + ".");
+        return -1;
+    }
+}
+
+int Engine::submitFrame(const uint8_t* src, int w, int h, size_t srcStride, uint8_t* dst, int dstW, int dstH, size_t dstStride) {
+    W2X_CUDA(cudaSetDevice(cfg.deviceId));
+    const int ticket = nextTicket;
+    PipeSlot& ps = pipe[ticket % kSlots];
+    if (ps.busy) { W2X_CUDA(cudaEventSynchronize(ps.evDone.get())); ps.busy = false; }
+    const size_t opitch = (size_t)dstW * 3;
+    ps.in.ensure((size_t)w * 3 * h);
+    ps.out.ensure(opitch * dstH);
+    uint8_t *dIn = ps.in.get<uint8_t>(), *dOut = ps.out.get<uint8_t>();
+    ensureFrameBuffers(w, h);
+    W2X_CUDA(cudaMemcpy2DAsync(dIn, (size_t)w * 3, src, srcStride, (size_t)w * 3, h, cudaMemcpyHostToDevice, h2dStream));
+    W2X_CUDA(cudaEventRecord(ps.evH2D.get(), h2dStream));
+    W2X_CUDA(cudaStreamWaitEvent(stream, ps.evH2D.get(), 0));
+    renderOnStream(dIn, w, h, (size_t)w * 3, dOut, opitch, stream, false, nullptr, 3, dstW, dstH);
+    W2X_CUDA(cudaEventRecord(ps.evComp.get(), stream));
+    W2X_CUDA(cudaStreamWaitEvent(d2hStream, ps.evComp.get(), 0));
+    W2X_CUDA(cudaMemcpy2DAsync(dst, dstStride, dOut, opitch, opitch, (size_t)dstH, cudaMemcpyDeviceToHost, d2hStream));
+    W2X_CUDA(cudaEventRecord(ps.evDone.get(), d2hStream));
+    ps.busy = true;
+    ++nextTicket;
+    return ticket;
 }
 
 // ------------------------------------------------------------------------------------------------

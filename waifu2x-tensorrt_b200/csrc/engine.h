@@ -157,6 +157,10 @@ public:
     // the colour-bled frame through the render pipeline, the alpha plane as a second model pass in the same batches (none when opaque)
     bool renderBgra(const uint8_t* src, int w, int h, size_t srcStride, uint8_t* dst, size_t dstStride);
     int submit(const uint8_t* src, int w, int h, size_t srcStride, uint8_t* dst, size_t dstStride);
+    // BGR host buffers -> render's canvas (w*scale x h*scale) reduced to dstW x dstH by an antialiased bicubic resample (include/w2x.h,
+    // w2x_render_resized): 1 <= dstW <= w*scale, 1 <= dstH <= h*scale, dst pitch >= 3 * dstW.  The canvas size is render, byte for byte.
+    bool renderResized(const uint8_t* src, int w, int h, size_t srcStride, uint8_t* dst, int dstW, int dstH, size_t dstStride);
+    int submitResized(const uint8_t* src, int w, int h, size_t srcStride, uint8_t* dst, int dstW, int dstH, size_t dstStride);
     bool wait(int ticket);
     // one image sharded over several engines (one per GPU) by bands of tile rows, seam rows exchanged peer-to-peer
     static bool renderBanded(Engine* const* engines, int count, const uint8_t* src, int w, int h, size_t srcStride, uint8_t* dst, size_t dstStride);
@@ -202,10 +206,16 @@ private:
     struct BandDone { int y0, y1; cudaEvent_t ev; };   // ... and have been stitched when `ev` fires
     // bands != nullptr (and no TTA): stitch progressively, one launch per finished tile row, and report the bands instead of one stitch at the end
     // pixelBytes 4: packed BGRA frames (dSrcPitch = 4w): alpha scan, colour bleed and alpha pass as the frame needs them; no bands
+    // dstW x dstH other than the canvas (BGR only): stitch into resize.canvas, then resample into dDst; with bands, the bands are output
+    // rows of dDst
     void renderOnStream(const uint8_t* dSrc, int w, int h, size_t srcPitch, uint8_t* dDst, size_t dstPitch, cudaStream_t s, bool timed,
-                        std::vector<BandDone>* bands = nullptr, int pixelBytes = 3);
-    // render / renderBgra: host frame -> staging buffers -> renderOnStream -> host frame, synchronous
-    void renderHostFrame(const uint8_t* src, int w, int h, size_t srcStride, uint8_t* dst, size_t dstStride, int pixelBytes);
+                        std::vector<BandDone>* bands = nullptr, int pixelBytes = 3, int dstW = 0, int dstH = 0);
+    // render / renderBgra / renderResized: host frame -> staging buffers -> renderOnStream -> host frame (dstW x dstH), synchronous
+    void renderHostFrame(const uint8_t* src, int w, int h, size_t srcStride, uint8_t* dst, size_t dstStride, int pixelBytes, int dstW, int dstH);
+    int submitFrame(const uint8_t* src, int w, int h, size_t srcStride, uint8_t* dst, int dstW, int dstH, size_t dstStride);
+    // the refusals of renderResized / submitResized (throws Error)
+    void checkResized(const uint8_t* src, int w, int h, const uint8_t* dst, int dstW, int dstH, size_t dstStride) const;
+    void ensureResize(int cw, int ch, int dw, int dh);
     void* dalloc(size_t bytes);
     Act allocAct(int h, int w, int c);
 
@@ -252,6 +262,15 @@ private:
     struct HostStaging { DeviceBuffer in, out; } staging;
     // BGRA frames: alpha-scan flags (2 ints) and the two ping-pong buffers of the colour bleed
     struct BgraScratch { DeviceBuffer flags, bleed[2]; } bgra;
+    // resized frames (ensureResize), valid for the key canvas cw x ch -> dw x dh; cw == 0: none
+    struct ResizeState {
+        int cw = 0, ch = 0, dw = 0, dh = 0;
+        DeviceBuffer canvas;             // u8 BGR [ch][cw][3], the stitched frame
+        DeviceBuffer tmp;                // f32 [ch][dw][3], the horizontal pass
+        DeviceBuffer tables[2];          // x, y: int first[n_out], int count[n_out], float w[n_out][taps]
+        ResampleTable tx{}, ty{};
+        std::vector<int> rowEnd;         // output row i reads canvas rows below rowEnd[i] (non-decreasing)
+    } resize;
     // pipelined submit
     static constexpr int kSlots = 3;
     struct PipeSlot {

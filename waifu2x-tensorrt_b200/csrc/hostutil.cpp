@@ -58,6 +58,49 @@ std::vector<float> blendRamp(int overlap) {
 }
 
 // ------------------------------------------------------------------------------------------------
+// Antialiased bicubic weights: the kernel is stretched by s = max(n_in / n_out, 1), so a reduction by r reads about 4r + 1 inputs.
+// ------------------------------------------------------------------------------------------------
+ResampleAxis resampleAxis(int nIn, int nOut) {
+    if (nIn < 1 || nOut < 1 || nOut > nIn) throw Error("resample: need 1 <= output size <= input size");
+    auto cubic = [](double x) {
+        const double a = -0.5;
+        x = std::fabs(x);
+        if (x < 1) return ((a + 2) * x - (a + 3)) * x * x + 1;
+        if (x < 2) return a * (((x - 5) * x + 8) * x - 4);
+        return 0.0;
+    };
+    const double r = (double)nIn / nOut, s = std::max(r, 1.0);
+    ResampleAxis ax;
+    ax.nIn = nIn;
+    ax.nOut = nOut;
+    ax.first.resize(nOut);
+    ax.count.resize(nOut);
+    std::vector<std::vector<double>> rows(nOut);
+    for (int i = 0; i < nOut; ++i) {
+        const double c = r * (i + 0.5);
+        const int lo = std::max((int)std::floor(c - 2 * s + 0.5), 0), hi = std::min((int)std::floor(c + 2 * s + 0.5), nIn);
+        std::vector<double>& wr = rows[i];
+        double sum = 0;
+        for (int j = lo; j < hi; ++j) {
+            wr.push_back(cubic((j - c + 0.5) / s));
+            sum += wr.back();
+        }
+        for (double& v : wr) v /= sum;
+        int b = 0, e = (int)wr.size();
+        while (e - b > 1 && wr[b] == 0.0) ++b;
+        while (e - b > 1 && wr[e - 1] == 0.0) --e;
+        wr = std::vector<double>(wr.begin() + b, wr.begin() + e);
+        ax.first[i] = lo + b;
+        ax.count[i] = e - b;
+        ax.taps = std::max(ax.taps, e - b);
+    }
+    ax.w.assign((size_t)nOut * ax.taps, 0.f);
+    for (int i = 0; i < nOut; ++i)
+        for (int k = 0; k < ax.count[i]; ++k) ax.w[(size_t)i * ax.taps + k] = (float)rows[i][k];
+    return ax;
+}
+
+// ------------------------------------------------------------------------------------------------
 // SHA-256 (FIPS 180-4), written from the standard.
 // ------------------------------------------------------------------------------------------------
 namespace {

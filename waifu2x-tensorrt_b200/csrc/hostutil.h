@@ -42,6 +42,18 @@ TileGrid calculateTiles(int inW, int inH, int outW, int outH, int tileW, int til
 // createTileWeights (img2img_load.cpp:29-52): ramp[i] = float(double(i + 1) / double(overlap + 1)), i in [0, overlap)
 std::vector<float> blendRamp(int overlap);
 
+// ---- antialiased bicubic reduction (w2x_render_resized) --------------------------------------------
+// One axis n_in -> n_out (1 <= n_out <= n_in): output index i reads inputs first[i] .. first[i] + count[i] - 1 with weights
+// w[i * taps + k] (k < count[i]; the rest of the row is 0).  The weights are torch's interpolate(mode="bicubic", antialias=True,
+// align_corners=False), i.e. PIL's BICUBIC (a = -0.5), computed in double, normalised to sum 1 and stored as float; zero weights at
+// either end of a window are dropped, so an identity axis is one tap of weight 1.  first[i] and first[i] + count[i] never decrease.
+struct ResampleAxis {
+    int nIn = 0, nOut = 0, taps = 0;
+    std::vector<int> first, count;
+    std::vector<float> w;
+};
+ResampleAxis resampleAxis(int nIn, int nOut);   // throws Error outside 1 <= nOut <= nIn
+
 // ---- sha256 (lowercase hex), json sidecar, naming (img2img_build.cpp:8-50,151-154; img2img_load.cpp:54-114) -----
 std::string sha256Hex(const std::string& data);
 std::string configHashString(const std::string& deviceName, const w2x_build_config& c);  // pre-hash string

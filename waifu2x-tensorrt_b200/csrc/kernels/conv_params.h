@@ -287,6 +287,17 @@ void launchAlphaScan(const uint8_t* bgra, size_t pixels, int* flags, cudaStream_
 // n > 0 known 8-neighbours takes their per-channel mean (2 sum + n) / 2n (grow != 0) and becomes known, any other is (0, 0, 0).  The
 // output alpha byte is 255 / 0 for known / unknown, or, when alphaOf != nullptr (last round), alphaOf's alpha byte.
 void launchAlphaBleedRound(const uint8_t* in, uint8_t* out, int w, int h, int grow, const uint8_t* alphaOf, cudaStream_t s);
+// Antialiased bicubic reduction (kernels/resample.cu): one axis table on the device, laid out as hostutil.h's ResampleAxis
+struct ResampleTable {
+    const int* first;    // [n_out] first input index
+    const int* count;    // [n_out] taps
+    const float* w;      // [n_out][taps] weights
+    int taps;
+};
+// horizontal pass: canvas rows [y0, y1) of a u8 BGR canvas -> rows [y0, y1) of tmp, f32 [rows][dstW][3]
+void launchResampleH(const uint8_t* canvas, size_t pitch, int y0, int y1, const ResampleTable& tx, int dstW, float* tmp, cudaStream_t s);
+// vertical pass: output rows [i0, i1) from tmp -> u8 BGR rows of dst, rint + clamp to [0, 255]
+void launchResampleV(const float* tmp, int dstW, const ResampleTable& ty, int i0, int i1, uint8_t* dst, size_t pitch, cudaStream_t s);
 void launchTtaReduce(const __half* outs, int tiles, int outT, float* mean, cudaStream_t s);
 void launchTtaReduce(const float* outs, int tiles, int outT, float* mean, cudaStream_t s);
 // NCHW f32 <-> NHWC4 fp16 / f32 (Img2Img::infer host entry, tests)

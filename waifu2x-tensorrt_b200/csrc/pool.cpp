@@ -59,7 +59,7 @@ bool EnginePool::load(const std::string& onnxPath, const w2x_render_config& cfg)
     return true;
 }
 
-int EnginePool::submit(const uint8_t* src, int w, int h, size_t srcStride, uint8_t* dst, size_t dstStride) {
+int EnginePool::submit(const uint8_t* src, int w, int h, size_t srcStride, uint8_t* dst, size_t dstStride, int dstW, int dstH) {
     int ticket;
     {
         std::unique_lock<std::mutex> lk(stateMu);
@@ -72,7 +72,7 @@ int EnginePool::submit(const uint8_t* src, int w, int h, size_t srcStride, uint8
     {
         std::unique_lock<std::mutex> lk(wk.mu);
         wk.cv.wait(lk, [&] { return (int)wk.queue.size() < kQueueDepth || wk.stop; });  // back-pressure on the producer
-        wk.queue.push_back(Job{src, w, h, srcStride, dst, dstStride, ticket});
+        wk.queue.push_back(Job{src, w, h, srcStride, dst, dstStride, dstW, dstH, ticket});
     }
     wk.cv.notify_all();
     return ticket;
@@ -106,7 +106,9 @@ void EnginePool::workerLoop(Worker* w) {
         }
         if (have) {
             w->cv.notify_all();  // a queue slot is free again
-            const int t = w->eng.impl.submit(job.src, job.w, job.h, job.srcStride, job.dst, job.dstStride);
+            Engine& e = w->eng.impl;
+            const int t = job.dstW > 0 ? e.submitResized(job.src, job.w, job.h, job.srcStride, job.dst, job.dstW, job.dstH, job.dstStride)
+                                       : e.submit(job.src, job.w, job.h, job.srcStride, job.dst, job.dstStride);
             if (t < 0) finish(job.ticket, false);
             else flight.push_back({t, job.ticket});
             continue;

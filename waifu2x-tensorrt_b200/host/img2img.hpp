@@ -102,6 +102,16 @@ public:
     int submit(const unsigned char* srcBgr, int width, int height, size_t srcStride, unsigned char* dstBgr, size_t dstStride) {
         return w2x_submit(h_, srcBgr, width, height, srcStride, dstBgr, dstStride);
     }
+
+    // extensions: the output reduced to dstWidth x dstHeight (at most the model's scale), see w2x_render_resized in include/w2x.h
+    bool renderResized(const unsigned char* srcBgr, int width, int height, size_t srcStride, unsigned char* dstBgr, int dstWidth, int dstHeight,
+                       size_t dstStride) {
+        return w2x_render_resized(h_, srcBgr, width, height, srcStride, dstBgr, dstWidth, dstHeight, dstStride) != 0;
+    }
+    int submitResized(const unsigned char* srcBgr, int width, int height, size_t srcStride, unsigned char* dstBgr, int dstWidth, int dstHeight,
+                      size_t dstStride) {
+        return w2x_submit_resized(h_, srcBgr, width, height, srcStride, dstBgr, dstWidth, dstHeight, dstStride);
+    }
     bool wait(int ticket) { return w2x_wait(h_, ticket) != 0; }
 
     w2x_engine* handle() const { return h_; }
@@ -137,6 +147,10 @@ public:
     }
     int submit(const unsigned char* srcBgr, int width, int height, size_t srcStride, unsigned char* dstBgr, size_t dstStride) {
         return w2x_pool_submit(h_, srcBgr, width, height, srcStride, dstBgr, dstStride);
+    }
+    int submitResized(const unsigned char* srcBgr, int width, int height, size_t srcStride, unsigned char* dstBgr, int dstWidth, int dstHeight,
+                      size_t dstStride) {
+        return w2x_pool_submit_resized(h_, srcBgr, width, height, srcStride, dstBgr, dstWidth, dstHeight, dstStride);
     }
     bool wait(int ticket) { return w2x_pool_wait(h_, ticket) != 0; }
     // the pool's index-th engine (borrowed), e.g. for w2x_render_bgra

@@ -42,6 +42,7 @@ struct Options {
     std::vector<fs::path> inputPaths;
     bool recursive = false, nosuffix = false, tta = false;
     bool alpha = false;  // extension: still images keep their alpha channel (BGRA through Img2Img::renderBgra, PNG out)
+    double outputScale = 0;  // extension (> 0 when given): output lround(w F) x lround(h F), at most --scale (Img2Img::submitResized)
     fs::path outputDirectory;
     double blend = 1.0 / 16.0;
     std::string codec = "libx264", pixelFormat = "yuv420p";
@@ -72,6 +73,8 @@ const char* kUsage =
     "    --blend FLOAT:{0.125,0.0625,0.03125,0}=0.0625   --tta\n"
     "    --codec TEXT=libx264   --pix_fmt TEXT=yuv420p   --crf INT:[0,51]=23   --ffmpegDir TEXT\n"
     "    --alpha                     Keep the alpha channel of still images (extension; videos are rendered without it)\n"
+    "    --outputScale FLOAT:(0,scale]   Output size round(F x input) instead of scale x input: the model's output reduced on the GPU\n"
+    "                                by an antialiased bicubic resample (extension; not with --alpha)\n"
     "  build                         Build model\n";
 
 int toInt(const std::string& name, const std::string& v) {
@@ -161,6 +164,13 @@ Options parse(int argc, char** argv) {
         }
         else if (inRender && a == "--tta") o.tta = true;
         else if (inRender && a == "--alpha") o.alpha = true;
+        else if (inRender && a == "--outputScale") {
+            const std::string v = value();
+            size_t pos = 0;
+            try { o.outputScale = std::stod(v, &pos); } catch (...) { pos = 0; }
+            if (v.empty() || pos != v.size() || !std::isfinite(o.outputScale)) throw ParseError(a + ": '" + v + "' is not a number");
+            if (o.outputScale <= 0) throw ParseError(a + ": must be positive");
+        }
         else if (inRender && a == "--codec") o.codec = value();
         else if (inRender && a == "--pix_fmt") o.pixelFormat = value();
         else if (inRender && a == "--crf") { o.crf = toInt(a, value()); if (o.crf < 0 || o.crf > 51) throw ParseError(a + ": value not in range 0 to 51"); }
@@ -172,6 +182,8 @@ Options parse(int argc, char** argv) {
         if (!seen.count(req)) throw ParseError(std::string(req) + " is required");
     if (o.command.empty()) throw ParseError("A subcommand is required");
     if (o.command == "render" && o.inputPaths.empty()) throw ParseError("--input is required");
+    if (o.outputScale > o.scale) throw ParseError("--outputScale: at most --scale (" + std::to_string(o.scale) + "); the resample only reduces the model's output");
+    if (o.outputScale > 0 && o.alpha) throw ParseError("--outputScale: not available with --alpha");
     return o;
 }
 
@@ -287,8 +299,11 @@ int main(int argc, char* argv[]) {
     } else if (!engine.load(modelPath, rc)) {
         return -1;
     }
-    auto submitFrame = [&](const unsigned char* src, int w, int h, size_t ss, unsigned char* dst, size_t ds) {
-        return pool ? pool->submit(src, w, h, ss, dst, ds) : engine.submit(src, w, h, ss, dst, ds);
+    auto submitFrame = [&](const unsigned char* src, int w, int h, size_t ss, unsigned char* dst, const FrameSize& ds) {
+        if (o.outputScale > 0)
+            return pool ? pool->submitResized(src, w, h, ss, dst, ds.width, ds.height, (size_t)ds.width * 3)
+                        : engine.submitResized(src, w, h, ss, dst, ds.width, ds.height, (size_t)ds.width * 3);
+        return pool ? pool->submit(src, w, h, ss, dst, (size_t)ds.width * 3) : engine.submit(src, w, h, ss, dst, (size_t)ds.width * 3);
     };
     auto waitFrame = [&](int ticket) { return pool ? pool->wait(ticket) : engine.wait(ticket); };
 
@@ -310,11 +325,17 @@ int main(int argc, char* argv[]) {
             const bool bgra = o.alpha && capture.getFrameCount() == 1;
             if (bgra) capture.setChannels(4).open(file.string());
             else if (o.alpha) logLine(trt::Severity::warn, "--alpha applies to still images; " + file.string() + " is rendered without alpha");
-            const FrameSize inSize = capture.getFrameSize(), outSize = inSize * o.scale;
+            const FrameSize inSize = capture.getFrameSize();
+            FrameSize outSize = inSize * o.scale;
+            std::string sizeTag;
+            if (o.outputScale > 0) {
+                outSize = {std::max(1, (int)std::lround(inSize.width * o.outputScale)), std::max(1, (int)std::lround(inSize.height * o.outputScale))};
+                sizeTag = "(" + std::to_string(outSize.width) + "x" + std::to_string(outSize.height) + ")";
+            }
             frameIndex = 0;
             frameCount = (size_t)capture.getFrameCount();
             if (!o.outputDirectory.empty()) file = o.outputDirectory / file.filename();
-            if (!o.nosuffix) file.replace_filename(file.stem().string() + suffix + file.extension().string());
+            if (!o.nosuffix) file.replace_filename(file.stem().string() + suffix + sizeTag + file.extension().string());
             if (frameCount == 1) {
                 file.replace_extension(".png");
                 writer.setFrameRate(1).setPixelFormat("").setCodec("");
@@ -402,7 +423,7 @@ int main(int argc, char* argv[]) {
                 while (waitFor(submitted, FILLED)) {
                     if (submitted - retired >= (size_t)kInFlight) retire();
                     const int s = (int)(submitted % kRing);
-                    tickets[s] = submitFrame(in[s].p, inSize.width, inSize.height, (size_t)inSize.width * 3, out[s].p, (size_t)outSize.width * 3);
+                    tickets[s] = submitFrame(in[s].p, inSize.width, inSize.height, (size_t)inSize.width * 3, out[s].p, outSize);
                     if (tickets[s] < 0) throw std::runtime_error("render failed");
                     setState(submitted, SUBMITTED);
                     ++submitted;

@@ -100,6 +100,8 @@ _SIGNATURES = {
     "w2x_render_device": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_size_t, C.c_void_p, C.c_size_t]),
     "w2x_render_bgra": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_size_t, C.c_void_p, C.c_size_t]),
     "w2x_submit": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_size_t, C.c_void_p, C.c_size_t]),
+    "w2x_render_resized": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_size_t, C.c_void_p, C.c_int, C.c_int, C.c_size_t]),
+    "w2x_submit_resized": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_size_t, C.c_void_p, C.c_int, C.c_int, C.c_size_t]),
     "w2x_render_banded": (C.c_int, [C.POINTER(C.c_void_p), C.c_int, C.c_void_p, C.c_int, C.c_int, C.c_size_t, C.c_void_p, C.c_size_t]),
     "w2x_wait": (C.c_int, [C.c_void_p, C.c_int]),
     "w2x_pool_create": (C.c_void_p, [C.POINTER(C.c_int), C.c_int]),
@@ -110,6 +112,7 @@ _SIGNATURES = {
     "w2x_pool_build": (C.c_int, [C.c_void_p, C.c_char_p, C.POINTER(_BuildConfig)]),
     "w2x_pool_load": (C.c_int, [C.c_void_p, C.c_char_p, C.POINTER(_RenderConfig)]),
     "w2x_pool_submit": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_size_t, C.c_void_p, C.c_size_t]),
+    "w2x_pool_submit_resized": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_size_t, C.c_void_p, C.c_int, C.c_int, C.c_size_t]),
     "w2x_pool_wait": (C.c_int, [C.c_void_p, C.c_int]),
     "w2x_pool_sync": (C.c_int, [C.c_void_p]),
     "w2x_sync": (C.c_int, [C.c_void_p]),
@@ -134,6 +137,8 @@ _SIGNATURES = {
     "w2x_stitch_tiles": (C.c_int, [C.c_int, C.c_void_p] + [C.c_int] * 8 + [C.c_void_p, C.c_size_t]),
     "w2x_tta_reduce": (C.c_int, [C.c_int, C.c_void_p, C.c_int, C.c_int, C.c_void_p]),
     "w2x_alpha_bleed": (C.c_int, [C.c_int, C.c_void_p, C.c_int, C.c_int, C.c_size_t, C.c_int, C.c_void_p]),
+    "w2x_resample": (C.c_int, [C.c_int, C.c_void_p, C.c_int, C.c_int, C.c_size_t, C.c_void_p, C.c_int, C.c_int, C.c_size_t]),
+    "w2x_resample_table": (C.c_int, [C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t]),
     "w2x_infer": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_void_p]),
     "w2x_layer_tensor": (C.c_longlong, [C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_size_t, C.POINTER(C.c_int)]),
     "w2x_selftest_conv": (C.c_double, [C.c_int] * 7 + [C.c_uint]),
@@ -301,6 +306,35 @@ def alpha_bleed(src_bgra: np.ndarray, rounds: int, device: int = 0) -> np.ndarra
     if not lib().w2x_alpha_bleed(device, _ptr(src), w, h, src.strides[0], int(rounds), _ptr(out)):
         raise RuntimeError("w2x_alpha_bleed failed")
     return out
+
+
+def resample_table(n_in: int, n_out: int):
+    """The resample's table of one axis n_in -> n_out (include/w2x_dev.h: w2x_resample_table; no GPU needed): (first int32 [n_out],
+    count int32 [n_out], weights float32 [n_out, taps]); output i reads inputs first[i] .. first[i] + count[i] - 1."""
+    l = lib()
+    taps = l.w2x_resample_table(int(n_in), int(n_out), None, None, None, 0)
+    if taps <= 0:
+        raise ValueError(f"resample_table: need 1 <= n_out <= n_in, got {n_in} -> {n_out}")
+    first, count = np.empty(n_out, np.int32), np.empty(n_out, np.int32)
+    weights = np.empty((n_out, taps), np.float32)
+    if l.w2x_resample_table(int(n_in), int(n_out), _ptr(first), _ptr(count), _ptr(weights), weights.size) != taps:
+        raise RuntimeError("w2x_resample_table failed")
+    return first, count, weights
+
+
+def resample(src_bgr: np.ndarray, size: Tuple[int, int], dst: Optional[np.ndarray] = None, device: int = 0) -> np.ndarray:
+    """The resample of Img2Img.render_resized alone (include/w2x_dev.h: w2x_resample): uint8 [H, W, 3] BGR -> uint8 [dst_h, dst_w, 3],
+    size = (dst_w, dst_h) with 1 <= dst_w <= W, 1 <= dst_h <= H.  src and a caller's dst may have strided rows."""
+    src = src_bgr if _rows_of_pixels(src_bgr, 3) else np.ascontiguousarray(src_bgr, dtype=np.uint8)
+    h, w = src.shape[:2]
+    dw, dh = int(size[0]), int(size[1])
+    if dst is None:
+        dst = np.empty((dh, dw, 3), np.uint8)
+    elif not _rows_of_pixels(dst, 3) or dst.shape[:2] != (dh, dw):
+        raise ValueError("dst must be uint8 [dst_h, dst_w, 3] with contiguous pixels")
+    if not lib().w2x_resample(device, _ptr(src), w, h, src.strides[0], _ptr(dst), dw, dh, dst.strides[0]):
+        raise RuntimeError("w2x_resample failed")
+    return dst
 
 
 def run_conv_layer(kind: int, x: np.ndarray, w_packed: np.ndarray, bias: np.ndarray, cout: int, skip: Optional[np.ndarray] = None,
@@ -478,6 +512,26 @@ class Img2Img:
             raise ValueError("dst must be uint8 [H, W, 4] with contiguous pixels")
         ok = self._l.w2x_render_bgra(self._h, _ptr(src), w, h, src.strides[0], _ptr(dst), dst.strides[0])
         return dst if ok else None
+
+    def render_resized(self, src: np.ndarray, size: Tuple[int, int], dst: Optional[np.ndarray] = None) -> Optional[np.ndarray]:
+        """src: uint8 [H, W, 3] BGR (rows may be strided); size = (dst_w, dst_h) with 1 <= dst_w <= W * scaling, 1 <= dst_h <= H * scaling.
+        Returns dst (uint8 [dst_h, dst_w, 3] BGR: render(src) reduced by an antialiased bicubic resample, include/w2x.h w2x_render_resized;
+        a caller's dst may have strided rows) or None on failure (the reason in last_error)."""
+        if not _rows_of_pixels(src, 3):
+            src = np.ascontiguousarray(src, dtype=np.uint8)
+        h, w = src.shape[:2]
+        dw, dh = int(size[0]), int(size[1])
+        if dst is None:
+            dst = np.empty((max(dh, 1), max(dw, 1), 3), np.uint8)
+        elif not _rows_of_pixels(dst, 3):
+            raise ValueError("dst must be uint8 [H, W, 3] with contiguous pixels")
+        ok = self._l.w2x_render_resized(self._h, _ptr(src), w, h, src.strides[0], _ptr(dst), dw, dh, dst.strides[0])
+        return dst if ok else None
+
+    def submit_resized(self, src_ptr: int, w: int, h: int, dst_ptr: int, size: Tuple[int, int]) -> int:
+        """submit with the output of render_resized: dst_ptr holds size[1] rows of 3 * size[0] bytes.  Returns a ticket for wait, or -1."""
+        dw, dh = int(size[0]), int(size[1])
+        return int(self._l.w2x_submit_resized(self._h, C.c_void_p(src_ptr), w, h, w * 3, C.c_void_p(dst_ptr), dw, dh, dw * 3))
 
     def infer(self, x_nchw: np.ndarray) -> Optional[np.ndarray]:
         x = np.ascontiguousarray(x_nchw, dtype=np.float32)
@@ -660,6 +714,11 @@ class Img2ImgPool:
 
     def submit(self, src_ptr: int, w: int, h: int, dst_ptr: int) -> int:
         return int(self._l.w2x_pool_submit(self._h, C.c_void_p(src_ptr), w, h, w * 3, C.c_void_p(dst_ptr), w * self.scaling * 3))
+
+    def submit_resized(self, src_ptr: int, w: int, h: int, dst_ptr: int, size: Tuple[int, int]) -> int:
+        """submit with the output of Img2Img.render_resized: dst_ptr holds size[1] rows of 3 * size[0] bytes."""
+        dw, dh = int(size[0]), int(size[1])
+        return int(self._l.w2x_pool_submit_resized(self._h, C.c_void_p(src_ptr), w, h, w * 3, C.c_void_p(dst_ptr), dw, dh, dw * 3))
 
     def wait(self, ticket: int) -> bool:
         return bool(self._l.w2x_pool_wait(self._h, ticket))
