@@ -125,6 +125,24 @@ W2X_API int w2x_render_resized(w2x_engine* e, const uint8_t* src_bgr, int width,
 W2X_API int w2x_submit_resized(w2x_engine* e, const uint8_t* src_bgr, int width, int height, size_t src_stride, uint8_t* dst_bgr,
                                int dst_width, int dst_height, size_t dst_stride);
 
+/* 16 bits per channel: src BGR u16 HWC (w x h) -> dst BGR u16 (w*scaling x h*scaling), native-endian samples, synchronous like
+ * w2x_render, with any loaded engine (fp16 or tf32, cunet/art or swin_unet, with or without TTA).
+ *  - Strides are in BYTES: src_stride >= 6 * width, dst_stride >= 6 * width * scaling.  Both strides and both pointers must be even.
+ *  - Input: each sample x becomes f32(x) * f32(1/65535) (one rounded multiply), rounded to the engine's element type.  Everything
+ *    else is exactly what w2x_render does: replicate padding, D4 augmentation, BGR -> RGB, the tile grid, batching, the TTA mean, the
+ *    blend weights and the fp32 accumulation order.
+ *  - Output: each sample is saturate_u16(rint(f32(v) * 65535)) of the same fp32 canvas v that w2x_render packs to u8, then RGB -> BGR.
+ *  - fp16 engines: fp16(f32(257 x) * f32(1/65535)) == fp16(f32(x) * f32(1/255)) for every u8 value x, so w2x_render_u16 of 257 * F runs
+ *    the model on exactly the tiles w2x_render of F does, blends the same canvas, and every output sample satisfies
+ *    |out16 - 257 * out8| <= 129.  tf32 engines see the two inputs one fp32 ulp apart and give no such guarantee.
+ * Returns 0 and logs the reason on failure (no engine loaded, null pointers, strides below 6 bytes per pixel, odd strides or pointers).
+ * Not available with an alpha channel, an output size other than the model's, or through w2x_render_banded / w2x_render_device. */
+W2X_API int w2x_render_u16(w2x_engine* e, const uint16_t* src_bgr, int width, int height, size_t src_stride, uint16_t* dst_bgr,
+                           size_t dst_stride);
+/* w2x_render_u16 through the pipeline of w2x_submit: returns a ticket >= 0 for w2x_wait, or -1 with the reason logged. */
+W2X_API int w2x_submit_u16(w2x_engine* e, const uint16_t* src_bgr, int width, int height, size_t src_stride, uint16_t* dst_bgr,
+                           size_t dst_stride);
+
 /* Same as w2x_render but src/dst are DEVICE pointers on cfg.deviceId; enqueued on the engine's stream,
  * returns without synchronising (w2x_sync to wait).  Used for the HBM-resident `value` measurement. */
 W2X_API int w2x_render_device(w2x_engine* e, const uint8_t* d_src_bgr, int width, int height, size_t src_stride,
@@ -161,6 +179,10 @@ W2X_API int w2x_pool_submit(w2x_pool* p, const uint8_t* src_bgr, int width, int 
  * logged through the pool's message callback. */
 W2X_API int w2x_pool_submit_resized(w2x_pool* p, const uint8_t* src_bgr, int width, int height, size_t src_stride, uint8_t* dst_bgr,
                                     int dst_width, int dst_height, size_t dst_stride);
+/* w2x_pool_submit with the frames of w2x_render_u16; a frame the engine refuses fails its w2x_pool_wait, with the reason logged through
+ * the pool's message callback. */
+W2X_API int w2x_pool_submit_u16(w2x_pool* p, const uint16_t* src_bgr, int width, int height, size_t src_stride, uint16_t* dst_bgr,
+                                size_t dst_stride);
 W2X_API int w2x_pool_wait(w2x_pool* p, int ticket);
 W2X_API int w2x_pool_sync(w2x_pool* p);
 W2X_API void* w2x_host_alloc(size_t bytes);   /* cudaHostAlloc (pinned) */

@@ -20,6 +20,17 @@ extern "C" {
  * dst BGRA packed (pitch 4 * width), alpha bytes copied from src.  Returns 1 on success. */
 W2X_API int w2x_alpha_bleed(int device, const uint8_t* src_bgra, int width, int height, size_t src_stride, int rounds, uint8_t* dst_bgra);
 
+/* The u16 twins of w2x_unpack_tiles / w2x_stitch_tiles (the kernels of w2x_render_u16), on host buffers:
+ *  - w2x_unpack_tiles_u16: u16 BGR frame (pitch src_stride >= 6 * width bytes) -> n fp16 RGB0 NHWC4 tiles, each sample x as
+ *    fp16(f32(x) * f32(1/65535)); rects, aug and the replicate padding as w2x_unpack_tiles.
+ *  - w2x_stitch_tiles_u16: fp16 NHWC4 tiles -> u16 BGR canvas (pitch dst_stride >= 6 * canvas_w bytes; the bytes between rows are left
+ *    alone), each sample saturate(rint(65535 v)) of the fp32 blend that w2x_stitch_tiles packs to u8.
+ * Return 1 on success. */
+W2X_API int w2x_unpack_tiles_u16(int device, const uint16_t* src_bgr, int width, int height, size_t src_stride, const w2x_rect* rects,
+                                 const int* aug, int n, int tile, uint16_t* out_f16_nhwc4);
+W2X_API int w2x_stitch_tiles_u16(int device, const uint16_t* tiles_f16_nhwc4, int count, int out_tile, int nx, int ny, int overlap_x,
+                                 int overlap_y, int canvas_w, int canvas_h, uint16_t* dst_bgr, size_t dst_stride);
+
 /* The resample of w2x_render_resized alone, on host buffers: src BGR (w x h, pitch src_stride >= 3 * width) -> dst BGR (dst_width x
  * dst_height, pitch dst_stride >= 3 * dst_width; the bytes between rows are left alone), 1 <= dst_width <= width, 1 <= dst_height <= height.
  * Returns 1 on success. */

@@ -86,6 +86,16 @@ int w2x_submit_resized(w2x_engine* e, const uint8_t* src, int width, int height,
     return e->impl.submitResized(src, width, height, src_stride, dst, dst_width, dst_height, dst_stride);
 }
 
+int w2x_render_u16(w2x_engine* e, const uint16_t* src, int width, int height, size_t src_stride, uint16_t* dst, size_t dst_stride) {
+    if (!e) return 0;
+    return e->impl.renderU16(src, width, height, src_stride, dst, dst_stride) ? 1 : 0;
+}
+
+int w2x_submit_u16(w2x_engine* e, const uint16_t* src, int width, int height, size_t src_stride, uint16_t* dst, size_t dst_stride) {
+    if (!e) return -1;
+    return e->impl.submitU16(src, width, height, src_stride, dst, dst_stride);
+}
+
 int w2x_render_device(w2x_engine* e, const uint8_t* src, int width, int height, size_t src_stride, uint8_t* dst, size_t dst_stride) {
     if (!e || !src || !dst) return 0;
     return e->impl.renderDevice(src, width, height, src_stride, dst, dst_stride) ? 1 : 0;
@@ -134,6 +144,10 @@ int w2x_pool_submit_resized(w2x_pool* p, const uint8_t* src, int width, int heig
         return -1;
     }
     try { return p->impl.submit(src, width, height, src_stride, dst, dst_stride, dst_width, dst_height); } catch (...) { return -1; }
+}
+int w2x_pool_submit_u16(w2x_pool* p, const uint16_t* src, int width, int height, size_t src_stride, uint16_t* dst, size_t dst_stride) {
+    if (!p || !src || !dst) return -1;   // the other refusals come from the engine that takes the frame, through w2x_pool_wait
+    try { return p->impl.submitU16(src, width, height, src_stride, dst, dst_stride); } catch (...) { return -1; }
 }
 int w2x_pool_wait(w2x_pool* p, int ticket) {
     try { return p && p->impl.wait(ticket) ? 1 : 0; } catch (...) { return 0; }
@@ -262,6 +276,60 @@ int w2x_stitch_tiles(int device, const uint16_t* tiles, int count, int out_tile,
         return 1;
     } catch (const std::exception& ex) {
         std::fprintf(stderr, "w2x_stitch_tiles: %s\n", ex.what());
+        return 0;
+    }
+}
+
+int w2x_unpack_tiles_u16(int device, const uint16_t* src, int width, int height, size_t src_stride, const w2x_rect* rects, const int* aug, int n,
+                         int tile, uint16_t* out) {
+    try {
+        if (!src || !rects || !out || n <= 0 || tile <= 0 || width <= 0 || height <= 0 || src_stride < (size_t)width * 6) return 0;
+        W2X_CUDA(cudaSetDevice(device));
+        std::vector<DeviceBuffer> b;
+        const size_t row = (size_t)width * 6;
+        uint8_t* dSrc = alloc<uint8_t>(b, row * height);
+        W2X_CUDA(cudaMemcpy2D(dSrc, row, src, src_stride, row, height, cudaMemcpyHostToDevice));
+        std::vector<TileSlot> slots(n);
+        for (int i = 0; i < n; ++i) slots[i] = {rects[i].x, rects[i].y, aug ? aug[i] : 0, 1};
+        TileSlot* dSlots = alloc<TileSlot>(b, n);
+        W2X_CUDA(cudaMemcpy(dSlots, slots.data(), sizeof(TileSlot) * n, cudaMemcpyHostToDevice));
+        const size_t elems = (size_t)n * tile * tile * 4;
+        __half* dOut = alloc<__half>(b, elems);
+        launchUnpack(dSrc, width, height, row, dSlots, n, tile, dOut, nullptr, 3, 2);
+        W2X_CUDA(cudaGetLastError());
+        W2X_CUDA(cudaMemcpy(out, dOut, elems * 2, cudaMemcpyDeviceToHost));
+        return 1;
+    } catch (const std::exception& ex) {
+        std::fprintf(stderr, "w2x_unpack_tiles_u16: %s\n", ex.what());
+        return 0;
+    }
+}
+
+int w2x_stitch_tiles_u16(int device, const uint16_t* tiles, int count, int out_tile, int nx, int ny, int overlap_x, int overlap_y,
+                         int canvas_w, int canvas_h, uint16_t* dst, size_t dst_stride) {
+    try {
+        if (!tiles || !dst || count != nx * ny || canvas_w <= 0 || canvas_h <= 0 || dst_stride < (size_t)canvas_w * 6) return 0;
+        W2X_CUDA(cudaSetDevice(device));
+        std::vector<DeviceBuffer> b;
+        const size_t elems = (size_t)count * out_tile * out_tile * 4;
+        __half* dT = alloc<__half>(b, elems);
+        W2X_CUDA(cudaMemcpy(dT, tiles, elems * 2, cudaMemcpyHostToDevice));
+        std::vector<float> rx = blendRamp(overlap_x), ry = blendRamp(overlap_y);
+        float* dRx = alloc<float>(b, rx.size() + 1);
+        float* dRy = alloc<float>(b, ry.size() + 1);
+        if (!rx.empty()) W2X_CUDA(cudaMemcpy(dRx, rx.data(), rx.size() * 4, cudaMemcpyHostToDevice));
+        if (!ry.empty()) W2X_CUDA(cudaMemcpy(dRy, ry.data(), ry.size() * 4, cudaMemcpyHostToDevice));
+        const size_t row = (size_t)canvas_w * 6;
+        uint8_t* dDst = alloc<uint8_t>(b, row * canvas_h);
+        StitchParams sp{};
+        sp.tiles = dT; sp.f32 = 0; sp.outT = out_tile; sp.nx = nx; sp.ny = ny; sp.ovx = overlap_x; sp.ovy = overlap_y;
+        sp.cw = canvas_w; sp.ch = canvas_h; sp.rampx = dRx; sp.rampy = dRy; sp.dst = dDst; sp.pitch = row; sp.u16 = 1;
+        launchStitch(sp, nullptr);
+        W2X_CUDA(cudaGetLastError());
+        W2X_CUDA(cudaMemcpy2D(dst, dst_stride, dDst, row, row, canvas_h, cudaMemcpyDeviceToHost));
+        return 1;
+    } catch (const std::exception& ex) {
+        std::fprintf(stderr, "w2x_stitch_tiles_u16: %s\n", ex.what());
         return 0;
     }
 }

@@ -1007,7 +1007,7 @@ void Engine::ensureResize(int cw, int ch, int dw, int dh) {
 }
 
 void Engine::renderOnStream(const uint8_t* dSrc, int w, int h, size_t srcPitch, uint8_t* dDst, size_t dstPitch, cudaStream_t s, bool timed,
-                            std::vector<BandDone>* bands, int pixelBytes, int dstW, int dstH) {
+                            std::vector<BandDone>* bands, int pixelBytes, int sampleBytes, int dstW, int dstH) {
     if (timed) { timing.used = 0; timing.spans.clear(); }
     auto span = [&](int kind, auto&& fn) {
         if (!timed) { fn(); return; }
@@ -1057,7 +1057,7 @@ void Engine::renderOnStream(const uint8_t* dSrc, int w, int h, size_t srcPitch, 
     // a resized frame is stitched into the engine's canvas and resampled from there into dDst
     const bool resized = dstW != cw || dstH != ch;
     if (resized) {
-        if (pixelBytes != 3) throw Error("resized output is BGR only");
+        if (pixelBytes != 3 || sampleBytes != 1) throw Error("resized output is u8 BGR only");
         ensureResize(cw, ch, dstW, dstH);
     }
     const TileGrid& grid = fc.grid;
@@ -1075,6 +1075,7 @@ void Engine::renderOnStream(const uint8_t* dSrc, int w, int h, size_t srcPitch, 
         sp.tile_map = cfg.tta ? nullptr : fc.tileMap.get<int>();
         sp.y_begin = yBegin; sp.y_end = yEnd;
         sp.bgra = pixelBytes == 4 ? 1 : 0;
+        sp.u16 = sampleBytes == 2 ? 1 : 0;
         sp.alpha_off = passes == 2 ? grid.count : 0;   // TTA: index of the reduced alpha tile; else the alpha step of the tile's slot
         launchStitch(sp, s);
         ++launches;
@@ -1101,7 +1102,7 @@ void Engine::renderOnStream(const uint8_t* dSrc, int w, int h, size_t srcPitch, 
     const bool frameWide = frameWideUnpack();
     if (frameWide)
         span(0, [&] {
-            unpackTiles(dSrc, w, h, srcPitch, fc.slots.get<TileSlot>(), realSteps, fc.unpacked.get(), s, pixelBytes);
+            unpackTiles(dSrc, w, h, srcPitch, fc.slots.get<TileSlot>(), realSteps, fc.unpacked.get(), s, pixelBytes, sampleBytes);
             ++launches;
         });
     for (int b = 0; b < fc.batchCount; ++b) {
@@ -1110,7 +1111,7 @@ void Engine::renderOnStream(const uint8_t* dSrc, int w, int h, size_t srcPitch, 
         if (nReal <= 0) continue;
         if (!frameWide)
             span(0, [&] {
-                unpackTiles(dSrc, w, h, srcPitch, fc.slots.get<TileSlot>() + (size_t)b * batch, nReal, actIn.p, s, pixelBytes);
+                unpackTiles(dSrc, w, h, srcPitch, fc.slots.get<TileSlot>() + (size_t)b * batch, nReal, actIn.p, s, pixelBytes, sampleBytes);
                 ++launches;
             });
         span(1, [&] { runModel(s, elemAt(fc.tileOut.get(), (size_t)b * batch * tileElems), nReal, frameWide ? elemAt(fc.unpacked.get(), (size_t)b * batch * inElems) : nullptr); });
@@ -1151,9 +1152,10 @@ void Engine::renderOnStream(const uint8_t* dSrc, int w, int h, size_t srcPitch, 
     W2X_CUDA(cudaGetLastError());
 }
 
-void Engine::unpackTiles(const uint8_t* src, int w, int h, size_t pitch, const TileSlot* slots, int n, void* out, cudaStream_t s, int pixelBytes) {
-    if (tf32()) launchUnpack(src, w, h, pitch, slots, n, tile, static_cast<float*>(out), s, pixelBytes);
-    else launchUnpack(src, w, h, pitch, slots, n, tile, static_cast<__half*>(out), s, pixelBytes);
+void Engine::unpackTiles(const uint8_t* src, int w, int h, size_t pitch, const TileSlot* slots, int n, void* out, cudaStream_t s, int pixelBytes,
+                         int sampleBytes) {
+    if (tf32()) launchUnpack(src, w, h, pitch, slots, n, tile, static_cast<float*>(out), s, pixelBytes, sampleBytes);
+    else launchUnpack(src, w, h, pitch, slots, n, tile, static_cast<__half*>(out), s, pixelBytes, sampleBytes);
 }
 
 void Engine::ttaReduce(const void* outs, int tiles, float* mean, cudaStream_t s) {
@@ -1215,7 +1217,7 @@ bool Engine::renderDevice(const uint8_t* dSrc, int w, int h, size_t srcStride, u
 bool Engine::render(const uint8_t* src, int w, int h, size_t srcStride, uint8_t* dst, size_t dstStride) {
     try {
         if (!isLoaded) throw Error("no engine loaded");
-        renderHostFrame(src, w, h, srcStride, dst, dstStride, 3, w * scale, h * scale);
+        renderHostFrame(src, w, h, srcStride, dst, dstStride, 3, 1, w * scale, h * scale);
         return true;
     } catch (const std::exception& ex) {
         ELOG(W2X_ERROR, std::string("Render failed unexpectedly: ") + ex.what() + ".");
@@ -1229,7 +1231,7 @@ bool Engine::renderBgra(const uint8_t* src, int w, int h, size_t srcStride, uint
         if (!src || !dst) throw Error("null image pointer");
         if (w <= 0 || h <= 0) throw Error("invalid frame size");
         if (srcStride < (size_t)w * 4 || dstStride < (size_t)w * scale * 4) throw Error("row stride is smaller than 4 bytes per pixel");
-        renderHostFrame(src, w, h, srcStride, dst, dstStride, 4, w * scale, h * scale);
+        renderHostFrame(src, w, h, srcStride, dst, dstStride, 4, 1, w * scale, h * scale);
         return true;
     } catch (const std::exception& ex) {
         ELOG(W2X_ERROR, std::string("Render failed unexpectedly: ") + ex.what() + ".");
@@ -1251,7 +1253,7 @@ bool Engine::renderResized(const uint8_t* src, int w, int h, size_t srcStride, u
         if (!isLoaded) throw Error("no engine loaded");
         checkResized(src, w, h, dst, dstW, dstH, dstStride);
         if (srcStride < (size_t)w * 3) throw Error("row stride is smaller than 3 bytes per pixel");
-        renderHostFrame(src, w, h, srcStride, dst, dstStride, 3, dstW, dstH);
+        renderHostFrame(src, w, h, srcStride, dst, dstStride, 3, 1, dstW, dstH);
         return true;
     } catch (const std::exception& ex) {
         ELOG(W2X_ERROR, std::string("Render failed unexpectedly: ") + ex.what() + ".");
@@ -1259,9 +1261,41 @@ bool Engine::renderResized(const uint8_t* src, int w, int h, size_t srcStride, u
     }
 }
 
-void Engine::renderHostFrame(const uint8_t* src, int w, int h, size_t srcStride, uint8_t* dst, size_t dstStride, int pixelBytes, int dstW, int dstH) {
+void Engine::checkU16(const uint16_t* src, int w, int h, size_t srcStride, const uint16_t* dst, size_t dstStride) const {
+    if (!src || !dst) throw Error("null image pointer");
+    if (w <= 0 || h <= 0) throw Error("invalid frame size");
+    if (srcStride < (size_t)w * 6 || dstStride < (size_t)w * scale * 6) throw Error("row stride is smaller than 6 bytes per pixel");
+    if ((srcStride | dstStride) & 1) throw Error("row stride is odd (u16 rows must be 2-byte aligned)");
+    if ((reinterpret_cast<uintptr_t>(src) | reinterpret_cast<uintptr_t>(dst)) & 1) throw Error("image pointer is odd (u16 samples must be 2-byte aligned)");
+}
+
+bool Engine::renderU16(const uint16_t* src, int w, int h, size_t srcStride, uint16_t* dst, size_t dstStride) {
+    try {
+        if (!isLoaded) throw Error("no engine loaded");
+        checkU16(src, w, h, srcStride, dst, dstStride);
+        renderHostFrame(reinterpret_cast<const uint8_t*>(src), w, h, srcStride, reinterpret_cast<uint8_t*>(dst), dstStride, 3, 2, w * scale, h * scale);
+        return true;
+    } catch (const std::exception& ex) {
+        ELOG(W2X_ERROR, std::string("Render failed unexpectedly: ") + ex.what() + ".");
+        return false;
+    }
+}
+
+int Engine::submitU16(const uint16_t* src, int w, int h, size_t srcStride, uint16_t* dst, size_t dstStride) {
+    try {
+        if (!isLoaded) throw Error("no engine loaded");
+        checkU16(src, w, h, srcStride, dst, dstStride);
+        return submitFrame(reinterpret_cast<const uint8_t*>(src), w, h, srcStride, reinterpret_cast<uint8_t*>(dst), w * scale, h * scale, dstStride, 2);
+    } catch (const std::exception& ex) {
+        ELOG(W2X_ERROR, std::string("Submit failed unexpectedly: ") + ex.what() + ".");
+        return -1;
+    }
+}
+
+void Engine::renderHostFrame(const uint8_t* src, int w, int h, size_t srcStride, uint8_t* dst, size_t dstStride, int pixelBytes, int sampleBytes,
+                             int dstW, int dstH) {
     W2X_CUDA(cudaSetDevice(cfg.deviceId));
-    const size_t ipitch = (size_t)w * pixelBytes, opitch = (size_t)dstW * pixelBytes;
+    const size_t ipitch = (size_t)w * pixelBytes * sampleBytes, opitch = (size_t)dstW * pixelBytes * sampleBytes;
     staging.in.ensure(ipitch * h);
     staging.out.ensure(opitch * dstH);
     uint8_t *dIn = staging.in.get<uint8_t>(), *dOut = staging.out.get<uint8_t>();
@@ -1270,7 +1304,7 @@ void Engine::renderHostFrame(const uint8_t* src, int w, int h, size_t srcStride,
     // ordered behind its band's stitch only, so the download of a band overlaps the batches still computing (the reference downloads
     // the whole canvas after the last batch, render.cpp:344).  With --tta, and for BGRA frames, there is one band: the whole frame.
     std::vector<BandDone> bands;
-    renderOnStream(dIn, w, h, ipitch, dOut, opitch, stream, true, &bands, pixelBytes, dstW, dstH);
+    renderOnStream(dIn, w, h, ipitch, dOut, opitch, stream, true, &bands, pixelBytes, sampleBytes, dstW, dstH);
     if (bands.empty()) {
         W2X_CUDA(cudaMemcpy2DAsync(dst, dstStride, dOut, opitch, opitch, (size_t)dstH, cudaMemcpyDeviceToHost, stream));  // render.cpp:344
     } else {
@@ -1307,20 +1341,20 @@ int Engine::submitResized(const uint8_t* src, int w, int h, size_t srcStride, ui
     }
 }
 
-int Engine::submitFrame(const uint8_t* src, int w, int h, size_t srcStride, uint8_t* dst, int dstW, int dstH, size_t dstStride) {
+int Engine::submitFrame(const uint8_t* src, int w, int h, size_t srcStride, uint8_t* dst, int dstW, int dstH, size_t dstStride, int sampleBytes) {
     W2X_CUDA(cudaSetDevice(cfg.deviceId));
     const int ticket = nextTicket;
     PipeSlot& ps = pipe[ticket % kSlots];
     if (ps.busy) { W2X_CUDA(cudaEventSynchronize(ps.evDone.get())); ps.busy = false; }
-    const size_t opitch = (size_t)dstW * 3;
-    ps.in.ensure((size_t)w * 3 * h);
+    const size_t ipitch = (size_t)w * 3 * sampleBytes, opitch = (size_t)dstW * 3 * sampleBytes;
+    ps.in.ensure(ipitch * h);
     ps.out.ensure(opitch * dstH);
     uint8_t *dIn = ps.in.get<uint8_t>(), *dOut = ps.out.get<uint8_t>();
     ensureFrameBuffers(w, h);
-    W2X_CUDA(cudaMemcpy2DAsync(dIn, (size_t)w * 3, src, srcStride, (size_t)w * 3, h, cudaMemcpyHostToDevice, h2dStream));
+    W2X_CUDA(cudaMemcpy2DAsync(dIn, ipitch, src, srcStride, ipitch, h, cudaMemcpyHostToDevice, h2dStream));
     W2X_CUDA(cudaEventRecord(ps.evH2D.get(), h2dStream));
     W2X_CUDA(cudaStreamWaitEvent(stream, ps.evH2D.get(), 0));
-    renderOnStream(dIn, w, h, (size_t)w * 3, dOut, opitch, stream, false, nullptr, 3, dstW, dstH);
+    renderOnStream(dIn, w, h, ipitch, dOut, opitch, stream, false, nullptr, 3, sampleBytes, dstW, dstH);
     W2X_CUDA(cudaEventRecord(ps.evComp.get(), stream));
     W2X_CUDA(cudaStreamWaitEvent(d2hStream, ps.evComp.get(), 0));
     W2X_CUDA(cudaMemcpy2DAsync(dst, dstStride, dOut, opitch, opitch, (size_t)dstH, cudaMemcpyDeviceToHost, d2hStream));

@@ -161,6 +161,10 @@ public:
     // w2x_render_resized): 1 <= dstW <= w*scale, 1 <= dstH <= h*scale, dst pitch >= 3 * dstW.  The canvas size is render, byte for byte.
     bool renderResized(const uint8_t* src, int w, int h, size_t srcStride, uint8_t* dst, int dstW, int dstH, size_t dstStride);
     int submitResized(const uint8_t* src, int w, int h, size_t srcStride, uint8_t* dst, int dstW, int dstH, size_t dstStride);
+    // u16 BGR host buffers (include/w2x.h, w2x_render_u16): strides in bytes, >= 6 per pixel, even, as are the pointers.  The input is
+    // scaled by f32(1/65535), the output is saturate(rint(65535 v)) of render's fp32 canvas; tiles, batches and blending are render's.
+    bool renderU16(const uint16_t* src, int w, int h, size_t srcStride, uint16_t* dst, size_t dstStride);
+    int submitU16(const uint16_t* src, int w, int h, size_t srcStride, uint16_t* dst, size_t dstStride);
     bool wait(int ticket);
     // one image sharded over several engines (one per GPU) by bands of tile rows, seam rows exchanged peer-to-peer
     static bool renderBanded(Engine* const* engines, int count, const uint8_t* src, int w, int h, size_t srcStride, uint8_t* dst, size_t dstStride);
@@ -197,7 +201,8 @@ private:
     bool tf32() const { return elemBytes == 4; }
     // element `i` of an activation / tile buffer of this engine's element type
     void* elemAt(void* base, size_t i) const { return static_cast<uint8_t*>(base) + i * elemBytes; }
-    void unpackTiles(const uint8_t* src, int w, int h, size_t pitch, const TileSlot* slots, int n, void* out, cudaStream_t s, int pixelBytes = 3);
+    void unpackTiles(const uint8_t* src, int w, int h, size_t pitch, const TileSlot* slots, int n, void* out, cudaStream_t s, int pixelBytes = 3,
+                     int sampleBytes = 1);
     void ttaReduce(const void* outs, int tiles, float* mean, cudaStream_t s);
     bool frameWideUnpack() const;
     // passes: 1 = the colour tiles, 2 = the colour tiles followed by the alpha tiles of a BGRA frame (renderBgra)
@@ -208,11 +213,16 @@ private:
     // pixelBytes 4: packed BGRA frames (dSrcPitch = 4w): alpha scan, colour bleed and alpha pass as the frame needs them; no bands
     // dstW x dstH other than the canvas (BGR only): stitch into resize.canvas, then resample into dDst; with bands, the bands are output
     // rows of dDst
+    // sampleBytes 2: u16 BGR frames in and out (pitches in bytes), canvas size only; the tiles, batches and bands are those of u8 frames
     void renderOnStream(const uint8_t* dSrc, int w, int h, size_t srcPitch, uint8_t* dDst, size_t dstPitch, cudaStream_t s, bool timed,
-                        std::vector<BandDone>* bands = nullptr, int pixelBytes = 3, int dstW = 0, int dstH = 0);
-    // render / renderBgra / renderResized: host frame -> staging buffers -> renderOnStream -> host frame (dstW x dstH), synchronous
-    void renderHostFrame(const uint8_t* src, int w, int h, size_t srcStride, uint8_t* dst, size_t dstStride, int pixelBytes, int dstW, int dstH);
-    int submitFrame(const uint8_t* src, int w, int h, size_t srcStride, uint8_t* dst, int dstW, int dstH, size_t dstStride);
+                        std::vector<BandDone>* bands = nullptr, int pixelBytes = 3, int sampleBytes = 1, int dstW = 0, int dstH = 0);
+    // render / renderBgra / renderResized / renderU16: host frame -> staging buffers -> renderOnStream -> host frame (dstW x dstH),
+    // synchronous
+    void renderHostFrame(const uint8_t* src, int w, int h, size_t srcStride, uint8_t* dst, size_t dstStride, int pixelBytes, int sampleBytes,
+                         int dstW, int dstH);
+    int submitFrame(const uint8_t* src, int w, int h, size_t srcStride, uint8_t* dst, int dstW, int dstH, size_t dstStride, int sampleBytes = 1);
+    // the refusals of renderU16 / submitU16 (throws Error)
+    void checkU16(const uint16_t* src, int w, int h, size_t srcStride, const uint16_t* dst, size_t dstStride) const;
     // the refusals of renderResized / submitResized (throws Error)
     void checkResized(const uint8_t* src, int w, int h, const uint8_t* dst, int dstW, int dstH, size_t dstStride) const;
     void ensureResize(int cw, int ch, int dw, int dh);
@@ -258,7 +268,7 @@ private:
         DeviceBuffer rampX, rampY;       // blend ramps of rampXLen / rampYLen entries
         int rampXLen = -1, rampYLen = -1;
     } fc;
-    // host-buffer paths: the frame on the device (render, renderBgra, renderBanded)
+    // host-buffer paths: the frame on the device (render, renderBgra, renderResized, renderU16, renderBanded), sized in bytes
     struct HostStaging { DeviceBuffer in, out; } staging;
     // BGRA frames: alpha-scan flags (2 ints) and the two ping-pong buffers of the colour bleed
     struct BgraScratch { DeviceBuffer flags, bleed[2]; } bgra;
@@ -274,7 +284,7 @@ private:
     // pipelined submit
     static constexpr int kSlots = 3;
     struct PipeSlot {
-        DeviceBuffer in, out;
+        DeviceBuffer in, out;            // bytes: u8 and u16 frames share them
         CudaEvent evH2D{cudaEventDisableTiming}, evComp{cudaEventDisableTiming}, evDone{cudaEventDisableTiming};
         bool busy = false;
     };

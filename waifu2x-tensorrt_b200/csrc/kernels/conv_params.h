@@ -259,11 +259,12 @@ void launchScaleWeights(const __half* w, __half* wOut, const float* scale, int n
 // alpha byte of a BGRA frame as R = G = B (the alpha pass of Engine::renderBgra)
 struct TileSlot { int x, y, aug, valid; };
 constexpr int kSlotAlpha = 2;
-// pixelBytes: 3 = BGR frame, 4 = BGRA frame
+// pixelBytes: 3 = BGR frame, 4 = BGRA frame; sampleBytes: 1 = u8 samples, 2 = native-endian u16 samples (BGR only, 2-byte aligned
+// frame and pitch)
 void launchUnpack(const uint8_t* frame, int w, int h, size_t pitch, const TileSlot* slots, int nslots, int tile,
-                  __half* out, cudaStream_t s, int pixelBytes = 3);
+                  __half* out, cudaStream_t s, int pixelBytes = 3, int sampleBytes = 1);
 void launchUnpack(const uint8_t* frame, int w, int h, size_t pitch, const TileSlot* slots, int nslots, int tile,
-                  float* out, cudaStream_t s, int pixelBytes = 3);  // tf32 engines: the reference's convertTo(CV_32F, 1/255) blob exactly
+                  float* out, cudaStream_t s, int pixelBytes = 3, int sampleBytes = 1);  // tf32 engines: the reference's convertTo(CV_32F, 1/255) blob exactly
 struct StitchParams {
     const void* tiles;   // [count][outT][outT][4] fp16 or f32
     int f32;             // element type of tiles
@@ -278,6 +279,8 @@ struct StitchParams {
     const int* tile_map;
     // BGRA canvas (4-byte pixels); alpha_off > 0: the alpha pass's tile of reference tile t is at slot(t) + alpha_off, else alpha = 255
     int bgra, alpha_off;
+    // u16 BGR canvas (6-byte pixels, saturate(rint(65535 v)) per sample); bgra must be 0
+    int u16;
 };
 void launchStitch(const StitchParams& p, cudaStream_t s);
 // BGRA frames (kernels/alpha.cu), packed w x h x 4 bytes on the device.

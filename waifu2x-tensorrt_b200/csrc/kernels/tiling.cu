@@ -77,17 +77,20 @@ template <> struct Px4<float> {
 // bytes each, 128 for BGRA) in shared memory with coalesced loads -- 32-bit words from the 4-byte-aligned start of each row segment
 // when the segment lies inside the frame, clamped byte loads on border blocks -- and then every thread converts four pixels, reading
 // the staged bytes at the mirrored / transposed position, and writes them with 8-byte stores (256 contiguous bytes per warp).
-// PS = source bytes per pixel: 3 (BGR) or 4 (BGRA; a slot with valid == kSlotAlpha reads the alpha byte into R, G and B).
+// PS = source samples per pixel: 3 (BGR) or 4 (BGRA; a slot with valid == kSlotAlpha reads the alpha byte into R, G and B).
+// S = source sample type: uint8_t (scaled by 1/255) or uint16_t (BGR only, scaled by 1/65535; 192 source bytes per staged row).
 constexpr int kUB = 32;             // block edge
 // staged bytes per source row: BGR 96 + up to 3 alignment bytes, rounded up to a word multiple; BGRA rows are word-aligned (128 bytes),
-// padded by one word so that the column reads of the transposed augmentations do not all hit one bank
-template <int PS> constexpr int kURow = PS == 3 ? 104 : 132;
+// padded by one word so that the column reads of the transposed augmentations do not all hit one bank; u16 BGR 192 + up to 2
+// alignment bytes, rounded up to an odd number of words (49) for the same reason
+template <int PS, typename S> constexpr int kURow = sizeof(S) == 2 ? 196 : PS == 3 ? 104 : 132;
 
-template <typename T, int PS>
+template <typename T, int PS, typename S = uint8_t>
 __global__ void __launch_bounds__(256) unpack_kernel(const uint8_t* __restrict__ frame, int w, int h, size_t pitch,
                                                      const TileSlot* __restrict__ slots, int tile, int wordOk,
                                                      T* __restrict__ out) {
-    constexpr int kRow = kURow<PS>;
+    static_assert(sizeof(S) == 1 || PS == 3, "u16 frames are BGR");
+    constexpr int kRow = kURow<PS, S>;
     __shared__ __align__(16) uint8_t sm[kUB * kRow];
     __shared__ int smOff[kUB];      // byte offset of local source column 0 inside each staged row (fast path: alignment slack)
     const int blocksPerSide = (tile + kUB - 1) / kUB;
@@ -118,6 +121,28 @@ __global__ void __launch_bounds__(256) unpack_kernel(const uint8_t* __restrict__
     for (int lr = ty; lr < rows; lr += 8) {
         const int sy = min(max(ts.y + rrMin + lr, 0), h - 1);
         const uint8_t* rowp = frame + (size_t)sy * pitch;
+        if constexpr (sizeof(S) == 2) {
+            // u16 BGR: the 192-byte segment starts 2-byte aligned.  Fast path: the words from the 4-byte-aligned start that cover it
+            // (48 or 49; the last one ends at most 2 bytes behind the segment, inside the row); else clamped sample loads.
+            const size_t segStart = (size_t)sy * pitch + (size_t)x0 * 6;
+            if (inside && wordOk && (size_t)(x0 + kUB) * 6 + 2 <= pitch) {
+                const size_t a = segStart & ~(size_t)3;
+                const int off = (int)(segStart - a), nw = (off + kUB * 6 + 3) >> 2;
+                for (int q = tx; q < nw; q += 32)
+                    *reinterpret_cast<uint32_t*>(sm + lr * kRow + 4 * q) = *reinterpret_cast<const uint32_t*>(frame + a + 4 * q);
+                if (tx == 0) smOff[lr] = off;
+            } else {
+                const uint16_t* rows16 = reinterpret_cast<const uint16_t*>(rowp);
+                uint16_t* d = reinterpret_cast<uint16_t*>(sm + lr * kRow);
+                for (int e = tx; e < cols * 3; e += 32) {
+                    const int cc = e / 3, ch = e - cc * 3;
+                    const int sx = min(max(x0 + cc, 0), w - 1);   // BORDER_REPLICATE
+                    d[e] = rows16[(size_t)sx * 3 + ch];
+                }
+                if (tx == 0) smOff[lr] = 0;
+            }
+            continue;
+        }
         const size_t segStart = (size_t)sy * pitch + (size_t)x0 * PS;  // byte offset of the segment from `frame`
         // fast path: whole 32-pixel segment inside the row and (BGR) at least 4 bytes of the row (or the next row) behind it; a BGRA
         // segment is word-aligned (wordOk includes pitch % 4 == 0) and read exactly
@@ -138,6 +163,21 @@ __global__ void __launch_bounds__(256) unpack_kernel(const uint8_t* __restrict__
         }
     }
     __syncthreads();
+    if constexpr (sizeof(S) == 2) {
+        const float k = 1.0f / 65535.0f;  // f32(1/65535): a u16 sample 257x gives the fp16 of the u8 sample x
+#pragma unroll
+        for (int i = 0; i < 4; ++i) {
+            const int r = r0 + ty + 8 * i, c = c0 + tx;
+            if (r >= tile || c >= tile) continue;
+            int rr, cc;
+            augSrcIndex(ts.aug, r, c, tile, rr, cc);
+            const int lr = rr - rrMin;
+            const uint16_t* px = reinterpret_cast<const uint16_t*>(sm + lr * kRow + smOff[lr] + (cc - ccMin) * 6);
+            const float b = __fmul_rn((float)px[0], k), g = __fmul_rn((float)px[1], k), rch = __fmul_rn((float)px[2], k);
+            storePx(outp, (size_t)r * tile + c, rch, g, b);
+        }
+        return;
+    }
     const float k = 1.0f / 255.0f;  // float(1.0/255.0), infer.cpp:19
 #pragma unroll
     for (int i = 0; i < 4; ++i) {
@@ -159,21 +199,22 @@ __global__ void __launch_bounds__(256) unpack_kernel(const uint8_t* __restrict__
 
 template <typename T>
 void launchUnpackT(const uint8_t* frame, int w, int h, size_t pitch, const TileSlot* slots, int nslots, int tile, T* out, cudaStream_t s,
-                   int pixelBytes) {
+                   int pixelBytes, int sampleBytes) {
     if (nslots <= 0) return;
     const int side = (tile + kUB - 1) / kUB;
     dim3 grid(side * side, nslots);
     const bool aligned = (reinterpret_cast<uintptr_t>(frame) & 3) == 0;
-    if (pixelBytes == 4) unpack_kernel<T, 4><<<grid, 256, 0, s>>>(frame, w, h, pitch, slots, tile, aligned && (pitch & 3) == 0 ? 1 : 0, out);
+    if (sampleBytes == 2) unpack_kernel<T, 3, uint16_t><<<grid, 256, 0, s>>>(frame, w, h, pitch, slots, tile, aligned ? 1 : 0, out);  // BGR
+    else if (pixelBytes == 4) unpack_kernel<T, 4><<<grid, 256, 0, s>>>(frame, w, h, pitch, slots, tile, aligned && (pitch & 3) == 0 ? 1 : 0, out);
     else unpack_kernel<T, 3><<<grid, 256, 0, s>>>(frame, w, h, pitch, slots, tile, aligned ? 1 : 0, out);
 }
 void launchUnpack(const uint8_t* frame, int w, int h, size_t pitch, const TileSlot* slots, int nslots, int tile, __half* out, cudaStream_t s,
-                  int pixelBytes) {
-    launchUnpackT(frame, w, h, pitch, slots, nslots, tile, out, s, pixelBytes);
+                  int pixelBytes, int sampleBytes) {
+    launchUnpackT(frame, w, h, pitch, slots, nslots, tile, out, s, pixelBytes, sampleBytes);
 }
 void launchUnpack(const uint8_t* frame, int w, int h, size_t pitch, const TileSlot* slots, int nslots, int tile, float* out, cudaStream_t s,
-                  int pixelBytes) {
-    launchUnpackT(frame, w, h, pitch, slots, nslots, tile, out, s, pixelBytes);
+                  int pixelBytes, int sampleBytes) {
+    launchUnpackT(frame, w, h, pitch, slots, nslots, tile, out, s, pixelBytes, sampleBytes);
 }
 
 // ---- stitch + pack ----------------------------------------------------------------------------------
@@ -194,12 +235,14 @@ __device__ __forceinline__ void loadTilePx(const void* tiles, size_t idx, float&
 // is computed once per block (threads 0..kSR-1) and broadcast through shared memory, and the tile reads of a warp are 256
 // contiguous bytes.  Along each axis a pixel is covered by at most two tiles (stride = outT - ov > outT / 2).  The packed BGR bytes
 // of a row (768 per block) are staged in shared memory and leave as 16-byte vector stores (scalar on unaligned canvases / tails).
-// PB = output bytes per pixel: 3 (BGR) or 4 (BGRA).  A BGRA pixel blends the alpha pass's tile of the same reference tile (slot +
+// PB = output samples per pixel: 3 (BGR) or 4 (BGRA); O = output sample type: uint8_t, or uint16_t (BGR only: 1536 bytes per block
+// row, saturate(rint(65535 v)) of the same fp32 canvas).  A BGRA pixel blends the alpha pass's tile of the same reference tile (slot +
 // alpha_off) with the same weights in the same order, and packs the mean of its three channels as alpha; without an alpha pass
 // (alpha_off == 0) alpha is 255.
 constexpr int kSW = 256, kSR = 16;
 
 __device__ __forceinline__ uint8_t packU8(float v) { return (uint8_t)min(max(__float2int_rn(__fmul_rn(v, 255.f)), 0), 255); }
+__device__ __forceinline__ uint16_t packU16(float v) { return (uint16_t)min(max(__float2int_rn(__fmul_rn(v, 65535.f)), 0), 65535); }
 
 struct StitchRow {
     int n;            // covering tile rows (0 past the band end)
@@ -207,9 +250,11 @@ struct StitchRow {
     float wt[2], wb[2];
 };
 
-template <bool F32, int PB>
+template <bool F32, int PB, typename O = uint8_t>
 __global__ void __launch_bounds__(kSW) stitch_kernel(StitchParams p, int vecOk) {
-    __shared__ __align__(16) uint8_t sm[kSR][kSW * PB];
+    static_assert(sizeof(O) == 1 || PB == 3, "u16 canvases are BGR");
+    constexpr int kOB = PB * (int)sizeof(O);   // output bytes per pixel
+    __shared__ __align__(16) uint8_t sm[kSR][kSW * kOB];
     __shared__ StitchRow rowInfo[kSR];
     const int ox0 = blockIdx.x * kSW, ox = ox0 + threadIdx.x;
     const int oyBase = p.y_begin + blockIdx.y * kSR;
@@ -308,6 +353,13 @@ __global__ void __launch_bounds__(kSW) stitch_kernel(StitchParams p, int vecOk) 
                 }
             }
         }
+        if constexpr (sizeof(O) == 2) {
+            uint16_t* d = reinterpret_cast<uint16_t*>(sm[row]) + threadIdx.x * 3;
+            d[0] = packU16(accb);
+            d[1] = packU16(accg);
+            d[2] = packU16(accr);
+            continue;
+        }
         // convertTo(CV_8UC3, 255): saturate_cast<uchar>(rint(v * 255)) (render.cpp:342), then RGB -> BGR (:343)
         uint8_t* d = sm[row] + threadIdx.x * PB;
         d[0] = packU8(accb);
@@ -316,23 +368,23 @@ __global__ void __launch_bounds__(kSW) stitch_kernel(StitchParams p, int vecOk) 
         if (PB == 4) d[3] = alpha ? packU8(__fdiv_rn(__fadd_rn(__fadd_rn(alr, alg), alb), 3.f)) : (uint8_t)255;
     }
     __syncthreads();
-    const int nbytes = min(kSW, p.cw - ox0) * PB;
+    const int nbytes = min(kSW, p.cw - ox0) * kOB;
     if (nbytes <= 0) return;
     const int rowsHere = min(kSR, p.y_end - oyBase);
     if (vecOk) {
-        const int nvec = nbytes >> 4;                       // 48 (BGRA: 64) vectors per full row
+        const int nvec = nbytes >> 4;                       // 48 (BGRA: 64, u16 BGR: 96) vectors per full row
         for (int v = threadIdx.x; v < nvec * rowsHere; v += kSW) {
             const int row = v / nvec, c = v - row * nvec;
-            reinterpret_cast<uint4*>(p.dst + (size_t)(oyBase + row) * p.pitch + (size_t)ox0 * PB)[c] = reinterpret_cast<const uint4*>(sm[row])[c];
+            reinterpret_cast<uint4*>(p.dst + (size_t)(oyBase + row) * p.pitch + (size_t)ox0 * kOB)[c] = reinterpret_cast<const uint4*>(sm[row])[c];
         }
         const int tail = nbytes - (nvec << 4);
         for (int b = threadIdx.x; b < tail * rowsHere; b += kSW) {
             const int row = b / tail, c = (nvec << 4) + b - row * tail;
-            p.dst[(size_t)(oyBase + row) * p.pitch + (size_t)ox0 * PB + c] = sm[row][c];
+            p.dst[(size_t)(oyBase + row) * p.pitch + (size_t)ox0 * kOB + c] = sm[row][c];
         }
     } else {
         for (int row = 0; row < rowsHere; ++row)
-            for (int b = threadIdx.x; b < nbytes; b += kSW) p.dst[(size_t)(oyBase + row) * p.pitch + (size_t)ox0 * PB + b] = sm[row][b];
+            for (int b = threadIdx.x; b < nbytes; b += kSW) p.dst[(size_t)(oyBase + row) * p.pitch + (size_t)ox0 * kOB + b] = sm[row][b];
     }
 }
 
@@ -341,9 +393,12 @@ void launchStitch(const StitchParams& pin, cudaStream_t s) {
     if (p.y_end <= 0) { p.y_begin = 0; p.y_end = p.ch; }  // whole canvas
     if (p.y_end <= p.y_begin) return;
     dim3 grid((p.cw + kSW - 1) / kSW, (p.y_end - p.y_begin + kSR - 1) / kSR);
-    // 16-byte stores need 16-byte aligned row segments: block columns start at multiples of 768 (BGRA: 1024) bytes
+    // 16-byte stores need 16-byte aligned row segments: block columns start at multiples of 768 (BGRA: 1024, u16 BGR: 1536) bytes
     const int vecOk = ((reinterpret_cast<uintptr_t>(p.dst) & 15) == 0 && (p.pitch & 15) == 0) ? 1 : 0;
-    if (p.bgra) {
+    if (p.u16) {
+        if (p.f32) stitch_kernel<true, 3, uint16_t><<<grid, kSW, 0, s>>>(p, vecOk);
+        else stitch_kernel<false, 3, uint16_t><<<grid, kSW, 0, s>>>(p, vecOk);
+    } else if (p.bgra) {
         if (p.f32) stitch_kernel<true, 4><<<grid, kSW, 0, s>>>(p, vecOk);
         else stitch_kernel<false, 4><<<grid, kSW, 0, s>>>(p, vecOk);
     } else {

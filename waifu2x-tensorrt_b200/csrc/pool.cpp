@@ -60,6 +60,14 @@ bool EnginePool::load(const std::string& onnxPath, const w2x_render_config& cfg)
 }
 
 int EnginePool::submit(const uint8_t* src, int w, int h, size_t srcStride, uint8_t* dst, size_t dstStride, int dstW, int dstH) {
+    return enqueue(Job{src, w, h, srcStride, dst, dstStride, dstW, dstH, 0, false});
+}
+
+int EnginePool::submitU16(const uint16_t* src, int w, int h, size_t srcStride, uint16_t* dst, size_t dstStride) {
+    return enqueue(Job{reinterpret_cast<const uint8_t*>(src), w, h, srcStride, reinterpret_cast<uint8_t*>(dst), dstStride, 0, 0, 0, true});
+}
+
+int EnginePool::enqueue(Job job) {
     int ticket;
     {
         std::unique_lock<std::mutex> lk(stateMu);
@@ -72,7 +80,8 @@ int EnginePool::submit(const uint8_t* src, int w, int h, size_t srcStride, uint8
     {
         std::unique_lock<std::mutex> lk(wk.mu);
         wk.cv.wait(lk, [&] { return (int)wk.queue.size() < kQueueDepth || wk.stop; });  // back-pressure on the producer
-        wk.queue.push_back(Job{src, w, h, srcStride, dst, dstStride, dstW, dstH, ticket});
+        job.ticket = ticket;
+        wk.queue.push_back(job);
     }
     wk.cv.notify_all();
     return ticket;
@@ -107,8 +116,10 @@ void EnginePool::workerLoop(Worker* w) {
         if (have) {
             w->cv.notify_all();  // a queue slot is free again
             Engine& e = w->eng.impl;
-            const int t = job.dstW > 0 ? e.submitResized(job.src, job.w, job.h, job.srcStride, job.dst, job.dstW, job.dstH, job.dstStride)
-                                       : e.submit(job.src, job.w, job.h, job.srcStride, job.dst, job.dstStride);
+            const int t = job.u16 ? e.submitU16(reinterpret_cast<const uint16_t*>(job.src), job.w, job.h, job.srcStride, reinterpret_cast<uint16_t*>(job.dst),
+                                                job.dstStride)
+                          : job.dstW > 0 ? e.submitResized(job.src, job.w, job.h, job.srcStride, job.dst, job.dstW, job.dstH, job.dstStride)
+                                         : e.submit(job.src, job.w, job.h, job.srcStride, job.dst, job.dstStride);
             if (t < 0) finish(job.ticket, false);
             else flight.push_back({t, job.ticket});
             continue;

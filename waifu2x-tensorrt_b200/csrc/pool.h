@@ -34,12 +34,15 @@ public:
     // frame `ticket` (0, 1, 2, ... in submission order) goes to engine ticket % size(); returns the ticket or -1.  dstW > 0: the output
     // is resized to dstW x dstH (Engine::submitResized)
     int submit(const uint8_t* src, int w, int h, size_t srcStride, uint8_t* dst, size_t dstStride, int dstW = 0, int dstH = 0);
+    // the same with u16 BGR frames (Engine::submitU16)
+    int submitU16(const uint16_t* src, int w, int h, size_t srcStride, uint16_t* dst, size_t dstStride);
     bool wait(int ticket);   // true when that frame's dst is complete; tickets may be waited on in any order, each once
     bool sync();             // every submitted frame has been retired
 
 private:
     struct Job {
         const uint8_t* src; int w, h; size_t srcStride; uint8_t* dst; size_t dstStride; int dstW, dstH; int ticket;
+        bool u16;   // src / dst are u16 BGR frames
     };
     struct Worker {
         w2x_engine eng;
@@ -54,6 +57,7 @@ private:
     static constexpr int kRing = 256;      // tickets in flight (submitted, not yet waited for) must stay below this
     static constexpr int kQueueDepth = 4;  // frames a worker may hold beyond the engine's own three in flight
 
+    int enqueue(Job job);   // assigns job.ticket
     void workerLoop(Worker* w);
     void finish(int ticket, bool ok);
 

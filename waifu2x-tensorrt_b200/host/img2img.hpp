@@ -112,6 +112,13 @@ public:
                       size_t dstStride) {
         return w2x_submit_resized(h_, srcBgr, width, height, srcStride, dstBgr, dstWidth, dstHeight, dstStride);
     }
+    // extensions: 16 bits per channel, native-endian u16 BGR in and out, strides in bytes, see w2x_render_u16 in include/w2x.h
+    bool renderU16(const uint16_t* srcBgr, int width, int height, size_t srcStride, uint16_t* dstBgr, size_t dstStride) {
+        return w2x_render_u16(h_, srcBgr, width, height, srcStride, dstBgr, dstStride) != 0;
+    }
+    int submitU16(const uint16_t* srcBgr, int width, int height, size_t srcStride, uint16_t* dstBgr, size_t dstStride) {
+        return w2x_submit_u16(h_, srcBgr, width, height, srcStride, dstBgr, dstStride);
+    }
     bool wait(int ticket) { return w2x_wait(h_, ticket) != 0; }
 
     w2x_engine* handle() const { return h_; }
@@ -151,6 +158,9 @@ public:
     int submitResized(const unsigned char* srcBgr, int width, int height, size_t srcStride, unsigned char* dstBgr, int dstWidth, int dstHeight,
                       size_t dstStride) {
         return w2x_pool_submit_resized(h_, srcBgr, width, height, srcStride, dstBgr, dstWidth, dstHeight, dstStride);
+    }
+    int submitU16(const uint16_t* srcBgr, int width, int height, size_t srcStride, uint16_t* dstBgr, size_t dstStride) {
+        return w2x_pool_submit_u16(h_, srcBgr, width, height, srcStride, dstBgr, dstStride);
     }
     bool wait(int ticket) { return w2x_pool_wait(h_, ticket) != 0; }
     // the pool's index-th engine (borrowed), e.g. for w2x_render_bgra

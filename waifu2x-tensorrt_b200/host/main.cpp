@@ -43,6 +43,7 @@ struct Options {
     bool recursive = false, nosuffix = false, tta = false;
     bool alpha = false;  // extension: still images keep their alpha channel (BGRA through Img2Img::renderBgra, PNG out)
     double outputScale = 0;  // extension (> 0 when given): output lround(w F) x lround(h F), at most --scale (Img2Img::submitResized)
+    int bitDepth = 8;        // extension: 16 = u16 BGR frames through Img2Img::submitU16, 16-bit PNG stills
     fs::path outputDirectory;
     double blend = 1.0 / 16.0;
     std::string codec = "libx264", pixelFormat = "yuv420p";
@@ -75,6 +76,9 @@ const char* kUsage =
     "    --alpha                     Keep the alpha channel of still images (extension; videos are rendered without it)\n"
     "    --outputScale FLOAT:(0,scale]   Output size round(F x input) instead of scale x input: the model's output reduced on the GPU\n"
     "                                by an antialiased bicubic resample (extension; not with --alpha)\n"
+    "    --bitDepth INT:{8,16}=8     Bits per channel of the frames the model sees and returns (extension): 16 decodes the input as\n"
+    "                                16-bit BGR and writes 16-bit PNG stills; a video keeps --codec / --pix_fmt, so it needs a deep\n"
+    "                                --pix_fmt (e.g. yuv420p10le) to keep the bits.  Not with --alpha or --outputScale\n"
     "  build                         Build model\n";
 
 int toInt(const std::string& name, const std::string& v) {
@@ -171,6 +175,7 @@ Options parse(int argc, char** argv) {
             if (v.empty() || pos != v.size() || !std::isfinite(o.outputScale)) throw ParseError(a + ": '" + v + "' is not a number");
             if (o.outputScale <= 0) throw ParseError(a + ": must be positive");
         }
+        else if (a == "--bitDepth") { o.bitDepth = toInt(a, value()); requireMember(a, o.bitDepth, {8, 16}); }
         else if (inRender && a == "--codec") o.codec = value();
         else if (inRender && a == "--pix_fmt") o.pixelFormat = value();
         else if (inRender && a == "--crf") { o.crf = toInt(a, value()); if (o.crf < 0 || o.crf > 51) throw ParseError(a + ": value not in range 0 to 51"); }
@@ -184,6 +189,9 @@ Options parse(int argc, char** argv) {
     if (o.command == "render" && o.inputPaths.empty()) throw ParseError("--input is required");
     if (o.outputScale > o.scale) throw ParseError("--outputScale: at most --scale (" + std::to_string(o.scale) + "); the resample only reduces the model's output");
     if (o.outputScale > 0 && o.alpha) throw ParseError("--outputScale: not available with --alpha");
+    if (seen.count("--bitDepth") && o.command != "render") throw ParseError("--bitDepth: applies to render only");
+    if (o.bitDepth == 16 && o.alpha) throw ParseError("--bitDepth: 16 is not available with --alpha");
+    if (o.bitDepth == 16 && o.outputScale > 0) throw ParseError("--bitDepth: 16 is not available with --outputScale");
     return o;
 }
 
@@ -299,7 +307,13 @@ int main(int argc, char* argv[]) {
     } else if (!engine.load(modelPath, rc)) {
         return -1;
     }
+    const bool deep = o.bitDepth == 16;
     auto submitFrame = [&](const unsigned char* src, int w, int h, size_t ss, unsigned char* dst, const FrameSize& ds) {
+        if (deep) {
+            const auto* s16 = reinterpret_cast<const uint16_t*>(src);
+            auto* d16 = reinterpret_cast<uint16_t*>(dst);
+            return pool ? pool->submitU16(s16, w, h, ss, d16, (size_t)ds.width * 6) : engine.submitU16(s16, w, h, ss, d16, (size_t)ds.width * 6);
+        }
         if (o.outputScale > 0)
             return pool ? pool->submitResized(src, w, h, ss, dst, ds.width, ds.height, (size_t)ds.width * 3)
                         : engine.submitResized(src, w, h, ss, dst, ds.width, ds.height, (size_t)ds.width * 3);
@@ -316,8 +330,8 @@ int main(int argc, char* argv[]) {
     std::vector<PinnedBuffer> in(kRing), out(kRing);
     VideoCapture capture;
     VideoWriter writer;
-    capture.setFfmpegDir(o.ffmpegDir);
-    writer.setFfmpegDir(o.ffmpegDir).setConstantRateFactor(o.crf);
+    capture.setFfmpegDir(o.ffmpegDir).setBitDepth(o.bitDepth);
+    writer.setFfmpegDir(o.ffmpegDir).setConstantRateFactor(o.crf).setBitDepth(o.bitDepth);
     try {
         for (auto& file : files) {
             capture.setChannels(3).open(file.string());
@@ -338,7 +352,7 @@ int main(int argc, char* argv[]) {
             if (!o.nosuffix) file.replace_filename(file.stem().string() + suffix + sizeTag + file.extension().string());
             if (frameCount == 1) {
                 file.replace_extension(".png");
-                writer.setFrameRate(1).setPixelFormat("").setCodec("");
+                writer.setFrameRate(1).setPixelFormat(deep ? "rgb48be" : "").setCodec("");   // 16-bit: a 16-bit PNG
             } else {
                 file.replace_extension(".mp4");
                 writer.setFrameRate(capture.getFrameRate()).setPixelFormat(o.pixelFormat).setCodec(o.codec);
@@ -360,7 +374,7 @@ int main(int argc, char* argv[]) {
                 fileIndex++;
                 continue;
             }
-            for (int s = 0; s < kRing; ++s) { in[s].reserve(inSize.bytes()); out[s].reserve(outSize.bytes()); }
+            for (int s = 0; s < kRing; ++s) { in[s].reserve(inSize.bytes(3, o.bitDepth)); out[s].reserve(outSize.bytes(3, o.bitDepth)); }
 
             std::mutex mu;
             std::condition_variable cv;
@@ -423,7 +437,7 @@ int main(int argc, char* argv[]) {
                 while (waitFor(submitted, FILLED)) {
                     if (submitted - retired >= (size_t)kInFlight) retire();
                     const int s = (int)(submitted % kRing);
-                    tickets[s] = submitFrame(in[s].p, inSize.width, inSize.height, (size_t)inSize.width * 3, out[s].p, outSize);
+                    tickets[s] = submitFrame(in[s].p, inSize.width, inSize.height, (size_t)inSize.width * 3 * (o.bitDepth / 8), out[s].p, outSize);
                     if (tickets[s] < 0) throw std::runtime_error("render failed");
                     setState(submitted, SUBMITTED);
                     ++submitted;

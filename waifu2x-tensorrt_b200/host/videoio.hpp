@@ -2,7 +2,8 @@
 // reference's VideoCapture (/root/reference/src/videoio/capture.{h,cpp}) and VideoWriter (writer.{h,cpp}) with the same
 // class names, method names, command lines (capture.cpp:65-68,96-99; writer.cpp:24-33) and error behaviour (std::exception
 // on failure), minus OpenCV: frames are raw BGR8 HWC buffers (cv::Mat overloads appear when <opencv2/core.hpp> was included).
-// setChannels(4) on either class switches the raw frames to BGRA8 (`-pix_fmt bgra` instead of `bgr24`, nothing else changes).
+// setChannels(4) on either class switches the raw frames to BGRA8 (`-pix_fmt bgra` instead of `bgr24`, nothing else changes), and
+// setBitDepth(16) to native-endian u16 BGR (`-pix_fmt bgr48le`; 16-bit BGRA is refused).
 //
 // Fixes relative to the reference (SURVEY 8f rank 1): the command prefix (`ffmpegDir`) is settable on BOTH classes and is
 // honoured by VideoWriter::open (the reference ignores it, writer.cpp:24); release() uses pclose on every platform (the
@@ -34,7 +35,7 @@ struct FrameSize {  // stands in for cv::Size2i
     bool operator==(const FrameSize& o) const { return width == o.width && height == o.height; }
     bool operator!=(const FrameSize& o) const { return !(*this == o); }
     FrameSize operator*(int s) const { return {width * s, height * s}; }
-    size_t bytes(int channels = 3) const { return (size_t)width * height * channels; }
+    size_t bytes(int channels = 3, int bitDepth = 8) const { return (size_t)width * height * channels * (bitDepth / 8); }
 };
 
 // A path inside the double quotes of the reference's command lines (capture.cpp:65-68,96-99; writer.cpp:24-33).  The reference pastes
@@ -49,11 +50,15 @@ inline std::string quotedPath(const std::string& path) {
     return q + "\"";
 }
 
-// ffmpeg's name of the raw frame layout with `channels` bytes per pixel
-inline const char* rawPixelFormat(int channels) {
-    if (channels == 3) return "bgr24";
-    if (channels == 4) return "bgra";
-    throw std::invalid_argument("channels must be 3 or 4");
+// ffmpeg's name of the raw frame layout with `channels` samples of `bitDepth` bits per pixel
+inline const char* rawPixelFormat(int channels, int bitDepth = 8) {
+    if (bitDepth != 8 && bitDepth != 16) throw std::invalid_argument("bit depth must be 8 or 16");
+    if (channels != 3 && channels != 4) throw std::invalid_argument("channels must be 3 or 4");
+    if (bitDepth == 16) {
+        if (channels == 4) throw std::invalid_argument("16-bit frames have 3 channels");
+        return "bgr48le";
+    }
+    return channels == 3 ? "bgr24" : "bgra";
 }
 
 class VideoCapture {
@@ -83,7 +88,7 @@ public:
             frameSize.height = std::stoi(props.at("height"));
             frameRate = fraction(props.at("r_frame_rate"));
             frameCount = props.at("nb_frames") == "n/a" ? 1 : std::stoi(props.at("nb_frames"));  // no frame count => an image
-            const std::string cmd = ffmpegDir + "ffmpeg -v error -i " + quotedPath(path) + " -f image2pipe -vcodec rawvideo -pix_fmt " + rawPixelFormat(channels) + " -";
+            const std::string cmd = ffmpegDir + "ffmpeg -v error -i " + quotedPath(path) + " -f image2pipe -vcodec rawvideo -pix_fmt " + rawPixelFormat(channels, bitDepth) + " -";
             pipe = popen(cmd.c_str(), "r");
             if (!pipe) throw std::runtime_error("could not open ffmpeg with command\"" + cmd + "\"");
             growPipe(pipe);
@@ -97,11 +102,11 @@ public:
 
     [[nodiscard]] bool isOpened() const noexcept { return opened; }
 
-    // capture.cpp:116-128: one blocking read of W*H*channels bytes; false after the last frame
+    // capture.cpp:116-128: one blocking read of W*H*channels*bitDepth/8 bytes; false after the last frame
     bool read(uint8_t* bgr) {
         if (!opened) throw std::runtime_error("video capture is not opened");
         if (frameIndex + 1 >= frameCount) return false;
-        const size_t want = frameSize.bytes(channels);
+        const size_t want = frameSize.bytes(channels, bitDepth);
         size_t got = 0;
         while (got < want) {
             const size_t n = fread(bgr + got, 1, want - got, pipe);
@@ -128,8 +133,11 @@ public:
     [[nodiscard]] const std::string& getFfmpegDir() const noexcept { return ffmpegDir; }
     VideoCapture& setFfmpegDir(const std::string& value) { ffmpegDir = value; return *this; }  // missing in the reference (capture.h)
     // 3 (BGR, the default) or 4 (BGRA); applies from the next open()
-    VideoCapture& setChannels(int value) { rawPixelFormat(value); channels = value; return *this; }
+    VideoCapture& setChannels(int value) { rawPixelFormat(value, bitDepth); channels = value; return *this; }
     [[nodiscard]] int getChannels() const noexcept { return channels; }
+    // 8 (the default) or 16 (3 channels only); applies from the next open()
+    VideoCapture& setBitDepth(int value) { rawPixelFormat(channels, value); bitDepth = value; return *this; }
+    [[nodiscard]] int getBitDepth() const noexcept { return bitDepth; }
     [[nodiscard]] const FrameSize& getFrameSize() const noexcept { return frameSize; }
     [[nodiscard]] double getFrameRate() const noexcept { return frameRate; }
     [[nodiscard]] int getFrameCount() const noexcept { return frameCount; }
@@ -162,6 +170,7 @@ private:
     int frameCount = -1;
     int frameIndex = -1;
     int channels = 3;
+    int bitDepth = 8;
 };
 
 class VideoWriter {
@@ -177,7 +186,7 @@ public:
         if (frameSize.width <= 0 || frameSize.height <= 0) throw std::invalid_argument("frame size must be greater than 0");
         if (outputFile.empty()) throw std::invalid_argument("output file is empty");
         const std::string cmd = ffmpegDir + "ffmpeg -v error -y -f rawvideo -vcodec rawvideo -s " + std::to_string(frameSize.width) + "x" +
-                                std::to_string(frameSize.height) + " -pix_fmt " + rawPixelFormat(channels) + (frameRate <= 0 ? "" : " -r " + std::to_string(frameRate)) +
+                                std::to_string(frameSize.height) + " -pix_fmt " + rawPixelFormat(channels, bitDepth) + (frameRate <= 0 ? "" : " -r " + std::to_string(frameRate)) +
                                 " -i -" + (codec.empty() ? "" : " -vcodec " + codec) + (pixelFormat.empty() ? "" : " -pix_fmt " + pixelFormat) +
                                 (crf < 0 ? "" : " -crf " + std::to_string(crf)) + (quality < 0 ? "" : " -q:v " + std::to_string(quality)) +
                                 " " + quotedPath(outputFile);
@@ -193,7 +202,8 @@ public:
     void write(const uint8_t* bgr, const FrameSize& size) {
         if (!opened) throw std::runtime_error("video writer is not opened");
         if (size != frameSize) throw std::invalid_argument("frame size does not match");
-        if (fwrite(bgr, 1, frameSize.bytes(channels), pipe) != frameSize.bytes(channels)) throw std::runtime_error("could not write frame to pipe");
+        const size_t n = frameSize.bytes(channels, bitDepth);
+        if (fwrite(bgr, 1, n, pipe) != n) throw std::runtime_error("could not write frame to pipe");
     }
 #ifdef OPENCV_CORE_HPP
     void write(const cv::Mat& frame) {
@@ -231,8 +241,11 @@ public:
     VideoWriter& setConstantRateFactor(int v) { guard(); crf = v; return *this; }
     VideoWriter& setQuality(int v) { guard(); quality = v; return *this; }
     // 3 (BGR, the default) or 4 (BGRA): the layout of the frames given to write()
-    VideoWriter& setChannels(int v) { guard(); rawPixelFormat(v); channels = v; return *this; }
+    VideoWriter& setChannels(int v) { guard(); rawPixelFormat(v, bitDepth); channels = v; return *this; }
     [[nodiscard]] int getChannels() const noexcept { return channels; }
+    // 8 (the default) or 16 (3 channels only): the sample size of the frames given to write()
+    VideoWriter& setBitDepth(int v) { guard(); rawPixelFormat(channels, v); bitDepth = v; return *this; }
+    [[nodiscard]] int getBitDepth() const noexcept { return bitDepth; }
 
 private:
     void guard() const {
@@ -247,4 +260,5 @@ private:
     int crf = -1, quality = -1;
     int lastStatus = 0;
     int channels = 3;
+    int bitDepth = 8;
 };

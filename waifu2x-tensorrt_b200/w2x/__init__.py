@@ -102,6 +102,8 @@ _SIGNATURES = {
     "w2x_submit": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_size_t, C.c_void_p, C.c_size_t]),
     "w2x_render_resized": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_size_t, C.c_void_p, C.c_int, C.c_int, C.c_size_t]),
     "w2x_submit_resized": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_size_t, C.c_void_p, C.c_int, C.c_int, C.c_size_t]),
+    "w2x_render_u16": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_size_t, C.c_void_p, C.c_size_t]),
+    "w2x_submit_u16": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_size_t, C.c_void_p, C.c_size_t]),
     "w2x_render_banded": (C.c_int, [C.POINTER(C.c_void_p), C.c_int, C.c_void_p, C.c_int, C.c_int, C.c_size_t, C.c_void_p, C.c_size_t]),
     "w2x_wait": (C.c_int, [C.c_void_p, C.c_int]),
     "w2x_pool_create": (C.c_void_p, [C.POINTER(C.c_int), C.c_int]),
@@ -113,6 +115,7 @@ _SIGNATURES = {
     "w2x_pool_load": (C.c_int, [C.c_void_p, C.c_char_p, C.POINTER(_RenderConfig)]),
     "w2x_pool_submit": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_size_t, C.c_void_p, C.c_size_t]),
     "w2x_pool_submit_resized": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_size_t, C.c_void_p, C.c_int, C.c_int, C.c_size_t]),
+    "w2x_pool_submit_u16": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_size_t, C.c_void_p, C.c_size_t]),
     "w2x_pool_wait": (C.c_int, [C.c_void_p, C.c_int]),
     "w2x_pool_sync": (C.c_int, [C.c_void_p]),
     "w2x_sync": (C.c_int, [C.c_void_p]),
@@ -135,6 +138,8 @@ _SIGNATURES = {
     "w2x_blend_ramp": (C.c_int, [C.c_int, C.POINTER(C.c_float)]),
     "w2x_unpack_tiles": (C.c_int, [C.c_int, C.c_void_p, C.c_int, C.c_int, C.c_size_t, C.POINTER(_Rect), C.POINTER(C.c_int), C.c_int, C.c_int, C.c_void_p]),
     "w2x_stitch_tiles": (C.c_int, [C.c_int, C.c_void_p] + [C.c_int] * 8 + [C.c_void_p, C.c_size_t]),
+    "w2x_unpack_tiles_u16": (C.c_int, [C.c_int, C.c_void_p, C.c_int, C.c_int, C.c_size_t, C.POINTER(_Rect), C.POINTER(C.c_int), C.c_int, C.c_int, C.c_void_p]),
+    "w2x_stitch_tiles_u16": (C.c_int, [C.c_int, C.c_void_p] + [C.c_int] * 8 + [C.c_void_p, C.c_size_t]),
     "w2x_tta_reduce": (C.c_int, [C.c_int, C.c_void_p, C.c_int, C.c_int, C.c_void_p]),
     "w2x_alpha_bleed": (C.c_int, [C.c_int, C.c_void_p, C.c_int, C.c_int, C.c_size_t, C.c_int, C.c_void_p]),
     "w2x_resample": (C.c_int, [C.c_int, C.c_void_p, C.c_int, C.c_int, C.c_size_t, C.c_void_p, C.c_int, C.c_int, C.c_size_t]),
@@ -284,6 +289,30 @@ def stitch_tiles(tiles_f16: np.ndarray, nx: int, ny: int, ov_x: int, ov_y: int, 
     return dst
 
 
+def unpack_tiles_u16(src_bgr: np.ndarray, rects: List[Tuple[int, int, int, int]], aug: List[int], tile: int, device: int = 0) -> np.ndarray:
+    """uint16 [H, W, 3] BGR (rows may be strided) -> float16 [n, tile, tile, 4] (RGB0), each sample x as fp16(f32(x) * f32(1/65535))."""
+    src = src_bgr if _rows_of_u16_pixels(src_bgr) else np.ascontiguousarray(src_bgr, dtype=np.uint16)
+    n = len(rects)
+    cr = (_Rect * n)(*[_Rect(*r) for r in rects])
+    ca = (C.c_int * n)(*aug)
+    out = np.empty((n, tile, tile, 4), np.float16)
+    ok = lib().w2x_unpack_tiles_u16(device, _ptr(src), src.shape[1], src.shape[0], src.strides[0], cr, ca, n, tile, _ptr(out))
+    if not ok:
+        raise RuntimeError("w2x_unpack_tiles_u16 failed")
+    return out
+
+
+def stitch_tiles_u16(tiles_f16: np.ndarray, nx: int, ny: int, ov_x: int, ov_y: int, canvas_w: int, canvas_h: int, device: int = 0) -> np.ndarray:
+    """stitch_tiles with a uint16 [canvas_h, canvas_w, 3] BGR canvas: saturate(rint(65535 v)) of the same fp32 blend."""
+    t = np.ascontiguousarray(tiles_f16, dtype=np.float16)
+    count, out_tile = t.shape[0], t.shape[1]
+    dst = np.empty((canvas_h, canvas_w, 3), np.uint16)
+    ok = lib().w2x_stitch_tiles_u16(device, _ptr(t), count, out_tile, nx, ny, ov_x, ov_y, canvas_w, canvas_h, _ptr(dst), dst.strides[0])
+    if not ok:
+        raise RuntimeError("w2x_stitch_tiles_u16 failed")
+    return dst
+
+
 def tta_reduce(outs_f16: np.ndarray, device: int = 0) -> np.ndarray:
     t = np.ascontiguousarray(outs_f16, dtype=np.float16)  # [tiles, 8, T, T, 4]
     tiles, _, ot = t.shape[0], t.shape[1], t.shape[2]
@@ -296,6 +325,12 @@ def tta_reduce(outs_f16: np.ndarray, device: int = 0) -> np.ndarray:
 def _rows_of_pixels(a: np.ndarray, channels: int) -> bool:
     """a is [H, W, channels] uint8 with contiguous pixels (rows may be strided)."""
     return a.dtype == np.uint8 and a.ndim == 3 and a.shape[2] == channels and a.strides[2] == 1 and a.strides[1] == channels
+
+
+def _rows_of_u16_pixels(a: np.ndarray) -> bool:
+    """a is [H, W, 3] uint16 with contiguous pixels (rows may be strided, by an even number of bytes)."""
+    return (a.dtype == np.uint16 and a.ndim == 3 and a.shape[2] == 3 and a.strides[2] == 2 and a.strides[1] == 6 and a.strides[0] % 2 == 0
+            and a.ctypes.data % 2 == 0)
 
 
 def alpha_bleed(src_bgra: np.ndarray, rounds: int, device: int = 0) -> np.ndarray:
@@ -533,6 +568,24 @@ class Img2Img:
         dw, dh = int(size[0]), int(size[1])
         return int(self._l.w2x_submit_resized(self._h, C.c_void_p(src_ptr), w, h, w * 3, C.c_void_p(dst_ptr), dw, dh, dw * 3))
 
+    def render_u16(self, src: np.ndarray, dst: Optional[np.ndarray] = None) -> Optional[np.ndarray]:
+        """src: uint16 [H, W, 3] BGR (rows may be strided).  Returns dst (uint16 [H*s, W*s, 3] BGR, include/w2x.h w2x_render_u16; a
+        caller's dst may have strided rows) or None on failure (the reason in last_error)."""
+        if not _rows_of_u16_pixels(src):
+            src = np.ascontiguousarray(src, dtype=np.uint16)
+        h, w = src.shape[:2]
+        if dst is None:
+            dst = np.empty((h * self.scaling, w * self.scaling, 3), np.uint16)
+        elif not _rows_of_u16_pixels(dst):
+            raise ValueError("dst must be uint16 [H, W, 3] with contiguous pixels")
+        ok = self._l.w2x_render_u16(self._h, _ptr(src), w, h, src.strides[0], _ptr(dst), dst.strides[0])
+        return dst if ok else None
+
+    def submit_u16(self, src_ptr: int, w: int, h: int, dst_ptr: int) -> int:
+        """submit with the frames of render_u16: src_ptr holds h rows of 6 * w bytes, dst_ptr h * s rows of 6 * w * s bytes.  Returns
+        a ticket for wait, or -1."""
+        return int(self._l.w2x_submit_u16(self._h, C.c_void_p(src_ptr), w, h, w * 6, C.c_void_p(dst_ptr), w * self.scaling * 6))
+
     def infer(self, x_nchw: np.ndarray) -> Optional[np.ndarray]:
         x = np.ascontiguousarray(x_nchw, dtype=np.float32)
         n = x.shape[0]
@@ -719,6 +772,10 @@ class Img2ImgPool:
         """submit with the output of Img2Img.render_resized: dst_ptr holds size[1] rows of 3 * size[0] bytes."""
         dw, dh = int(size[0]), int(size[1])
         return int(self._l.w2x_pool_submit_resized(self._h, C.c_void_p(src_ptr), w, h, w * 3, C.c_void_p(dst_ptr), dw, dh, dw * 3))
+
+    def submit_u16(self, src_ptr: int, w: int, h: int, dst_ptr: int) -> int:
+        """submit with the frames of Img2Img.render_u16: src_ptr holds h rows of 6 * w bytes, dst_ptr h * s rows of 6 * w * s bytes."""
+        return int(self._l.w2x_pool_submit_u16(self._h, C.c_void_p(src_ptr), w, h, w * 6, C.c_void_p(dst_ptr), w * self.scaling * 6))
 
     def wait(self, ticket: int) -> bool:
         return bool(self._l.w2x_pool_wait(self._h, ticket))
