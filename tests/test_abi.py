@@ -69,3 +69,45 @@ def test_errors_do_not_cross_the_boundary(built_lib):
     assert e.render(__import__("numpy").zeros((8, 8, 3), "uint8")) is None
     assert "no engine loaded" in e.last_error
     e.close()
+
+
+def test_frame_entry_points_refuse_without_an_engine(built_lib):
+    """Every frame entry point of the C ABI fails (0 for the render calls, -1 for the submit calls) on a NULL handle, and on an engine
+    that has loaded nothing, with the reason "no engine loaded".  The pool's engines refuse the frame through w2x_pool_wait."""
+    import numpy as np
+    import w2x
+    l = built_lib
+    src, dst = np.zeros((8, 8, 4), np.uint8), np.zeros((16, 16, 4), np.uint8)
+    src16, dst16 = np.zeros((8, 8, 3), np.uint16), np.zeros((16, 16, 3), np.uint16)
+    p = lambda a: C.c_void_p(a.ctypes.data)
+    bgr, bgra, u16 = (p(src), 8, 8, 24, p(dst), 48), (p(src), 8, 8, 32, p(dst), 64), (p(src16), 8, 8, 48, p(dst16), 96)
+    resized = (p(src), 8, 8, 24, p(dst), 12, 12, 36)
+    engine_calls = [("w2x_render", bgr, 0), ("w2x_render_bgra", bgra, 0), ("w2x_render_resized", resized, 0), ("w2x_render_u16", u16, 0),
+                    ("w2x_render_device", bgr, 0), ("w2x_submit", bgr, -1), ("w2x_submit_resized", resized, -1), ("w2x_submit_u16", u16, -1)]
+    pool_calls = [("w2x_pool_submit", bgr), ("w2x_pool_submit_resized", resized), ("w2x_pool_submit_u16", u16)]
+
+    e = w2x.Img2Img()
+    msgs = []
+    e.setMessageCallback(lambda sev, m: msgs.append(m))
+    for name, args, bad in engine_calls:
+        assert getattr(l, name)(None, *args) == bad, name
+        msgs.clear()
+        assert getattr(l, name)(e._h, *args) == bad, name
+        assert len(msgs) == 1 and "no engine loaded" in msgs[0] and "no engine loaded" in e.last_error, (name, msgs)
+    assert l.w2x_render_banded(None, 1, *bgr) == 0
+    msgs.clear()
+    assert l.w2x_render_banded((C.c_void_p * 1)(e._h), 1, *bgr) == 0
+    assert len(msgs) == 1 and "no engine loaded" in msgs[0], msgs
+    e.close()
+
+    pool = w2x.Img2ImgPool([0])
+    msgs = []
+    pool.setMessageCallback(lambda sev, m: msgs.append(m))
+    for name, args in pool_calls:
+        assert getattr(l, name)(None, *args) == -1, name
+        msgs.clear()
+        ticket = getattr(l, name)(pool._h, *args)
+        assert ticket >= 0, name
+        assert l.w2x_pool_wait(pool._h, ticket) == 0, name
+        assert len(msgs) == 1 and "no engine loaded" in msgs[0], (name, msgs)
+    pool.close()

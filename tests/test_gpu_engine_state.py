@@ -78,3 +78,40 @@ def test_rejected_frame_does_not_poison_the_engine(kind, built_lib, cunet2x):
     assert np.array_equal(got, want)
     fresh.close()
     e.close()
+
+
+def test_bgr_frames_with_null_pointers_or_short_strides_are_refused_up_front(built_lib, cunet2x):
+    """w2x_render, w2x_submit, w2x_render_device and w2x_render_banded refuse a null image pointer and a row stride below 3 bytes per
+    pixel with a message, before any copy or launch; the engine then renders what it rendered before."""
+    import ctypes as C
+    import w2x
+    l = w2x.lib()
+    e = _engine(cunet2x)
+    f = _frame("render", 40, 30, 4)
+    want = e.render(f)
+    assert want is not None, e.last_error
+    msgs = []
+    e.setMessageCallback(lambda s, m: msgs.append(m))
+    src, dst = np.ascontiguousarray(f), np.zeros_like(want)
+    d_src, d_dst = e.device_alloc(src.nbytes), e.device_alloc(dst.nbytes)
+    p = lambda a: C.c_void_p(a.ctypes.data)
+    banded = lambda h, *args: l.w2x_render_banded((C.c_void_p * 1)(h), 1, *args)
+    calls = [(l.w2x_render, p(src), p(dst), 0), (l.w2x_submit, p(src), p(dst), -1),
+             (l.w2x_render_device, C.c_void_p(d_src), C.c_void_p(d_dst), 0), (banded, p(src), p(dst), 0)]
+
+    def refusal(fn, bad, *args):
+        msgs.clear()
+        assert fn(e._h, *args) == bad and len(msgs) == 1, msgs
+        return msgs[0]
+
+    n0 = e.launch_count
+    for fn, s, d, bad in calls:
+        assert "null image pointer" in refusal(fn, bad, None, 40, 30, 120, d, 240)
+        assert "null image pointer" in refusal(fn, bad, s, 40, 30, 120, None, 240)
+        assert "smaller than 3 bytes per pixel" in refusal(fn, bad, s, 40, 30, 119, d, 240)
+        assert "smaller than 3 bytes per pixel" in refusal(fn, bad, s, 40, 30, 120, d, 239)
+    assert e.launch_count == n0
+    assert np.array_equal(e.render(f), want)
+    e.device_free(d_src)
+    e.device_free(d_dst)
+    e.close()

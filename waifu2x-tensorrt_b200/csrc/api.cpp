@@ -31,6 +31,58 @@ template <class T> T* alloc(std::vector<DeviceBuffer>& bufs, size_t count) {
     bufs.emplace_back(count * sizeof(T) + 16);
     return bufs.back().get<T>();
 }
+
+// the stage hooks w2x_unpack_tiles(_u16) and w2x_stitch_tiles(_u16): a host frame of `format` <-> fp16 tiles on the device
+int unpackTiles(const char* name, PixelFormat format, int device, const void* src, int width, int height, size_t src_stride, const w2x_rect* rects,
+                const int* aug, int n, int tile, uint16_t* out) {
+    try {
+        W2X_CUDA(cudaSetDevice(device));
+        std::vector<DeviceBuffer> b;
+        const size_t row = (size_t)width * bytesPerPixel(format);
+        uint8_t* dSrc = alloc<uint8_t>(b, row * height);
+        W2X_CUDA(cudaMemcpy2D(dSrc, row, src, src_stride, row, height, cudaMemcpyHostToDevice));
+        std::vector<TileSlot> slots(n);
+        for (int i = 0; i < n; ++i) slots[i] = {rects[i].x, rects[i].y, aug ? aug[i] : 0, 1};
+        TileSlot* dSlots = alloc<TileSlot>(b, n);
+        W2X_CUDA(cudaMemcpy(dSlots, slots.data(), sizeof(TileSlot) * n, cudaMemcpyHostToDevice));
+        const size_t elems = (size_t)n * tile * tile * 4;
+        __half* dOut = alloc<__half>(b, elems);
+        launchUnpack(dSrc, width, height, row, dSlots, n, tile, dOut, nullptr, format);
+        W2X_CUDA(cudaGetLastError());
+        W2X_CUDA(cudaMemcpy(out, dOut, elems * 2, cudaMemcpyDeviceToHost));
+        return 1;
+    } catch (const std::exception& ex) {
+        std::fprintf(stderr, "%s: %s\n", name, ex.what());
+        return 0;
+    }
+}
+
+int stitchTiles(const char* name, PixelFormat format, int device, const uint16_t* tiles, int count, int out_tile, int nx, int ny, int overlap_x,
+                int overlap_y, int canvas_w, int canvas_h, void* dst, size_t dst_stride) {
+    try {
+        W2X_CUDA(cudaSetDevice(device));
+        std::vector<DeviceBuffer> b;
+        const size_t elems = (size_t)count * out_tile * out_tile * 4;
+        __half* dT = alloc<__half>(b, elems);
+        W2X_CUDA(cudaMemcpy(dT, tiles, elems * 2, cudaMemcpyHostToDevice));
+        std::vector<float> rx = blendRamp(overlap_x), ry = blendRamp(overlap_y);
+        float* dRx = alloc<float>(b, rx.size() + 1);
+        float* dRy = alloc<float>(b, ry.size() + 1);
+        if (!rx.empty()) W2X_CUDA(cudaMemcpy(dRx, rx.data(), rx.size() * 4, cudaMemcpyHostToDevice));
+        if (!ry.empty()) W2X_CUDA(cudaMemcpy(dRy, ry.data(), ry.size() * 4, cudaMemcpyHostToDevice));
+        const size_t row = (size_t)canvas_w * bytesPerPixel(format);
+        uint8_t* dDst = alloc<uint8_t>(b, row * canvas_h);
+        StitchParams sp = stitchGrid(out_tile, nx, ny, overlap_x, overlap_y, canvas_w, canvas_h, dRx, dRy);
+        sp.tiles = dT; sp.dst = dDst; sp.pitch = row; sp.format = format;
+        launchStitch(sp, nullptr);
+        W2X_CUDA(cudaGetLastError());
+        W2X_CUDA(cudaMemcpy2D(dst, dst_stride, dDst, row, row, canvas_h, cudaMemcpyDeviceToHost));
+        return 1;
+    } catch (const std::exception& ex) {
+        std::fprintf(stderr, "%s: %s\n", name, ex.what());
+        return 0;
+    }
+}
 }  // namespace
 
 extern "C" {
@@ -65,56 +117,56 @@ int w2x_load(w2x_engine* e, const char* onnx_path, const w2x_render_config* cfg)
 }
 
 int w2x_render(w2x_engine* e, const uint8_t* src, int width, int height, size_t src_stride, uint8_t* dst, size_t dst_stride) {
-    if (!e || !src || !dst) return 0;
-    return e->impl.render(src, width, height, src_stride, dst, dst_stride) ? 1 : 0;
+    if (!e) return 0;
+    return e->impl.render(Frame{PixelFormat::Bgr8, src, width, height, src_stride, dst, dst_stride}) ? 1 : 0;
 }
 
 int w2x_render_bgra(w2x_engine* e, const uint8_t* src, int width, int height, size_t src_stride, uint8_t* dst, size_t dst_stride) {
     if (!e) return 0;
-    return e->impl.renderBgra(src, width, height, src_stride, dst, dst_stride) ? 1 : 0;
+    return e->impl.render(Frame{PixelFormat::Bgra8, src, width, height, src_stride, dst, dst_stride}) ? 1 : 0;
 }
 
 int w2x_render_resized(w2x_engine* e, const uint8_t* src, int width, int height, size_t src_stride, uint8_t* dst, int dst_width, int dst_height,
                        size_t dst_stride) {
     if (!e) return 0;
-    return e->impl.renderResized(src, width, height, src_stride, dst, dst_width, dst_height, dst_stride) ? 1 : 0;
+    return e->impl.render(Frame{PixelFormat::Bgr8, src, width, height, src_stride, dst, dst_stride, Frame::Size{dst_width, dst_height}}) ? 1 : 0;
 }
 
 int w2x_submit_resized(w2x_engine* e, const uint8_t* src, int width, int height, size_t src_stride, uint8_t* dst, int dst_width, int dst_height,
                        size_t dst_stride) {
     if (!e) return -1;
-    return e->impl.submitResized(src, width, height, src_stride, dst, dst_width, dst_height, dst_stride);
+    return e->impl.submit(Frame{PixelFormat::Bgr8, src, width, height, src_stride, dst, dst_stride, Frame::Size{dst_width, dst_height}});
 }
 
 int w2x_render_u16(w2x_engine* e, const uint16_t* src, int width, int height, size_t src_stride, uint16_t* dst, size_t dst_stride) {
     if (!e) return 0;
-    return e->impl.renderU16(src, width, height, src_stride, dst, dst_stride) ? 1 : 0;
+    return e->impl.render(Frame{PixelFormat::Bgr16, src, width, height, src_stride, dst, dst_stride}) ? 1 : 0;
 }
 
 int w2x_submit_u16(w2x_engine* e, const uint16_t* src, int width, int height, size_t src_stride, uint16_t* dst, size_t dst_stride) {
     if (!e) return -1;
-    return e->impl.submitU16(src, width, height, src_stride, dst, dst_stride);
+    return e->impl.submit(Frame{PixelFormat::Bgr16, src, width, height, src_stride, dst, dst_stride});
 }
 
 int w2x_render_device(w2x_engine* e, const uint8_t* src, int width, int height, size_t src_stride, uint8_t* dst, size_t dst_stride) {
-    if (!e || !src || !dst) return 0;
-    return e->impl.renderDevice(src, width, height, src_stride, dst, dst_stride) ? 1 : 0;
+    if (!e) return 0;
+    return e->impl.renderDevice(Frame{PixelFormat::Bgr8, src, width, height, src_stride, dst, dst_stride}) ? 1 : 0;
 }
 
 int w2x_submit(w2x_engine* e, const uint8_t* src, int width, int height, size_t src_stride, uint8_t* dst, size_t dst_stride) {
-    if (!e || !src || !dst) return -1;
-    return e->impl.submit(src, width, height, src_stride, dst, dst_stride);
+    if (!e) return -1;
+    return e->impl.submit(Frame{PixelFormat::Bgr8, src, width, height, src_stride, dst, dst_stride});
 }
 
 int w2x_render_banded(w2x_engine* const* engines, int count, const uint8_t* src, int width, int height, size_t src_stride,
                       uint8_t* dst, size_t dst_stride) {
-    if (!engines || count < 1 || count > 16 || !src || !dst) return 0;
+    if (!engines || count < 1 || count > 16) return 0;
     Engine* es[16];
     for (int i = 0; i < count; ++i) {
         if (!engines[i]) return 0;
         es[i] = &engines[i]->impl;
     }
-    return Engine::renderBanded(es, count, src, width, height, src_stride, dst, dst_stride) ? 1 : 0;
+    return Engine::renderBanded(es, count, Frame{PixelFormat::Bgr8, src, width, height, src_stride, dst, dst_stride}) ? 1 : 0;
 }
 
 w2x_pool* w2x_pool_create(const int* device_ids, int count) {
@@ -131,23 +183,27 @@ int w2x_pool_load(w2x_pool* p, const char* onnx_path, const w2x_render_config* c
     try { return p && onnx_path && cfg && p->impl.load(onnx_path, *cfg) ? 1 : 0; } catch (...) { return 0; }
 }
 int w2x_pool_submit(w2x_pool* p, const uint8_t* src, int width, int height, size_t src_stride, uint8_t* dst, size_t dst_stride) {
-    if (!p || !src || !dst) return -1;
-    try { return p->impl.submit(src, width, height, src_stride, dst, dst_stride); } catch (...) { return -1; }
+    if (!p) return -1;
+    try { return p->impl.submit(Frame{PixelFormat::Bgr8, src, width, height, src_stride, dst, dst_stride}); } catch (...) { return -1; }
 }
 int w2x_pool_submit_resized(w2x_pool* p, const uint8_t* src, int width, int height, size_t src_stride, uint8_t* dst, int dst_width, int dst_height,
                             size_t dst_stride) {
-    if (!p || !src || !dst) return -1;
+    if (!p) return -1;
     if (dst_width < 1 || dst_height < 1) {   // the other refusals come from the engine that takes the frame, through w2x_pool_wait
         if (w2x_engine* e = p->impl.engine(0))
             e->impl.log(W2X_ERROR, "Submit failed: output size " + std::to_string(dst_width) + "x" + std::to_string(dst_height) + " is below 1x1.",
                         __FUNCTION__, __LINE__);
         return -1;
     }
-    try { return p->impl.submit(src, width, height, src_stride, dst, dst_stride, dst_width, dst_height); } catch (...) { return -1; }
+    try {
+        return p->impl.submit(Frame{PixelFormat::Bgr8, src, width, height, src_stride, dst, dst_stride, Frame::Size{dst_width, dst_height}});
+    } catch (...) {
+        return -1;
+    }
 }
 int w2x_pool_submit_u16(w2x_pool* p, const uint16_t* src, int width, int height, size_t src_stride, uint16_t* dst, size_t dst_stride) {
-    if (!p || !src || !dst) return -1;   // the other refusals come from the engine that takes the frame, through w2x_pool_wait
-    try { return p->impl.submitU16(src, width, height, src_stride, dst, dst_stride); } catch (...) { return -1; }
+    if (!p) return -1;   // the refusals come from the engine that takes the frame, through w2x_pool_wait
+    try { return p->impl.submit(Frame{PixelFormat::Bgr16, src, width, height, src_stride, dst, dst_stride}); } catch (...) { return -1; }
 }
 int w2x_pool_wait(w2x_pool* p, int ticket) {
     try { return p && p->impl.wait(ticket) ? 1 : 0; } catch (...) { return 0; }
@@ -230,108 +286,28 @@ int w2x_blend_ramp(int overlap, float* ramp) {
 
 int w2x_unpack_tiles(int device, const uint8_t* src, int width, int height, size_t src_stride, const w2x_rect* rects,
                      const int* aug, int n, int tile, uint16_t* out) {
-    try {
-        if (!src || !rects || !out || n <= 0 || tile <= 0) return 0;
-        W2X_CUDA(cudaSetDevice(device));
-        std::vector<DeviceBuffer> b;
-        uint8_t* dSrc = alloc<uint8_t>(b, (size_t)width * 3 * height);
-        W2X_CUDA(cudaMemcpy2D(dSrc, (size_t)width * 3, src, src_stride, (size_t)width * 3, height, cudaMemcpyHostToDevice));
-        std::vector<TileSlot> slots(n);
-        for (int i = 0; i < n; ++i) slots[i] = {rects[i].x, rects[i].y, aug ? aug[i] : 0, 1};
-        TileSlot* dSlots = alloc<TileSlot>(b, n);
-        W2X_CUDA(cudaMemcpy(dSlots, slots.data(), sizeof(TileSlot) * n, cudaMemcpyHostToDevice));
-        const size_t elems = (size_t)n * tile * tile * 4;
-        __half* dOut = alloc<__half>(b, elems);
-        launchUnpack(dSrc, width, height, (size_t)width * 3, dSlots, n, tile, dOut, nullptr);
-        W2X_CUDA(cudaGetLastError());
-        W2X_CUDA(cudaMemcpy(out, dOut, elems * 2, cudaMemcpyDeviceToHost));
-        return 1;
-    } catch (const std::exception& ex) {
-        std::fprintf(stderr, "w2x_unpack_tiles: %s\n", ex.what());
-        return 0;
-    }
+    if (!src || !rects || !out || n <= 0 || tile <= 0) return 0;
+    return unpackTiles("w2x_unpack_tiles", PixelFormat::Bgr8, device, src, width, height, src_stride, rects, aug, n, tile, out);
 }
 
 int w2x_stitch_tiles(int device, const uint16_t* tiles, int count, int out_tile, int nx, int ny, int overlap_x, int overlap_y,
                      int canvas_w, int canvas_h, uint8_t* dst, size_t dst_stride) {
-    try {
-        if (!tiles || !dst || count != nx * ny) return 0;
-        W2X_CUDA(cudaSetDevice(device));
-        std::vector<DeviceBuffer> b;
-        const size_t elems = (size_t)count * out_tile * out_tile * 4;
-        __half* dT = alloc<__half>(b, elems);
-        W2X_CUDA(cudaMemcpy(dT, tiles, elems * 2, cudaMemcpyHostToDevice));
-        std::vector<float> rx = blendRamp(overlap_x), ry = blendRamp(overlap_y);
-        float* dRx = alloc<float>(b, rx.size() + 1);
-        float* dRy = alloc<float>(b, ry.size() + 1);
-        if (!rx.empty()) W2X_CUDA(cudaMemcpy(dRx, rx.data(), rx.size() * 4, cudaMemcpyHostToDevice));
-        if (!ry.empty()) W2X_CUDA(cudaMemcpy(dRy, ry.data(), ry.size() * 4, cudaMemcpyHostToDevice));
-        uint8_t* dDst = alloc<uint8_t>(b, (size_t)canvas_w * 3 * canvas_h);
-        StitchParams sp{};
-        sp.tiles = dT; sp.f32 = 0; sp.outT = out_tile; sp.nx = nx; sp.ny = ny; sp.ovx = overlap_x; sp.ovy = overlap_y;
-        sp.cw = canvas_w; sp.ch = canvas_h; sp.rampx = dRx; sp.rampy = dRy; sp.dst = dDst; sp.pitch = (size_t)canvas_w * 3;
-        launchStitch(sp, nullptr);
-        W2X_CUDA(cudaGetLastError());
-        W2X_CUDA(cudaMemcpy2D(dst, dst_stride, dDst, (size_t)canvas_w * 3, (size_t)canvas_w * 3, canvas_h, cudaMemcpyDeviceToHost));
-        return 1;
-    } catch (const std::exception& ex) {
-        std::fprintf(stderr, "w2x_stitch_tiles: %s\n", ex.what());
-        return 0;
-    }
+    if (!tiles || !dst || count != nx * ny) return 0;
+    return stitchTiles("w2x_stitch_tiles", PixelFormat::Bgr8, device, tiles, count, out_tile, nx, ny, overlap_x, overlap_y, canvas_w, canvas_h, dst,
+                       dst_stride);
 }
 
 int w2x_unpack_tiles_u16(int device, const uint16_t* src, int width, int height, size_t src_stride, const w2x_rect* rects, const int* aug, int n,
                          int tile, uint16_t* out) {
-    try {
-        if (!src || !rects || !out || n <= 0 || tile <= 0 || width <= 0 || height <= 0 || src_stride < (size_t)width * 6) return 0;
-        W2X_CUDA(cudaSetDevice(device));
-        std::vector<DeviceBuffer> b;
-        const size_t row = (size_t)width * 6;
-        uint8_t* dSrc = alloc<uint8_t>(b, row * height);
-        W2X_CUDA(cudaMemcpy2D(dSrc, row, src, src_stride, row, height, cudaMemcpyHostToDevice));
-        std::vector<TileSlot> slots(n);
-        for (int i = 0; i < n; ++i) slots[i] = {rects[i].x, rects[i].y, aug ? aug[i] : 0, 1};
-        TileSlot* dSlots = alloc<TileSlot>(b, n);
-        W2X_CUDA(cudaMemcpy(dSlots, slots.data(), sizeof(TileSlot) * n, cudaMemcpyHostToDevice));
-        const size_t elems = (size_t)n * tile * tile * 4;
-        __half* dOut = alloc<__half>(b, elems);
-        launchUnpack(dSrc, width, height, row, dSlots, n, tile, dOut, nullptr, 3, 2);
-        W2X_CUDA(cudaGetLastError());
-        W2X_CUDA(cudaMemcpy(out, dOut, elems * 2, cudaMemcpyDeviceToHost));
-        return 1;
-    } catch (const std::exception& ex) {
-        std::fprintf(stderr, "w2x_unpack_tiles_u16: %s\n", ex.what());
-        return 0;
-    }
+    if (!src || !rects || !out || n <= 0 || tile <= 0 || width <= 0 || height <= 0 || src_stride < (size_t)width * 6) return 0;
+    return unpackTiles("w2x_unpack_tiles_u16", PixelFormat::Bgr16, device, src, width, height, src_stride, rects, aug, n, tile, out);
 }
 
 int w2x_stitch_tiles_u16(int device, const uint16_t* tiles, int count, int out_tile, int nx, int ny, int overlap_x, int overlap_y,
                          int canvas_w, int canvas_h, uint16_t* dst, size_t dst_stride) {
-    try {
-        if (!tiles || !dst || count != nx * ny || canvas_w <= 0 || canvas_h <= 0 || dst_stride < (size_t)canvas_w * 6) return 0;
-        W2X_CUDA(cudaSetDevice(device));
-        std::vector<DeviceBuffer> b;
-        const size_t elems = (size_t)count * out_tile * out_tile * 4;
-        __half* dT = alloc<__half>(b, elems);
-        W2X_CUDA(cudaMemcpy(dT, tiles, elems * 2, cudaMemcpyHostToDevice));
-        std::vector<float> rx = blendRamp(overlap_x), ry = blendRamp(overlap_y);
-        float* dRx = alloc<float>(b, rx.size() + 1);
-        float* dRy = alloc<float>(b, ry.size() + 1);
-        if (!rx.empty()) W2X_CUDA(cudaMemcpy(dRx, rx.data(), rx.size() * 4, cudaMemcpyHostToDevice));
-        if (!ry.empty()) W2X_CUDA(cudaMemcpy(dRy, ry.data(), ry.size() * 4, cudaMemcpyHostToDevice));
-        const size_t row = (size_t)canvas_w * 6;
-        uint8_t* dDst = alloc<uint8_t>(b, row * canvas_h);
-        StitchParams sp{};
-        sp.tiles = dT; sp.f32 = 0; sp.outT = out_tile; sp.nx = nx; sp.ny = ny; sp.ovx = overlap_x; sp.ovy = overlap_y;
-        sp.cw = canvas_w; sp.ch = canvas_h; sp.rampx = dRx; sp.rampy = dRy; sp.dst = dDst; sp.pitch = row; sp.u16 = 1;
-        launchStitch(sp, nullptr);
-        W2X_CUDA(cudaGetLastError());
-        W2X_CUDA(cudaMemcpy2D(dst, dst_stride, dDst, row, row, canvas_h, cudaMemcpyDeviceToHost));
-        return 1;
-    } catch (const std::exception& ex) {
-        std::fprintf(stderr, "w2x_stitch_tiles_u16: %s\n", ex.what());
-        return 0;
-    }
+    if (!tiles || !dst || count != nx * ny || canvas_w <= 0 || canvas_h <= 0 || dst_stride < (size_t)canvas_w * 6) return 0;
+    return stitchTiles("w2x_stitch_tiles_u16", PixelFormat::Bgr16, device, tiles, count, out_tile, nx, ny, overlap_x, overlap_y, canvas_w, canvas_h,
+                       dst, dst_stride);
 }
 
 int w2x_alpha_bleed(int device, const uint8_t* src, int width, int height, size_t src_stride, int rounds, uint8_t* dst) {

@@ -1006,8 +1006,10 @@ void Engine::ensureResize(int cw, int ch, int dw, int dh) {
     resize.dh = dh;
 }
 
-void Engine::renderOnStream(const uint8_t* dSrc, int w, int h, size_t srcPitch, uint8_t* dDst, size_t dstPitch, cudaStream_t s, bool timed,
-                            std::vector<BandDone>* bands, int pixelBytes, int sampleBytes, int dstW, int dstH) {
+void Engine::renderOnStream(const Frame& d, cudaStream_t s, bool timed, std::vector<BandDone>* bands) {
+    const int w = d.w, h = d.h;
+    const uint8_t* dSrc = static_cast<const uint8_t*>(d.src);
+    uint8_t* dDst = static_cast<uint8_t*>(d.dst);
     if (timed) { timing.used = 0; timing.spans.clear(); }
     auto span = [&](int kind, auto&& fn) {
         if (!timed) { fn(); return; }
@@ -1020,7 +1022,7 @@ void Engine::renderOnStream(const uint8_t* dSrc, int w, int h, size_t srcPitch, 
         timing.spans.push_back({kind, i0, timing.used - 1});
     };
     int passes = 1;
-    if (pixelBytes == 4) {
+    if (d.format == PixelFormat::Bgra8) {
         // The alpha plane decides the schedule: no alpha < 255, no alpha pass; some alpha == 0, the colour bleed first.  Both count as
         // unpack time.
         bgra.flags.ensure(2 * sizeof(int));
@@ -1052,30 +1054,23 @@ void Engine::renderOnStream(const uint8_t* dSrc, int w, int h, size_t srcPitch, 
     }
     ensureFrameBuffers(w, h, passes);
     const int cw = w * scale, ch = h * scale;
-    if (dstW <= 0) dstW = cw;
-    if (dstH <= 0) dstH = ch;
+    const Frame::Size out = outputSize(d);
+    const int dstW = out.w, dstH = out.h;
     // a resized frame is stitched into the engine's canvas and resampled from there into dDst
     const bool resized = dstW != cw || dstH != ch;
-    if (resized) {
-        if (pixelBytes != 3 || sampleBytes != 1) throw Error("resized output is u8 BGR only");
-        ensureResize(cw, ch, dstW, dstH);
-    }
+    if (resized) ensureResize(cw, ch, dstW, dstH);
     const TileGrid& grid = fc.grid;
-    const bool progressive = pixelBytes == 3 && bands != nullptr && !cfg.tta && !fc.rowBands.empty();
+    const bool progressive = d.format != PixelFormat::Bgra8 && bands != nullptr && !cfg.tta && !fc.rowBands.empty();
     if (bands) bands->clear();
     auto stitchRows = [&](int yBegin, int yEnd) {
-        StitchParams sp{};
-        sp.outT = outTile; sp.nx = grid.nx; sp.ny = grid.ny; sp.ovx = grid.outOvX; sp.ovy = grid.outOvY;
-        sp.cw = cw; sp.ch = ch;
-        sp.rampx = fc.rampX.get<float>(); sp.rampy = fc.rampY.get<float>();
+        StitchParams sp = stitchGrid(outTile, grid.nx, grid.ny, grid.outOvX, grid.outOvY, cw, ch, fc.rampX.get<float>(), fc.rampY.get<float>());
         sp.dst = resized ? resize.canvas.get<uint8_t>() : dDst;
-        sp.pitch = resized ? (size_t)cw * 3 : dstPitch;
+        sp.pitch = resized ? (size_t)cw * 3 : d.dstStride;
         sp.tiles = cfg.tta ? fc.ttaMean.get() : fc.tileOut.get();
         sp.f32 = (cfg.tta || tf32()) ? 1 : 0;
         sp.tile_map = cfg.tta ? nullptr : fc.tileMap.get<int>();
         sp.y_begin = yBegin; sp.y_end = yEnd;
-        sp.bgra = pixelBytes == 4 ? 1 : 0;
-        sp.u16 = sampleBytes == 2 ? 1 : 0;
+        sp.format = d.format;
         sp.alpha_off = passes == 2 ? grid.count : 0;   // TTA: index of the reduced alpha tile; else the alpha step of the tile's slot
         launchStitch(sp, s);
         ++launches;
@@ -1089,7 +1084,7 @@ void Engine::renderOnStream(const uint8_t* dSrc, int w, int h, size_t srcPitch, 
         const int i0 = rowsOut;
         while (rowsOut < dstH && resize.rowEnd[rowsOut] <= y1) ++rowsOut;
         if (rowsOut > i0) {
-            launchResampleV(resize.tmp.get<float>(), dstW, resize.ty, i0, rowsOut, dDst, dstPitch, s);
+            launchResampleV(resize.tmp.get<float>(), dstW, resize.ty, i0, rowsOut, dDst, d.dstStride, s);
             ++launches;
         }
         return std::make_pair(i0, rowsOut);
@@ -1102,7 +1097,7 @@ void Engine::renderOnStream(const uint8_t* dSrc, int w, int h, size_t srcPitch, 
     const bool frameWide = frameWideUnpack();
     if (frameWide)
         span(0, [&] {
-            unpackTiles(dSrc, w, h, srcPitch, fc.slots.get<TileSlot>(), realSteps, fc.unpacked.get(), s, pixelBytes, sampleBytes);
+            unpackTiles(dSrc, w, h, d.srcStride, fc.slots.get<TileSlot>(), realSteps, fc.unpacked.get(), s, d.format);
             ++launches;
         });
     for (int b = 0; b < fc.batchCount; ++b) {
@@ -1111,7 +1106,7 @@ void Engine::renderOnStream(const uint8_t* dSrc, int w, int h, size_t srcPitch, 
         if (nReal <= 0) continue;
         if (!frameWide)
             span(0, [&] {
-                unpackTiles(dSrc, w, h, srcPitch, fc.slots.get<TileSlot>() + (size_t)b * batch, nReal, actIn.p, s, pixelBytes, sampleBytes);
+                unpackTiles(dSrc, w, h, d.srcStride, fc.slots.get<TileSlot>() + (size_t)b * batch, nReal, actIn.p, s, d.format);
                 ++launches;
             });
         span(1, [&] { runModel(s, elemAt(fc.tileOut.get(), (size_t)b * batch * tileElems), nReal, frameWide ? elemAt(fc.unpacked.get(), (size_t)b * batch * inElems) : nullptr); });
@@ -1152,10 +1147,10 @@ void Engine::renderOnStream(const uint8_t* dSrc, int w, int h, size_t srcPitch, 
     W2X_CUDA(cudaGetLastError());
 }
 
-void Engine::unpackTiles(const uint8_t* src, int w, int h, size_t pitch, const TileSlot* slots, int n, void* out, cudaStream_t s, int pixelBytes,
-                         int sampleBytes) {
-    if (tf32()) launchUnpack(src, w, h, pitch, slots, n, tile, static_cast<float*>(out), s, pixelBytes, sampleBytes);
-    else launchUnpack(src, w, h, pitch, slots, n, tile, static_cast<__half*>(out), s, pixelBytes, sampleBytes);
+void Engine::unpackTiles(const uint8_t* src, int w, int h, size_t pitch, const TileSlot* slots, int n, void* out, cudaStream_t s,
+                         PixelFormat format) {
+    if (tf32()) launchUnpack(src, w, h, pitch, slots, n, tile, static_cast<float*>(out), s, format);
+    else launchUnpack(src, w, h, pitch, slots, n, tile, static_cast<__half*>(out), s, format);
 }
 
 void Engine::ttaReduce(const void* outs, int tiles, float* mean, cudaStream_t s) {
@@ -1202,11 +1197,44 @@ float Engine::timerElapsedMs(int i0, int i1) {
     return ms;
 }
 
-bool Engine::renderDevice(const uint8_t* dSrc, int w, int h, size_t srcStride, uint8_t* dDst, size_t dstStride) {
+void Engine::checkFrame(const Frame& f, FramePath path) const {
+    if (!isLoaded) throw Error("no engine loaded");
+    if (!f.src || !f.dst) throw Error("null image pointer");
+    if (f.w <= 0 || f.h <= 0) throw Error("invalid frame size");
+    if (f.format == PixelFormat::Bgra8 && path != FramePath::Render) throw Error("BGRA frames are rendered synchronously only");
+    if (f.out && f.format != PixelFormat::Bgr8) throw Error("resized output is u8 BGR only");
+    if ((path == FramePath::Device || path == FramePath::Banded) && (f.format != PixelFormat::Bgr8 || f.out))
+        throw Error("device and row-band frames are u8 BGR at the model's scale");
+    const Frame::Size out = outputSize(f);
+    if (out.w < 1 || out.w > f.w * scale || out.h < 1 || out.h > f.h * scale)
+        throw Error("output size " + std::to_string(out.w) + "x" + std::to_string(out.h) + " is outside 1x1 .. " + std::to_string(f.w * scale) + "x" +
+                    std::to_string(f.h * scale) + " (the resample only reduces the model's " + std::to_string(scale) + "x output)");
+    const size_t bpp = bytesPerPixel(f.format);
+    if (f.srcStride < (size_t)f.w * bpp || f.dstStride < (size_t)out.w * bpp)
+        throw Error("row stride is smaller than " + std::to_string(bpp) + " bytes per pixel");
+    if (f.format == PixelFormat::Bgr16) {
+        if ((f.srcStride | f.dstStride) & 1) throw Error("row stride is odd (u16 rows must be 2-byte aligned)");
+        if ((reinterpret_cast<uintptr_t>(f.src) | reinterpret_cast<uintptr_t>(f.dst)) & 1)
+            throw Error("image pointer is odd (u16 samples must be 2-byte aligned)");
+    }
+}
+
+namespace {
+// f with its buffers replaced by packed ones of pitch srcPitch / dstPitch (the engine's copies on the device)
+Frame packedOnDevice(Frame f, const void* src, size_t srcPitch, void* dst, size_t dstPitch) {
+    f.src = src;
+    f.srcStride = srcPitch;
+    f.dst = dst;
+    f.dstStride = dstPitch;
+    return f;
+}
+}  // namespace
+
+bool Engine::renderDevice(const Frame& f) {
     try {
-        if (!isLoaded) throw Error("no engine loaded");
+        checkFrame(f, FramePath::Device);
         W2X_CUDA(cudaSetDevice(cfg.deviceId));
-        renderOnStream(dSrc, w, h, srcStride, dDst, dstStride, stream, true);
+        renderOnStream(f, stream, true);
         return true;
     } catch (const std::exception& ex) {
         ELOG(W2X_ERROR, std::string("Render failed unexpectedly: ") + ex.what() + ".");
@@ -1214,154 +1242,70 @@ bool Engine::renderDevice(const uint8_t* dSrc, int w, int h, size_t srcStride, u
     }
 }
 
-bool Engine::render(const uint8_t* src, int w, int h, size_t srcStride, uint8_t* dst, size_t dstStride) {
+// host frame -> staging buffers -> renderOnStream -> host frame, synchronous
+bool Engine::render(const Frame& f) {
     try {
-        if (!isLoaded) throw Error("no engine loaded");
-        renderHostFrame(src, w, h, srcStride, dst, dstStride, 3, 1, w * scale, h * scale);
-        return true;
-    } catch (const std::exception& ex) {
-        ELOG(W2X_ERROR, std::string("Render failed unexpectedly: ") + ex.what() + ".");
-        return false;
-    }
-}
-
-bool Engine::renderBgra(const uint8_t* src, int w, int h, size_t srcStride, uint8_t* dst, size_t dstStride) {
-    try {
-        if (!isLoaded) throw Error("no engine loaded");
-        if (!src || !dst) throw Error("null image pointer");
-        if (w <= 0 || h <= 0) throw Error("invalid frame size");
-        if (srcStride < (size_t)w * 4 || dstStride < (size_t)w * scale * 4) throw Error("row stride is smaller than 4 bytes per pixel");
-        renderHostFrame(src, w, h, srcStride, dst, dstStride, 4, 1, w * scale, h * scale);
-        return true;
-    } catch (const std::exception& ex) {
-        ELOG(W2X_ERROR, std::string("Render failed unexpectedly: ") + ex.what() + ".");
-        return false;
-    }
-}
-
-void Engine::checkResized(const uint8_t* src, int w, int h, const uint8_t* dst, int dstW, int dstH, size_t dstStride) const {
-    if (!src || !dst) throw Error("null image pointer");
-    if (w <= 0 || h <= 0) throw Error("invalid frame size");
-    if (dstW < 1 || dstW > w * scale || dstH < 1 || dstH > h * scale)
-        throw Error("output size " + std::to_string(dstW) + "x" + std::to_string(dstH) + " is outside 1x1 .. " + std::to_string(w * scale) + "x" +
-                    std::to_string(h * scale) + " (the resample only reduces the model's " + std::to_string(scale) + "x output)");
-    if (dstStride < (size_t)dstW * 3) throw Error("row stride is smaller than 3 bytes per pixel");
-}
-
-bool Engine::renderResized(const uint8_t* src, int w, int h, size_t srcStride, uint8_t* dst, int dstW, int dstH, size_t dstStride) {
-    try {
-        if (!isLoaded) throw Error("no engine loaded");
-        checkResized(src, w, h, dst, dstW, dstH, dstStride);
-        if (srcStride < (size_t)w * 3) throw Error("row stride is smaller than 3 bytes per pixel");
-        renderHostFrame(src, w, h, srcStride, dst, dstStride, 3, 1, dstW, dstH);
-        return true;
-    } catch (const std::exception& ex) {
-        ELOG(W2X_ERROR, std::string("Render failed unexpectedly: ") + ex.what() + ".");
-        return false;
-    }
-}
-
-void Engine::checkU16(const uint16_t* src, int w, int h, size_t srcStride, const uint16_t* dst, size_t dstStride) const {
-    if (!src || !dst) throw Error("null image pointer");
-    if (w <= 0 || h <= 0) throw Error("invalid frame size");
-    if (srcStride < (size_t)w * 6 || dstStride < (size_t)w * scale * 6) throw Error("row stride is smaller than 6 bytes per pixel");
-    if ((srcStride | dstStride) & 1) throw Error("row stride is odd (u16 rows must be 2-byte aligned)");
-    if ((reinterpret_cast<uintptr_t>(src) | reinterpret_cast<uintptr_t>(dst)) & 1) throw Error("image pointer is odd (u16 samples must be 2-byte aligned)");
-}
-
-bool Engine::renderU16(const uint16_t* src, int w, int h, size_t srcStride, uint16_t* dst, size_t dstStride) {
-    try {
-        if (!isLoaded) throw Error("no engine loaded");
-        checkU16(src, w, h, srcStride, dst, dstStride);
-        renderHostFrame(reinterpret_cast<const uint8_t*>(src), w, h, srcStride, reinterpret_cast<uint8_t*>(dst), dstStride, 3, 2, w * scale, h * scale);
-        return true;
-    } catch (const std::exception& ex) {
-        ELOG(W2X_ERROR, std::string("Render failed unexpectedly: ") + ex.what() + ".");
-        return false;
-    }
-}
-
-int Engine::submitU16(const uint16_t* src, int w, int h, size_t srcStride, uint16_t* dst, size_t dstStride) {
-    try {
-        if (!isLoaded) throw Error("no engine loaded");
-        checkU16(src, w, h, srcStride, dst, dstStride);
-        return submitFrame(reinterpret_cast<const uint8_t*>(src), w, h, srcStride, reinterpret_cast<uint8_t*>(dst), w * scale, h * scale, dstStride, 2);
-    } catch (const std::exception& ex) {
-        ELOG(W2X_ERROR, std::string("Submit failed unexpectedly: ") + ex.what() + ".");
-        return -1;
-    }
-}
-
-void Engine::renderHostFrame(const uint8_t* src, int w, int h, size_t srcStride, uint8_t* dst, size_t dstStride, int pixelBytes, int sampleBytes,
-                             int dstW, int dstH) {
-    W2X_CUDA(cudaSetDevice(cfg.deviceId));
-    const size_t ipitch = (size_t)w * pixelBytes * sampleBytes, opitch = (size_t)dstW * pixelBytes * sampleBytes;
-    staging.in.ensure(ipitch * h);
-    staging.out.ensure(opitch * dstH);
-    uint8_t *dIn = staging.in.get<uint8_t>(), *dOut = staging.out.get<uint8_t>();
-    W2X_CUDA(cudaMemcpy2DAsync(dIn, ipitch, src, srcStride, ipitch, h, cudaMemcpyHostToDevice, stream));  // render.cpp:226
-    // every kernel of the frame is queued first; the output then leaves band by band (rows that are final after a tile row), each copy
-    // ordered behind its band's stitch only, so the download of a band overlaps the batches still computing (the reference downloads
-    // the whole canvas after the last batch, render.cpp:344).  With --tta, and for BGRA frames, there is one band: the whole frame.
-    std::vector<BandDone> bands;
-    renderOnStream(dIn, w, h, ipitch, dOut, opitch, stream, true, &bands, pixelBytes, sampleBytes, dstW, dstH);
-    if (bands.empty()) {
-        W2X_CUDA(cudaMemcpy2DAsync(dst, dstStride, dOut, opitch, opitch, (size_t)dstH, cudaMemcpyDeviceToHost, stream));  // render.cpp:344
-    } else {
-        for (const BandDone& bd : bands) {
-            W2X_CUDA(cudaStreamWaitEvent(d2hStream, bd.ev, 0));
-            W2X_CUDA(cudaMemcpy2DAsync(dst + (size_t)bd.y0 * dstStride, dstStride, dOut + (size_t)bd.y0 * opitch, opitch, opitch, (size_t)(bd.y1 - bd.y0),
-                                       cudaMemcpyDeviceToHost, d2hStream));
+        checkFrame(f, FramePath::Render);
+        W2X_CUDA(cudaSetDevice(cfg.deviceId));
+        const Frame::Size out = outputSize(f);
+        const size_t ipitch = (size_t)f.w * bytesPerPixel(f.format), opitch = (size_t)out.w * bytesPerPixel(f.format);
+        staging.in.ensure(ipitch * f.h);
+        staging.out.ensure(opitch * out.h);
+        uint8_t *dIn = staging.in.get<uint8_t>(), *dOut = staging.out.get<uint8_t>();
+        uint8_t* dst = static_cast<uint8_t*>(f.dst);
+        W2X_CUDA(cudaMemcpy2DAsync(dIn, ipitch, f.src, f.srcStride, ipitch, f.h, cudaMemcpyHostToDevice, stream));  // render.cpp:226
+        // every kernel of the frame is queued first; the output then leaves band by band (rows that are final after a tile row), each copy
+        // ordered behind its band's stitch only, so the download of a band overlaps the batches still computing (the reference downloads
+        // the whole canvas after the last batch, render.cpp:344).  With --tta, and for BGRA frames, there is one band: the whole frame.
+        std::vector<BandDone> bands;
+        renderOnStream(packedOnDevice(f, dIn, ipitch, dOut, opitch), stream, true, &bands);
+        if (bands.empty()) {
+            W2X_CUDA(cudaMemcpy2DAsync(dst, f.dstStride, dOut, opitch, opitch, (size_t)out.h, cudaMemcpyDeviceToHost, stream));  // render.cpp:344
+        } else {
+            for (const BandDone& bd : bands) {
+                W2X_CUDA(cudaStreamWaitEvent(d2hStream, bd.ev, 0));
+                W2X_CUDA(cudaMemcpy2DAsync(dst + (size_t)bd.y0 * f.dstStride, f.dstStride, dOut + (size_t)bd.y0 * opitch, opitch, opitch,
+                                           (size_t)(bd.y1 - bd.y0), cudaMemcpyDeviceToHost, d2hStream));
+            }
+            W2X_CUDA(cudaStreamSynchronize(d2hStream));
         }
-        W2X_CUDA(cudaStreamSynchronize(d2hStream));
+        W2X_CUDA(cudaStreamSynchronize(stream));  // the sync the reference leaves commented out (render.cpp:345)
+        return true;
+    } catch (const std::exception& ex) {
+        ELOG(W2X_ERROR, std::string("Render failed unexpectedly: ") + ex.what() + ".");
+        return false;
     }
-    W2X_CUDA(cudaStreamSynchronize(stream));  // the sync the reference leaves commented out (render.cpp:345)
 }
 
 // Pipelined frames: H2D (copy stream) -> compute (engine stream) -> D2H (copy stream), kSlots frames in flight.
-int Engine::submit(const uint8_t* src, int w, int h, size_t srcStride, uint8_t* dst, size_t dstStride) {
+int Engine::submit(const Frame& f) {
     try {
-        if (!isLoaded) throw Error("no engine loaded");
-        return submitFrame(src, w, h, srcStride, dst, w * scale, h * scale, dstStride);
+        checkFrame(f, FramePath::Submit);
+        W2X_CUDA(cudaSetDevice(cfg.deviceId));
+        const int ticket = nextTicket;
+        PipeSlot& ps = pipe[ticket % kSlots];
+        if (ps.busy) { W2X_CUDA(cudaEventSynchronize(ps.evDone.get())); ps.busy = false; }
+        const Frame::Size out = outputSize(f);
+        const size_t ipitch = (size_t)f.w * bytesPerPixel(f.format), opitch = (size_t)out.w * bytesPerPixel(f.format);
+        ps.in.ensure(ipitch * f.h);
+        ps.out.ensure(opitch * out.h);
+        uint8_t *dIn = ps.in.get<uint8_t>(), *dOut = ps.out.get<uint8_t>();
+        ensureFrameBuffers(f.w, f.h);
+        W2X_CUDA(cudaMemcpy2DAsync(dIn, ipitch, f.src, f.srcStride, ipitch, f.h, cudaMemcpyHostToDevice, h2dStream));
+        W2X_CUDA(cudaEventRecord(ps.evH2D.get(), h2dStream));
+        W2X_CUDA(cudaStreamWaitEvent(stream, ps.evH2D.get(), 0));
+        renderOnStream(packedOnDevice(f, dIn, ipitch, dOut, opitch), stream, false);
+        W2X_CUDA(cudaEventRecord(ps.evComp.get(), stream));
+        W2X_CUDA(cudaStreamWaitEvent(d2hStream, ps.evComp.get(), 0));
+        W2X_CUDA(cudaMemcpy2DAsync(f.dst, f.dstStride, dOut, opitch, opitch, (size_t)out.h, cudaMemcpyDeviceToHost, d2hStream));
+        W2X_CUDA(cudaEventRecord(ps.evDone.get(), d2hStream));
+        ps.busy = true;
+        ++nextTicket;
+        return ticket;
     } catch (const std::exception& ex) {
         ELOG(W2X_ERROR, std::string("Submit failed unexpectedly: ") + ex.what() + ".");
         return -1;
     }
-}
-
-int Engine::submitResized(const uint8_t* src, int w, int h, size_t srcStride, uint8_t* dst, int dstW, int dstH, size_t dstStride) {
-    try {
-        if (!isLoaded) throw Error("no engine loaded");
-        checkResized(src, w, h, dst, dstW, dstH, dstStride);
-        if (srcStride < (size_t)w * 3) throw Error("row stride is smaller than 3 bytes per pixel");
-        return submitFrame(src, w, h, srcStride, dst, dstW, dstH, dstStride);
-    } catch (const std::exception& ex) {
-        ELOG(W2X_ERROR, std::string("Submit failed unexpectedly: ") + ex.what() + ".");
-        return -1;
-    }
-}
-
-int Engine::submitFrame(const uint8_t* src, int w, int h, size_t srcStride, uint8_t* dst, int dstW, int dstH, size_t dstStride, int sampleBytes) {
-    W2X_CUDA(cudaSetDevice(cfg.deviceId));
-    const int ticket = nextTicket;
-    PipeSlot& ps = pipe[ticket % kSlots];
-    if (ps.busy) { W2X_CUDA(cudaEventSynchronize(ps.evDone.get())); ps.busy = false; }
-    const size_t ipitch = (size_t)w * 3 * sampleBytes, opitch = (size_t)dstW * 3 * sampleBytes;
-    ps.in.ensure(ipitch * h);
-    ps.out.ensure(opitch * dstH);
-    uint8_t *dIn = ps.in.get<uint8_t>(), *dOut = ps.out.get<uint8_t>();
-    ensureFrameBuffers(w, h);
-    W2X_CUDA(cudaMemcpy2DAsync(dIn, ipitch, src, srcStride, ipitch, h, cudaMemcpyHostToDevice, h2dStream));
-    W2X_CUDA(cudaEventRecord(ps.evH2D.get(), h2dStream));
-    W2X_CUDA(cudaStreamWaitEvent(stream, ps.evH2D.get(), 0));
-    renderOnStream(dIn, w, h, ipitch, dOut, opitch, stream, false, nullptr, 3, sampleBytes, dstW, dstH);
-    W2X_CUDA(cudaEventRecord(ps.evComp.get(), stream));
-    W2X_CUDA(cudaStreamWaitEvent(d2hStream, ps.evComp.get(), 0));
-    W2X_CUDA(cudaMemcpy2DAsync(dst, dstStride, dOut, opitch, opitch, (size_t)dstH, cudaMemcpyDeviceToHost, d2hStream));
-    W2X_CUDA(cudaEventRecord(ps.evDone.get(), d2hStream));
-    ps.busy = true;
-    ++nextTicket;
-    return ticket;
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -1374,7 +1318,7 @@ int Engine::submitFrame(const uint8_t* src, int w, int h, size_t srcStride, uint
 // buffer.  No collective, no NCCL, no host synchronisation between the devices until the final wait; the result is
 // byte-identical to the single-GPU render (same tiles, same fp32 add order).
 // ------------------------------------------------------------------------------------------------
-bool Engine::renderBanded(Engine* const* es, int count, const uint8_t* src, int w, int h, size_t srcStride, uint8_t* dst, size_t dstStride) {
+bool Engine::renderBanded(Engine* const* es, int count, const Frame& f) {
     if (!es || count < 1 || !es[0]) return false;
     Engine& e0 = *es[0];
     try {
@@ -1385,6 +1329,11 @@ bool Engine::renderBanded(Engine* const* es, int count, const uint8_t* src, int 
                 es[r]->elemBytes != e0.elemBytes)
                 throw Error("row-band render needs identically configured engines");
         }
+        e0.checkFrame(f, FramePath::Banded);
+        const uint8_t* src = static_cast<const uint8_t*>(f.src);
+        uint8_t* dst = static_cast<uint8_t*>(f.dst);
+        const int w = f.w, h = f.h;
+        const size_t srcStride = f.srcStride, dstStride = f.dstStride;
         const int scale = e0.scale, outT = e0.outTile, tile = e0.tile, batch = e0.batch;
         const bool tta = e0.cfg.tta != 0;
         const int spt = tta ? 8 : 1;  // model runs per tile
@@ -1446,7 +1395,7 @@ bool Engine::renderBanded(Engine* const* es, int count, const uint8_t* src, int 
             for (int bi = 0; bi < b.steps / batch; ++bi) {
                 const int nReal = std::min(batch, realSteps - bi * batch);
                 if (nReal <= 0) break;
-                e.unpackTiles(dIn, w, bandH, (size_t)w * 3, dSlots + (size_t)bi * batch, nReal, e.actIn.p, e.stream);
+                e.unpackTiles(dIn, w, bandH, (size_t)w * 3, dSlots + (size_t)bi * batch, nReal, e.actIn.p, e.stream, PixelFormat::Bgr8);
                 ++e.launches;
                 W2X_CUDA(cudaGetLastError());
                 e.runModel(e.stream, e.elemAt(e.band.tiles.get(), (size_t)bi * batch * tileElems), nReal);
@@ -1482,10 +1431,8 @@ bool Engine::renderBanded(Engine* const* es, int count, const uint8_t* src, int 
                 uint8_t* dstRow = tilesBase + (size_t)(tta ? b.own : b.steps) * tileBytes + rowOff;
                 W2X_CUDA(cudaMemcpy2DAsync(dstRow, tileBytes, srcRow, tileBytes, stripBytes, (size_t)g.nx, cudaMemcpyDefault, e.stream));
             }
-            StitchParams sp{};
+            StitchParams sp = stitchGrid(outT, g.nx, g.ny, g.outOvX, g.outOvY, cw, ch, e.fc.rampX.get<float>(), e.fc.rampY.get<float>());
             sp.tiles = tilesBase; sp.f32 = elemBytes == 4 ? 1 : 0; sp.tile_map = e.band.map.get<int>();
-            sp.outT = outT; sp.nx = g.nx; sp.ny = g.ny; sp.ovx = g.outOvX; sp.ovy = g.outOvY;
-            sp.cw = cw; sp.ch = ch; sp.rampx = e.fc.rampX.get<float>(); sp.rampy = e.fc.rampY.get<float>();
             // the band's output rows land at the top of its (band-sized) output buffer
             sp.dst = e.staging.out.get<uint8_t>() - (size_t)b.yBegin * cw * 3; sp.pitch = (size_t)cw * 3;
             sp.y_begin = b.yBegin; sp.y_end = b.yEnd;

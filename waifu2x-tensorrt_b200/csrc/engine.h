@@ -6,6 +6,7 @@
 
 #include <array>
 #include <cstring>
+#include <optional>
 #include <string>
 #include <utility>
 #include <vector>
@@ -142,6 +143,26 @@ ConvParams makeDown2Params(const Act& in, const Act& out, const __half* w, const
 ConvParams makeUp2Params(const Act& in, const Act& out, const __half* w, const float* bias, int cout, float slope, const Act* skip, int skipOff);
 ConvParams makeUp4Params(const Act& in, const Act& out, const __half* w, const float* bias);
 
+// One frame through the engine: src (w x h pixels of `format`) -> dst (the canvas, w*scale x h*scale, or `out` when set), strides in
+// bytes, at least the pixel size times the row's width.  The formats (include/w2x.h):
+//  - Bgr8: render's frames.  `out` reduces the canvas by an antialiased bicubic resample (w2x_render_resized), 1x1 .. the canvas; the
+//    canvas size itself is render, byte for byte.
+//  - Bgra8: the B, G, R of the colour-bled frame through the render pipeline, the alpha plane as a second model pass in the same
+//    batches (none when opaque).  Synchronous host frames only.
+//  - Bgr16: u16 samples, even strides and pointers; the input is scaled by f32(1/65535), the output is saturate(rint(65535 v)) of
+//    render's fp32 canvas.  Tiles, batches and blending are render's.
+// Engine::checkFrame decides which frames each entry point takes.
+struct Frame {
+    struct Size { int w, h; };
+    PixelFormat format = PixelFormat::Bgr8;
+    const void* src = nullptr;
+    int w = 0, h = 0;
+    size_t srcStride = 0;
+    void* dst = nullptr;
+    size_t dstStride = 0;
+    std::optional<Size> out;   // the resized output size (Bgr8 only); unset: the canvas
+};
+
 class Engine {
 public:
     Engine();
@@ -151,23 +172,16 @@ public:
 
     bool build(const std::string& onnxPath, const w2x_build_config& cfg);
     bool load(const std::string& onnxPath, const w2x_render_config& cfg);
-    bool render(const uint8_t* src, int w, int h, size_t srcStride, uint8_t* dst, size_t dstStride);
-    bool renderDevice(const uint8_t* dSrc, int w, int h, size_t srcStride, uint8_t* dDst, size_t dstStride);
-    // BGRA host buffers (w x h, pitch >= 4w) -> BGRA (w*scale x h*scale, pitch >= 4*w*scale), synchronous like render: the B, G, R of
-    // the colour-bled frame through the render pipeline, the alpha plane as a second model pass in the same batches (none when opaque)
-    bool renderBgra(const uint8_t* src, int w, int h, size_t srcStride, uint8_t* dst, size_t dstStride);
-    int submit(const uint8_t* src, int w, int h, size_t srcStride, uint8_t* dst, size_t dstStride);
-    // BGR host buffers -> render's canvas (w*scale x h*scale) reduced to dstW x dstH by an antialiased bicubic resample (include/w2x.h,
-    // w2x_render_resized): 1 <= dstW <= w*scale, 1 <= dstH <= h*scale, dst pitch >= 3 * dstW.  The canvas size is render, byte for byte.
-    bool renderResized(const uint8_t* src, int w, int h, size_t srcStride, uint8_t* dst, int dstW, int dstH, size_t dstStride);
-    int submitResized(const uint8_t* src, int w, int h, size_t srcStride, uint8_t* dst, int dstW, int dstH, size_t dstStride);
-    // u16 BGR host buffers (include/w2x.h, w2x_render_u16): strides in bytes, >= 6 per pixel, even, as are the pointers.  The input is
-    // scaled by f32(1/65535), the output is saturate(rint(65535 v)) of render's fp32 canvas; tiles, batches and blending are render's.
-    bool renderU16(const uint16_t* src, int w, int h, size_t srcStride, uint16_t* dst, size_t dstStride);
-    int submitU16(const uint16_t* src, int w, int h, size_t srcStride, uint16_t* dst, size_t dstStride);
+    // host frames, synchronous: dst is complete on return
+    bool render(const Frame& f);
+    // host frames through the copy / compute / copy pipeline (kSlots frames in flight): a ticket for wait, or -1
+    int submit(const Frame& f);
+    // device frames (Bgr8, canvas size) enqueued on the engine's stream, not synchronised
+    bool renderDevice(const Frame& f);
     bool wait(int ticket);
-    // one image sharded over several engines (one per GPU) by bands of tile rows, seam rows exchanged peer-to-peer
-    static bool renderBanded(Engine* const* engines, int count, const uint8_t* src, int w, int h, size_t srcStride, uint8_t* dst, size_t dstStride);
+    // one host frame (Bgr8, canvas size) sharded over several engines (one per GPU) by bands of tile rows, seam rows exchanged
+    // peer-to-peer
+    static bool renderBanded(Engine* const* engines, int count, const Frame& f);
     bool sync();
     bool infer(const float* inNchw, int n, float* outNchw);
     int profileLayers(int repeats, char (*names)[48], float* ms, double* flops, int cap);
@@ -201,30 +215,24 @@ private:
     bool tf32() const { return elemBytes == 4; }
     // element `i` of an activation / tile buffer of this engine's element type
     void* elemAt(void* base, size_t i) const { return static_cast<uint8_t*>(base) + i * elemBytes; }
-    void unpackTiles(const uint8_t* src, int w, int h, size_t pitch, const TileSlot* slots, int n, void* out, cudaStream_t s, int pixelBytes = 3,
-                     int sampleBytes = 1);
+    void unpackTiles(const uint8_t* src, int w, int h, size_t pitch, const TileSlot* slots, int n, void* out, cudaStream_t s, PixelFormat format);
     void ttaReduce(const void* outs, int tiles, float* mean, cudaStream_t s);
     bool frameWideUnpack() const;
-    // passes: 1 = the colour tiles, 2 = the colour tiles followed by the alpha tiles of a BGRA frame (renderBgra)
+    // passes: 1 = the colour tiles, 2 = the colour tiles followed by the alpha tiles of a Bgra8 frame
     void ensureFrameBuffers(int w, int h, int passes = 1);
     struct RowBand { int y0, y1, batch; };             // output rows [y0, y1) are final once batch `batch` has run (row-major tile order)
     struct BandDone { int y0, y1; cudaEvent_t ev; };   // ... and have been stitched when `ev` fires
+    // The entry points that take a frame, and every refusal they make (throws Error): no engine, null pointers, sizes, strides,
+    // alignment, and the formats and output sizes each one takes.
+    enum class FramePath { Render, Submit, Device, Banded };
+    void checkFrame(const Frame& f, FramePath path) const;
+    Frame::Size outputSize(const Frame& f) const { return f.out ? *f.out : Frame::Size{f.w * scale, f.h * scale}; }
+    // d: a checked frame whose src and dst are on this device
     // bands != nullptr (and no TTA): stitch progressively, one launch per finished tile row, and report the bands instead of one stitch at the end
-    // pixelBytes 4: packed BGRA frames (dSrcPitch = 4w): alpha scan, colour bleed and alpha pass as the frame needs them; no bands
-    // dstW x dstH other than the canvas (BGR only): stitch into resize.canvas, then resample into dDst; with bands, the bands are output
-    // rows of dDst
-    // sampleBytes 2: u16 BGR frames in and out (pitches in bytes), canvas size only; the tiles, batches and bands are those of u8 frames
-    void renderOnStream(const uint8_t* dSrc, int w, int h, size_t srcPitch, uint8_t* dDst, size_t dstPitch, cudaStream_t s, bool timed,
-                        std::vector<BandDone>* bands = nullptr, int pixelBytes = 3, int sampleBytes = 1, int dstW = 0, int dstH = 0);
-    // render / renderBgra / renderResized / renderU16: host frame -> staging buffers -> renderOnStream -> host frame (dstW x dstH),
-    // synchronous
-    void renderHostFrame(const uint8_t* src, int w, int h, size_t srcStride, uint8_t* dst, size_t dstStride, int pixelBytes, int sampleBytes,
-                         int dstW, int dstH);
-    int submitFrame(const uint8_t* src, int w, int h, size_t srcStride, uint8_t* dst, int dstW, int dstH, size_t dstStride, int sampleBytes = 1);
-    // the refusals of renderU16 / submitU16 (throws Error)
-    void checkU16(const uint16_t* src, int w, int h, size_t srcStride, const uint16_t* dst, size_t dstStride) const;
-    // the refusals of renderResized / submitResized (throws Error)
-    void checkResized(const uint8_t* src, int w, int h, const uint8_t* dst, int dstW, int dstH, size_t dstStride) const;
+    // Bgra8: alpha scan, colour bleed and alpha pass as the frame needs them; no bands
+    // d.out other than the canvas: stitch into resize.canvas, then resample into d.dst; with bands, the bands are output rows of d.dst
+    // Bgr16: the tiles, batches and bands are those of Bgr8 frames
+    void renderOnStream(const Frame& d, cudaStream_t s, bool timed, std::vector<BandDone>* bands = nullptr);
     void ensureResize(int cw, int ch, int dw, int dh);
     void* dalloc(size_t bytes);
     Act allocAct(int h, int w, int c);
@@ -268,7 +276,7 @@ private:
         DeviceBuffer rampX, rampY;       // blend ramps of rampXLen / rampYLen entries
         int rampXLen = -1, rampYLen = -1;
     } fc;
-    // host-buffer paths: the frame on the device (render, renderBgra, renderResized, renderU16, renderBanded), sized in bytes
+    // host-buffer paths: the frame on the device (render, renderBanded), sized in bytes
     struct HostStaging { DeviceBuffer in, out; } staging;
     // BGRA frames: alpha-scan flags (2 ints) and the two ping-pong buffers of the colour bleed
     struct BgraScratch { DeviceBuffer flags, bleed[2]; } bgra;

@@ -1,4 +1,4 @@
-// Memory-bound kernels of the BGRA path (Engine::renderBgra): the alpha scan that decides whether a frame needs the colour bleed and
+// Memory-bound kernels of the BGRA path (Bgra8 frames): the alpha scan that decides whether a frame needs the colour bleed and
 // the alpha model pass, and one round of the colour bleed.  Frames are packed w x h BGRA on the device (one 32-bit word per pixel,
 // alpha in the top byte).
 #include <cuda_runtime.h>

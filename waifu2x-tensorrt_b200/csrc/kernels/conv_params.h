@@ -256,15 +256,17 @@ void launchScaleWeights(const __half* w, __half* wOut, const float* scale, int n
 
 // tiling (kernels/tiling.cu)
 // input rect origin, D4 op, valid: 0 = zero dummy slot (img2img_render.cpp:281), 1 = the frame's B, G, R bytes, kSlotAlpha = the
-// alpha byte of a BGRA frame as R = G = B (the alpha pass of Engine::renderBgra)
+// alpha byte of a BGRA frame as R = G = B (the alpha pass of a Bgra8 render)
 struct TileSlot { int x, y, aug, valid; };
 constexpr int kSlotAlpha = 2;
-// pixelBytes: 3 = BGR frame, 4 = BGRA frame; sampleBytes: 1 = u8 samples, 2 = native-endian u16 samples (BGR only, 2-byte aligned
-// frame and pitch)
+// The pixel layout of a frame in and out: packed B, G, R (, A) u8 samples, or native-endian u16 B, G, R samples (2-byte aligned frame
+// and pitch)
+enum class PixelFormat { Bgr8, Bgra8, Bgr16 };
+constexpr int bytesPerPixel(PixelFormat f) { return f == PixelFormat::Bgr8 ? 3 : f == PixelFormat::Bgra8 ? 4 : 6; }
 void launchUnpack(const uint8_t* frame, int w, int h, size_t pitch, const TileSlot* slots, int nslots, int tile,
-                  __half* out, cudaStream_t s, int pixelBytes = 3, int sampleBytes = 1);
+                  __half* out, cudaStream_t s, PixelFormat format);
 void launchUnpack(const uint8_t* frame, int w, int h, size_t pitch, const TileSlot* slots, int nslots, int tile,
-                  float* out, cudaStream_t s, int pixelBytes = 3, int sampleBytes = 1);  // tf32 engines: the reference's convertTo(CV_32F, 1/255) blob exactly
+                  float* out, cudaStream_t s, PixelFormat format);  // tf32 engines: the reference's convertTo(CV_32F, 1/255) blob exactly
 struct StitchParams {
     const void* tiles;   // [count][outT][outT][4] fp16 or f32
     int f32;             // element type of tiles
@@ -277,11 +279,20 @@ struct StitchParams {
     // (i, j) lives at slot tile_map[i * ny + j] of `tiles` (nullptr = identity, the reference's column-major order)
     int y_begin, y_end;
     const int* tile_map;
-    // BGRA canvas (4-byte pixels); alpha_off > 0: the alpha pass's tile of reference tile t is at slot(t) + alpha_off, else alpha = 255
-    int bgra, alpha_off;
-    // u16 BGR canvas (6-byte pixels, saturate(rint(65535 v)) per sample); bgra must be 0
-    int u16;
+    // the canvas: Bgr16 packs saturate(rint(65535 v)) per sample.  Bgra8 with alpha_off > 0: the alpha pass's tile of reference tile t
+    // is at slot(t) + alpha_off, else alpha = 255
+    PixelFormat format;
+    int alpha_off;
 };
+// A StitchParams of the tile grid (output tile size, tile counts, blend overlaps, canvas size, blend ramps); the rest is zero: fp16
+// tiles in the reference's order, a Bgr8 canvas, the whole canvas
+inline StitchParams stitchGrid(int outT, int nx, int ny, int ovx, int ovy, int cw, int ch, const float* rampx, const float* rampy) {
+    StitchParams p{};
+    p.outT = outT; p.nx = nx; p.ny = ny; p.ovx = ovx; p.ovy = ovy;
+    p.cw = cw; p.ch = ch;
+    p.rampx = rampx; p.rampy = rampy;
+    return p;
+}
 void launchStitch(const StitchParams& p, cudaStream_t s);
 // BGRA frames (kernels/alpha.cu), packed w x h x 4 bytes on the device.
 // flags[0] = 1 if some alpha < 255, flags[1] = 1 if some alpha == 0; flags must be zeroed

@@ -1,4 +1,4 @@
-// Antialiased bicubic reduction of a u8 BGR canvas (Engine::renderResized): a horizontal pass from the canvas into an fp32 image of
+// Antialiased bicubic reduction of a u8 BGR canvas (frames with an output size): a horizontal pass from the canvas into an fp32 image of
 // dst_w columns, then a vertical pass from that image into the u8 destination.  Both passes read host-built per-axis tables
 // (hostutil.h, resampleAxis); nothing is rounded between them.  The horizontal pass works on any band of canvas rows and the vertical
 // pass on any band of output rows, so the engine can resample a frame band by band while the model still computes the rest.

@@ -199,22 +199,26 @@ __global__ void __launch_bounds__(256) unpack_kernel(const uint8_t* __restrict__
 
 template <typename T>
 void launchUnpackT(const uint8_t* frame, int w, int h, size_t pitch, const TileSlot* slots, int nslots, int tile, T* out, cudaStream_t s,
-                   int pixelBytes, int sampleBytes) {
+                   PixelFormat format) {
     if (nslots <= 0) return;
     const int side = (tile + kUB - 1) / kUB;
     dim3 grid(side * side, nslots);
     const bool aligned = (reinterpret_cast<uintptr_t>(frame) & 3) == 0;
-    if (sampleBytes == 2) unpack_kernel<T, 3, uint16_t><<<grid, 256, 0, s>>>(frame, w, h, pitch, slots, tile, aligned ? 1 : 0, out);  // BGR
-    else if (pixelBytes == 4) unpack_kernel<T, 4><<<grid, 256, 0, s>>>(frame, w, h, pitch, slots, tile, aligned && (pitch & 3) == 0 ? 1 : 0, out);
-    else unpack_kernel<T, 3><<<grid, 256, 0, s>>>(frame, w, h, pitch, slots, tile, aligned ? 1 : 0, out);
+    switch (format) {
+    case PixelFormat::Bgr16: unpack_kernel<T, 3, uint16_t><<<grid, 256, 0, s>>>(frame, w, h, pitch, slots, tile, aligned ? 1 : 0, out); break;
+    case PixelFormat::Bgra8:
+        unpack_kernel<T, 4><<<grid, 256, 0, s>>>(frame, w, h, pitch, slots, tile, aligned && (pitch & 3) == 0 ? 1 : 0, out);
+        break;
+    case PixelFormat::Bgr8: unpack_kernel<T, 3><<<grid, 256, 0, s>>>(frame, w, h, pitch, slots, tile, aligned ? 1 : 0, out); break;
+    }
 }
 void launchUnpack(const uint8_t* frame, int w, int h, size_t pitch, const TileSlot* slots, int nslots, int tile, __half* out, cudaStream_t s,
-                  int pixelBytes, int sampleBytes) {
-    launchUnpackT(frame, w, h, pitch, slots, nslots, tile, out, s, pixelBytes, sampleBytes);
+                  PixelFormat format) {
+    launchUnpackT(frame, w, h, pitch, slots, nslots, tile, out, s, format);
 }
 void launchUnpack(const uint8_t* frame, int w, int h, size_t pitch, const TileSlot* slots, int nslots, int tile, float* out, cudaStream_t s,
-                  int pixelBytes, int sampleBytes) {
-    launchUnpackT(frame, w, h, pitch, slots, nslots, tile, out, s, pixelBytes, sampleBytes);
+                  PixelFormat format) {
+    launchUnpackT(frame, w, h, pitch, slots, nslots, tile, out, s, format);
 }
 
 // ---- stitch + pack ----------------------------------------------------------------------------------
@@ -395,15 +399,19 @@ void launchStitch(const StitchParams& pin, cudaStream_t s) {
     dim3 grid((p.cw + kSW - 1) / kSW, (p.y_end - p.y_begin + kSR - 1) / kSR);
     // 16-byte stores need 16-byte aligned row segments: block columns start at multiples of 768 (BGRA: 1024, u16 BGR: 1536) bytes
     const int vecOk = ((reinterpret_cast<uintptr_t>(p.dst) & 15) == 0 && (p.pitch & 15) == 0) ? 1 : 0;
-    if (p.u16) {
+    switch (p.format) {
+    case PixelFormat::Bgr16:
         if (p.f32) stitch_kernel<true, 3, uint16_t><<<grid, kSW, 0, s>>>(p, vecOk);
         else stitch_kernel<false, 3, uint16_t><<<grid, kSW, 0, s>>>(p, vecOk);
-    } else if (p.bgra) {
+        break;
+    case PixelFormat::Bgra8:
         if (p.f32) stitch_kernel<true, 4><<<grid, kSW, 0, s>>>(p, vecOk);
         else stitch_kernel<false, 4><<<grid, kSW, 0, s>>>(p, vecOk);
-    } else {
+        break;
+    case PixelFormat::Bgr8:
         if (p.f32) stitch_kernel<true, 3><<<grid, kSW, 0, s>>>(p, vecOk);
         else stitch_kernel<false, 3><<<grid, kSW, 0, s>>>(p, vecOk);
+        break;
     }
 }
 

@@ -59,12 +59,9 @@ bool EnginePool::load(const std::string& onnxPath, const w2x_render_config& cfg)
     return true;
 }
 
-int EnginePool::submit(const uint8_t* src, int w, int h, size_t srcStride, uint8_t* dst, size_t dstStride, int dstW, int dstH) {
-    return enqueue(Job{src, w, h, srcStride, dst, dstStride, dstW, dstH, 0, false});
-}
-
-int EnginePool::submitU16(const uint16_t* src, int w, int h, size_t srcStride, uint16_t* dst, size_t dstStride) {
-    return enqueue(Job{reinterpret_cast<const uint8_t*>(src), w, h, srcStride, reinterpret_cast<uint8_t*>(dst), dstStride, 0, 0, 0, true});
+int EnginePool::submit(const Frame& frame) {
+    if (!frame.src || !frame.dst) return -1;
+    return enqueue(Job{frame, 0});
 }
 
 int EnginePool::enqueue(Job job) {
@@ -115,11 +112,7 @@ void EnginePool::workerLoop(Worker* w) {
         }
         if (have) {
             w->cv.notify_all();  // a queue slot is free again
-            Engine& e = w->eng.impl;
-            const int t = job.u16 ? e.submitU16(reinterpret_cast<const uint16_t*>(job.src), job.w, job.h, job.srcStride, reinterpret_cast<uint16_t*>(job.dst),
-                                                job.dstStride)
-                          : job.dstW > 0 ? e.submitResized(job.src, job.w, job.h, job.srcStride, job.dst, job.dstW, job.dstH, job.dstStride)
-                                         : e.submit(job.src, job.w, job.h, job.srcStride, job.dst, job.dstStride);
+            const int t = w->eng.impl.submit(job.frame);
             if (t < 0) finish(job.ticket, false);
             else flight.push_back({t, job.ticket});
             continue;

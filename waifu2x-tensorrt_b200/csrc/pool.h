@@ -31,19 +31,14 @@ public:
     void setMessageCallback(w2x_message_cb cb, void* user);
     bool build(const std::string& onnxPath, const w2x_build_config& cfg);   // once per distinct device name in the pool
     bool load(const std::string& onnxPath, const w2x_render_config& cfg);   // every engine, cfg.deviceId replaced by its own
-    // frame `ticket` (0, 1, 2, ... in submission order) goes to engine ticket % size(); returns the ticket or -1.  dstW > 0: the output
-    // is resized to dstW x dstH (Engine::submitResized)
-    int submit(const uint8_t* src, int w, int h, size_t srcStride, uint8_t* dst, size_t dstStride, int dstW = 0, int dstH = 0);
-    // the same with u16 BGR frames (Engine::submitU16)
-    int submitU16(const uint16_t* src, int w, int h, size_t srcStride, uint16_t* dst, size_t dstStride);
+    // frame `ticket` (0, 1, 2, ... in submission order) goes to engine ticket % size(); returns the ticket or -1.  A null image pointer is
+    // refused here; the engine's other refusals (Engine::submit) fail the ticket's wait.
+    int submit(const Frame& frame);
     bool wait(int ticket);   // true when that frame's dst is complete; tickets may be waited on in any order, each once
     bool sync();             // every submitted frame has been retired
 
 private:
-    struct Job {
-        const uint8_t* src; int w, h; size_t srcStride; uint8_t* dst; size_t dstStride; int dstW, dstH; int ticket;
-        bool u16;   // src / dst are u16 BGR frames
-    };
+    struct Job { Frame frame; int ticket; };
     struct Worker {
         w2x_engine eng;
         int device = 0;

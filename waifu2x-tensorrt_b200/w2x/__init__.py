@@ -291,7 +291,7 @@ def stitch_tiles(tiles_f16: np.ndarray, nx: int, ny: int, ov_x: int, ov_y: int, 
 
 def unpack_tiles_u16(src_bgr: np.ndarray, rects: List[Tuple[int, int, int, int]], aug: List[int], tile: int, device: int = 0) -> np.ndarray:
     """uint16 [H, W, 3] BGR (rows may be strided) -> float16 [n, tile, tile, 4] (RGB0), each sample x as fp16(f32(x) * f32(1/65535))."""
-    src = src_bgr if _rows_of_u16_pixels(src_bgr) else np.ascontiguousarray(src_bgr, dtype=np.uint16)
+    src = src_bgr if _rows_of_pixels(src_bgr, 3, np.uint16) else np.ascontiguousarray(src_bgr, dtype=np.uint16)
     n = len(rects)
     cr = (_Rect * n)(*[_Rect(*r) for r in rects])
     ca = (C.c_int * n)(*aug)
@@ -322,20 +322,26 @@ def tta_reduce(outs_f16: np.ndarray, device: int = 0) -> np.ndarray:
     return mean
 
 
-def _rows_of_pixels(a: np.ndarray, channels: int) -> bool:
-    """a is [H, W, channels] uint8 with contiguous pixels (rows may be strided)."""
-    return a.dtype == np.uint8 and a.ndim == 3 and a.shape[2] == channels and a.strides[2] == 1 and a.strides[1] == channels
+def _rows_of_pixels(a: np.ndarray, channels: int, dtype) -> bool:
+    """a is [H, W, channels] of dtype with contiguous pixels (rows may be strided, by whole samples from an aligned start)."""
+    n = np.dtype(dtype).itemsize
+    return (a.dtype == dtype and a.ndim == 3 and a.shape[2] == channels and a.strides[2] == n and a.strides[1] == channels * n
+            and a.strides[0] % n == 0 and a.ctypes.data % n == 0)
 
 
-def _rows_of_u16_pixels(a: np.ndarray) -> bool:
-    """a is [H, W, 3] uint16 with contiguous pixels (rows may be strided, by an even number of bytes)."""
-    return (a.dtype == np.uint16 and a.ndim == 3 and a.shape[2] == 3 and a.strides[2] == 2 and a.strides[1] == 6 and a.strides[0] % 2 == 0
-            and a.ctypes.data % 2 == 0)
+def _call_packed(owner, fn, src_ptr: int, w: int, h: int, dst_ptr: int, pixel_bytes: int, size: Optional[Tuple[int, int]] = None) -> int:
+    """fn, a frame entry point of owner (Img2Img or Img2ImgPool), on packed rows: src_ptr holds h rows of w pixels, dst_ptr the
+    canvas (w * scaling x h * scaling), or with size = (dst_w, dst_h), dst_h rows of dst_w pixels."""
+    src, dst = C.c_void_p(src_ptr), C.c_void_p(dst_ptr)
+    if size is None:
+        return int(fn(owner._h, src, w, h, w * pixel_bytes, dst, w * owner.scaling * pixel_bytes))
+    dw, dh = int(size[0]), int(size[1])
+    return int(fn(owner._h, src, w, h, w * pixel_bytes, dst, dw, dh, dw * pixel_bytes))
 
 
 def alpha_bleed(src_bgra: np.ndarray, rounds: int, device: int = 0) -> np.ndarray:
     """The colour bleed of w2x_render_bgra (include/w2x_dev.h: w2x_alpha_bleed): uint8 [H, W, 4] BGRA -> uint8 [H, W, 4], alpha unchanged."""
-    src = src_bgra if _rows_of_pixels(src_bgra, 4) else np.ascontiguousarray(src_bgra, dtype=np.uint8)
+    src = src_bgra if _rows_of_pixels(src_bgra, 4, np.uint8) else np.ascontiguousarray(src_bgra, dtype=np.uint8)
     h, w = src.shape[:2]
     out = np.empty((h, w, 4), np.uint8)
     if not lib().w2x_alpha_bleed(device, _ptr(src), w, h, src.strides[0], int(rounds), _ptr(out)):
@@ -360,12 +366,12 @@ def resample_table(n_in: int, n_out: int):
 def resample(src_bgr: np.ndarray, size: Tuple[int, int], dst: Optional[np.ndarray] = None, device: int = 0) -> np.ndarray:
     """The resample of Img2Img.render_resized alone (include/w2x_dev.h: w2x_resample): uint8 [H, W, 3] BGR -> uint8 [dst_h, dst_w, 3],
     size = (dst_w, dst_h) with 1 <= dst_w <= W, 1 <= dst_h <= H.  src and a caller's dst may have strided rows."""
-    src = src_bgr if _rows_of_pixels(src_bgr, 3) else np.ascontiguousarray(src_bgr, dtype=np.uint8)
+    src = src_bgr if _rows_of_pixels(src_bgr, 3, np.uint8) else np.ascontiguousarray(src_bgr, dtype=np.uint8)
     h, w = src.shape[:2]
     dw, dh = int(size[0]), int(size[1])
     if dst is None:
         dst = np.empty((dh, dw, 3), np.uint8)
-    elif not _rows_of_pixels(dst, 3) or dst.shape[:2] != (dh, dw):
+    elif not _rows_of_pixels(dst, 3, np.uint8) or dst.shape[:2] != (dh, dw):
         raise ValueError("dst must be uint8 [dst_h, dst_w, 3] with contiguous pixels")
     if not lib().w2x_resample(device, _ptr(src), w, h, src.strides[0], _ptr(dst), dw, dh, dst.strides[0]):
         raise RuntimeError("w2x_resample failed")
@@ -535,56 +541,46 @@ class Img2Img:
         return dst if ok else None
 
     # extensions
+    def _render_frame(self, fn, src: np.ndarray, dst: Optional[np.ndarray], channels: int, dtype, size: Optional[Tuple[int, int]] = None):
+        """fn (w2x_render_bgra / _resized / _u16) from src, whose rows may be strided (else it is copied), into the caller's dst, which
+        must have contiguous pixels, or a new one: the canvas (H*s x W*s), or size = (dst_w, dst_h) (at least 1 x 1).  Returns dst, or None
+        on failure (the reason in last_error)."""
+        if not _rows_of_pixels(src, channels, dtype):
+            src = np.ascontiguousarray(src, dtype=dtype)
+        h, w = src.shape[:2]
+        if dst is None:
+            shape = (h * self.scaling, w * self.scaling) if size is None else (max(int(size[1]), 1), max(int(size[0]), 1))
+            dst = np.empty(shape + (channels,), dtype)
+        elif not _rows_of_pixels(dst, channels, dtype):
+            raise ValueError(f"dst must be {np.dtype(dtype).name} [H, W, {channels}] with contiguous pixels")
+        out_size = () if size is None else (int(size[0]), int(size[1]))
+        ok = fn(self._h, _ptr(src), w, h, src.strides[0], _ptr(dst), *out_size, dst.strides[0])
+        return dst if ok else None
+
     def render_bgra(self, src: np.ndarray, dst: Optional[np.ndarray] = None) -> Optional[np.ndarray]:
         """src: uint8 [H, W, 4] BGRA (rows may be strided).  Returns dst (uint8 [H*s, W*s, 4] BGRA; a caller's dst may have strided rows)
         or None on failure (the reason in last_error)."""
-        if not _rows_of_pixels(src, 4):
-            src = np.ascontiguousarray(src, dtype=np.uint8)
-        h, w = src.shape[:2]
-        if dst is None:
-            dst = np.empty((h * self.scaling, w * self.scaling, 4), np.uint8)
-        elif not _rows_of_pixels(dst, 4):
-            raise ValueError("dst must be uint8 [H, W, 4] with contiguous pixels")
-        ok = self._l.w2x_render_bgra(self._h, _ptr(src), w, h, src.strides[0], _ptr(dst), dst.strides[0])
-        return dst if ok else None
+        return self._render_frame(self._l.w2x_render_bgra, src, dst, 4, np.uint8)
 
     def render_resized(self, src: np.ndarray, size: Tuple[int, int], dst: Optional[np.ndarray] = None) -> Optional[np.ndarray]:
         """src: uint8 [H, W, 3] BGR (rows may be strided); size = (dst_w, dst_h) with 1 <= dst_w <= W * scaling, 1 <= dst_h <= H * scaling.
         Returns dst (uint8 [dst_h, dst_w, 3] BGR: render(src) reduced by an antialiased bicubic resample, include/w2x.h w2x_render_resized;
         a caller's dst may have strided rows) or None on failure (the reason in last_error)."""
-        if not _rows_of_pixels(src, 3):
-            src = np.ascontiguousarray(src, dtype=np.uint8)
-        h, w = src.shape[:2]
-        dw, dh = int(size[0]), int(size[1])
-        if dst is None:
-            dst = np.empty((max(dh, 1), max(dw, 1), 3), np.uint8)
-        elif not _rows_of_pixels(dst, 3):
-            raise ValueError("dst must be uint8 [H, W, 3] with contiguous pixels")
-        ok = self._l.w2x_render_resized(self._h, _ptr(src), w, h, src.strides[0], _ptr(dst), dw, dh, dst.strides[0])
-        return dst if ok else None
+        return self._render_frame(self._l.w2x_render_resized, src, dst, 3, np.uint8, size)
 
     def submit_resized(self, src_ptr: int, w: int, h: int, dst_ptr: int, size: Tuple[int, int]) -> int:
         """submit with the output of render_resized: dst_ptr holds size[1] rows of 3 * size[0] bytes.  Returns a ticket for wait, or -1."""
-        dw, dh = int(size[0]), int(size[1])
-        return int(self._l.w2x_submit_resized(self._h, C.c_void_p(src_ptr), w, h, w * 3, C.c_void_p(dst_ptr), dw, dh, dw * 3))
+        return _call_packed(self, self._l.w2x_submit_resized, src_ptr, w, h, dst_ptr, 3, size)
 
     def render_u16(self, src: np.ndarray, dst: Optional[np.ndarray] = None) -> Optional[np.ndarray]:
         """src: uint16 [H, W, 3] BGR (rows may be strided).  Returns dst (uint16 [H*s, W*s, 3] BGR, include/w2x.h w2x_render_u16; a
         caller's dst may have strided rows) or None on failure (the reason in last_error)."""
-        if not _rows_of_u16_pixels(src):
-            src = np.ascontiguousarray(src, dtype=np.uint16)
-        h, w = src.shape[:2]
-        if dst is None:
-            dst = np.empty((h * self.scaling, w * self.scaling, 3), np.uint16)
-        elif not _rows_of_u16_pixels(dst):
-            raise ValueError("dst must be uint16 [H, W, 3] with contiguous pixels")
-        ok = self._l.w2x_render_u16(self._h, _ptr(src), w, h, src.strides[0], _ptr(dst), dst.strides[0])
-        return dst if ok else None
+        return self._render_frame(self._l.w2x_render_u16, src, dst, 3, np.uint16)
 
     def submit_u16(self, src_ptr: int, w: int, h: int, dst_ptr: int) -> int:
         """submit with the frames of render_u16: src_ptr holds h rows of 6 * w bytes, dst_ptr h * s rows of 6 * w * s bytes.  Returns
         a ticket for wait, or -1."""
-        return int(self._l.w2x_submit_u16(self._h, C.c_void_p(src_ptr), w, h, w * 6, C.c_void_p(dst_ptr), w * self.scaling * 6))
+        return _call_packed(self, self._l.w2x_submit_u16, src_ptr, w, h, dst_ptr, 6)
 
     def infer(self, x_nchw: np.ndarray) -> Optional[np.ndarray]:
         x = np.ascontiguousarray(x_nchw, dtype=np.float32)
@@ -660,10 +656,10 @@ class Img2Img:
         return out
 
     def render_device(self, d_src: int, w: int, h: int, d_dst: int) -> bool:
-        return bool(self._l.w2x_render_device(self._h, C.c_void_p(d_src), w, h, w * 3, C.c_void_p(d_dst), w * self.scaling * 3))
+        return bool(_call_packed(self, self._l.w2x_render_device, d_src, w, h, d_dst, 3))
 
     def submit(self, src_ptr: int, w: int, h: int, dst_ptr: int) -> int:
-        return int(self._l.w2x_submit(self._h, C.c_void_p(src_ptr), w, h, w * 3, C.c_void_p(dst_ptr), w * self.scaling * 3))
+        return _call_packed(self, self._l.w2x_submit, src_ptr, w, h, dst_ptr, 3)
 
     def wait(self, ticket: int) -> bool:
         return bool(self._l.w2x_wait(self._h, ticket))
@@ -766,16 +762,15 @@ class Img2ImgPool:
         return ok
 
     def submit(self, src_ptr: int, w: int, h: int, dst_ptr: int) -> int:
-        return int(self._l.w2x_pool_submit(self._h, C.c_void_p(src_ptr), w, h, w * 3, C.c_void_p(dst_ptr), w * self.scaling * 3))
+        return _call_packed(self, self._l.w2x_pool_submit, src_ptr, w, h, dst_ptr, 3)
 
     def submit_resized(self, src_ptr: int, w: int, h: int, dst_ptr: int, size: Tuple[int, int]) -> int:
         """submit with the output of Img2Img.render_resized: dst_ptr holds size[1] rows of 3 * size[0] bytes."""
-        dw, dh = int(size[0]), int(size[1])
-        return int(self._l.w2x_pool_submit_resized(self._h, C.c_void_p(src_ptr), w, h, w * 3, C.c_void_p(dst_ptr), dw, dh, dw * 3))
+        return _call_packed(self, self._l.w2x_pool_submit_resized, src_ptr, w, h, dst_ptr, 3, size)
 
     def submit_u16(self, src_ptr: int, w: int, h: int, dst_ptr: int) -> int:
         """submit with the frames of Img2Img.render_u16: src_ptr holds h rows of 6 * w bytes, dst_ptr h * s rows of 6 * w * s bytes."""
-        return int(self._l.w2x_pool_submit_u16(self._h, C.c_void_p(src_ptr), w, h, w * 6, C.c_void_p(dst_ptr), w * self.scaling * 6))
+        return _call_packed(self, self._l.w2x_pool_submit_u16, src_ptr, w, h, dst_ptr, 6)
 
     def wait(self, ticket: int) -> bool:
         return bool(self._l.w2x_pool_wait(self._h, ticket))
